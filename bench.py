@@ -2,6 +2,7 @@
 """bench.py -- expanded states/sec of the frontier-expansion path (BASELINE.json's metric).
 
     python bench.py --gpus 1 --steps K --warmup W            # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                   # ... and write what its last timed step computed (below)
     python bench.py --impl reference --steps K --warmup W    # the reference algorithm on host cores
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   # one rank per GPU
 
@@ -66,7 +67,13 @@ def parse():
     ap.add_argument('--bfs-depth', type=int, default=10)
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-parity', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed to DIR/*.npy (float64), for comparing two builds')
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if a.dump_outputs and a.impl != 'b200':
+        ap.error('--dump-outputs applies to the CUDA arm (--impl b200)')
     world = int(os.environ.get('WORLD_SIZE', '1'))
     d = {'C1': (10, 'simple', 300_000), 'C2': (255, 'simple', 0), 'C3': (15, 'aggressive', PER_GPU_BEAM['C3'] * world),
          'C4': (15, 'balanced', PER_GPU_BEAM['C4'] * world), 'C5': (15, 'competitive', 20_000)}[a.config]
@@ -161,7 +168,7 @@ def _market_seed0():
 
 
 def python_reference_rate(a):
-    """the unmodified Python reference (baseline/_ref, staged by build() where /root/reference exists) on one core"""
+    """the unmodified Python reference (baseline/_ref, staged by build() from SPLENDOR_REFERENCE) on one core"""
     ref = ROOT / 'baseline' / '_ref'
     if a.config == 'C5' or a.config == 'C2' or not (ref / 'src' / 'solver.py').exists():
         return None
@@ -194,7 +201,7 @@ def run_reference(a):
     if int(os.environ.get('RANK', '0')) != 0:
         return
     beam = min(a.beam, CPU_SAMPLE_BEAM) if a.config != 'C2' else 0
-    steps, warm = max(1, min(a.steps, 3)), min(a.warmup, 1)
+    steps, warm = a.steps, min(a.warmup, 1)
     small = argparse.Namespace(**vars(a))
     for _ in range(warm):
         cpu_solve(small, min(beam, 20_000) if a.config != 'C2' else 0)
@@ -220,6 +227,61 @@ def run_reference(a):
     }))
 
 
+# ------------------------------------------------------------------ --dump-outputs
+# DIR/levels.npy      [levels, 9]  per-level counters of the last timed solve, columns LEVEL_FIELDS (NaN: not reported)
+# DIR/queue.npy       [rows, Wq]    its final queue (one GPU only): each record as Wq little-endian 32-bit words
+#                                   (speedrun: lo, hi, aux, link -> Wq = 8; realistic mode: 96-byte records -> Wq = 24)
+# DIR/queue_rows.npy  [rows]        queue rank of each dumped record: all of them, or a fixed seeded sample
+# DIR/path.npy        [moves+1, Wp] the winning line of the last timed public-API solve (not C2), one state per row
+#                                   (speedrun: State.record() as lo, hi, aux -> Wp = 6; realistic mode:
+#                                   MultiPlayerState.record(), link all ones -> Wp = 24)
+# Every value is an integer held exactly in float64.
+LEVEL_FIELDS = ('level', 'ended', 'frontier', 'expanded', 'generated', 'unique', 'kept', 'goal_rank', 'visited')
+QUEUE_DUMP_BYTES = 48 << 20  # queue sample + its row indices; the whole dump stays under 64 MB
+
+
+def _words(rows_u8):
+    import numpy as np
+    return np.ascontiguousarray(rows_u8).view('<u4').astype(np.float64)
+
+
+def level_array(infos):
+    import numpy as np
+    return np.array([[float(i.get(f, np.nan)) for f in LEVEL_FIELDS] for i in infos], dtype=np.float64).reshape(-1, len(LEVEL_FIELDS))
+
+
+def queue_sample(sol, a, torch):
+    """-> (queue ranks, record words) of a finished single-GPU solver's queue; above the QUEUE_DUMP_BYTES budget a
+    sample of ranks drawn with seed 0, in queue order"""
+    import numpy as np
+    fr = sol.frontier()  # C5: host records [n]; otherwise a device int64 tensor [n, 4]
+    n, rec_bytes = fr.shape[0], (96 if a.config == 'C5' else 32)
+    cap = QUEUE_DUMP_BYTES // (8 * (rec_bytes // 4 + 1))
+    rows = np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+    if a.config == 'C5':
+        raw = fr[rows].view(np.uint8)
+    else:
+        raw = fr[torch.from_numpy(rows).to(fr.device)].cpu().numpy().view(np.uint8)
+    return rows.astype(np.float64), _words(raw.reshape(-1, rec_bytes))
+
+
+def path_array(path, a):
+    import numpy as np
+    if a.config == 'C5':
+        raw = np.concatenate([p.record() for p in path]).view(np.uint8)
+    else:
+        m64 = (1 << 64) - 1
+        raw = np.array([(k & m64, k >> 64, aux) for k, aux in (p.record() for p in path)], dtype=np.uint64).view(np.uint8)
+    return _words(raw.reshape(len(path), -1))
+
+
+def dump_outputs(d, arrays):
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(d, name + '.npy'), arr)
+
+
 # ------------------------------------------------------------------ GPU arm
 class Runner:
     """one search of the workload on the device through the same solver classes the public API uses"""
@@ -242,17 +304,18 @@ class Runner:
             return GroupedShardedSolver(eng, comm, self.k, self.aux, a.goal, a.heuristic, beam, a.noise, keep_links=keep_links)
         return ShardedSolver(CudaBackend(eng), comm, self.k, self.aux, a.goal, a.config != 'C2', a.heuristic, beam, a.tie, a.noise, keep_links=keep_links)
 
-    def run(self, beam, digest=False):
-        """-> (per-level infos, sha256 over every level's queue or None)"""
+    def run(self, beam, digest=False, keep=False):
+        """-> (per-level infos, sha256 over every level's queue or None); keep=True leaves the finished solver open
+        as self.kept (its final queue is read after the timed region; the caller closes it)"""
         if self.comm.world > 1 and not getattr(self, 'key_sharded', False):
             from splendor_rl_gym_b200.sharded import DictionaryOverflow
             try:
-                return self._run(beam, digest)
+                return self._run(beam, digest, keep)
             except DictionaryOverflow:  # e.g. `balanced` at wide beams: as State.solve() does, rerun on the key-sharded driver
                 self.key_sharded = True
-        return self._run(beam, digest)
+        return self._run(beam, digest, keep)
 
-    def _run(self, beam, digest=False):
+    def _run(self, beam, digest=False, keep=False):
         a = self.a
         sol = self.solver(beam)
         h = hashlib.sha256() if digest else None
@@ -271,9 +334,14 @@ class Runner:
                     else:
                         fr = sol.gather_frontier() if self.comm.world > 1 else sol.frontier()
                         h.update(fr.cpu().numpy().tobytes())
-        finally:
+        except BaseException:
             if hasattr(sol, 'close'):
                 sol.close()
+            raise
+        if keep:
+            self.kept = sol
+        elif hasattr(sol, 'close'):
+            sol.close()
         return infos, (h.hexdigest() if digest else None)
 
 
@@ -339,8 +407,8 @@ def run_b200(a):
     t0 = time.time()
     ev0.record()
     all_infos = []
-    for _ in range(a.steps):
-        all_infos.append(runner.run(a.beam)[0])
+    for s in range(a.steps):
+        all_infos.append(runner.run(a.beam, keep=bool(a.dump_outputs) and s == a.steps - 1)[0])
     ev1.record()
     torch.cuda.synchronize()
     t1 = time.time()
@@ -359,6 +427,13 @@ def run_b200(a):
     ms = float(tm.item())
     value = expanded / (ms * 1e-3)
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    outputs = {}
+    if a.dump_outputs:  # the last timed solve: its per-level counters and, on one GPU, its final queue
+        outputs['levels'] = level_array(all_infos[-1])
+        if comm.world == 1:
+            outputs['queue_rows'], outputs['queue'] = queue_sample(runner.kept, a, torch)
+        if hasattr(runner.kept, 'close'):
+            runner.kept.close()
 
     # ---- end to end through the public API (host inputs / outputs inside the timed region)
     def api_solve(stats):
@@ -405,6 +480,10 @@ def run_b200(a):
         if world > 1:
             dist.destroy_process_group()
         return
+    if a.dump_outputs:
+        if path:  # the winning line the last timed API solve returned
+            outputs['path'] = path_array(path, a)
+        dump_outputs(a.dump_outputs, outputs)
 
     infos = all_infos[-1]
     lv = [i for i in infos if i['expanded'] and i.get('generated')]
