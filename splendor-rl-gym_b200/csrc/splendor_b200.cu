@@ -74,7 +74,6 @@ struct spl_ctx {
     uint16_t *d_gemrank = nullptr;
     uint16_t *d_rankgems = nullptr;   // inverse of d_gemrank
     DevBuf brec, ntk8, boff2, run_start, run_wpre, cls_list;
-    int tie_link_top = 0;  // > 0: the beam cut breaks score ties on the records' link words (arrival order)
     // constant tables
     DevTables *d_tabs = nullptr;
     uint32_t *d_takes_idx = nullptr;
@@ -462,11 +461,26 @@ static int run_count(spl_ctx *c, const Rec *front, int64_t n, cudaStream_t st) {
     return read_ctr(c, st);
 }
 
-// det policy: split the score ties at the threshold (d_sel->prefix) by key, larger first
+// How the beam cut orders the states that tie on score.
+enum CutTies {
+    TIES_ARRIVAL,      // arrival order, the input being in arrival order (stable policy)
+    TIES_KEY,          // larger key first (det policy)
+    TIES_KEY_ORDERED,  // larger key first, the input being in key order already: only the score is sorted
+    TIES_LINK,         // arrival order read from the records' link words, the input being unordered (grouped level)
+};
+struct CutMode {
+    CutTies ties = TIES_ARRIVAL;
+    int link_bits = 0;  // TIES_LINK: the tie word is 2^link_bits - 1 - link
+    bool by_key() const { return ties != TIES_ARRIVAL; }                      // a key threshold splits the ties
+    bool sorts_keys() const { return ties == TIES_KEY || ties == TIES_LINK; }  // the rank sort has key passes
+    int lt() const { return ties == TIES_LINK ? link_bits : 0; }
+};
+
+// key policies: split the score ties at the threshold (d_sel->prefix) by key, larger first
 static int select_ties_by_key(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int ks, int64_t n, int64_t k,
-                              uint64_t sk_min, cudaStream_t st) {
+                              uint64_t sk_min, CutMode mode, cudaStream_t st) {
     const unsigned grid = std::min<unsigned>(nblk(n), 148 * 8);
-    const int lt = c->tie_link_top;
+    const int lt = mode.lt();
     if (lt) {
         // arrival-order ties: collect the tie words (2^lt - 1 - link) of the threshold score once, then select among them
         const int64_t ntie = (int64_t)c->h_sel->tie_count;
@@ -505,7 +519,7 @@ static int select_ties_by_key(spl_ctx *c, const uint64_t *sk, const uint64_t *kb
 // radix select of the k-th largest element under (score desc[, key desc]); leaves the thresholds and
 // the tie quota in d_sel / h_sel (score in x = sk - sk_min space).
 static int run_select(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int ks, int64_t n, int64_t k, uint64_t sk_min,
-                      uint64_t sk_max, int det, cudaStream_t st) {
+                      uint64_t sk_max, CutMode mode, cudaStream_t st) {
     const int nbits = bitlen(sk_max - sk_min);
     const unsigned grid = std::min<unsigned>(nblk(n), 148 * 8);
     memset(c->h_sel, 0, sizeof(SelState));
@@ -526,7 +540,7 @@ static int run_select(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int ks
     CK(c, cudaMemcpyAsync(c->h_sel, c->d_sel, sizeof(SelState), cudaMemcpyDeviceToHost, st));
     CK(c, cudaStreamSynchronize(st));
     c->d2h_bytes += sizeof(SelState);
-    if (det && c->h_sel->k_rem < c->h_sel->tie_count) CKS(c, select_ties_by_key(c, sk, kb, ks, n, k, sk_min, st));
+    if (mode.by_key() && c->h_sel->k_rem < c->h_sel->tie_count) CKS(c, select_ties_by_key(c, sk, kb, ks, n, k, sk_min, mode, st));
     return SPL_OK;
 }
 
@@ -534,7 +548,7 @@ static int run_select(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int ks
 // element.  Leaves d_sel / h_sel as run_select does plus rank_t; *used = 0 when the level has more
 // than DICT_MAX distinct scores (nothing decided: the caller falls back to the radix select).
 static int run_dict_select(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int ks, int64_t n, int64_t k,
-                           uint64_t sk_min, int det, int *used, cudaStream_t st, int keep_all = -1) {
+                           uint64_t sk_min, CutMode mode, int *used, cudaStream_t st, int keep_all = -1) {
     if (keep_all < 0) keep_all = k >= n;
     *used = 0;
     if (c->dict_skip > 0) { --c->dict_skip; return SPL_OK; }
@@ -556,7 +570,7 @@ static int run_dict_select(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, i
         return SPL_OK;
     }
     *used = 1;
-    if (det && !keep_all && c->h_sel->k_rem < c->h_sel->tie_count) CKS(c, select_ties_by_key(c, sk, kb, ks, n, k, sk_min, st));
+    if (mode.by_key() && !keep_all && c->h_sel->k_rem < c->h_sel->tie_count) CKS(c, select_ties_by_key(c, sk, kb, ks, n, k, sk_min, mode, st));
     return SPL_OK;
 }
 
@@ -586,71 +600,91 @@ static int sort_pass(spl_ctx *c, int wide, int cur, const uint64_t *dig, int64_t
     return SPL_OK;
 }
 
-// beam cut + rank sort.  stable: arrival-order cut, stable descending sort by score.  det: cut and sort
-// by (score desc, key desc).  On return idx[*which] holds the kept source indices in rank order.
-static int do_cut_sort(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int ks, int64_t n, int64_t cap_kept, int keep_all,
-                       int all_ties, uint64_t sk_min, uint64_t sk_max, int det, int use_dict, int *which, int64_t *kept_out,
-                       cudaStream_t st);
-
-// n = elements of sk / recs; n_valid of them are states (the rest are unused slots, sk == 0)
-static int run_cut_sort(spl_ctx *c, const uint64_t *sk, const Rec *recs, int64_t n, int64_t k, uint64_t sk_min,
-                        uint64_t sk_max, int det, int *which, int64_t *kept_out, cudaStream_t st, int64_t n_valid = -1) {
-    if (n_valid < 0) n_valid = n;
-    const int keep_all = n_valid <= k;
-    const uint64_t *kb = reinterpret_cast<const uint64_t *>(recs);
-    const int ks = 4;
-    int use_dict = 0;
-    CKS(c, run_dict_select(c, sk, kb, ks, n, std::min(n_valid, k), sk_min, det, &use_dict, st, keep_all));
-    if (!keep_all && !use_dict) CKS(c, run_select(c, sk, kb, ks, n, k, sk_min, sk_max, det, st));
-    const int all_ties = keep_all || c->h_sel->tie_count != ~0ull;
-    CKS(c, do_cut_sort(c, sk, kb, ks, n, std::min(n_valid, k), keep_all, all_ties, sk_min, sk_max, det, use_dict, which, kept_out, st));
-    if (*kept_out != std::min(n_valid, k))
-        return fail(c, SPL_E_CUDA, "internal: cut kept %lld states, expected %lld", (long long)*kept_out, (long long)std::min(n_valid, k));
+// Stable sort of the (sort word, slot) pairs c->y[*cur] / c->idx[*cur] [0, n) by the words' low `nbits` bits: one-sweep
+// passes below OS_MAX_ITEMS pairs, 8-bit LSD passes at and above it.
+static int sort_pairs(spl_ctx *c, int64_t n, int nbits, int *cur, cudaStream_t st) {
+    if (n <= 1 || nbits <= 0) return SPL_OK;
+    if (n < OS_MAX_ITEMS) {
+        uint64_t *const yk[2] = {c->y[0].as<uint64_t>(), c->y[1].as<uint64_t>()};
+        uint32_t *const yi[2] = {c->idx[0].as<uint32_t>(), c->idx[1].as<uint32_t>()};
+        return onesweep_sort(c, yk, yi, n, 0, nbits, cur, st);
+    }
+    const unsigned nt = nblk(n, SORT_TILE);
+    const size_t msz = (size_t)SORT_BINS * nt;
+    CK(c, c->matrix.ensure(msz * 4, 0, st));
+    CK(c, c->matrix2.ensure(msz * 4, 0, st));
+    for (int shift = 0; shift < nbits; shift += SORT_BITS) {
+        CKS(c, sort_pass(c, 0, *cur, c->y[*cur].as<uint64_t>(), n, shift, nt, msz, st));
+        *cur ^= 1;
+    }
     return SPL_OK;
 }
 
-// cut by the thresholds currently in d_sel / h_sel (x-space score threshold `prefix`, arrival quota
-// `k_rem` for the stable policy, key threshold khi/klo for det), then rank-sort the survivors.
+// Packed beam cut by the thresholds in d_sel: one sort word per survivor (its score's rank in `dict` << link_bits | link
+// word), then the (word, slot) pairs sorted ascending -- best first -- into c->y[*cur] / c->idx[*cur].  At most `cap`
+// survivors.
+static int cut_packed(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int ks, int64_t n, int64_t cap, uint64_t sk_min,
+                      int keep_all, int all_ties, const ScoreDict *dict, int link_bits, int *cur, int64_t *kept_out,
+                      cudaStream_t st) {
+    for (int b = 0; b < 2; ++b) {
+        CK(c, c->y[b].ensure((size_t)cap * 8 + 8, 0, st));
+        CK(c, c->idx[b].ensure((size_t)cap * 4 + 4, 0, st));
+    }
+    const unsigned ct = nblk(n, TILE * CUTP_ITEMS);
+    CKS(c, prep_status(c, 2, ct, st));
+    CKS(c, zero_ctr(c, st));
+    cut_pack_kernel<<<ct, TILE, 0, st>>>(sk, kb, ks, n, sk_min, keep_all, all_ties, c->d_sel, dict, link_bits, c->y[0].as<uint64_t>(),
+                                          c->idx[0].as<uint32_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1);
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    uint64_t last = 0;  // survivors written: the inclusive prefix published by the last cut tile
+    CK(c, cudaMemcpyAsync(&last, c->status[2].as<uint64_t>() + (ct - 1), 8, cudaMemcpyDeviceToHost, st));
+    CK(c, cudaStreamSynchronize(st));
+    c->d2h_bytes += 8;
+    const int64_t kept = (int64_t)(last & ((1ull << 62) - 1));
+    if (kept > cap) return fail(c, SPL_E_CUDA, "internal: cut kept %lld > capacity %lld", (long long)kept, (long long)cap);
+    *cur = 0;
+    *kept_out = kept;
+    return sort_pairs(c, kept, bitlen(c->h_sel->rank_t) + link_bits, cur, st);
+}
+
+// beam cut + rank sort by the thresholds currently in d_sel / h_sel (x-space score threshold `prefix`, arrival quota
+// `k_rem` for arrival ties, key threshold khi/klo for key ties).  Arrival ties: arrival-order cut, stable descending sort
+// by score.  Key ties: cut and sort by (score desc, key desc).  On return idx[*which] holds the kept source indices in
+// rank order.
 static int do_cut_sort(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int ks, int64_t n, int64_t cap_kept, int keep_all,
-                       int all_ties, uint64_t sk_min, uint64_t sk_max, int det, int use_dict, int *which, int64_t *kept_out,
+                       int all_ties, uint64_t sk_min, uint64_t sk_max, CutMode mode, int use_dict, int *which, int64_t *kept_out,
                        cudaStream_t st) {
+    if (mode.ties == TIES_LINK && use_dict)
+        return cut_packed(c, sk, kb, ks, n, cap_kept, sk_min, keep_all, all_ties, c->d_dict, mode.link_bits, which, kept_out, st);
     int64_t kept = cap_kept;
     const uint64_t T = keep_all ? 0 : c->h_sel->prefix;
     for (int b = 0; b < 2; ++b) {
         CK(c, c->y[b].ensure((size_t)kept * 8 + 8, 0, st));
         CK(c, c->idx[b].ensure((size_t)kept * 4 + 4, 0, st));
-        if (det) {
+        if (mode.by_key()) {
             CK(c, c->kl[b].ensure((size_t)kept * 8 + 8, 0, st));
             CK(c, c->kh[b].ensure((size_t)kept * 8 + 8, 0, st));
         }
     }
-    const int lt0 = det == 1 ? c->tie_link_top : 0;
-    const unsigned ct = nblk(n, TILE * ((lt0 && use_dict) ? CUTP_ITEMS : CUT_ITEMS));
+    const unsigned ct = nblk(n, TILE * CUT_ITEMS);
     CKS(c, prep_status(c, 1, ct, st));
     CKS(c, prep_status(c, 2, ct, st));
     CKS(c, reset_ticket(c, 1, st));
     uint64_t vary_lo = 0, vary_hi = 0;
-    const int lt = det == 1 ? c->tie_link_top : 0;
-    const int pack = lt && use_dict;  // one sort word: score rank << lt | link
-    if (pack) {
-        CKS(c, zero_ctr(c, st));
-        cut_pack_kernel<<<ct, TILE, 0, st>>>(sk, kb, ks, n, sk_min, keep_all, all_ties, c->d_sel, c->d_dict, lt, c->y[0].as<uint64_t>(),
-                                              c->idx[0].as<uint32_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1);
-        ++c->launches;
-        CK(c, cudaGetLastError());
-    } else if (det) {
+    if (mode.by_key()) {
         CKS(c, zero_ctr(c, st));
         if (use_dict)
             cut_det_kernel<true><<<ct, TILE, 0, st>>>(sk, kb, ks, n, sk_min, sk_max, keep_all, all_ties, c->d_sel, c->d_dict,
                                                        c->y[0].as<uint64_t>(), c->kl[0].as<uint64_t>(), c->kh[0].as<uint64_t>(),
-                                                       c->idx[0].as<uint32_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1, lt, pack);
+                                                       c->idx[0].as<uint32_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1, mode.lt(), 0);
         else
             cut_det_kernel<false><<<ct, TILE, 0, st>>>(sk, kb, ks, n, sk_min, sk_max, keep_all, all_ties, c->d_sel, nullptr,
                                                         c->y[0].as<uint64_t>(), c->kl[0].as<uint64_t>(), c->kh[0].as<uint64_t>(),
-                                                        c->idx[0].as<uint32_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1, lt, 0);
+                                                        c->idx[0].as<uint32_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1, mode.lt(), 0);
         ++c->launches;
         CK(c, cudaGetLastError());
-        if (det == 1 && !pack) {  // which key bits vary among the survivors (constant digits need no sort pass)
+        if (mode.sorts_keys()) {  // which key bits vary among the survivors (constant digits need no sort pass)
             CKS(c, read_ctr(c, st));
             vary_lo = c->h_ctr->key_or[0] ^ c->h_ctr->key_and[0];
             vary_hi = (c->h_ctr->key_or[1] ^ c->h_ctr->key_and[1]) & HI_KEY_MASK;
@@ -668,43 +702,39 @@ static int do_cut_sort(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int k
         CK(c, cudaGetLastError());
     }
     {   // survivors actually written, from the inclusive prefixes published by the last cut tile
+        const bool quota = mode.ties == TIES_ARRIVAL && !keep_all;  // the threshold score's ties fill the arrival quota
         uint64_t last = 0, last_tie = 0;
         CK(c, cudaMemcpyAsync(&last, c->status[2].as<uint64_t>() + (ct - 1), 8, cudaMemcpyDeviceToHost, st));
-        if (!det && !keep_all)
-            CK(c, cudaMemcpyAsync(&last_tie, c->status[1].as<uint64_t>() + (ct - 1), 8, cudaMemcpyDeviceToHost, st));
+        if (quota) CK(c, cudaMemcpyAsync(&last_tie, c->status[1].as<uint64_t>() + (ct - 1), 8, cudaMemcpyDeviceToHost, st));
         CK(c, cudaStreamSynchronize(st));
-        c->d2h_bytes += 16;
+        c->d2h_bytes += quota ? 16 : 8;
         constexpr uint64_t VAL = (1ull << 62) - 1;
-        kept = (int64_t)(last & VAL);  // det: kept states; stable: states above the threshold
-        if (!det && !keep_all) kept += (int64_t)std::min<uint64_t>(last_tie & VAL, c->h_sel->k_rem);
+        kept = (int64_t)(last & VAL);  // key ties: kept states; arrival ties: states above the threshold
+        if (quota) kept += (int64_t)std::min<uint64_t>(last_tie & VAL, c->h_sel->k_rem);
         if (kept > cap_kept) return fail(c, SPL_E_CUDA, "internal: cut kept %lld > capacity %lld", (long long)kept, (long long)cap_kept);
     }
     // y = sk_max - sk in [0, sk_max - sk_min - T], or (dictionary) the score's descending rank in [0, rank_t]
-    const int nbits = (use_dict ? bitlen(c->h_sel->rank_t) : bitlen((sk_max - sk_min) - T)) + (pack ? lt : 0);
+    const int nbits = use_dict ? bitlen(c->h_sel->rank_t) : bitlen((sk_max - sk_min) - T);
     int cur = 0;
-    const unsigned nt = nblk(kept, SORT_TILE);
     if (kept > 1 && (nbits > 0 || vary_lo || vary_hi)) {
-        const size_t msz = (size_t)SORT_BINS * nt;
-        CK(c, c->matrix.ensure(msz * 4, 0, st));
-        CK(c, c->matrix2.ensure(msz * 4, 0, st));
-        if (det == 1 && !pack) {  // least significant first: key.lo, key.hi, then the score
+        if (mode.sorts_keys()) {  // least significant first: key.lo, key.hi, then the score
+            const unsigned nt = nblk(kept, SORT_TILE);
+            const size_t msz = (size_t)SORT_BINS * nt;
+            CK(c, c->matrix.ensure(msz * 4, 0, st));
+            CK(c, c->matrix2.ensure(msz * 4, 0, st));
             for (int shift = 0; shift < 64; shift += SORT_BITS)
                 if ((vary_lo >> shift) & 0xff) { CKS(c, sort_pass(c, 1, cur, c->kl[cur].as<uint64_t>(), kept, shift, nt, msz, st)); cur ^= 1; }
             for (int shift = 0; shift < 41; shift += SORT_BITS)
                 if ((vary_hi >> shift) & 0xff) { CKS(c, sort_pass(c, 1, cur, c->kh[cur].as<uint64_t>(), kept, shift, nt, msz, st)); cur ^= 1; }
-        }
-        if (!(det == 1 && !pack) && kept < OS_MAX_ITEMS) {  // (sort word, slot) pairs: one-sweep passes of 10 bits
-            uint64_t *const yk[2] = {c->y[0].as<uint64_t>(), c->y[1].as<uint64_t>()};
-            uint32_t *const yi[2] = {c->idx[0].as<uint32_t>(), c->idx[1].as<uint32_t>()};
-            CKS(c, onesweep_sort(c, yk, yi, kept, 0, nbits, &cur, st));
-        } else {
             for (int shift = 0; shift < nbits; shift += SORT_BITS) {
-                CKS(c, sort_pass(c, det == 1 && !pack, cur, c->y[cur].as<uint64_t>(), kept, shift, nt, msz, st));
+                CKS(c, sort_pass(c, 1, cur, c->y[cur].as<uint64_t>(), kept, shift, nt, msz, st));
                 cur ^= 1;
             }
+        } else {
+            CKS(c, sort_pairs(c, kept, nbits, &cur, st));
         }
     }
-    if (det == 2 && kept > 0) {  // keys were in rank order already: the stable score sort kept them so; rebuild the key words
+    if (mode.ties == TIES_KEY_ORDERED && kept > 0) {  // keys were in rank order already: the stable score sort kept them so; rebuild the key words
         key_words_kernel<<<nblk(kept), TILE, 0, st>>>(c->idx[cur].as<uint32_t>(), kept, kb, ks, c->kl[cur].as<uint64_t>(),
                                                        c->kh[cur].as<uint64_t>());
         ++c->launches;
@@ -712,6 +742,23 @@ static int do_cut_sort(spl_ctx *c, const uint64_t *sk, const uint64_t *kb, int k
     }
     *which = cur;
     *kept_out = kept;
+    return SPL_OK;
+}
+
+// n = elements of sk / recs; n_valid of them are states (the rest are unused slots, sk == 0)
+static int run_cut_sort(spl_ctx *c, const uint64_t *sk, const Rec *recs, int64_t n, int64_t k, uint64_t sk_min,
+                        uint64_t sk_max, CutMode mode, int *which, int64_t *kept_out, cudaStream_t st, int64_t n_valid = -1) {
+    if (n_valid < 0) n_valid = n;
+    const int keep_all = n_valid <= k;
+    const uint64_t *kb = reinterpret_cast<const uint64_t *>(recs);
+    const int ks = 4;
+    int use_dict = 0;
+    CKS(c, run_dict_select(c, sk, kb, ks, n, std::min(n_valid, k), sk_min, mode, &use_dict, st, keep_all));
+    if (!keep_all && !use_dict) CKS(c, run_select(c, sk, kb, ks, n, k, sk_min, sk_max, mode, st));
+    const int all_ties = keep_all || c->h_sel->tie_count != ~0ull;
+    CKS(c, do_cut_sort(c, sk, kb, ks, n, std::min(n_valid, k), keep_all, all_ties, sk_min, sk_max, mode, use_dict, which, kept_out, st));
+    if (*kept_out != std::min(n_valid, k))
+        return fail(c, SPL_E_CUDA, "internal: cut kept %lld states, expected %lld", (long long)*kept_out, (long long)std::min(n_valid, k));
     return SPL_OK;
 }
 
@@ -816,7 +863,8 @@ int32_t spl_topk(spl_ctx *c, const double *scores, const spl_key *keys, int64_t 
         ++c->launches;
         recs = c->tmp_rec.as<Rec>();
     }
-    CKS(c, run_cut_sort(c, c->sk.as<uint64_t>(), recs, n, k, smin, smax, tie_policy == SPL_TIE_KEY, &which, &kept, st));
+    CKS(c, run_cut_sort(c, c->sk.as<uint64_t>(), recs, n, k, smin, smax, CutMode{tie_policy == SPL_TIE_KEY ? TIES_KEY : TIES_ARRIVAL},
+                        &which, &kept, st));
     idx_widen_kernel<<<nblk(kept), TILE, 0, st>>>(c->idx[which].as<uint32_t>(), kept, out_idx);
     ++c->launches;
     CK(c, cudaGetLastError());
@@ -1086,18 +1134,20 @@ int32_t spl_dtopk_cut(spl_ctx *c, int32_t tie_policy, int32_t keep_all, int32_t 
     const int64_t n = c->dtopk_n;
     *kept_host = 0;
     if (n == 0) return SPL_OK;
-    const int det = tie_policy == SPL_TIE_KEY ? 1 : tie_policy == SPL_TIE_KEY_ORDERED ? 2 : 0;
-    if (det && !c->dtopk_recs) return fail(c, SPL_E_STATE, "spl_dtopk_cut: det policy needs keys in spl_dtopk_begin");
+    CutMode mode;
+    if (tie_policy == SPL_TIE_KEY) mode.ties = TIES_KEY;
+    else if (tie_policy == SPL_TIE_KEY_ORDERED) mode.ties = TIES_KEY_ORDERED;
+    if (mode.by_key() && !c->dtopk_recs) return fail(c, SPL_E_STATE, "spl_dtopk_cut: det policy needs keys in spl_dtopk_begin");
     int which = 0;
     int64_t kept = 0;
     CKS(c, do_cut_sort(c, c->sk.as<uint64_t>(), c->dtopk_keys, 2, n, n, keep_all, all_ties, sk_min_global, sk_max_global,
-                       det, 0, &which, &kept, st));
+                       mode, 0, &which, &kept, st));
     if (kept) {
         idx_widen_kernel<<<nblk(kept), TILE, 0, st>>>(c->idx[which].as<uint32_t>(), kept, out_idx);
         ++c->launches;
         if (out_y) CK(c, cudaMemcpyAsync(out_y, c->y[which].p, (size_t)kept * 8, cudaMemcpyDeviceToDevice, st));
-        if (det && out_klo) CK(c, cudaMemcpyAsync(out_klo, c->kl[which].p, (size_t)kept * 8, cudaMemcpyDeviceToDevice, st));
-        if (det && out_khi) CK(c, cudaMemcpyAsync(out_khi, c->kh[which].p, (size_t)kept * 8, cudaMemcpyDeviceToDevice, st));
+        if (mode.by_key() && out_klo) CK(c, cudaMemcpyAsync(out_klo, c->kl[which].p, (size_t)kept * 8, cudaMemcpyDeviceToDevice, st));
+        if (mode.by_key() && out_khi) CK(c, cudaMemcpyAsync(out_khi, c->kh[which].p, (size_t)kept * 8, cudaMemcpyDeviceToDevice, st));
         CK(c, cudaGetLastError());
         CK(c, cudaStreamSynchronize(st));
     }
@@ -1176,9 +1226,63 @@ struct LinkCols {
     }
 };
 
-struct spl_solver {
-    spl_ctx *c = nullptr;
-    int goal = 15, use_h = 0, heuristic = 0, tie = 0, noise = 0, keep_links = 1;
+// What a solver holds while it is open: the queue buffers, lent by its context (the last solve's, so that their memory
+// is reused), and per level the queue's parent links and, on the card-set-sharded driver, its global ranks.
+struct SolverBufs {
+    spl_ctx *c;
+    int keep_links = 1;
+    DevBuf front, uniq, grank;
+    LinkCols links, ranks;
+    explicit SolverBufs(spl_ctx *ctx) : c(ctx) {
+        front.swap(c->pool_front);
+        uniq.swap(c->pool_uniq);
+        grank.swap(c->pool_grank);
+        std::sort(c->pool_links.begin(), c->pool_links.end(), [](DevBuf *a, DevBuf *b) { return a->cap > b->cap; });
+    }
+    ~SolverBufs() {
+        if (c->active == this) c->active = nullptr;
+        c->pool_front.swap(front);  // keep the big buffers for the next solve on this context
+        c->pool_uniq.swap(uniq);
+        c->pool_grank.swap(grank);
+        for (auto *b : links.dev) c->pool_links.push_back(b);
+        for (auto *b : ranks.dev) c->pool_links.push_back(b);
+    }
+    void activate() { c->active = this; }
+};
+
+// Append the columns of a level whose queue is front[0..n): the parent links (from 96-byte realistic records when
+// `realistic`) and, with `with_ranks`, the global ranks in grank.  Then spill the oldest columns to pinned host memory
+// past the context's link budget, which the columns of a level share evenly.
+static int save_links(SolverBufs *s, int64_t n, bool realistic, bool with_ranks, cudaStream_t st) {
+    spl_ctx *c = s->c;
+    const bool keep = s->keep_links && n > 0;
+    const size_t need = keep ? (size_t)n * 8 : 0;
+    const int ncols = with_ranks ? 2 : 1;
+    LinkCols *cols[2] = {&s->links, &s->ranks};
+    DevBuf *buf[2] = {nullptr, nullptr};
+    for (int i = 0; i < ncols; ++i) {
+        buf[i] = take_link_buf(c, need);  // columns of earlier solves on this context
+        cols[i]->push(buf[i], s->keep_links ? n : 0);
+    }
+    if (!keep) return SPL_OK;
+    for (int i = 0; i < ncols; ++i)
+        if (buf[i]->cap < need) CK(c, buf[i]->ensure(link_bytes(n), 0, st));
+    if (realistic)
+        r_links_kernel<<<nblk(n), TILE, 0, st>>>(s->front.as<RRec>(), n, buf[0]->as<uint64_t>());
+    else
+        unpack_rec_kernel<<<nblk(n), TILE, 0, st>>>(s->front.as<Rec>(), n, nullptr, nullptr, buf[0]->as<uint64_t>());
+    ++c->launches;
+    if (with_ranks) CK(c, cudaMemcpyAsync(buf[1]->p, s->grank.p, need, cudaMemcpyDeviceToDevice, st));
+    CK(c, cudaGetLastError());
+    uint64_t moved = 0;
+    for (int i = 0; i < ncols; ++i) CK(c, cols[i]->spill(c->link_budget / ncols, &moved, st));
+    c->d2h_bytes += moved;
+    c->spilled_bytes += moved;
+    return SPL_OK;
+}
+
+struct spl_solver : SolverBufs {
+    int goal = 15, use_h = 0, heuristic = 0, tie = 0, noise = 0;
     bool realistic = false;
     bool grouped = false;  // beam search on the card-set-grouped level (spl_m2.cuh); otherwise the key-table level
     spl_rconfig rcfg{};
@@ -1187,39 +1291,12 @@ struct spl_solver {
     int64_t pend_n = 0, pend_uniq = 0;
     spl_level_info pend_info{};
     int64_t beam = 300000;
-    DevBuf front, uniq;
     int64_t n_front = 0;
     int level = 0;
     bool ended = false;
     int64_t goal_rank = -1;
-    LinkCols links;                // per level: link column of the queue
-    ~spl_solver() {
-        if (c->active == this) c->active = nullptr;
-        c->pool_front.swap(front);
-        c->pool_uniq.swap(uniq);
-        for (auto *b : links.dev) c->pool_links.push_back(b);
-    }
+    explicit spl_solver(spl_ctx *ctx) : SolverBufs(ctx) {}
 };
-
-static int save_links(spl_solver *s, cudaStream_t st) {
-    spl_ctx *c = s->c;
-    const bool keep = s->keep_links && s->n_front > 0;
-    DevBuf *b = take_link_buf(c, keep ? (size_t)s->n_front * 8 : 0);
-    s->links.push(b, s->keep_links ? s->n_front : 0);
-    if (!keep) return SPL_OK;
-    if (b->cap < (size_t)s->n_front * 8) CK(c, b->ensure(link_bytes(s->n_front), 0, st));
-    if (s->realistic)
-        r_links_kernel<<<nblk(s->n_front), TILE, 0, st>>>(s->front.as<RRec>(), s->n_front, b->as<uint64_t>());
-    else
-        unpack_rec_kernel<<<nblk(s->n_front), TILE, 0, st>>>(s->front.as<Rec>(), s->n_front, nullptr, nullptr, b->as<uint64_t>());
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    uint64_t moved = 0;
-    CK(c, s->links.spill(c->link_budget, &moved, st));
-    c->d2h_bytes += moved;
-    c->spilled_bytes += moved;
-    return SPL_OK;
-}
 
 // ------------------------------------------------------------------ card-set-grouped level (spl_m2.cuh)
 // grow the node table so that `need` more card sets keep its load factor <= 0.6 (if memory allows)
@@ -1250,7 +1327,16 @@ static int ensure_nodes(spl_ctx *c, uint64_t need, cudaStream_t st) {
     return SPL_OK;
 }
 
-// stable LSD sort of packed 64-bit items on bits [lo_bit, 64): result in c->y[*cur]
+// the root's card set into the node table (the grouped level's visited set), with the counters zeroed
+static int add_grouped_root(spl_ctx *c, uint64_t lo, uint64_t hi, cudaStream_t st) {
+    m2_root_kernel<<<1, 1, 0, st>>>(c->nodes, c->nn, lo, hi, c->d_gemrank, c->d_ctr);
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    c->node_occ = 1;
+    c->occupied = 1;
+    return SPL_OK;
+}
+
 // One-sweep stable LSD sort (spl_m2.cuh 2b) of k[*cur][0..n) by bits lo_bit .. lo_bit + nbits - 1, ping-ponging between
 // k[0] / k[1]; with a payload column (pl != nullptr) the pairs move together.  n < OS_MAX_ITEMS.
 static int onesweep_sort(spl_ctx *c, uint64_t *const k[2], uint32_t *const pl[2], int64_t n, int lo_bit, int nbits, int *cur, cudaStream_t st) {
@@ -1286,8 +1372,7 @@ static int onesweep_sort(spl_ctx *c, uint64_t *const k[2], uint32_t *const pl[2]
 // (rounds below 2^30 items), else 8-bit LSD passes with per-pass histogram + scan.
 static int sort_items(spl_ctx *c, int64_t n_items, int *cur, cudaStream_t st) {
     const unsigned snt = nblk(n_items, SORT_TILE);
-    static const bool no_onesweep = getenv("SPL_NO_ONESWEEP") != nullptr;
-    if (n_items < OS_MAX_ITEMS && !no_onesweep) {
+    if (n_items < OS_MAX_ITEMS) {
         uint64_t *const k[2] = {c->y[0].as<uint64_t>(), c->y[1].as<uint64_t>()};
         return onesweep_sort(c, k, nullptr, n_items, ITEM_KEY_LO, 64 - ITEM_KEY_LO, cur, st);
     }
@@ -1312,6 +1397,95 @@ static int sort_items(spl_ctx *c, int64_t n_items, int *cur, cudaStream_t st) {
     return SPL_OK;
 }
 
+// One round of a grouped level after its fan-out, the same on one GPU and on the card-set-sharded driver.
+struct GroupRound {
+    const Rec *front = nullptr;      // the round's parents
+    const Rec *brec = nullptr;       // the buy records: the round's own (one GPU) or those this rank received (sharded)
+    int64_t np = 0, n_items = 0;     // parents; items packed in c->y[0], the parents' first
+    uint64_t n_cands = 0;            // candidates (gem takes + buy records): the most winners the round can have
+    int64_t rank_base = 0;           // queue rank of front[0] (one GPU) ...
+    const uint64_t *grank = nullptr; // ... or the parents' global ranks (sharded)
+    bool unordered = false;          // the records arrive in no particular order (sharded): the warp kernel sorts them
+    DevBuf *out = nullptr;           // winners go to out / c->sk from slot out_base on
+    int64_t out_base = 0;
+    int heuristic = 0, noise = 0, level = 0;
+};
+struct RoundTimes { float sort, prep, thread, warp, cta; };  // CUDA-event ms: item sort + runs, node table + buffers, the kernels
+
+// Sort the round's items by card-set hash, find the runs of equal key, then deduplicate every run against the node
+// table: thread kernel over all runs, then the warp kernel and the CTA kernel over the runs each one queued.  The caller
+// has zeroed the counters; they hold the round's on return.
+static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, RoundTimes *t, cudaStream_t st) {
+    CK(c, cudaEventRecord(c->ev[1], st));
+    int cur = 0;
+    CKS(c, sort_items(c, R.n_items, &cur, st));
+    const unsigned rt = nblk(R.n_items, TILE * RUN_ITEMS);  // runs of equal key + candidate-weight prefix
+    CK(c, c->run_start.ensure((size_t)R.n_items * 4 + 8, 0, st));
+    CK(c, c->run_wpre.ensure((size_t)R.n_items * 4 + 8, 0, st));
+    CKS(c, prep_status(c, 1, rt, st));
+    CKS(c, prep_status(c, 2, rt, st));
+    CKS(c, reset_ticket(c, 1, st));
+    m2_runs_kernel<<<rt, TILE, 0, st>>>(c->y[cur].as<uint64_t>(), R.n_items, (uint32_t)R.np, c->ntk8.as<uint8_t>(), c->run_start.as<uint32_t>(),
+                                         c->run_wpre.as<uint32_t>(), c->status[1].as<uint64_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1);
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    CK(c, cudaEventRecord(c->ev[2], st));
+    CKS(c, read_ctr(c, st));
+    const uint64_t n_runs = c->h_ctr->n_runs;
+    // every run holds at least one card set; more than one only when two sets share the 30 sorted hash bits
+    CKS(c, ensure_nodes(c, n_runs + n_runs / 8 + 64, st));
+    CK(c, c->cls_list.ensure((size_t)n_runs * 8 + 16, 0, st));
+    const size_t n_out = (size_t)R.out_base + (size_t)R.n_cands;
+    CK(c, R.out->ensure(n_out * 32, (size_t)R.out_base * 32, st));
+    CK(c, c->sk.ensure(n_out * 8, (size_t)R.out_base * 8, st));
+    GroupArgs A;
+    A.front = R.front; A.brec = R.brec; A.iv = c->y[cur].as<uint64_t>();
+    A.run_start = c->run_start.as<uint32_t>(); A.run_wpre = c->run_wpre.as<uint32_t>();
+    A.np = (uint32_t)R.np; A.rank_base = R.rank_base; A.grank = R.grank; A.unordered = R.unordered;
+    A.warp_max = R.unordered ? std::min<uint32_t>(BIG_W, BSORT_MAX) : BIG_W;  // the warp kernel sorts at most BSORT_MAX records of a run itself
+    A.tabs = c->d_tabs; A.takes_idx = c->d_takes_idx; A.takes_edges = c->d_takes_edges; A.gemrank = c->d_gemrank; A.rankgems = c->d_rankgems;
+    A.nodes = c->nodes; A.nn = c->nn; A.out = R.out->as<Rec>(); A.out_sk = c->sk.as<uint64_t>(); A.out_base = (uint64_t)R.out_base;
+    for (int k = 0; k < NUM_CLS; ++k) A.cls_list[k] = nullptr;
+    A.cls_list[CLS_WARP] = c->cls_list.as<uint32_t>();
+    A.cls_list[CLS_CTA] = c->cls_list.as<uint32_t>() + n_runs;
+    A.h = R.heuristic; A.noise_mode = R.noise; A.L = c->luts; A.ctr = c->d_ctr;
+    CK(c, cudaEventRecord(c->ev[3], st));
+    if (R.unordered) m2_group_tiny_kernel<true><<<nblk((int64_t)n_runs), TILE, 0, st>>>(A, (uint32_t)n_runs);
+    else m2_group_tiny_kernel<false><<<nblk((int64_t)n_runs), TILE, 0, st>>>(A, (uint32_t)n_runs);
+    CK(c, cudaEventRecord(c->ev[4], st));
+    CKS(c, reset_ticket(c, 2, st));  // the warp kernel draws its runs from ticket 2
+    if (R.unordered) m2_group_warp_kernel<true><<<148 * SPL_WARP_CTAS, TILE, sizeof(WarpSmem), st>>>(A);
+    else m2_group_warp_kernel<false><<<148 * SPL_WARP_CTAS, TILE, offsetof(WarpSmem, bsort), st>>>(A);  // no sort area
+    CK(c, cudaEventRecord(c->ev[5], st));
+    m2_group_big_kernel<<<148 * 5, TILE, sizeof(BigSmem), st>>>(A);
+    c->launches += 3;
+    CK(c, cudaGetLastError());
+    CK(c, cudaEventRecord(c->ev[6], st));
+    CKS(c, read_ctr(c, st));
+    const Counters &h = *c->h_ctr;
+    cudaEventElapsedTime(&t->sort, c->ev[1], c->ev[2]);
+    cudaEventElapsedTime(&t->prep, c->ev[2], c->ev[3]);
+    cudaEventElapsedTime(&t->thread, c->ev[3], c->ev[4]);
+    cudaEventElapsedTime(&t->warp, c->ev[4], c->ev[5]);
+    cudaEventElapsedTime(&t->cta, c->ev[5], c->ev[6]);
+    if (getenv("SPL_DEBUG"))
+        fprintf(stderr, "[grouped] L%d np=%lld items=%lld runs=%llu cls=%u/%u/%u new_nodes=%u winners=%llu | sort+runs %.2f prep %.2f thread %.2f warp %.2f cta %.2f ms | nodes %llu/%llu\n",
+                R.level, (long long)R.np, (long long)R.n_items, (unsigned long long)n_runs,
+                (unsigned)(n_runs - h.n_cls[CLS_WARP] - h.n_cls[CLS_CTA]), h.n_cls[CLS_WARP], h.n_cls[CLS_CTA], h.n_new_nodes,
+                (unsigned long long)h.n_emitted, t->sort, t->prep, t->thread, t->warp, t->cta, (unsigned long long)c->node_occ,
+                (unsigned long long)c->nn);
+    if (h.error == 3)
+        return fail(c, SPL_E_CUDA, "level %d: more than %d card sets share one 30-bit sort key in a run of the warp kernel (or more than %d in one of the CTA kernel)",
+                    R.level, MAX_SETS, BIG_DONE);
+    if (h.error)
+        return fail(c, SPL_E_TABLE_FULL, "card-set table full during level %d (device error %u; %llu slots, max_node_bytes=%llu)", R.level,
+                    h.error, (unsigned long long)c->nn, (unsigned long long)c->max_node_bytes);
+    c->node_occ += h.n_new_nodes;
+    c->occupied += h.n_emitted;
+    *n_new_out = (int64_t)h.n_emitted;
+    return SPL_OK;
+}
+
 // expand + dedup (+ score) of the whole queue `front[0..n)` in rounds of parents; winners are appended to
 // s->uniq / c->sk in no particular order (their link words carry the arrival order)
 static int grouped_expand(spl_solver *s, const Rec *front, int64_t n, int64_t *n_uniq_out, int64_t *n_slots_out, int64_t *generated_out,
@@ -1323,7 +1497,7 @@ static int grouped_expand(spl_solver *s, const Rec *front, int64_t n, int64_t *n
     for (int64_t p0 = 0; p0 < n; p0 += chunk) {
         const int64_t np = std::min<int64_t>(chunk, n - p0);
         const unsigned nt = nblk(np);
-        // ---- 1. fan-out: buys offsets, take counts, sort keys of the parents
+        // fan-out: buys offsets, take counts, sort keys of the parents
         CKS(c, zero_ctr(c, st));
         CK(c, cudaEventRecord(c->ev[0], st));
         CK(c, c->boff2.ensure((size_t)np * 4 + 4, 0, st));
@@ -1352,82 +1526,21 @@ static int grouped_expand(spl_solver *s, const Rec *front, int64_t n, int64_t *n
             ++c->launches;
             CK(c, cudaGetLastError());
         }
-        CK(c, cudaEventRecord(c->ev[7], st));
-        // ---- 2. stable LSD sort of the items by the high half of their card-set hash
-        int cur = 0;
-        CKS(c, sort_items(c, n_items, &cur, st));
-        // ---- 3. runs of equal key + candidate-weight prefix
-        const unsigned rt = nblk(n_items, TILE * RUN_ITEMS);
-        CK(c, c->run_start.ensure((size_t)n_items * 4 + 8, 0, st));
-        CK(c, c->run_wpre.ensure((size_t)n_items * 4 + 8, 0, st));
-        CKS(c, prep_status(c, 1, rt, st));
-        CKS(c, prep_status(c, 2, rt, st));
-        CKS(c, reset_ticket(c, 1, st));
-        m2_runs_kernel<<<rt, TILE, 0, st>>>(c->y[cur].as<uint64_t>(), n_items, (uint32_t)np,
-                                             c->ntk8.as<uint8_t>(), c->run_start.as<uint32_t>(), c->run_wpre.as<uint32_t>(),
-                                             c->status[1].as<uint64_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1);
-        ++c->launches;
-        CK(c, cudaGetLastError());
-        CK(c, cudaEventRecord(c->ev[1], st));
-        CKS(c, read_ctr(c, st));
-        const uint64_t n_runs = c->h_ctr->n_runs;
-        // every run holds at least one card set; more than one only when two sets share the 30 sorted hash bits
-        CKS(c, ensure_nodes(c, n_runs + n_runs / 8 + 64, st));
-        CK(c, c->cls_list.ensure((size_t)n_runs * 8 + 16, 0, st));
-        CK(c, s->uniq.ensure((size_t)(n_slots + (int64_t)total) * 32, (size_t)n_slots * 32, st));
-        CK(c, c->sk.ensure((size_t)(n_slots + (int64_t)total) * 8, (size_t)n_slots * 8, st));
-        // ---- 4. per-run dedup: warp kernel, then the CTA kernel over the runs it queued
-        GroupArgs A;
-        A.front = front + p0; A.brec = c->brec.as<Rec>(); A.iv = c->y[cur].as<uint64_t>();
-        A.run_start = c->run_start.as<uint32_t>(); A.run_wpre = c->run_wpre.as<uint32_t>();
-        A.np = (uint32_t)np; A.rank_base = p0; A.grank = nullptr; A.unordered = 0; A.warp_max = BIG_W; A.tabs = c->d_tabs; A.takes_idx = c->d_takes_idx; A.takes_edges = c->d_takes_edges;
-        A.gemrank = c->d_gemrank; A.rankgems = c->d_rankgems; A.nodes = c->nodes; A.nn = c->nn; A.out = s->uniq.as<Rec>();
-        A.out_sk = c->sk.as<uint64_t>(); A.out_base = (uint64_t)n_slots;
-        for (int k = 0; k < NUM_CLS; ++k) A.cls_list[k] = nullptr;
-        A.cls_list[CLS_WARP] = c->cls_list.as<uint32_t>();
-        A.cls_list[CLS_CTA] = c->cls_list.as<uint32_t>() + n_runs;
-        A.h = s->heuristic; A.noise_mode = s->noise; A.L = c->luts; A.ctr = c->d_ctr;
-        CK(c, cudaEventRecord(c->ev[2], st));
-        // dispatch + thread kernel over all runs, then the warp kernel and the CTA kernel over the runs it queued
-        m2_group_tiny_kernel<false><<<nblk((int64_t)n_runs), TILE, 0, st>>>(A, (uint32_t)n_runs);
-        CK(c, cudaEventRecord(c->ev[4], st));
-        CKS(c, reset_ticket(c, 2, st));  // the warp kernel draws its runs from ticket 2
-        m2_group_warp_kernel<false><<<148 * SPL_WARP_CTAS, TILE, offsetof(WarpSmem, bsort), st>>>(A);
-        CK(c, cudaEventRecord(c->ev[5], st));
-        CK(c, cudaEventRecord(c->ev[6], st));
-        m2_group_big_kernel<<<148 * 5, TILE, sizeof(BigSmem), st>>>(A);
-        c->launches += 3;
-        CK(c, cudaGetLastError());
-        CK(c, cudaEventRecord(c->ev[3], st));
-        CKS(c, read_ctr(c, st));
-        if (c->h_ctr->error)
-            return fail(c, c->h_ctr->error == 3 ? SPL_E_CUDA : SPL_E_TABLE_FULL,
-                        c->h_ctr->error == 3 ? "internal: more than %d card sets share one sort key (level %d)" : "card-set table full during level %d (code %d)",
-                        c->h_ctr->error == 3 ? BIG_DONE : s->level, c->h_ctr->error == 3 ? s->level : (int)c->h_ctr->error);
-        const int64_t n_new = (int64_t)c->h_ctr->n_emitted;
-        c->node_occ += c->h_ctr->n_new_nodes;
-        c->occupied += n_new;
+        GroupRound R;
+        R.front = front + p0; R.brec = c->brec.as<Rec>(); R.np = np; R.n_items = n_items; R.n_cands = total; R.rank_base = p0;
+        R.out = &s->uniq; R.out_base = n_slots; R.heuristic = s->heuristic; R.noise = s->noise; R.level = s->level;
+        int64_t n_new = 0;
+        RoundTimes t;
+        CKS(c, group_round(c, R, &n_new, &t, st));
         if (n_new) { sk_min = std::min<uint64_t>(sk_min, c->h_ctr->sk_min); sk_max = std::max<uint64_t>(sk_max, c->h_ctr->sk_max); }
         n_uniq += n_new;
         n_slots += n_new;  // dense output
-        float t;
-        cudaEventElapsedTime(&t, c->ev[0], c->ev[7]); ms[0] += t;   // fan-out + buy records
-        cudaEventElapsedTime(&t, c->ev[7], c->ev[1]); ms[2] += t;   // item sort + runs (grouping)
-        cudaEventElapsedTime(&t, c->ev[2], c->ev[3]); ms[1] += t;   // per-run dedup + emit + score (the dominant stage)
-        cudaEventElapsedTime(&t, c->ev[4], c->ev[5]); ms[5] += t;   // ... of which the warp kernel
-        if (getenv("SPL_DEBUG")) {
-            float tt = 0, ts = 0, tm = 0, tb = 0, tc = 0, tso = 0;
-            cudaEventElapsedTime(&tt, c->ev[2], c->ev[4]);
-            cudaEventElapsedTime(&ts, c->ev[4], c->ev[5]);
-            cudaEventElapsedTime(&tm, c->ev[5], c->ev[6]);
-            cudaEventElapsedTime(&tb, c->ev[6], c->ev[3]);
-            cudaEventElapsedTime(&tc, c->ev[0], c->ev[7]);
-            cudaEventElapsedTime(&tso, c->ev[7], c->ev[1]);
-            fprintf(stderr, "[grouped] L%d p0=%lld np=%lld takes=%llu buys=%llu runs=%llu cls=%u/%u/%u new_nodes=%u winners=%lld | count+buys %.2f sort+runs %.2f thread %.2f warp %.2f (-) %.2f cta %.2f ms | nodes %llu/%llu\n",
-                    s->level, (long long)p0, (long long)np, (unsigned long long)n_takes, (unsigned long long)n_buys,
-                    (unsigned long long)n_runs, (unsigned)(n_runs - c->h_ctr->n_cls[CLS_WARP] - c->h_ctr->n_cls[CLS_CTA]), c->h_ctr->n_cls[CLS_WARP], c->h_ctr->n_cls[CLS_CTA], c->h_ctr->n_new_nodes,
-                    (long long)n_new, tc, tso, tt, ts, tm, tb, (unsigned long long)c->node_occ, (unsigned long long)c->nn);
-        }
+        float t_count;
+        cudaEventElapsedTime(&t_count, c->ev[0], c->ev[1]);
+        ms[0] += t_count;                        // fan-out + buy records
+        ms[2] += t.sort;                         // item sort + runs (grouping)
+        ms[1] += t.thread + t.warp + t.cta;      // per-run dedup + emit + score (the dominant stage)
+        ms[5] += t.warp;                         // ... of which the warp kernel
     }
     *n_uniq_out = n_uniq;
     *n_slots_out = n_slots;
@@ -1446,11 +1559,9 @@ static int grouped_expand(spl_solver *s, const Rec *front, int64_t n, int64_t *n
 //                      -> spl_gs_tie_pick) x passes] -> spl_gs_cut (local survivors, sorted by their sort word)
 //           ranks:  sample sort of the sort words across ranks (spl_gs_partition / spl_gs_rank_sort + all-to-all) ->
 //                   spl_gs_adopt (next queue = survivors with their global ranks)
-struct spl_gsolver {
-    spl_ctx *c = nullptr;
-    int rank = 0, world = 1, goal = 15, heuristic = 0, noise = 0, keep_links = 1;
+struct spl_gsolver : SolverBufs {
+    int rank = 0, world = 1, goal = 15, heuristic = 0, noise = 0;
     int64_t beam = 0;
-    DevBuf front, grank, uniq;
     int64_t n_local = 0, n_global = 1;
     int level = 0;
     // round
@@ -1463,38 +1574,8 @@ struct spl_gsolver {
     // cut
     int lt = 0, cut_cur = 0;
     int64_t kept_local = 0;
-    LinkCols link_cols, rank_cols;  // per level: links / global ranks of the local queue (path reconstruction)
-    ~spl_gsolver() {
-        if (c->active == this) c->active = nullptr;
-        c->pool_front.swap(front);  // keep the big buffers for the next solve on this context
-        c->pool_uniq.swap(uniq);
-        c->pool_grank.swap(grank);
-        for (auto *b : link_cols.dev) c->pool_links.push_back(b);
-        for (auto *b : rank_cols.dev) c->pool_links.push_back(b);
-    }
+    explicit spl_gsolver(spl_ctx *ctx) : SolverBufs(ctx) {}
 };
-
-static int gs_save_links(spl_gsolver *s, cudaStream_t st) {
-    spl_ctx *c = s->c;
-    const bool keep = s->keep_links && s->n_local > 0;
-    const size_t need = keep ? (size_t)s->n_local * 8 : 0;
-    DevBuf *lb = take_link_buf(c, need), *rb = take_link_buf(c, need);  // columns of earlier solves on this context
-    s->link_cols.push(lb, s->keep_links ? s->n_local : 0);
-    s->rank_cols.push(rb, s->keep_links ? s->n_local : 0);
-    if (!keep) return SPL_OK;
-    if (lb->cap < need) CK(c, lb->ensure(link_bytes(s->n_local), 0, st));
-    if (rb->cap < need) CK(c, rb->ensure(link_bytes(s->n_local), 0, st));
-    unpack_rec_kernel<<<nblk(s->n_local), TILE, 0, st>>>(s->front.as<Rec>(), s->n_local, nullptr, nullptr, lb->as<uint64_t>());
-    ++c->launches;
-    CK(c, cudaMemcpyAsync(rb->p, s->grank.p, (size_t)s->n_local * 8, cudaMemcpyDeviceToDevice, st));
-    CK(c, cudaGetLastError());
-    uint64_t moved = 0;  // the two columns share the budget
-    CK(c, s->link_cols.spill(c->link_budget / 2, &moved, st));
-    CK(c, s->rank_cols.spill(c->link_budget / 2, &moved, st));
-    c->d2h_bytes += moved;
-    c->spilled_bytes += moved;
-    return SPL_OK;
-}
 
 extern "C" {
 
@@ -1507,13 +1588,9 @@ int32_t spl_gs_create(spl_ctx *c, int32_t rank, int32_t world, const spl_key *ro
     CK(c, enter_device(c));
     cudaStream_t st = 0;
     CKS(c, reset_visited(c, st));
-    spl_gsolver *s = new spl_gsolver();
-    s->c = c; s->rank = rank; s->world = world; s->goal = goal; s->heuristic = heuristic; s->beam = beam; s->noise = noise;
+    spl_gsolver *s = new spl_gsolver(c);
+    s->rank = rank; s->world = world; s->goal = goal; s->heuristic = heuristic; s->beam = beam; s->noise = noise;
     s->keep_links = keep_links;
-    s->front.swap(c->pool_front);
-    s->uniq.swap(c->pool_uniq);
-    s->grank.swap(c->pool_grank);
-    std::sort(c->pool_links.begin(), c->pool_links.end(), [](DevBuf *a, DevBuf *b) { return a->cap > b->cap; });
     uint64_t m0, m1;
     mask_words(root_key->lo, root_key->hi & HI_KEY_MASK, m0, m1);
     int rc = SPL_OK;
@@ -1528,18 +1605,13 @@ int32_t spl_gs_create(spl_ctx *c, int32_t rank, int32_t world, const spl_key *ro
         c->h2d_bytes += 40;
         if (e != cudaSuccess) rc = fail(c, SPL_E_CUDA, "root upload: %s", cudaGetErrorString(e));
         if (rc == SPL_OK) rc = zero_ctr(c, st);
-        if (rc == SPL_OK) {
-            m2_root_kernel<<<1, 1, 0, st>>>(c->nodes, c->nn, r.lo, r.hi, c->d_gemrank, c->d_ctr);
-            ++c->launches;
-            c->node_occ = 1;
-            c->occupied = 1;
-        }
+        if (rc == SPL_OK) rc = add_grouped_root(c, r.lo, r.hi, st);
         s->n_local = 1;
     }
-    if (rc == SPL_OK) rc = gs_save_links(s, st);
+    if (rc == SPL_OK) rc = save_links(s, s->n_local, false, true, st);
     if (rc == SPL_OK && cudaStreamSynchronize(st) != cudaSuccess) rc = fail(c, SPL_E_CUDA, "spl_gs_create: sync failed");
     if (rc != SPL_OK) { delete s; return rc; }
-    c->active = s;
+    s->activate();
     *out = s;
     return SPL_OK;
 }
@@ -1727,67 +1799,19 @@ int32_t spl_gs_round_group(spl_gsolver *s, const void *recv_dev, int64_t n_recv,
         return fail(c, SPL_E_INVALID, "round holds %llu candidates (>= 2^32): use smaller rank windows", (unsigned long long)total);
     CK(c, c->y[0].ensure((size_t)n_items * 8 + 8, (size_t)np * 8, st));
     CK(c, c->y[1].ensure((size_t)n_items * 8 + 8, 0, st));
+    CKS(c, zero_ctr(c, st));  // a rank without parents in this round skipped the one in spl_gs_round_begin
     if (n_recv) {
         gs_recv_items_kernel<<<nblk(n_recv), TILE, 0, st>>>(reinterpret_cast<const Rec *>(recv_dev), n_recv, (uint32_t)np, c->y[0].as<uint64_t>());
         ++c->launches;
     }
-    const bool dbg = getenv("SPL_DEBUG") != nullptr;
-    CK(c, cudaEventRecord(c->ev[0], st));
-    int cur = 0;
-    CKS(c, sort_items(c, n_items, &cur, st));
-    const unsigned rt = nblk(n_items, TILE * RUN_ITEMS);
-    CK(c, c->run_start.ensure((size_t)n_items * 4 + 8, 0, st));
-    CK(c, c->run_wpre.ensure((size_t)n_items * 4 + 8, 0, st));
-    CKS(c, zero_ctr(c, st));
-    CKS(c, prep_status(c, 1, rt, st));
-    CKS(c, prep_status(c, 2, rt, st));
-    m2_runs_kernel<<<rt, TILE, 0, st>>>(c->y[cur].as<uint64_t>(), n_items, (uint32_t)np, c->ntk8.as<uint8_t>(), c->run_start.as<uint32_t>(),
-                                         c->run_wpre.as<uint32_t>(), c->status[1].as<uint64_t>(), c->status[2].as<uint64_t>(), c->d_ctr, 1);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    const uint64_t n_runs = c->h_ctr->n_runs;
-    CKS(c, ensure_nodes(c, n_runs + n_runs / 8 + 64, st));
-    CK(c, c->cls_list.ensure((size_t)n_runs * 8 + 16, 0, st));
-    CK(c, s->uniq.ensure((size_t)(s->n_uniq + (int64_t)total) * 32, (size_t)s->n_uniq * 32, st));
-    CK(c, c->sk.ensure((size_t)(s->n_uniq + (int64_t)total) * 8, (size_t)s->n_uniq * 8, st));
-    GroupArgs A;
-    A.front = s->front.as<Rec>() + s->r_p0; A.brec = reinterpret_cast<const Rec *>(recv_dev); A.iv = c->y[cur].as<uint64_t>();
-    A.run_start = c->run_start.as<uint32_t>(); A.run_wpre = c->run_wpre.as<uint32_t>();
-    A.np = (uint32_t)np; A.rank_base = 0; A.grank = s->grank.as<uint64_t>() + s->r_p0; A.unordered = 1;
-    A.warp_max = std::min<uint32_t>(BIG_W, BSORT_MAX);  // the warp kernel sorts at most BSORT_MAX records of a run itself
-    A.tabs = c->d_tabs; A.takes_idx = c->d_takes_idx; A.takes_edges = c->d_takes_edges; A.gemrank = c->d_gemrank; A.rankgems = c->d_rankgems;
-    A.nodes = c->nodes; A.nn = c->nn; A.out = s->uniq.as<Rec>(); A.out_sk = c->sk.as<uint64_t>(); A.out_base = (uint64_t)s->n_uniq;
-    for (int k = 0; k < NUM_CLS; ++k) A.cls_list[k] = nullptr;
-    A.cls_list[CLS_WARP] = c->cls_list.as<uint32_t>();
-    A.cls_list[CLS_CTA] = c->cls_list.as<uint32_t>() + n_runs;
-    A.h = s->heuristic; A.noise_mode = s->noise; A.L = c->luts; A.ctr = c->d_ctr;
-    CK(c, cudaEventRecord(c->ev[1], st));
-    m2_group_tiny_kernel<true><<<nblk((int64_t)n_runs), TILE, 0, st>>>(A, (uint32_t)n_runs);
-    CK(c, cudaEventRecord(c->ev[2], st));
-    CKS(c, reset_ticket(c, 2, st));
-    m2_group_warp_kernel<true><<<148 * SPL_WARP_CTAS, TILE, sizeof(WarpSmem), st>>>(A);
-    CK(c, cudaEventRecord(c->ev[3], st));
-    m2_group_big_kernel<<<148 * 5, TILE, sizeof(BigSmem), st>>>(A);
-    CK(c, cudaEventRecord(c->ev[4], st));
-    c->launches += 3;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    float t1 = 0, t2 = 0, t3 = 0, t4 = 0;
-    cudaEventElapsedTime(&t1, c->ev[0], c->ev[1]); cudaEventElapsedTime(&t2, c->ev[1], c->ev[2]);
-    cudaEventElapsedTime(&t3, c->ev[2], c->ev[3]); cudaEventElapsedTime(&t4, c->ev[3], c->ev[4]);
-    s->ms[0] += t1; s->ms[1] += t2; s->ms[2] += t3; s->ms[3] += t4;
-    if (dbg) {
-        fprintf(stderr, "[gs r%d] L%d np=%lld recv=%lld takes=%llu runs=%llu warp=%u cta=%u winners=%llu | sort+runs %.2f tiny %.2f warp %.2f cta %.2f ms\n",
-                s->rank, s->level, (long long)np, (long long)n_recv, (unsigned long long)s->r_takes, (unsigned long long)n_runs,
-                c->h_ctr->n_cls[CLS_WARP], c->h_ctr->n_cls[CLS_CTA], (unsigned long long)c->h_ctr->n_emitted, t1, t2, t3, t4);
-    }
-    if (c->h_ctr->error)
-        return fail(c, c->h_ctr->error == 3 ? SPL_E_CUDA : SPL_E_TABLE_FULL, "sharded level %d: device error code %u (2 = card-set table full, 3 = too many card sets under one sort key)",
-                    s->level, c->h_ctr->error);
-    const int64_t n_new = (int64_t)c->h_ctr->n_emitted;
-    c->node_occ += c->h_ctr->n_new_nodes;
-    c->occupied += n_new;
+    GroupRound R;
+    R.front = s->front.as<Rec>() + s->r_p0; R.brec = reinterpret_cast<const Rec *>(recv_dev); R.np = np; R.n_items = n_items;
+    R.n_cands = total; R.grank = s->grank.as<uint64_t>() + s->r_p0; R.unordered = true; R.out = &s->uniq; R.out_base = s->n_uniq;
+    R.heuristic = s->heuristic; R.noise = s->noise; R.level = s->level;
+    int64_t n_new = 0;
+    RoundTimes t;
+    CKS(c, group_round(c, R, &n_new, &t, st));
+    s->ms[0] += t.sort + t.prep; s->ms[1] += t.thread; s->ms[2] += t.warp; s->ms[3] += t.cta;
     s->n_uniq += n_new;
     *n_new_host = n_new;
     return SPL_OK;
@@ -1914,40 +1938,10 @@ int32_t spl_gs_cut(spl_gsolver *s, int32_t have_tie_threshold, int64_t *kept_loc
     *y_sorted_dev = nullptr;
     s->cut_cur = 0;
     if (n == 0) return SPL_OK;
-    for (int b = 0; b < 2; ++b) {
-        CK(c, c->y[b].ensure((size_t)n * 8 + 8, 0, st));
-        CK(c, c->idx[b].ensure((size_t)n * 4 + 4, 0, st));
-    }
-    const unsigned ct = nblk(n, TILE * CUTP_ITEMS);
-    CKS(c, prep_status(c, 2, ct, st));
-    CKS(c, zero_ctr(c, st));
-    cut_pack_kernel<<<ct, TILE, 0, st>>>(c->sk.as<uint64_t>(), reinterpret_cast<const uint64_t *>(s->uniq.p), 4, n, 0, 0, have_tie_threshold ? 0 : 1,
-                                          c->d_sel, c->d_dict2, s->lt, c->y[0].as<uint64_t>(), c->idx[0].as<uint32_t>(), c->status[2].as<uint64_t>(),
-                                          c->d_ctr, 1);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    uint64_t last = 0;
-    CK(c, cudaMemcpyAsync(&last, c->status[2].as<uint64_t>() + (ct - 1), 8, cudaMemcpyDeviceToHost, st));
-    CK(c, cudaStreamSynchronize(st));
-    c->d2h_bytes += 8;
-    const int64_t kept = (int64_t)(last & ((1ull << 62) - 1));
     int cur = 0;
-    if (kept > 1) {
-        const unsigned nt = nblk(kept, SORT_TILE);
-        const size_t msz = (size_t)SORT_BINS * nt;
-        CK(c, c->matrix.ensure(msz * 4, 0, st));
-        CK(c, c->matrix2.ensure(msz * 4, 0, st));
-        if (kept < OS_MAX_ITEMS) {
-            uint64_t *const yk[2] = {c->y[0].as<uint64_t>(), c->y[1].as<uint64_t>()};
-            uint32_t *const yi[2] = {c->idx[0].as<uint32_t>(), c->idx[1].as<uint32_t>()};
-            CKS(c, onesweep_sort(c, yk, yi, kept, 0, nbits, &cur, st));
-        } else {
-            for (int shift = 0; shift < nbits; shift += SORT_BITS) {
-                CKS(c, sort_pass(c, 0, cur, c->y[cur].as<uint64_t>(), kept, shift, nt, msz, st));
-                cur ^= 1;
-            }
-        }
-    }
+    int64_t kept = 0;
+    CKS(c, cut_packed(c, c->sk.as<uint64_t>(), reinterpret_cast<const uint64_t *>(s->uniq.p), 4, n, n, 0, 0, have_tie_threshold ? 0 : 1,
+                      c->d_dict2, s->lt, &cur, &kept, st));
     s->cut_cur = cur;
     *kept_local_host = s->kept_local = kept;
     *y_sorted_dev = c->y[cur].as<uint64_t>();
@@ -2025,7 +2019,7 @@ int32_t spl_gs_adopt(spl_gsolver *s, const int64_t *granks_dev, int64_t n_global
     s->n_global = n_global_next;
     s->level += 1;
     if (dbg) CK(c, cudaEventRecord(c->ev[1], st));
-    CKS(c, gs_save_links(s, st));
+    CKS(c, save_links(s, s->n_local, false, true, st));
     if (dbg) CK(c, cudaEventRecord(c->ev[2], st));
     CK(c, cudaStreamSynchronize(st));
     if (dbg) {
@@ -2047,25 +2041,25 @@ int32_t spl_gs_frontier(spl_gsolver *s, const void **recs_dev, const uint64_t **
 
 // link (parent rank << 8 | ordinal) of the state with global rank `grank` in the queue of `level`, if this rank holds it
 int32_t spl_gs_link_at(spl_gsolver *s, int32_t level, int64_t grank, int32_t *found_host, uint64_t *link_host) {
-    if (!s || !found_host || !link_host || level < 0 || level >= (int)s->rank_cols.dev.size()) return SPL_E_INVALID;
+    if (!s || !found_host || !link_host || level < 0 || level >= (int)s->ranks.dev.size()) return SPL_E_INVALID;
     spl_ctx *c = s->c;
     if (!s->keep_links) return fail(c, SPL_E_STATE, "spl_gs_link_at: solver was created with keep_links = 0");
     CK(c, enter_device(c));
     *found_host = 0;
     *link_host = 0;
-    const int64_t n = s->rank_cols.n[level];
+    const int64_t n = s->ranks.n[level];
     int64_t lo = 0, hi = n;
     while (lo < hi) {
         const int64_t mid = (lo + hi) >> 1;
         uint64_t v = 0;
-        CK(c, s->rank_cols.read(level, mid, &v));
+        CK(c, s->ranks.read(level, mid, &v));
         if ((int64_t)v < grank) lo = mid + 1; else hi = mid;
     }
     if (lo < n) {
         uint64_t v = 0;
-        CK(c, s->rank_cols.read(level, lo, &v));
+        CK(c, s->ranks.read(level, lo, &v));
         if ((int64_t)v == grank) {
-            CK(c, s->link_cols.read(level, lo, link_host));
+            CK(c, s->links.read(level, lo, link_host));
             *found_host = 1;
         }
     }
@@ -2085,13 +2079,10 @@ static int speedrun_cut(spl_solver *s, spl_level_info *info, int64_t n, int64_t 
     if (s->use_h && n_uniq > 0) {
         int which = 0;
         CK(c, cudaEventRecord(c->ev[4], st));
-        // grouped level: the winners are unordered, so `stable` ties are broken on the link words (arrival order)
-        const bool link_ties = s->grouped && s->tie == SPL_TIE_STABLE;
-        c->tie_link_top = link_ties ? 8 + bitlen((uint64_t)n) : 0;
-        const int rc_cut = run_cut_sort(c, c->sk.as<uint64_t>(), s->uniq.as<Rec>(), n_slots, s->beam, sk_min, sk_max,
-                                        s->tie == SPL_TIE_KEY || link_ties, &which, &kept, st, n_uniq);
-        c->tie_link_top = 0;
-        CKS(c, rc_cut);
+        CutMode mode;
+        if (s->tie == SPL_TIE_KEY) mode.ties = TIES_KEY;
+        else if (s->grouped) mode = {TIES_LINK, 8 + bitlen((uint64_t)n)};  // unordered winners: arrival order is in their links
+        CKS(c, run_cut_sort(c, c->sk.as<uint64_t>(), s->uniq.as<Rec>(), n_slots, s->beam, sk_min, sk_max, mode, &which, &kept, st, n_uniq));
         CK(c, cudaEventRecord(c->ev[5], st));
         CK(c, s->front.ensure((size_t)kept * 32, 0, st));
         gather_rec_kernel<<<nblk(kept), TILE, 0, st>>>(s->uniq.as<Rec>(), c->idx[which].as<uint32_t>(), kept, s->front.as<Rec>());
@@ -2118,7 +2109,7 @@ static int speedrun_cut(spl_solver *s, spl_level_info *info, int64_t n, int64_t 
     }
     s->n_front = kept;
     s->level += 1;
-    CKS(c, save_links(s, st));
+    CKS(c, save_links(s, s->n_front, s->realistic, false, st));
     CK(c, cudaStreamSynchronize(st));
     return SPL_OK;
 }
@@ -2315,7 +2306,7 @@ static int realistic_cut(spl_solver *s, spl_level_info *info, int64_t n, int64_t
         CKS(c, read_ctr(c, st));
         const uint64_t smin = c->h_ctr->sk_min, smax = c->h_ctr->sk_max;
         int which = 0;
-        CKS(c, run_cut_sort(c, c->sk.as<uint64_t>(), nullptr, n_new, s->beam, smin, smax, 0, &which, &kept, st));
+        CKS(c, run_cut_sort(c, c->sk.as<uint64_t>(), nullptr, n_new, s->beam, smin, smax, CutMode{}, &which, &kept, st));
         if (s->level < 1000) {  // at the turn limit the queue just expanded stays in place (see below)
             CK(c, s->front.ensure((size_t)kept * 96, 0, st));
             r_gather_kernel<uint32_t><<<nblk(kept), TILE, 0, st>>>(s->uniq.as<RRec>(), c->idx[which].as<uint32_t>(), kept, s->front.as<RRec>());
@@ -2341,7 +2332,7 @@ static int realistic_cut(spl_solver *s, spl_level_info *info, int64_t n, int64_t
     }
     s->n_front = kept;
     s->level += 1;
-    CKS(c, save_links(s, st));
+    CKS(c, save_links(s, s->n_front, s->realistic, false, st));
     CK(c, cudaStreamSynchronize(st));
     return SPL_OK;
 }
@@ -2358,15 +2349,12 @@ int32_t spl_solver_create(spl_ctx *c, const spl_key *root_key, uint64_t root_aux
     NO_LIVE_SOLVER(c, "spl_solver_create");
     CK(c, enter_device(c));
     cudaStream_t st = 0;
-    spl_solver *s = new spl_solver();
-    s->c = c; s->goal = goal; s->use_h = use_h; s->heuristic = heuristic; s->beam = beam; s->tie = tie;
+    spl_solver *s = new spl_solver(c);
+    s->goal = goal; s->use_h = use_h; s->heuristic = heuristic; s->beam = beam; s->tie = tie;
     s->noise = noise; s->keep_links = keep_links;
     // beam search with on-device scoring runs on the card-set-grouped level; exhaustive BFS (queue order == arrival
     // order), the reference's hash identity and externally drawn noise (arrival-ordered draws) on the key table
     s->grouped = use_h && noise != SPL_NOISE_EXTERNAL && c->identity == IDENT_KEY && !getenv("SPL_NO_GROUPED");
-    s->front.swap(c->pool_front);
-    s->uniq.swap(c->pool_uniq);
-    std::sort(c->pool_links.begin(), c->pool_links.end(), [](DevBuf *a, DevBuf *b) { return a->cap > b->cap; });
     int rc = reset_visited(c, st);
     if (rc == SPL_OK) {
         Rec r{root_key->lo, root_key->hi & HI_KEY_MASK, root_aux, ~0ull};
@@ -2383,10 +2371,7 @@ int32_t spl_solver_create(spl_ctx *c, const spl_key *root_key, uint64_t root_aux
             cudaError_t e = c->cand_slot.ensure(4, 0, st);
             if (e != cudaSuccess) rc = fail(c, SPL_E_NOMEM, "cand_slot alloc");
             else if (s->grouped) {
-                m2_root_kernel<<<1, 1, 0, st>>>(c->nodes, c->nn, root_key->lo, root_key->hi & HI_KEY_MASK, c->d_gemrank, c->d_ctr);
-                ++c->launches;
-                c->occupied = 1;
-                c->node_occ = 1;
+                rc = add_grouped_root(c, root_key->lo, root_key->hi & HI_KEY_MASK, st);
             } else {
                 if (c->identity == IDENT_PYHASH)
                     probe_list_kernel<IDENT_PYHASH><<<1, TILE, 0, st>>>(reinterpret_cast<const spl_key *>(s->front.p), 1, c->table,
@@ -2400,10 +2385,10 @@ int32_t spl_solver_create(spl_ctx *c, const spl_key *root_key, uint64_t root_aux
         }
     }
     s->n_front = 1;
-    if (rc == SPL_OK) rc = save_links(s, st);
+    if (rc == SPL_OK) rc = save_links(s, s->n_front, false, false, st);
     if (rc == SPL_OK && cudaStreamSynchronize(st) != cudaSuccess) rc = fail(c, SPL_E_CUDA, "solver create sync failed");
     if (rc != SPL_OK) { delete s; return rc; }
-    c->active = s;
+    s->activate();
     *out = s;
     return SPL_OK;
 }
@@ -2602,11 +2587,9 @@ int32_t spl_rsolver_create(spl_ctx *c, const spl_rconfig *cfg, const void *root_
     CK(c, enter_device(c));
     cudaStream_t st = 0;
     CKS(c, upload_rconfig(c, cfg, st));
-    spl_solver *s = new spl_solver();
-    s->c = c; s->realistic = true; s->rcfg = *cfg; s->use_h = 1; s->beam = beam; s->keep_links = keep_links;
+    spl_solver *s = new spl_solver(c);
+    s->realistic = true; s->rcfg = *cfg; s->use_h = 1; s->beam = beam; s->keep_links = keep_links;
     s->goal = cfg->target_points;
-    s->front.swap(c->pool_front);
-    s->uniq.swap(c->pool_uniq);
     c->rcfg_dirty = false;
     int rc = reset_visited(c, st);
     if (rc == SPL_OK) {
@@ -2638,10 +2621,10 @@ int32_t spl_rsolver_create(spl_ctx *c, const spl_rconfig *cfg, const void *root_
             c->occupied = 1;
         }
     }
-    if (rc == SPL_OK) rc = save_links(s, st);
+    if (rc == SPL_OK) rc = save_links(s, s->n_front, true, false, st);
     if (rc == SPL_OK && cudaStreamSynchronize(st) != cudaSuccess) rc = fail(c, SPL_E_CUDA, "rsolver create sync failed");
     if (rc != SPL_OK) { delete s; return rc; }
-    c->active = s;
+    s->activate();
     *out = s;
     return SPL_OK;
 }

@@ -290,7 +290,18 @@ class Engine:
                            keep_links)
 
 
-class LevelSolver:
+class Stepper:
+    """run() of the level solvers: step() is one `while queue` iteration that appends its counters to self.infos"""
+
+    def run(self, max_levels=None):
+        while not self.ended:
+            self.step()
+            if max_levels is not None and len(self.infos) >= max_levels:
+                break
+        return self.infos
+
+
+class LevelSolver(Stepper):
     """spl_solver_*: one object per solve(); step() == one `while queue` iteration (src/solver.py:434-457)."""
 
     def __init__(self, eng: Engine, root_key, root_aux, goal_pts, use_heuristic, heuristic, beam_width, tie, noise,
@@ -318,13 +329,6 @@ class LevelSolver:
         self.infos.append(d)
         self.ended = bool(li.ended)
         return d
-
-    def run(self, max_levels=None):
-        while not self.ended:
-            self.step()
-            if max_levels is not None and len(self.infos) >= max_levels:
-                break
-        return self.infos
 
     def frontier(self) -> torch.Tensor:
         """Current queue as an int64 tensor [n, 4] = (lo, hi, aux, link) viewing library memory."""

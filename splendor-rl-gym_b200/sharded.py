@@ -29,7 +29,7 @@ import torch
 import torch.distributed as dist
 
 from ._lib import Key as _Key, check, lib
-from .engine import NOISE_IDS, TIE_IDS, Engine, _DevArray, heuristic_id
+from .engine import NOISE_IDS, TIE_IDS, Engine, Stepper, _DevArray, heuristic_id
 
 import os
 import time
@@ -52,6 +52,20 @@ def _tick(name, t0):
 
 def _bitlen(x: int) -> int:
     return int(x).bit_length()
+
+
+def _radix_select(comm, top, hist, pick):
+    """global radix select over the `top` high bits, SEL_BITS (or the bits left) per pass, most significant first:
+    hist(shift, bits, first) -> this rank's histogram of the pass (a device tensor), all-reduced here before
+    pick(shift, first) narrows the selection"""
+    first = True
+    while top > 0:
+        bits = min(SEL_BITS, top)
+        shift = top - bits
+        comm.all_reduce(hist(shift, bits, first), dist.ReduceOp.SUM)
+        pick(shift, first)
+        first = False
+        top = shift
 
 
 class Comm:
@@ -242,7 +256,7 @@ class CudaBackend:
                                  int(sorted_a), self.eng._stream()), self.eng._h)
 
 
-class ShardedSolver:
+class ShardedSolver(Stepper):
     """State.solve (src/solver.py:390-464) over a frontier sharded across `comm.world` ranks.
 
     Queue layout: global rank space [0, N) cut into blocks of `block_parents` ranks; block b lives on rank
@@ -459,30 +473,16 @@ class ShardedSolver:
         if not keep_all:
             nbits = _bitlen(smax - smin)
             b.dtopk_set([0, K, 0, u_total, 0, 0])
-            top, first, init_k = nbits, True, True
-            while top > 0:
-                bits = min(SEL_BITS, top)
-                shift = top - bits
-                hist = b.dtopk_hist(0, shift, bits, first, smin)
-                comm.all_reduce(hist, dist.ReduceOp.SUM)
-                b.dtopk_pick(0, shift, first, init_k, K)
-                first = init_k = False
-                top = shift
+            _radix_select(comm, nbits, lambda shift, bits, first: b.dtopk_hist(0, shift, bits, first, smin),
+                          lambda shift, first: b.dtopk_pick(0, shift, first, first, K))
             state = b.dtopk_get()
             quota, tie_count = state[1], state[3]
             if quota < tie_count:  # split the score ties by key (det) / by arrival (stable, synthetic key)
                 all_ties = False
                 # synthetic arrival keys are < 2^bitlen(u_total) with a zero high word: skip the constant digits
                 for word, wbits in (((1, 41), (2, 64)) if self.tie == 'det' else ((2, _bitlen(u_total)),)):
-                    top, first = wbits, True
-                    while top > 0:
-                        bits = min(SEL_BITS, top)
-                        shift = top - bits
-                        hist = b.dtopk_hist(word, shift, bits, first, smin)
-                        comm.all_reduce(hist, dist.ReduceOp.SUM)
-                        b.dtopk_pick(word, shift, first, False, K)
-                        first = False
-                        top = shift
+                    _radix_select(comm, wbits, lambda shift, bits, first: b.dtopk_hist(word, shift, bits, first, smin),
+                                  lambda shift, first: b.dtopk_pick(word, shift, first, False, K))
         t0 = _tick('bc_select', t0)
         # stable: the synthetic arrival keys fall with the local index, so the local sort only needs the score
         idx, y, kl, kh = b.dtopk_cut('det' if self.tie == 'det' else 'det_ordered', keep_all, all_ties, smin, smax, u_local)
@@ -506,13 +506,6 @@ class ShardedSolver:
         return out, grank, k_total
 
     # ------------------------------------------------------------------ driver helpers
-    def run(self, max_levels=None):
-        while not self.ended:
-            self.step()
-            if max_levels is not None and len(self.infos) >= max_levels:
-                break
-        return self.infos
-
     def path(self):
         """(ranks, ordinals) of the winning line, walking the distributed link columns (src/solver.py:459-464)."""
         dev = self.b.device
@@ -602,7 +595,7 @@ class PeerRecv:
         self._fence()  # every mapping exists before anyone stores through one
 
 
-class GroupedShardedSolver:
+class GroupedShardedSolver(Stepper):
     """Beam search of State.solve (src/solver.py:390-464) over a queue sharded BY CARD SET (spl_gs_* entry points,
     csrc/spl_shard.cuh): a queue state lives on the rank that owns its cards, so its gem-take successors are
     deduplicated on the generating GPU by the fused on-chip walk and only card buys travel (32-byte records, one
@@ -660,6 +653,11 @@ class GroupedShardedSolver:
 
     def _dev(self, ptr, shape, typestr='<i8'):
         return torch.as_tensor(_DevArray(ptr, shape, typestr), device=self.eng.tdev)
+
+    def _tie_hist(self, shift, bits, first):
+        hp = C.c_void_p()
+        check(lib.spl_gs_tie_hist(self._h, shift, bits, int(first), C.byref(hp), self._st()), self.eng._h)
+        return self._dev(hp.value, (1 << SEL_BITS,), '<i4')
 
     # ---------------------------------------------------------------- one `while queue` iteration
     def step(self) -> dict:
@@ -738,16 +736,7 @@ class GroupedShardedSolver:
         if need.value:  # split the ties of the threshold score by arrival order
             lt = C.c_int32()
             check(lib.spl_gs_tie_begin(self._h, C.byref(lt), self._st()), eng._h)
-            top, first = lt.value, True
-            while top > 0:
-                bits = min(SEL_BITS, top)
-                shift = top - bits
-                hp = C.c_void_p()
-                check(lib.spl_gs_tie_hist(self._h, shift, bits, int(first), C.byref(hp), self._st()), eng._h)
-                comm.all_reduce(self._dev(hp.value, (1 << SEL_BITS,), '<i4'), dist.ReduceOp.SUM)
-                check(lib.spl_gs_tie_pick(self._h, shift, int(first), self._st()), eng._h)
-                first = False
-                top = shift
+            _radix_select(comm, lt.value, self._tie_hist, lambda shift, first: check(lib.spl_gs_tie_pick(self._h, shift, int(first), self._st()), eng._h))
         kept, yp, ybits = C.c_int64(), C.c_void_p(), C.c_int32()
         t0 = _tick('threshold', t0)
         check(lib.spl_gs_cut(self._h, need.value, C.byref(kept), C.byref(yp), C.byref(ybits), self._st()), eng._h)
@@ -800,13 +789,6 @@ class GroupedShardedSolver:
         ranks_recv = torch.empty(max(n_recv, 1), dtype=torch.int64, device=dev)
         check(lib.spl_gs_rank_sort(self._h, recv_y.data_ptr() if n_recv else None, n_recv, y_bits, base, ranks_recv.data_ptr(), self._st()), eng._h)
         return comm.all_to_all_rows(ranks_recv[:n_recv], recv_counts, send_counts)
-
-    def run(self, max_levels=None):
-        while not self.ended:
-            self.step()
-            if max_levels is not None and len(self.infos) >= max_levels:
-                break
-        return self.infos
 
     def frontier_local(self):
         """(records [n, 4] int64, global ranks [n] int64) of this rank's share of the queue (device views)"""
