@@ -348,10 +348,47 @@ int32_t spl_rpack(spl_ctx *ctx, const spl_rconfig *cfg, const void *recs_dev, in
 /* max(p.pts for p in state.players) per record: the progress line at :832-836 */
 int32_t spl_rmaxpts(spl_ctx *ctx, const spl_rconfig *cfg, const void *recs_dev, int64_t n, uint8_t *out_dev, void *stream);
 /* MultiPlayerState.solve (:750-860): beam always applied, ties by arrival order, game over when play
- * returns to the player who triggered the final round.  Steps / path / destroy via spl_solver_*. */
+ * returns to the player who triggered the final round.  Steps / path / destroy via spl_solver_*.  This is the
+ * single-GPU search; a search spread over several GPUs runs only when asked (see the key-sharded block below). */
 int32_t spl_rsolver_create(spl_ctx *ctx, const spl_rconfig *cfg, const void *root_rec_host, int64_t beam_width,
                            int32_t keep_links, spl_solver **out);
 int32_t spl_rsolver_frontier(spl_solver *s, const void **recs_dev, int64_t *n_host);
+
+/* ---- realistic mode on the key-sharded driver (sharded.py: RCudaBackend + RShardedSolver) ---------------------------
+ * MultiPlayerState.solve(shard=True) / --realistic --shard: the level loop of :820-852 over a queue spread block-cyclically
+ * across ranks, with the same per-level steps as spl_expand_rows .. spl_compact_winners above, on 96-byte records and
+ * 384-bit identity keys.  Every level holds the same records, in the same order, as spl_rsolver.  Ties by arrival order,
+ * noise const | hash (the config's; spl_rscore scores the records).  Realistic mode shards only when asked.
+ *   spl_rexpand_rows     successors of front records (:568-748), link = (rank_base + parent) << 8 | ordinal;
+ *                        SPL_E_CAPACITY + the needed count when cap is too small
+ *   spl_rroute_keys      the candidates' packed keys (spl_rpack) in (owner, arrival) order, send_keys_dev[n][6], + per-owner
+ *                        counts; owner = low 32 bits of the key hash, the owner's bucket comes from the high bits.  The
+ *                        permutation stays in the context for spl_rcompact_winners
+ *   spl_rdedup_flags     owner side (:840-843): first-arrival insert of a received key list (index = arrival) into the
+ *                        realistic visited table -> one winner byte each; keys inserted by earlier calls lose.  The table
+ *                        grows as spl_rsolver's does; SPL_E_TABLE_FULL when it cannot take the list (no state is dropped)
+ *   spl_rcompact_winners source side: winner bytes (in send order) -> the winning records in arrival order; SPL_E_STATE
+ *                        unless it follows spl_rroute_keys on the same candidates
+ *   spl_rmove_rows       out[i] = rows[idx[i]] (scatter = 0) or out[idx[i]] = rows[i] (scatter = 1), 96-byte records
+ *   spl_rfirst_goal      first queue index whose game is over (:827-829: players[cur].pts >= target), -1 if none
+ *   spl_rreset_visited   forget every visited state of the context: the realistic table and, as spl_rsolver_create does,
+ *                        the speedrun table (spl_reset_visited clears only that one).  The epoch counter restarts, so a
+ *                        long-lived context never runs out of epochs; each spl_rdedup_flags call takes one (at most
+ *                        2^23 - 1 calls between two resets)
+ *   spl_rvisited_count   states in the realistic visited table (spl_visited_count counts the speedrun table's) */
+int32_t spl_rexpand_rows(spl_ctx *ctx, const spl_rconfig *cfg, const void *front_recs_dev, int64_t n, int64_t rank_base,
+                         void *out_recs_dev, int64_t cap, int64_t *n_out_host, void *stream);
+int32_t spl_rroute_keys(spl_ctx *ctx, const spl_rconfig *cfg, const void *cand_recs_dev, int64_t n, int32_t n_ranks,
+                        uint64_t *send_keys_dev, int64_t *counts_host, void *stream);
+int32_t spl_rdedup_flags(spl_ctx *ctx, const uint64_t *keys_dev, int64_t n, uint8_t *flags_dev, void *stream);
+int32_t spl_rcompact_winners(spl_ctx *ctx, const void *cand_recs_dev, int64_t n, const uint8_t *flags_send_order_dev,
+                             void *out_recs_dev, int64_t *n_out_host, void *stream);
+int32_t spl_rmove_rows(spl_ctx *ctx, const void *recs_dev, const int64_t *idx_dev, int64_t n, void *out_recs_dev,
+                       int32_t scatter, void *stream);
+int32_t spl_rfirst_goal(spl_ctx *ctx, const spl_rconfig *cfg, const void *front_recs_dev, int64_t n, int64_t *rank_host,
+                        void *stream);
+int32_t spl_rreset_visited(spl_ctx *ctx, void *stream);
+int32_t spl_rvisited_count(spl_ctx *ctx, int64_t *n_host);
 
 #ifdef __cplusplus
 }

@@ -11,6 +11,7 @@ _HERE = Path(__file__).resolve().parent
 LIB_PATH = Path(os.environ.get('SPLENDOR_B200_LIB', _HERE / 'libsplendor_b200.so'))  # override: kernel A/B experiments
 
 SPL_OK = 0
+SPL_E_CAPACITY = -6  # caller buffer too small; the call reports the size it needs
 ERRORS = {-1: 'SPL_E_INVALID', -2: 'SPL_E_NODEVICE', -3: 'SPL_E_CUDA', -4: 'SPL_E_NOMEM',
           -5: 'SPL_E_TABLE_FULL', -6: 'SPL_E_CAPACITY', -7: 'SPL_E_STATE'}
 
@@ -88,6 +89,14 @@ def _load():
         'spl_rpack': (i32, [vp, vp, vp, i64, vp, vp]),
         'spl_rsolver_create': (i32, [vp, vp, vp, i64, i32, C.POINTER(vp)]),
         'spl_rsolver_frontier': (i32, [vp, C.POINTER(vp), C.POINTER(i64)]),
+        'spl_rexpand_rows': (i32, [vp, vp, vp, i64, i64, vp, i64, C.POINTER(i64), vp]),
+        'spl_rroute_keys': (i32, [vp, vp, vp, i64, i32, vp, vp, vp]),
+        'spl_rdedup_flags': (i32, [vp, vp, i64, vp, vp]),
+        'spl_rcompact_winners': (i32, [vp, vp, i64, vp, vp, C.POINTER(i64), vp]),
+        'spl_rmove_rows': (i32, [vp, vp, vp, i64, vp, i32, vp]),
+        'spl_rfirst_goal': (i32, [vp, vp, vp, i64, C.POINTER(i64), vp]),
+        'spl_rreset_visited': (i32, [vp, vp]),
+        'spl_rvisited_count': (i32, [vp, C.POINTER(i64)]),
         'spl_solver_create': (i32, [vp, C.POINTER(Key), u64, i32, i32, i32, i64, i32, i32, i32, C.POINTER(vp)]),
         'spl_solver_destroy': (i32, [vp]),
         'spl_solver_step': (i32, [vp, C.POINTER(LevelInfo), vp]),

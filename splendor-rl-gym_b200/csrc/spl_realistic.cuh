@@ -492,4 +492,101 @@ __global__ void __launch_bounds__(TILE) r_links_kernel(const RRec *__restrict__ 
     if (i < n) out[i] = recs[i].link;
 }
 
+// ------------------------------------------------------------------ key-sharded driver (sharded.py: RCudaBackend)
+// Owner rank of a state: the LOW 32 bits of r_key_hash, mapped onto [0, n_ranks) by a multiply-shift.  The owner's
+// table takes the bucket from the HIGH bits (__umul64hi(hash, nb) with nb < 2^32 buckets), so which rank owns a state
+// says nothing about its bucket there, and every owner fills its whole table evenly.
+__device__ __forceinline__ uint32_t r_owner_of(uint64_t h, uint32_t n_ranks) {
+    return (uint32_t)(((h & 0xffffffffull) * n_ranks) >> 32);
+}
+// packed key + owner (sort digit) + identity permutation of every candidate
+__global__ void __launch_bounds__(TILE) r_route_pack_kernel(const RRec *__restrict__ cand, int64_t n, const RConfigDev *__restrict__ cfg,
+                                                            uint32_t n_ranks, uint64_t *__restrict__ keys, uint64_t *__restrict__ owner,
+                                                            uint32_t *__restrict__ idx, Counters *ctr) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i >= n) return;
+    RRec s;
+    ld_rrec(cand + i, s);
+    uint64_t key[RKEY_WORDS];
+    if (!r_pack_key(*cfg, s, key)) atomicExch(&ctr->error, 4u);
+#pragma unroll
+    for (int k = 0; k < RKEY_WORDS; ++k) keys[i * RKEY_WORDS + k] = key[k];
+    owner[i] = r_owner_of(r_key_hash(key), n_ranks);
+    idx[i] = (uint32_t)i;
+}
+// send buffer: the keys in (owner, arrival) order; perm keeps that order for r_compact_kernel's caller
+__global__ void __launch_bounds__(TILE) r_gather_keys_kernel(const uint64_t *__restrict__ keys, const uint32_t *__restrict__ idx,
+                                                             int64_t n, uint64_t *__restrict__ out, uint32_t *__restrict__ perm) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t j = idx[i];
+#pragma unroll
+    for (int k = 0; k < RKEY_WORDS; ++k) out[i * RKEY_WORDS + k] = keys[(int64_t)j * RKEY_WORDS + k];
+    perm[i] = j;
+}
+// first-arrival insert of a list of packed keys (arrival index = list index)
+__global__ void __launch_bounds__(TILE) r_probe_keys_kernel(const uint64_t *__restrict__ keys, int64_t n, RBucket *__restrict__ table,
+                                                            uint64_t nb, uint64_t tag, uint32_t *__restrict__ cand_slot, Counters *ctr) {
+    const int64_t t = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    uint32_t n_new = 0;
+    if (t < n) {
+        uint64_t key[RKEY_WORDS];
+#pragma unroll
+        for (int k = 0; k < RKEY_WORDS; ++k) key[k] = keys[t * RKEY_WORDS + k];
+        cand_slot[t] = r_probe(table, nb, tag, key, ~(uint32_t)t, n_new, &ctr->error);
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) n_new += __shfl_xor_sync(0xffffffffu, n_new, d);
+    if ((threadIdx.x & 31) == 0 && n_new) atomicAdd(&ctr->n_new, (unsigned long long)n_new);
+}
+// winner byte per listed key: its bucket still holds its own arrival index
+__global__ void __launch_bounds__(TILE) r_win_flags_kernel(const uint32_t *__restrict__ cand_slot, const RBucket *__restrict__ table,
+                                                           int64_t n, uint8_t *__restrict__ flags) {
+    const int64_t t = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (t < n) {
+        const uint32_t sl = cand_slot[t];
+        flags[t] = sl != R_DEAD && ~ld_cg_u32(&table[sl].tinv) == (uint32_t)t;
+    }
+}
+// stable compaction of the flagged records (arrival order preserved): 8 records per thread, look-back scan
+__global__ void __launch_bounds__(TILE) r_compact_kernel(const RRec *__restrict__ recs, const uint8_t *__restrict__ flags, int64_t n,
+                                                         RRec *__restrict__ out, uint64_t *status, Counters *ctr, int ticket_id) {
+    __shared__ uint32_t warp_sums[TILE / 32 + 1];
+    __shared__ uint32_t s_tile;
+    __shared__ uint64_t s_base;
+    if (threadIdx.x == 0) s_tile = atomicAdd(&ctr->ticket[ticket_id], 1u);
+    __syncthreads();
+    const uint32_t tile = s_tile;
+    const int64_t b0 = ((int64_t)tile * TILE + threadIdx.x) * 8;
+    uint32_t mask = 0;
+    for (int q = 0; q < 8; ++q)
+        if (b0 + q < n && flags[b0 + q]) mask |= 1u << q;
+    uint32_t tot;
+    const uint32_t ex = block_excl_scan(__popc(mask), warp_sums, tot);
+    if (threadIdx.x < 32) {
+        const uint64_t e = lookback_exclusive(status, tile, tot, 0);
+        if (threadIdx.x == 0) {
+            s_base = e;
+            if (((int64_t)tile + 1) * TILE * 8 >= n) ctr->n_emitted = e + tot;
+        }
+    }
+    __syncthreads();
+    uint64_t pos = s_base + ex;
+    for (; mask; mask &= mask - 1) {
+        RRec r;
+        ld_rrec(recs + b0 + (__ffs(mask) - 1), r);
+        st_rrec(out + pos++, r);
+    }
+}
+// out[i] = recs[idx[i]] (gather) or out[idx[i]] = recs[i] (scatter)
+__global__ void __launch_bounds__(TILE) r_move_kernel(const RRec *__restrict__ recs, const int64_t *__restrict__ idx, int64_t n,
+                                                      RRec *__restrict__ out, int scatter) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i < n) {
+        RRec r;
+        ld_rrec(recs + (scatter ? i : idx[i]), r);
+        st_rrec(out + (scatter ? idx[i] : i), r);
+    }
+}
+
 }  // namespace spl

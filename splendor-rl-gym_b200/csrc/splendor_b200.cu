@@ -93,6 +93,10 @@ struct spl_ctx {
     DevBuf off, cand_slot, tmp_rec, tmp_rec2, sk, y[2], idx[2], kl[2], kh[2], matrix, matrix2, os_hist, os_status;
     DevBuf pool_front, pool_uniq, pool_grank;  // frontier buffers lent to the active solver
     DevBuf rcfg, rcand, rvmask, ridx64, rtmp;  // realistic mode scratch
+    DevBuf rkeys, rperm;       // spl_rroute_keys: packed keys of the candidates, their (owner, arrival) permutation
+    int64_t rroute_n = -1;     // candidates of the last spl_rroute_keys (its permutation lives in rperm)
+    spl_rconfig rcfg_host{};   // what c->rcfg holds (valid when rcfg_have)
+    bool rcfg_have = false;
     RBucket *rtable = nullptr;  // realistic mode: exact-key visited table (64-byte buckets, one state each)
     uint64_t rnb = 0, rocc = 0, rslots_hint = 0;
     std::vector<DevBuf *> pool_links;  // link columns of finished solves, reused by the next one
@@ -2137,10 +2141,18 @@ static int upload_rconfig(spl_ctx *c, const spl_rconfig *cfg, cudaStream_t st) {
     }
     CK(c, c->rcfg.ensure(sizeof h, 0, st));
     c->rcfg_dirty = true;
+    c->rcfg_have = false;
     CK(c, cudaMemcpyAsync(c->rcfg.p, &h, sizeof h, cudaMemcpyHostToDevice, st));
     CK(c, cudaStreamSynchronize(st));  // h is a stack object
     c->h2d_bytes += sizeof h;
+    c->rcfg_host = *cfg;
+    c->rcfg_have = true;
     return SPL_OK;
+}
+// upload only when the device copy holds another config (the sharded driver passes the same one every round)
+static int use_rconfig(spl_ctx *c, const spl_rconfig *cfg, cudaStream_t st) {
+    if (cfg && c->rcfg_have && memcmp(&c->rcfg_host, cfg, sizeof *cfg) == 0) return SPL_OK;
+    return upload_rconfig(c, cfg, st);
 }
 
 // realistic mode's visited table: allocate / grow so that `need` more states keep the load factor <= 0.6
@@ -2633,6 +2645,166 @@ int32_t spl_rsolver_frontier(spl_solver *s, const void **recs, int64_t *n) {
     if (!s || !recs || !n || !s->realistic) return SPL_E_INVALID;
     *recs = s->front.p;
     *n = s->n_front;
+    return SPL_OK;
+}
+
+// ---- realistic mode on the key-sharded driver: rows are 96-byte RRec records
+int32_t spl_rexpand_rows(spl_ctx *c, const spl_rconfig *cfg, const void *front, int64_t n, int64_t rank_base, void *out, int64_t cap,
+                         int64_t *n_out, void *stream) {
+    if (!c || !cfg || !n_out || n < 0 || n > (16ll << 20) || rank_base < 0) return fail(c, SPL_E_INVALID, "spl_rexpand_rows: bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    *n_out = 0;
+    if (n == 0) return SPL_OK;
+    CKS(c, use_rconfig(c, cfg, st));
+    const unsigned nt = nblk(n);
+    CK(c, c->off.ensure((size_t)n * 4 + 4, 0, st));
+    CK(c, c->rvmask.ensure((size_t)n * 4 + 4, 0, st));
+    CKS(c, zero_ctr(c, st));
+    CKS(c, prep_status(c, 0, nt, st));
+    r_count_scan_kernel<<<nt, TILE, 0, st>>>(reinterpret_cast<const RRec *>(front), n, c->rcfg.as<RConfigDev>(), c->off.as<uint32_t>(),
+                                              c->rvmask.as<uint32_t>(), c->status[0].as<uint64_t>(), c->d_ctr, 0);
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    CKS(c, read_ctr(c, st));
+    const int64_t total = (int64_t)c->h_ctr->total_cands;
+    *n_out = total;
+    if (total > cap) return fail(c, SPL_E_CAPACITY, "spl_rexpand_rows: %lld successors, capacity %lld", (long long)total, (long long)cap);
+    if (total == 0) return SPL_OK;
+    r_expand_kernel<<<nt, TILE, 0, st>>>(reinterpret_cast<const RRec *>(front), n, c->rcfg.as<RConfigDev>(), c->off.as<uint32_t>(),
+                                          c->rvmask.as<uint32_t>(), rank_base, reinterpret_cast<RRec *>(out));
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    return SPL_OK;
+}
+
+int32_t spl_rroute_keys(spl_ctx *c, const spl_rconfig *cfg, const void *cand, int64_t n, int32_t n_ranks, uint64_t *send_keys,
+                        int64_t *counts_host, void *stream) {
+    if (!c || !cfg || !counts_host || n < 0 || n >= (1ll << 32) || n_ranks < 1 || n_ranks > 255 || (n && !send_keys))
+        return fail(c, SPL_E_INVALID, "spl_rroute_keys: bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    for (int g = 0; g < n_ranks; ++g) counts_host[g] = 0;
+    c->rroute_n = -1;
+    if (n == 0) { c->rroute_n = 0; return SPL_OK; }
+    CKS(c, use_rconfig(c, cfg, st));
+    for (int b = 0; b < 2; ++b) {
+        CK(c, c->y[b].ensure((size_t)n * 8 + 8, 0, st));
+        CK(c, c->idx[b].ensure((size_t)n * 4 + 4, 0, st));
+    }
+    CK(c, c->rkeys.ensure((size_t)n * RKEY_WORDS * 8, 0, st));
+    CK(c, c->rperm.ensure((size_t)n * 4, 0, st));
+    CKS(c, zero_ctr(c, st));
+    r_route_pack_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const RRec *>(cand), n, c->rcfg.as<RConfigDev>(), (uint32_t)n_ranks,
+                                                   c->rkeys.as<uint64_t>(), c->y[0].as<uint64_t>(), c->idx[0].as<uint32_t>(), c->d_ctr);
+    ++c->launches;
+    const unsigned nt = nblk(n, SORT_TILE);
+    const size_t msz = (size_t)SORT_BINS * nt;
+    CK(c, c->matrix.ensure(msz * 4, 0, st));
+    CK(c, c->matrix2.ensure(msz * 4, 0, st));
+    CKS(c, sort_pass(c, 0, 0, c->y[0].as<uint64_t>(), n, 0, nt, msz, st));  // one stable pass: digit = owner
+    r_gather_keys_kernel<<<nblk(n), TILE, 0, st>>>(c->rkeys.as<uint64_t>(), c->idx[1].as<uint32_t>(), n, send_keys, c->rperm.as<uint32_t>());
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    // per-owner counts = differences of the digit-major scanned histogram at tile 0
+    std::vector<uint32_t> base(n_ranks + 1);
+    for (int g = 0; g <= n_ranks; ++g)
+        CK(c, cudaMemcpyAsync(&base[g], c->matrix2.as<uint32_t>() + (size_t)g * nt, 4, cudaMemcpyDeviceToHost, st));
+    c->d2h_bytes += 4 * (n_ranks + 1);
+    CKS(c, read_ctr(c, st));
+    if (c->h_ctr->error == 4) return fail(c, SPL_E_INVALID, "a player saved 1024 gems or more: outside the packed identity key");
+    for (int g = 0; g < n_ranks; ++g) counts_host[g] = base[g + 1] - base[g];
+    c->rroute_n = n;
+    return SPL_OK;
+}
+
+int32_t spl_rdedup_flags(spl_ctx *c, const uint64_t *keys, int64_t n, uint8_t *flags, void *stream) {
+    if (!c || n < 0 || n >= (1ll << 32) || (n && (!keys || !flags))) return fail(c, SPL_E_INVALID, "spl_rdedup_flags: bad arguments");
+    NO_LIVE_SOLVER(c, "spl_rdedup_flags");
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    if (n == 0) return SPL_OK;
+    CKS(c, zero_ctr(c, st));
+    CKS(c, ensure_rtable(c, (uint64_t)n, st));
+    uint64_t tag;
+    CKS(c, next_epoch(c, tag));
+    CK(c, c->cand_slot.ensure((size_t)n * 4, 0, st));
+    CKS(c, zero_ctr(c, st));
+    r_probe_keys_kernel<<<nblk(n), TILE, 0, st>>>(keys, n, c->rtable, c->rnb, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
+    r_win_flags_kernel<<<nblk(n), TILE, 0, st>>>(c->cand_slot.as<uint32_t>(), c->rtable, n, flags);
+    c->launches += 2;
+    CK(c, cudaGetLastError());
+    CKS(c, read_ctr(c, st));
+    c->rocc += c->h_ctr->n_new;  // counted before the error check, so that spl_rreset_visited clears a partial insert too
+    if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "spl_rdedup_flags: probe overflow (realistic visited table full, %llu buckets)",
+                                     (unsigned long long)c->rnb);
+    return SPL_OK;
+}
+
+int32_t spl_rcompact_winners(spl_ctx *c, const void *cand, int64_t n, const uint8_t *flags_partitioned, void *out, int64_t *n_out,
+                             void *stream) {
+    if (!c || !n_out || n < 0 || n != c->rroute_n)
+        return fail(c, SPL_E_STATE, "spl_rcompact_winners: must follow spl_rroute_keys on the same candidates");
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    *n_out = 0;
+    if (n == 0) return SPL_OK;
+    CK(c, c->rtmp.ensure((size_t)n + 8, 0, st));
+    scatter_flags_kernel<<<nblk(n), TILE, 0, st>>>(flags_partitioned, c->rperm.as<uint32_t>(), n, c->rtmp.as<uint8_t>());
+    const unsigned nt = nblk(n, TILE * 8);
+    CKS(c, zero_ctr(c, st));
+    CKS(c, prep_status(c, 0, nt, st));
+    r_compact_kernel<<<nt, TILE, 0, st>>>(reinterpret_cast<const RRec *>(cand), c->rtmp.as<uint8_t>(), n, reinterpret_cast<RRec *>(out),
+                                          c->status[0].as<uint64_t>(), c->d_ctr, 0);
+    c->launches += 2;
+    CK(c, cudaGetLastError());
+    CKS(c, read_ctr(c, st));
+    *n_out = (int64_t)c->h_ctr->n_emitted;
+    return SPL_OK;
+}
+
+int32_t spl_rmove_rows(spl_ctx *c, const void *rows, const int64_t *idx, int64_t n, void *out, int32_t scatter, void *stream) {
+    if (!c || n < 0 || (n && (!rows || !idx || !out))) return fail(c, SPL_E_INVALID, "spl_rmove_rows: bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    if (n == 0) return SPL_OK;
+    r_move_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const RRec *>(rows), idx, n, reinterpret_cast<RRec *>(out), scatter);
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    return SPL_OK;
+}
+
+int32_t spl_rfirst_goal(spl_ctx *c, const spl_rconfig *cfg, const void *front, int64_t n, int64_t *rank_host, void *stream) {
+    if (!c || !cfg || !rank_host || n < 0 || (n && !front)) return fail(c, SPL_E_INVALID, "spl_rfirst_goal: bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    *rank_host = -1;
+    if (n == 0) return SPL_OK;
+    CKS(c, use_rconfig(c, cfg, st));
+    CKS(c, zero_ctr(c, st));
+    r_goal_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const RRec *>(front), n, c->rcfg.as<RConfigDev>(), c->d_ctr);
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    CKS(c, read_ctr(c, st));
+    if (c->h_ctr->goal_rank != 0x7fffffffffffffffll) *rank_host = c->h_ctr->goal_rank;
+    return SPL_OK;
+}
+
+int32_t spl_rreset_visited(spl_ctx *c, void *stream) {
+    if (!c) return SPL_E_INVALID;
+    NO_LIVE_SOLVER(c, "spl_rreset_visited");
+    cudaStream_t st = (cudaStream_t)stream;
+    // the speedrun table is cleared too, as spl_rsolver_create does: both tables share the epoch counter, which can only
+    // restart at 0 once neither holds a tag (every spl_rdedup_flags call takes one epoch; TAG_MAX bounds them per search)
+    CKS(c, reset_visited(c, st));
+    if (c->rtable && c->rocc) CK(c, cudaMemsetAsync(c->rtable, 0, c->rnb * 64, st));
+    c->rocc = 0;
+    return SPL_OK;
+}
+
+int32_t spl_rvisited_count(spl_ctx *c, int64_t *n_host) {
+    if (!c || !n_host) return SPL_E_INVALID;
+    *n_host = (int64_t)c->rocc;
     return SPL_OK;
 }
 

@@ -1,7 +1,8 @@
 """Realistic multi-player mode: the reference's GameConfig / GemPool / CardMarket / PlayerState /
 MultiPlayerState surface (src/solver.py:25-200, 471-860) driven by the CUDA library.
 
-`MultiPlayerState.solve()` -> spl_rsolver_* ; `__iter__` -> spl_rexpand on one record; the
+`MultiPlayerState.solve()` -> spl_rsolver_* (with `shard=True`: RShardedSolver over the ranks of the process group,
+sharded.py) ; `__iter__` -> spl_rexpand on one record; the
 competitive heuristic -> spl_rscore.  The card market order (optionally shuffled with Python's
 `random.Random(seed)` exactly as CardMarket.from_full_deck does) is computed here on the host and
 handed to the kernels as an input table.  The reference draws tie-break noise from the unseeded
@@ -273,11 +274,24 @@ class MultiPlayerState:
 
     def solve(self, *, use_heuristic: bool = True, heuristic_name: str = 'competitive', beam_width: int = 20_000,
               verbose: bool = True, noise: str = 'const', device: int | None = None, engine: Engine | None = None,
-              stats: list | None = None) -> list['MultiPlayerState']:
+              stats: list | None = None, shard: bool = False) -> list['MultiPlayerState']:
         """Beam search over the multi-player game; arguments and return value as src/solver.py:750-860
-        (`use_heuristic` / `heuristic_name` are ignored there too: the beam is always applied)."""
+        (`use_heuristic` / `heuristic_name` are ignored there too: the beam is always applied).
+
+        Without `shard`, every process solves the whole game on its own GPU (under torchrun: one replica per rank).
+        `shard=True` spreads one search over the ranks of the default process group (a world of 1 when none is
+        initialised): every rank calls solve() collectively, each holds a slice of the queue and of the visited set,
+        so a beam too wide for one GPU's visited table can run, and every level equals the single-GPU search.  It
+        supports noise 'const' and 'hash' ('mt' raises ValueError).  With `verbose`, rank 0 prints the banner and the
+        `turn=... Queue size:` lines; the `max_pts=` progress lines are not printed on the sharded path."""
         from .solver import _engine
+        if shard and noise == 'mt':
+            raise ValueError("solve(shard=True) supports noise 'const' and 'hash', not 'mt'")
         eng = engine or _engine(device)
+        if shard:
+            import torch.distributed as dist
+            if dist.is_available() and dist.is_initialized() and dist.get_rank() != 0:
+                verbose = False
         if verbose:
             print('=' * 60)
             print('REALISTIC MODE SOLVER')
@@ -292,6 +306,34 @@ class MultiPlayerState:
             print('=' * 60)
             print()
         rcfg = self.rconfig(noise)
+        if shard:
+            ordinals = self._solve_sharded(eng, rcfg, beam_width, verbose, stats)
+        else:
+            ordinals = self._solve_local(eng, rcfg, beam_width, verbose, stats)
+        path = [self]
+        for o in ordinals:
+            path.append(path[-1]._successors(eng, noise)[o])
+        return path
+
+    def _solve_sharded(self, eng: Engine, rcfg: RConfig, beam_width: int, verbose: bool, stats) -> list[int]:
+        from .sharded import Comm, RCudaBackend, RShardedSolver
+        comm = Comm(eng.tdev)
+        sol = RShardedSolver(RCudaBackend(eng, rcfg, self.record()), comm, beam_width)
+        turn = 0
+        while True:
+            if verbose and turn % 100 == 0:
+                print(f'{turn=:<10} Queue size: {sol.N}')
+            info = sol.step()
+            if stats is not None:
+                stats.append(info)
+            turn += 1
+            if info['ended']:
+                break
+        if turn > 1000 and comm.rank == 0:
+            print('Warning: Reached turn limit (1000)')
+        return sol.path()[1]
+
+    def _solve_local(self, eng: Engine, rcfg: RConfig, beam_width: int, verbose: bool, stats) -> list[int]:
         sol = eng.rsolver(rcfg, self.record(), beam_width)
         try:
             turn = 0
@@ -321,7 +363,4 @@ class MultiPlayerState:
                 sol.noise_source.finish()
         finally:
             sol.close()
-        path = [self]
-        for o in ordinals:
-            path.append(path[-1]._successors(eng, noise)[o])
-        return path
+        return ordinals

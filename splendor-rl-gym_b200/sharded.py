@@ -19,8 +19,9 @@ Per level (G ranks; the queue is block-distributed by global rank: rank g holds 
      counts against the other ranks' sorted sort-words (all-gather + spl_count_less); survivors
      are sent to the rank that owns their global-rank block (all-to-all)          (:452-456)
 
-The compute primitives come from a `backend` object (CudaBackend below wraps the C ABI); the
-collectives go through torch.distributed (NCCL on GPUs, gloo in the CPU tests).
+The compute primitives come from a `backend` object (CudaBackend below wraps the C ABI; RCudaBackend the realistic-mode
+calls that RShardedSolver runs the same levels with); the collectives go through torch.distributed (NCCL on GPUs, gloo
+in the CPU tests).
 """
 import ctypes as C
 
@@ -28,7 +29,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from ._lib import Key as _Key, check, lib
+from ._lib import SPL_E_CAPACITY, Key as _Key, check, lib
 from .engine import NOISE_IDS, TIE_IDS, Engine, Stepper, _DevArray, heuristic_id
 
 import os
@@ -69,16 +70,24 @@ def _radix_select(comm, top, hist, pick):
 
 
 class Comm:
-    """Thin wrapper over torch.distributed (world size 1 works without a process group)."""
+    """Thin wrapper over torch.distributed (world size 1 works without a process group).  Over a gloo process group the
+    collectives of device tensors are staged through host memory, so that several ranks can share one GPU (a multi-rank
+    check of the device code on a machine with fewer GPUs than ranks; NCCL needs one GPU per rank)."""
 
     def __init__(self, device):
         self.on = dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
         self.rank = dist.get_rank() if self.on else 0
         self.world = dist.get_world_size() if self.on else 1
         self.device = device
+        self.stage = self.on and device.type == 'cuda' and dist.get_backend() == 'gloo'
 
     def gather_ints(self, *vals):
         """all_gather of a few python ints -> int64 array [world, len(vals)]"""
+        if self.stage:
+            t = torch.tensor(vals, dtype=torch.int64).reshape(1, -1)
+            out = torch.empty((self.world, t.shape[1]), dtype=torch.int64)
+            dist.all_gather(list(out.unbind(0)), t[0])
+            return out.numpy()
         t = torch.tensor(vals, dtype=torch.int64, device=self.device).reshape(1, -1)
         if not self.on:
             return t.cpu().numpy()
@@ -87,7 +96,11 @@ class Comm:
         return out.cpu().numpy()
 
     def all_reduce(self, t, op):
-        if self.on:
+        if self.stage:
+            h = t.cpu()
+            dist.all_reduce(h, op=op)
+            t.copy_(h)
+        elif self.on:
             dist.all_reduce(t, op=op)
         return t
 
@@ -95,28 +108,82 @@ class Comm:
         """variable all-to-all of rows (dim 0); send is grouped by destination rank"""
         if not self.on:
             return send
-        out = torch.empty((int(sum(recv_counts)),) + tuple(send.shape[1:]), dtype=send.dtype, device=send.device)
-        dist.all_to_all_single(out, send.contiguous(), [int(x) for x in recv_counts], [int(x) for x in send_counts])
-        return out
+        src = send.contiguous().cpu() if self.stage else send.contiguous()
+        out = torch.empty((int(sum(recv_counts)),) + tuple(send.shape[1:]), dtype=send.dtype, device=src.device)
+        dist.all_to_all_single(out, src, [int(x) for x in recv_counts], [int(x) for x in send_counts])
+        return out.to(send.device) if self.stage else out
 
     def all_gather_v(self, t, counts):
         """all_gather of 1-D tensors of different lengths -> list of tensors"""
         if not self.on:
             return [t]
         m = int(max(counts)) if len(counts) else 0
-        pad = torch.zeros(m, dtype=t.dtype, device=t.device)
+        dev = torch.device('cpu') if self.stage else t.device
+        pad = torch.zeros(m, dtype=t.dtype, device=dev)
         pad[:t.shape[0]] = t
-        outs = [torch.empty(m, dtype=t.dtype, device=t.device) for _ in range(self.world)]
+        outs = [torch.empty(m, dtype=t.dtype, device=dev) for _ in range(self.world)]
         dist.all_gather(outs, pad)
-        return [o[:int(c)] for o, c in zip(outs, counts)]
+        return [o[:int(c)].to(t.device) for o, c in zip(outs, counts)]
 
 
-class CudaBackend:
-    """Compute primitives of one rank, all through the C ABI of libsplendor_b200.so."""
+class _CutOps:
+    """The score-generic calls of the global beam cut (distributed radix select, local cut, global ranks): the same for
+    speedrun and realistic rows, since they see only scores and sort words."""
 
     def __init__(self, eng: Engine):
         self.eng = eng
         self.device = eng.tdev
+
+    # ---- distributed top-k passes
+    def dtopk_begin(self, scores, keys):
+        a, b = C.c_uint64(), C.c_uint64()
+        check(lib.spl_dtopk_begin(self.eng._h, scores.data_ptr(), keys.data_ptr() if keys is not None else None,
+                                  scores.shape[0], C.byref(a), C.byref(b), self.eng._stream()), self.eng._h)
+        return a.value, b.value
+
+    def dtopk_hist(self, word, shift, bits, first, smin):
+        p = C.c_void_p()
+        check(lib.spl_dtopk_hist(self.eng._h, word, shift, bits, int(first), smin, C.byref(p), self.eng._stream()), self.eng._h)
+        if getattr(self, '_hist_ptr', None) != p.value:  # the histogram lives at a fixed address inside the context
+            self._hist_ptr = p.value
+            self._hist = torch.as_tensor(_DevArray(p.value, (1 << SEL_BITS,), '<i4'), device=self.device)
+        return self._hist
+
+    def dtopk_pick(self, word, shift, first, init_k, k):
+        check(lib.spl_dtopk_pick(self.eng._h, word, shift, int(first), int(init_k), k, self.eng._stream()), self.eng._h)
+
+    def dtopk_get(self):
+        st = (C.c_uint64 * 6)()
+        check(lib.spl_dtopk_get(self.eng._h, st, self.eng._stream()), self.eng._h)
+        return list(st)
+
+    def dtopk_set(self, state):
+        check(lib.spl_dtopk_set(self.eng._h, (C.c_uint64 * 6)(*state), self.eng._stream()), self.eng._h)
+
+    def dtopk_cut(self, tie, keep_all, all_ties, smin, smax, n):
+        det = tie in ('det', 'det_ordered')
+        idx = torch.empty(max(n, 1), dtype=torch.int64, device=self.device)
+        y = torch.empty(max(n, 1), dtype=torch.int64, device=self.device)
+        kl = torch.empty(max(n, 1) if det else 1, dtype=torch.int64, device=self.device)
+        kh = torch.empty(max(n, 1) if det else 1, dtype=torch.int64, device=self.device)
+        kept = C.c_int64()
+        check(lib.spl_dtopk_cut(self.eng._h, TIE_IDS[tie], int(keep_all), int(all_ties), smin, smax, idx.data_ptr(),
+                                y.data_ptr(), kl.data_ptr() if det else None, kh.data_ptr() if det else None,
+                                C.byref(kept), self.eng._stream()), self.eng._h)
+        m = kept.value
+        return idx[:m], y[:m], (kl[:m] if det else None), (kh[:m] if det else None)
+
+    def count_less(self, words, inclusive, a, b, out, accumulate, sorted_a=False):
+        (ay, akl, akh), (by, bkl, bkh) = a, b
+        check(lib.spl_count_less(self.eng._h, words, int(inclusive), ay.data_ptr(),
+                                 akl.data_ptr() if words == 3 else None, akh.data_ptr() if words == 3 else None,
+                                 ay.shape[0], by.data_ptr(), bkl.data_ptr() if words == 3 else None,
+                                 bkh.data_ptr() if words == 3 else None, by.shape[0], out.data_ptr(), int(accumulate),
+                                 int(sorted_a), self.eng._stream()), self.eng._h)
+
+
+class CudaBackend(_CutOps):
+    """Compute primitives of one rank, all through the C ABI of libsplendor_b200.so."""
 
     def reset_visited(self):
         self.eng.reset_visited()
@@ -208,53 +275,6 @@ class CudaBackend:
                                 self.eng._stream()), self.eng._h)
         return out[:n_out]
 
-    # ---- distributed top-k passes
-    def dtopk_begin(self, scores, keys):
-        a, b = C.c_uint64(), C.c_uint64()
-        check(lib.spl_dtopk_begin(self.eng._h, scores.data_ptr(), keys.data_ptr() if keys is not None else None,
-                                  scores.shape[0], C.byref(a), C.byref(b), self.eng._stream()), self.eng._h)
-        return a.value, b.value
-
-    def dtopk_hist(self, word, shift, bits, first, smin):
-        p = C.c_void_p()
-        check(lib.spl_dtopk_hist(self.eng._h, word, shift, bits, int(first), smin, C.byref(p), self.eng._stream()), self.eng._h)
-        if getattr(self, '_hist_ptr', None) != p.value:  # the histogram lives at a fixed address inside the context
-            self._hist_ptr = p.value
-            self._hist = torch.as_tensor(_DevArray(p.value, (1 << SEL_BITS,), '<i4'), device=self.device)
-        return self._hist
-
-    def dtopk_pick(self, word, shift, first, init_k, k):
-        check(lib.spl_dtopk_pick(self.eng._h, word, shift, int(first), int(init_k), k, self.eng._stream()), self.eng._h)
-
-    def dtopk_get(self):
-        st = (C.c_uint64 * 6)()
-        check(lib.spl_dtopk_get(self.eng._h, st, self.eng._stream()), self.eng._h)
-        return list(st)
-
-    def dtopk_set(self, state):
-        check(lib.spl_dtopk_set(self.eng._h, (C.c_uint64 * 6)(*state), self.eng._stream()), self.eng._h)
-
-    def dtopk_cut(self, tie, keep_all, all_ties, smin, smax, n):
-        det = tie in ('det', 'det_ordered')
-        idx = torch.empty(max(n, 1), dtype=torch.int64, device=self.device)
-        y = torch.empty(max(n, 1), dtype=torch.int64, device=self.device)
-        kl = torch.empty(max(n, 1) if det else 1, dtype=torch.int64, device=self.device)
-        kh = torch.empty(max(n, 1) if det else 1, dtype=torch.int64, device=self.device)
-        kept = C.c_int64()
-        check(lib.spl_dtopk_cut(self.eng._h, TIE_IDS[tie], int(keep_all), int(all_ties), smin, smax, idx.data_ptr(),
-                                y.data_ptr(), kl.data_ptr() if det else None, kh.data_ptr() if det else None,
-                                C.byref(kept), self.eng._stream()), self.eng._h)
-        m = kept.value
-        return idx[:m], y[:m], (kl[:m] if det else None), (kh[:m] if det else None)
-
-    def count_less(self, words, inclusive, a, b, out, accumulate, sorted_a=False):
-        (ay, akl, akh), (by, bkl, bkh) = a, b
-        check(lib.spl_count_less(self.eng._h, words, int(inclusive), ay.data_ptr(),
-                                 akl.data_ptr() if words == 3 else None, akh.data_ptr() if words == 3 else None,
-                                 ay.shape[0], by.data_ptr(), bkl.data_ptr() if words == 3 else None,
-                                 bkh.data_ptr() if words == 3 else None, by.shape[0], out.data_ptr(), int(accumulate),
-                                 int(sorted_a), self.eng._stream()), self.eng._h)
-
 
 class ShardedSolver(Stepper):
     """State.solve (src/solver.py:390-464) over a frontier sharded across `comm.world` ranks.
@@ -263,7 +283,13 @@ class ShardedSolver(Stepper):
     b % G (block-cyclic), so that ROUND r = blocks r*G .. r*G+G-1 covers a contiguous range of global ranks,
     rank 0's block first.  Rounds are processed in order, each bounded in memory; within a round the
     receive buffers are concatenated by source rank -- hence every owner sees candidates in global arrival
-    order, and anything inserted by an earlier round is simply "visited" (it arrived earlier)."""
+    order, and anything inserted by an earlier round is simply "visited" (it arrived earlier).
+
+    Rows are int64 tensors [n, ROW_COLS] with the parent link in column LINK_COL: here the 32-byte speedrun
+    records {lo, hi, aux, link}; RShardedSolver runs the same levels on realistic mode's 96-byte records."""
+
+    ROW_COLS, LINK_COL = 4, 3
+    TURN_LIMIT = None  # level after which the search stops with the queue it has (realistic mode: 1000)
 
     def __init__(self, backend, comm: Comm, root_key: int, root_aux: int, goal_pts: int, use_heuristic: bool,
                  heuristic: str, beam_width: int, tie: str = 'stable', noise: str = 'const',
@@ -275,13 +301,7 @@ class ShardedSolver(Stepper):
         self.goal, self.use_h, self.h, self.beam, self.tie, self.noise = goal_pts, use_heuristic, heuristic, beam_width, tie, noise
         self.C = int(block_parents)
         self.keep_links = keep_links
-        dev = backend.device
-        m64 = (1 << 64) - 1
-
-        def s64(x):
-            x &= m64
-            return x - (1 << 64) if x >> 63 else x
-        root = torch.tensor([[s64(root_key), s64(root_key >> 64), s64(root_aux), -1]], dtype=torch.int64, device=dev)
+        root = self._root_row(root_key, root_aux)
         backend.reset_visited()  # trail = {}
         # the root is block 0 (rank 0); its key is registered in the visited set of its owner
         self.front = root if comm.rank == 0 else root[:0]
@@ -300,6 +320,14 @@ class ShardedSolver(Stepper):
             self.noise_source = MTNoise()
         self.links = []  # per level: local link column (block-cyclic local order)
         self._save_links()
+
+    def _root_row(self, root_key, root_aux):
+        m64 = (1 << 64) - 1
+
+        def s64(x):
+            x &= m64
+            return x - (1 << 64) if x >> 63 else x
+        return torch.tensor([[s64(root_key), s64(root_key >> 64), s64(root_aux), -1]], dtype=torch.int64, device=self.b.device)
 
     def _ident(self, rows):
         """what the visited set compares: the exact (cards, gems) key, or (identity='pyhash') the reference's 64-bit
@@ -327,7 +355,7 @@ class ShardedSolver(Stepper):
         return b % G, (b // G) * C + x % C
 
     def _save_links(self):
-        self.links.append(self.front[:, 3].clone() if self.keep_links else None)
+        self.links.append(self.front[:, self.LINK_COL].clone() if self.keep_links else None)
 
     def _redistribute(self, rows, x, dst, n_total_after):
         """send rows with global ranks x (tensor) to their block-cyclic owners; scatter into dst (grown as needed)"""
@@ -351,7 +379,7 @@ class ShardedSolver(Stepper):
             # first allocation of a level: size it for the growth seen in the previous level (no regrow copies)
             guess = self._local_count(int(self.N * self._growth * 1.08) + 1024, me) if dst is None else 0
             cap = max(need, guess, int(1.5 * (dst.shape[0] if dst is not None else 0)), 1024)
-            nd = torch.empty((cap, 4), dtype=torch.int64, device=dev)
+            nd = torch.empty((cap, self.ROW_COLS), dtype=torch.int64, device=dev)
             if dst is not None and self._dst_used:
                 nd[:self._dst_used] = dst[:self._dst_used]
             dst = nd
@@ -387,7 +415,7 @@ class ShardedSolver(Stepper):
             size = max(0, min(C, N - blk * C))
             parents = front[r * C: r * C + size]
             # 2. expand this rank's block of the round
-            cand = b.expand_rows(parents, blk * C) if size else torch.empty((0, 4), dtype=torch.int64, device=dev)
+            cand = b.expand_rows(parents, blk * C) if size else torch.empty((0, self.ROW_COLS), dtype=torch.int64, device=dev)
             m = cand.shape[0]
             t0 = _tick('expand', t0)
             # 3. route keys to their owners
@@ -430,7 +458,8 @@ class ShardedSolver(Stepper):
         info['kept'] = n_next
         info['visited'] = int(vis[:, 0].sum())
         self.infos.append(info)
-        if n_next == 0:  # frontier exhausted: `puzzle` stays the last dequeued state
+        if n_next == 0 or (self.TURN_LIMIT is not None and self.level >= self.TURN_LIMIT):
+            # frontier exhausted (or the turn limit): `puzzle` stays the last dequeued state
             self.ended, self.goal_rank = True, N - 1
             info['ended'] = 1
             return info
@@ -529,14 +558,144 @@ class ShardedSolver(Stepper):
         """the whole current queue on every rank, in global rank order (tests / small cases only)"""
         G, dev = self.comm.world, self.b.device
         sizes = [self._local_count(self.N, g) for g in range(G)]
-        out = torch.empty((self.N, 4), dtype=torch.int64, device=dev)
-        cols = [self.comm.all_gather_v(self.front[:, c].contiguous(), sizes) for c in range(4)]
+        out = torch.empty((self.N, self.ROW_COLS), dtype=torch.int64, device=dev)
+        cols = [self.comm.all_gather_v(self.front[:, c].contiguous(), sizes) for c in range(self.ROW_COLS)]
         for g in range(G):
             if sizes[g]:
                 x = self._global_of_local(torch.arange(sizes[g], dtype=torch.int64, device=dev), g)
-                out[x] = torch.stack([cols[c][g] for c in range(4)], dim=1)
+                out[x] = torch.stack([cols[c][g] for c in range(self.ROW_COLS)], dim=1)
         return out
 
+
+class RCudaBackend(_CutOps):
+    """Compute primitives of one rank for realistic mode (MultiPlayerState, csrc/spl_realistic.cuh), with the method
+    names of CudaBackend.  Rows are 96-byte records as int64 [n, 12]: players in columns 0-7, vis/cur in 8-9, link in
+    10, spare in 11; keys are the 384-bit exact identity (spl_rpack) as int64 [n, 6].  Scores come from spl_rscore
+    with the config's noise (`const` or `hash`); `root` is the record the search starts from (default: the config's
+    new game)."""
+
+    def __init__(self, eng: Engine, rcfg, root=None):
+        super().__init__(eng)
+        self.rcfg = rcfg
+        self.noise = {v: k for k, v in NOISE_IDS.items()}[rcfg.noise]
+        self.goal = rcfg.target_points
+        self._fanout = 27.0  # successors per parent the next expand_rows allocates for
+        if root is None:
+            from .realistic import RREC_DTYPE
+            root = np.zeros(1, RREC_DTYPE)
+            root['vis'][0] = [rcfg.deck[t][k] if k < rcfg.deck_len[t] else 255 for t in range(3) for k in range(4)]
+            root['link'] = (1 << 64) - 1
+        self.root = np.ascontiguousarray(root).reshape(-1)[:1].copy()
+
+    def _call(self, rc):
+        check(rc, self.eng._h)
+
+    def root_row(self):
+        return torch.from_numpy(self.root.view(np.int64).reshape(1, 12).copy()).to(self.device)
+
+    def reset_visited(self):
+        self._call(lib.spl_rreset_visited(self.eng._h, self.eng._stream()))
+
+    def visited_count(self):
+        n = C.c_int64()
+        self._call(lib.spl_rvisited_count(self.eng._h, C.byref(n)))
+        return n.value
+
+    def first_goal(self, front, goal):
+        """first queue index whose game is over (players[cur].pts >= the config's target), -1 if none"""
+        r = C.c_int64()
+        self._call(lib.spl_rfirst_goal(self.eng._h, C.byref(self.rcfg), front.data_ptr(), front.shape[0], C.byref(r),
+                                       self.eng._stream()))
+        return r.value
+
+    def expand_rows(self, front, rank_base):
+        """successors of the local queue slice as rows [m, 12]; link = (rank_base + parent) << 8 | ordinal.  The buffer is
+        sized from the successors per parent of the previous call (at most 27: 12 buys, 10 colour triples, 5 double
+        takes) rather than the worst case, so that device memory stays free for the visited table; when it is too small
+        the call reports the exact count and runs again."""
+        n = front.shape[0]
+        cap = max(64, int(n * self._fanout) + 1024)
+        while True:
+            out = torch.empty((cap, 12), dtype=torch.int64, device=self.device)
+            m = C.c_int64()
+            rc = lib.spl_rexpand_rows(self.eng._h, C.byref(self.rcfg), front.data_ptr(), n, rank_base, out.data_ptr(), cap,
+                                      C.byref(m), self.eng._stream())
+            if rc == SPL_E_CAPACITY:
+                cap = m.value
+                continue
+            self._call(rc)
+            if n:
+                self._fanout = min(27.0, 1.1 * m.value / n)
+            return out[:m.value]
+
+    def route_keys(self, cand, world):
+        """identity keys [m, 6] of the candidates grouped by owner rank (arrival order inside a group) + per-owner counts"""
+        m = cand.shape[0]
+        send = torch.empty((max(m, 1), 6), dtype=torch.int64, device=self.device)
+        counts = (C.c_int64 * world)()
+        self._call(lib.spl_rroute_keys(self.eng._h, C.byref(self.rcfg), cand.data_ptr(), m, world, send.data_ptr(), counts,
+                                       self.eng._stream()))
+        return send[:m], np.array(counts[:], dtype=np.int64)
+
+    def dedup_flags(self, keys):
+        """owner side: one winner byte per received key (first arrival of a never-seen state)"""
+        n = keys.shape[0]
+        flags = torch.empty(max(n, 1), dtype=torch.uint8, device=self.device)
+        self._call(lib.spl_rdedup_flags(self.eng._h, keys.data_ptr(), n, flags.data_ptr(), self.eng._stream()))
+        return flags[:n]
+
+    def compact_winners(self, cand, flags_send_order):
+        """source side: the winning rows in arrival order"""
+        m = cand.shape[0]
+        out = torch.empty((max(m, 1), 12), dtype=torch.int64, device=self.device)
+        k = C.c_int64()
+        self._call(lib.spl_rcompact_winners(self.eng._h, cand.data_ptr(), m, flags_send_order.data_ptr(), out.data_ptr(),
+                                            C.byref(k), self.eng._stream()))
+        return out[:k.value]
+
+    def score(self, heuristic, noise, rows, draws=None):
+        """multi_competitive_heuristic of every row (the config's noise; `heuristic` is the reference's ignored name)"""
+        n = rows.shape[0]
+        out = torch.empty(n, dtype=torch.float64, device=self.device)
+        self._call(lib.spl_rscore(self.eng._h, C.byref(self.rcfg), rows.data_ptr(), n, out.data_ptr(), self.eng._stream()))
+        return out
+
+    def scatter_into(self, dst, rows, pos):
+        """dst[pos[i]] = rows[i] for 96-byte rows (dst is an existing [n, 12] int64 tensor)"""
+        self._call(lib.spl_rmove_rows(self.eng._h, rows.contiguous().data_ptr(), pos.contiguous().data_ptr(), pos.shape[0],
+                                      dst.data_ptr(), 1, self.eng._stream()))
+
+    def move_rows(self, rows, idx, n_out, scatter):
+        """gather (out[i] = rows[idx[i]]) or scatter (out[idx[i]] = rows[i]) of 96-byte rows"""
+        out = torch.empty((max(n_out, 1), 12), dtype=torch.int64, device=self.device)
+        self._call(lib.spl_rmove_rows(self.eng._h, rows.data_ptr(), idx.data_ptr(), idx.shape[0], out.data_ptr(), int(scatter),
+                                      self.eng._stream()))
+        return out[:n_out]
+
+
+class RShardedSolver(ShardedSolver):
+    """MultiPlayerState.solve (src/solver.py:750-860) on the key-sharded choreography of ShardedSolver: 96-byte records,
+    the exact 384-bit identity as the routing and visited key, the beam always applied, score ties by arrival order (the
+    reference's stable sort; it has no key tie-break), noise `const` or `hash` from the backend's config.  Every level
+    holds the same records, in the same order, with the same links, as the single-GPU realistic solver (spl_rsolver).
+    `backend` is an RCudaBackend (or a stand-in with its methods and `root_row`, `noise`, `goal`)."""
+
+    ROW_COLS, LINK_COL = 12, 10
+    TURN_LIMIT = 1000  # the reference leaves its loop after the iteration with turn == 1000 (src/solver.py:846-852)
+
+    def __init__(self, backend, comm: Comm, beam_width: int, tie: str = 'stable', block_parents: int = 1 << 20,
+                 keep_links: bool = True, identity: str = 'key'):
+        if tie != 'stable':
+            raise ValueError(f"realistic mode breaks score ties by arrival order only (tie='stable'), not {tie!r}")
+        if identity != 'key':
+            raise ValueError(f"realistic mode dedups on its exact identity key only (identity='key'), not {identity!r}")
+        if backend.noise not in ('const', 'hash'):
+            raise ValueError(f"the sharded realistic search supports noise 'const' and 'hash', not {backend.noise!r}")
+        super().__init__(backend, comm, 0, 0, backend.goal, True, 'competitive', beam_width, tie, backend.noise,
+                         block_parents=block_parents, keep_links=keep_links, identity=identity)
+
+    def _root_row(self, root_key, root_aux):
+        return self.b.root_row()
 
 
 class DictionaryOverflow(RuntimeError):

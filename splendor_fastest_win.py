@@ -32,6 +32,9 @@ def cli():
     ap.add_argument('--players', type=int, default=2, help='number of players for realistic mode')
     ap.add_argument('--shuffle', action='store_true', help='shuffle the card market in realistic mode')
     ap.add_argument('--seed', type=int, default=None, help='market shuffle seed (the reference passes none)')
+    ap.add_argument('--shard', action='store_true',
+                    help='realistic mode under torchrun: spread one search over the ranks (queue and visited set) '
+                         'instead of solving the whole game on every rank')
     if len(sys.argv) == 1:
         ap.print_help()
         ap.exit()
@@ -47,14 +50,14 @@ def cli():
         dist.init_process_group('nccl', device_id=torch.device('cuda', local))
     from splendor_rl_gym_b200 import Color, GameConfig, MultiPlayerState, State
     rank0 = int(os.environ.get('RANK', '0')) == 0
-    if a.realistic:  # reference CLI lines 95-129 (realistic mode is not sharded: under torchrun every rank solves
-        try:          # the same game on its own GPU and rank 0 reports)
+    if a.realistic:  # reference CLI lines 95-129 (under torchrun every rank solves the same game on its own GPU and
+        try:          # rank 0 reports; with --shard the ranks share one search)
             cfg = GameConfig(num_players=a.players, target_points=a.goal_pts,
                              gems_per_color={2: 4, 3: 5, 4: 7}.get(a.players, 4), infinite_resources=False)
             solution = MultiPlayerState.newgame(config=cfg, shuffle_market=a.shuffle, seed=a.seed).solve(
                 use_heuristic=True, heuristic_name='competitive',
                 beam_width=a.beam_width if a.beam_width != 300_000 else 20_000, verbose=not a.quiet and rank0,
-                device=local if world > 1 else a.device)
+                device=local if world > 1 else a.device, shard=a.shard)
             last = solution[-1]
             if rank0:
                 print(f'\n{"=" * 60}')
