@@ -356,20 +356,18 @@ int32_t spl_rsolver_frontier(spl_solver *s, const void **recs_dev, int64_t *n_ho
 
 /* ---- realistic mode on the key-sharded driver (sharded.py: RCudaBackend + RShardedSolver) ---------------------------
  * MultiPlayerState.solve(shard=True) / --realistic --shard: the level loop of :820-852 over a queue spread block-cyclically
- * across ranks, with the same per-level steps as spl_expand_rows .. spl_compact_winners above, on 96-byte records and
- * 384-bit identity keys.  Every level holds the same records, in the same order, as spl_rsolver.  Ties by arrival order,
- * noise const | hash (the config's; spl_rscore scores the records).  Realistic mode shards only when asked.
- *   spl_rexpand_rows     successors of front records (:568-748), link = (rank_base + parent) << 8 | ordinal;
- *                        SPL_E_CAPACITY + the needed count when cap is too small
- *   spl_rroute_keys      the candidates' packed keys (spl_rpack) in (owner, arrival) order, send_keys_dev[n][6], + per-owner
- *                        counts; owner = low 32 bits of the key hash, the owner's bucket comes from the high bits.  The
- *                        permutation stays in the context for spl_rcompact_winners
- *   spl_rdedup_flags     owner side (:840-843): first-arrival insert of a received key list (index = arrival) into the
- *                        realistic visited table -> one winner byte each; keys inserted by earlier calls lose.  The table
- *                        grows as spl_rsolver's does; SPL_E_TABLE_FULL when it cannot take the list (no state is dropped)
- *   spl_rcompact_winners source side: winner bytes (in send order) -> the winning records in arrival order; SPL_E_STATE
- *                        unless it follows spl_rroute_keys on the same candidates
- *   spl_rmove_rows       out[i] = rows[idx[i]] (scatter = 0) or out[idx[i]] = rows[i] (scatter = 1), 96-byte records
+ * across ranks, with the same per-level steps as spl_expand_rows .. spl_move_rows above.  Every level holds the same
+ * records, in the same order, as spl_rsolver.  Ties by arrival order, noise const | hash (the config's; spl_rscore scores
+ * the records).  Realistic mode shards only when asked.  Each spl_r* row call is its speedrun twin on 96-byte records and
+ * 384-bit identity keys, with these differences:
+ *   spl_rexpand_rows     successors follow :568-748 under the config; rank_base must be >= 0
+ *   spl_rroute_keys      send_keys_dev[n][6] holds the packed keys (spl_rpack); owner = low 32 bits of the key hash, the
+ *                        owner's bucket comes from the high bits.  SPL_E_INVALID when a key cannot be packed.  Its
+ *                        permutation is kept apart from spl_route_keys': only spl_rcompact_winners may follow it
+ *   spl_rdedup_flags     (:840-843) inserts into the realistic visited table, which grows as spl_rsolver's does;
+ *                        SPL_E_TABLE_FULL when it cannot take the list (no state is dropped)
+ *   spl_rcompact_winners SPL_E_STATE unless it follows spl_rroute_keys on the same candidates
+ *   spl_rmove_rows       96-byte records
  *   spl_rfirst_goal      first queue index whose game is over (:827-829: players[cur].pts >= target), -1 if none
  *   spl_rreset_visited   forget every visited state of the context: the realistic table and, as spl_rsolver_create does,
  *                        the speedrun table (spl_reset_visited clears only that one).  The epoch counter restarts, so a

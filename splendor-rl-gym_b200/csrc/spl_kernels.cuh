@@ -1353,60 +1353,10 @@ __global__ void __launch_bounds__(TILE) gather_keys_kernel(const Rec *__restrict
         out[i].hi = hi;
     }
 }
-// winner byte per listed candidate: its slot still holds its own arrival index
-__global__ void __launch_bounds__(TILE) win_flags_kernel(const uint32_t *__restrict__ cand_slot,
-                                                         const uint64_t *__restrict__ table, int64_t n,
-                                                         uint8_t *__restrict__ flags) {
-    const int64_t t = (int64_t)blockIdx.x * TILE + threadIdx.x;
-    if (t < n) {
-        const uint32_t s = cand_slot[t];
-        flags[t] = s != DEAD && ~ld_cg_u32(slot_tword(table, s)) == (uint32_t)t;
-    }
-}
 __global__ void __launch_bounds__(TILE) scatter_flags_kernel(const uint8_t *__restrict__ part, const uint32_t *__restrict__ idx,
                                                              int64_t n, uint8_t *__restrict__ arrival) {
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
     if (i < n) arrival[idx[i]] = part[i];
-}
-// stable compaction of the flagged rows (arrival order preserved): 8 rows per thread, look-back scan
-__global__ void __launch_bounds__(TILE) compact_rows_kernel(const Rec *__restrict__ rows, const uint8_t *__restrict__ flags,
-                                                            int64_t n, Rec *__restrict__ out, uint64_t *status,
-                                                            Counters *ctr, int ticket_id) {
-    __shared__ uint32_t warp_sums[TILE / 32 + 1];
-    __shared__ uint32_t s_tile;
-    __shared__ uint64_t s_base;
-    if (threadIdx.x == 0) s_tile = atomicAdd(&ctr->ticket[ticket_id], 1u);
-    __syncthreads();
-    const uint32_t tile = s_tile;
-    const int64_t b0 = ((int64_t)tile * TILE + threadIdx.x) * 8;
-    uint32_t mask = 0;
-    if (b0 + 8 <= n) {
-        const uint64_t f = *reinterpret_cast<const uint64_t *>(flags + b0);
-#pragma unroll
-        for (int q = 0; q < 8; ++q) mask |= (uint32_t)((f >> (8 * q)) & 1) << q;
-    } else {
-        for (int q = 0; q < 8; ++q)
-            if (b0 + q < n && flags[b0 + q]) mask |= 1u << q;
-    }
-    uint32_t tot;
-    const uint32_t ex = block_excl_scan(__popc(mask), warp_sums, tot);
-    if (threadIdx.x < 32) {
-        const uint64_t e = lookback_exclusive(status, tile, tot, 0);
-        if (threadIdx.x == 0) {
-            s_base = e;
-            if (((int64_t)tile + 1) * TILE * 8 >= n) ctr->n_emitted = e + tot;
-        }
-    }
-    __syncthreads();
-    uint64_t pos = s_base + ex;
-    while (mask) {
-        const int q = __ffs(mask) - 1;
-        mask &= mask - 1;
-        Rec r;
-        ld_rec(rows + b0 + q, r);
-        st_rec(out + pos, r);
-        ++pos;
-    }
 }
 
 // scores of rows[i] with the i-th externally drawn randint (noise policy `mt`): order-preserving keys + range
@@ -1442,16 +1392,6 @@ __global__ void __launch_bounds__(TILE) score_rows_kernel(const Rec *__restrict_
         Rec r;
         ld_rec(rows + i, r);
         out[i] = score_state(h, noise_mode, r.lo, r.hi & HI_KEY_MASK, r.aux, L, draws ? draws[i] : 50);
-    }
-}
-// out[i] = rows[idx[i]] (gather) or out[idx[i]] = rows[i] (scatter), 64-bit indices
-__global__ void __launch_bounds__(TILE) move_rows_kernel(const Rec *__restrict__ rows, const int64_t *__restrict__ idx,
-                                                         int64_t n, Rec *__restrict__ out, int scatter) {
-    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
-    if (i < n) {
-        Rec r;
-        ld_rec(rows + (scatter ? i : idx[i]), r);
-        st_rec(out + (scatter ? idx[i] : i), r);
     }
 }
 

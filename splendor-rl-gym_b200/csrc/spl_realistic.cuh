@@ -41,12 +41,13 @@ struct RConfigDev {
     uint8_t pos_of[SPL_NUM_CARDS];  // position of a card inside its tier's deck sequence
 };
 
-__device__ __forceinline__ void ld_rrec(const RRec *p, RRec &r) {
+// the RRec overloads of ld_rec / st_rec (spl_common.cuh): three 32-byte sectors
+__device__ __forceinline__ void ld_rec(const RRec *p, RRec &r) {
     const ulonglong4 *s = reinterpret_cast<const ulonglong4 *>(p);
     ulonglong4 *d = reinterpret_cast<ulonglong4 *>(&r);
     d[0] = s[0]; d[1] = s[1]; d[2] = s[2];
 }
-__device__ __forceinline__ void st_rrec(RRec *p, const RRec &r) {
+__device__ __forceinline__ void st_rec(RRec *p, const RRec &r) {
     const ulonglong4 *s = reinterpret_cast<const ulonglong4 *>(&r);
     ulonglong4 *d = reinterpret_cast<ulonglong4 *>(p);
     d[0] = s[0]; d[1] = s[1]; d[2] = s[2];
@@ -253,7 +254,7 @@ __global__ void __launch_bounds__(TILE) r_probe_kernel(const RRec *__restrict__ 
     uint32_t n_new = 0;
     if (t < n) {
         RRec s;
-        ld_rrec(cand + t, s);
+        ld_rec(cand + t, s);
         uint64_t key[RKEY_WORDS];
         if (!r_pack_key(*cfg, s, key)) atomicExch(&ctr->error, 4u);
         cand_slot[t] = r_probe(table, nb, tag, key, ~(uint32_t)t, n_new, &ctr->error);
@@ -317,7 +318,7 @@ __global__ void __launch_bounds__(TILE) r_pack_kernel(const RRec *__restrict__ r
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
     if (i >= n) return;
     RRec s;
-    ld_rrec(recs + i, s);
+    ld_rec(recs + i, s);
     uint64_t key[RKEY_WORDS];
     r_pack_key(*cfg, s, key);
 #pragma unroll
@@ -388,7 +389,7 @@ __global__ void __launch_bounds__(TILE) r_count_scan_kernel(const RRec *__restri
     uint32_t cnt = 0, m = 0;
     if (p < n) {
         RRec s;
-        ld_rrec(front + p, s);
+        ld_rec(front + p, s);
         int bonus[NCOL], pts;
         r_derive(*cfg, s.p[s.cur], bonus, pts);
         m = r_valid_mask(*cfg, s, bonus);
@@ -417,7 +418,7 @@ __global__ void __launch_bounds__(TILE) r_expand_kernel(const RRec *__restrict__
     const int64_t p = (int64_t)blockIdx.x * TILE + threadIdx.x;
     if (p >= n) return;
     RRec s;
-    ld_rrec(front + p, s);
+    ld_rec(front + p, s);
     int bonus[NCOL], pts;
     r_derive(*cfg, s.p[s.cur], bonus, pts);
     uint32_t m = vmask[p], ord = 0;
@@ -429,7 +430,7 @@ __global__ void __launch_bounds__(TILE) r_expand_kernel(const RRec *__restrict__
         r_make_child(*cfg, s, bonus, slot, o);
         o.link = ((uint64_t)(rank_base + p) << 8) | ord;
         o.spare = 0;
-        st_rrec(cand + t, o);
+        st_rec(cand + t, o);
         ++t;
         ++ord;
     }
@@ -441,8 +442,8 @@ __global__ void __launch_bounds__(TILE) r_gather_kernel(const RRec *__restrict__
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
     if (i < n) {
         RRec r;
-        ld_rrec(src + idx[i], r);
-        st_rrec(dst + i, r);
+        ld_rec(src + idx[i], r);
+        st_rec(dst + i, r);
     }
 }
 
@@ -454,7 +455,7 @@ __global__ void __launch_bounds__(TILE) r_score_kernel(const RRec *__restrict__ 
     uint64_t kmin = ~0ull, kmax = 0;
     if (i < n) {
         RRec s;
-        ld_rrec(recs + i, s);
+        ld_rec(recs + i, s);
         const double sc = r_score(*cfg, s, L, draws ? draws[i] : 50);
         if (raw) raw[i] = sc;
         if (sk) {
@@ -506,7 +507,7 @@ __global__ void __launch_bounds__(TILE) r_route_pack_kernel(const RRec *__restri
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
     if (i >= n) return;
     RRec s;
-    ld_rrec(cand + i, s);
+    ld_rec(cand + i, s);
     uint64_t key[RKEY_WORDS];
     if (!r_pack_key(*cfg, s, key)) atomicExch(&ctr->error, 4u);
 #pragma unroll
@@ -514,7 +515,7 @@ __global__ void __launch_bounds__(TILE) r_route_pack_kernel(const RRec *__restri
     owner[i] = r_owner_of(r_key_hash(key), n_ranks);
     idx[i] = (uint32_t)i;
 }
-// send buffer: the keys in (owner, arrival) order; perm keeps that order for r_compact_kernel's caller
+// send buffer: the keys in (owner, arrival) order; perm keeps that order for spl_rcompact_winners
 __global__ void __launch_bounds__(TILE) r_gather_keys_kernel(const uint64_t *__restrict__ keys, const uint32_t *__restrict__ idx,
                                                              int64_t n, uint64_t *__restrict__ out, uint32_t *__restrict__ perm) {
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
@@ -539,18 +540,27 @@ __global__ void __launch_bounds__(TILE) r_probe_keys_kernel(const uint64_t *__re
     for (int d = 16; d; d >>= 1) n_new += __shfl_xor_sync(0xffffffffu, n_new, d);
     if ((threadIdx.x & 31) == 0 && n_new) atomicAdd(&ctr->n_new, (unsigned long long)n_new);
 }
-// winner byte per listed key: its bucket still holds its own arrival index
-__global__ void __launch_bounds__(TILE) r_win_flags_kernel(const uint32_t *__restrict__ cand_slot, const RBucket *__restrict__ table,
-                                                           int64_t n, uint8_t *__restrict__ flags) {
+// the ~t word of a realistic bucket: the slot_tword overload win_flags_kernel reads
+__device__ __forceinline__ const uint32_t *slot_tword(const RBucket *table, uint32_t sl) { return &table[sl].tinv; }
+
+// ------------------------------------------------------------------ row layer of the key-sharded driver, for both row kinds:
+// R = Rec (speedrun, 32 B) or RRec (realistic, 96 B) through the ld_rec / st_rec overloads; Table = the speedrun table's
+// uint64_t words or RBucket through the slot_tword overloads (R_DEAD == DEAD)
+// winner byte per listed candidate: its slot still holds its own arrival index
+template <typename Table>
+__global__ void __launch_bounds__(TILE) win_flags_kernel(const uint32_t *__restrict__ cand_slot, const Table *__restrict__ table,
+                                                         int64_t n, uint8_t *__restrict__ flags) {
     const int64_t t = (int64_t)blockIdx.x * TILE + threadIdx.x;
     if (t < n) {
-        const uint32_t sl = cand_slot[t];
-        flags[t] = sl != R_DEAD && ~ld_cg_u32(&table[sl].tinv) == (uint32_t)t;
+        const uint32_t s = cand_slot[t];
+        flags[t] = s != DEAD && ~ld_cg_u32(slot_tword(table, s)) == (uint32_t)t;
     }
 }
-// stable compaction of the flagged records (arrival order preserved): 8 records per thread, look-back scan
-__global__ void __launch_bounds__(TILE) r_compact_kernel(const RRec *__restrict__ recs, const uint8_t *__restrict__ flags, int64_t n,
-                                                         RRec *__restrict__ out, uint64_t *status, Counters *ctr, int ticket_id) {
+// stable compaction of the flagged rows (arrival order preserved): 8 rows per thread, look-back scan
+template <typename R>
+__global__ void __launch_bounds__(TILE) compact_rows_kernel(const R *__restrict__ rows, const uint8_t *__restrict__ flags,
+                                                            int64_t n, R *__restrict__ out, uint64_t *status,
+                                                            Counters *ctr, int ticket_id) {
     __shared__ uint32_t warp_sums[TILE / 32 + 1];
     __shared__ uint32_t s_tile;
     __shared__ uint64_t s_base;
@@ -559,8 +569,14 @@ __global__ void __launch_bounds__(TILE) r_compact_kernel(const RRec *__restrict_
     const uint32_t tile = s_tile;
     const int64_t b0 = ((int64_t)tile * TILE + threadIdx.x) * 8;
     uint32_t mask = 0;
-    for (int q = 0; q < 8; ++q)
-        if (b0 + q < n && flags[b0 + q]) mask |= 1u << q;
+    if (b0 + 8 <= n) {
+        const uint64_t f = *reinterpret_cast<const uint64_t *>(flags + b0);
+#pragma unroll
+        for (int q = 0; q < 8; ++q) mask |= (uint32_t)((f >> (8 * q)) & 1) << q;
+    } else {
+        for (int q = 0; q < 8; ++q)
+            if (b0 + q < n && flags[b0 + q]) mask |= 1u << q;
+    }
     uint32_t tot;
     const uint32_t ex = block_excl_scan(__popc(mask), warp_sums, tot);
     if (threadIdx.x < 32) {
@@ -572,20 +588,24 @@ __global__ void __launch_bounds__(TILE) r_compact_kernel(const RRec *__restrict_
     }
     __syncthreads();
     uint64_t pos = s_base + ex;
-    for (; mask; mask &= mask - 1) {
-        RRec r;
-        ld_rrec(recs + b0 + (__ffs(mask) - 1), r);
-        st_rrec(out + pos++, r);
+    while (mask) {
+        const int q = __ffs(mask) - 1;
+        mask &= mask - 1;
+        R r;
+        ld_rec(rows + b0 + q, r);
+        st_rec(out + pos, r);
+        ++pos;
     }
 }
-// out[i] = recs[idx[i]] (gather) or out[idx[i]] = recs[i] (scatter)
-__global__ void __launch_bounds__(TILE) r_move_kernel(const RRec *__restrict__ recs, const int64_t *__restrict__ idx, int64_t n,
-                                                      RRec *__restrict__ out, int scatter) {
+// out[i] = rows[idx[i]] (gather) or out[idx[i]] = rows[i] (scatter), 64-bit indices
+template <typename R>
+__global__ void __launch_bounds__(TILE) move_rows_kernel(const R *__restrict__ rows, const int64_t *__restrict__ idx,
+                                                         int64_t n, R *__restrict__ out, int scatter) {
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
     if (i < n) {
-        RRec r;
-        ld_rrec(recs + (scatter ? i : idx[i]), r);
-        st_rrec(out + (scatter ? idx[i] : i), r);
+        R r;
+        ld_rec(rows + (scatter ? i : idx[i]), r);
+        st_rec(out + (scatter ? idx[i] : i), r);
     }
 }
 

@@ -878,6 +878,20 @@ int32_t spl_topk(spl_ctx *c, const double *scores, const spl_key *keys, int64_t 
 }
 
 // ---- multi-GPU building blocks ----------------------------------------------------------------
+// Per-owner counts from the digit-major scanned histogram in c->matrix2 (nt tiles per digit): owner g's candidates start
+// at digit g, tile 0, and the last owner's end at n.  read_owner_starts queues the reads of the first n_read starts (the
+// sort paths read n_ranks + 1); owner_counts takes the differences once the caller has synchronised the stream.
+static int read_owner_starts(spl_ctx *c, unsigned nt, int n_read, std::vector<uint32_t> &start, cudaStream_t st) {
+    start.resize(n_read);
+    for (int g = 0; g < n_read; ++g)
+        CK(c, cudaMemcpyAsync(&start[g], c->matrix2.as<uint32_t>() + (size_t)g * nt, 4, cudaMemcpyDeviceToHost, st));
+    c->d2h_bytes += 4 * n_read;
+    return SPL_OK;
+}
+static void owner_counts(const std::vector<uint32_t> &start, int n_ranks, int64_t n, int64_t *counts_host) {
+    for (int g = 0; g < n_ranks; ++g) counts_host[g] = (g + 1 < n_ranks ? start[g + 1] : (uint32_t)n) - start[g];
+}
+
 int32_t spl_owner_partition(spl_ctx *c, const spl_key *keys, int64_t n, int32_t n_ranks, int64_t *perm, int64_t *counts_host,
                             void *stream) {
     if (!c || !counts_host || n < 0 || n >= (1ll << 32) || n_ranks < 1 || n_ranks > 256)
@@ -899,13 +913,10 @@ int32_t spl_owner_partition(spl_ctx *c, const spl_key *keys, int64_t n, int32_t 
     CKS(c, sort_pass(c, 0, 0, c->y[0].as<uint64_t>(), n, 0, nt, msz, st));  // one stable pass: digit = owner
     idx_widen_kernel<<<nblk(n), TILE, 0, st>>>(c->idx[1].as<uint32_t>(), n, perm);
     ++c->launches;
-    // per-owner counts = differences of the digit-major scanned histogram at tile 0
-    std::vector<uint32_t> base(n_ranks + 1);
-    for (int g = 0; g <= n_ranks; ++g)
-        CK(c, cudaMemcpyAsync(&base[g], c->matrix2.as<uint32_t>() + (size_t)g * nt, 4, cudaMemcpyDeviceToHost, st));
+    std::vector<uint32_t> start;
+    CKS(c, read_owner_starts(c, nt, n_ranks + 1, start, st));
     CK(c, cudaStreamSynchronize(st));
-    c->d2h_bytes += 4 * (n_ranks + 1);
-    for (int g = 0; g < n_ranks; ++g) counts_host[g] = (g + 1 < SORT_BINS ? base[g + 1] : (uint32_t)n) - base[g];
+    owner_counts(start, n_ranks, n, counts_host);
     return SPL_OK;
 }
 
@@ -960,13 +971,10 @@ int32_t spl_route_keys(spl_ctx *c, const void *cand_rows, int64_t n, int32_t n_r
                                                    c->idx[1].as<uint32_t>());
         c->launches += 3;
         CK(c, cudaGetLastError());
-        std::vector<uint32_t> base(n_ranks + 1);
-        for (int g = 0; g < n_ranks; ++g)
-            CK(c, cudaMemcpyAsync(&base[g], c->matrix2.as<uint32_t>() + (size_t)g * nt, 4, cudaMemcpyDeviceToHost, st));
+        std::vector<uint32_t> start;
+        CKS(c, read_owner_starts(c, nt, n_ranks, start, st));
         CK(c, cudaStreamSynchronize(st));
-        base[n_ranks] = (uint32_t)n;
-        c->d2h_bytes += 4 * n_ranks;
-        for (int g = 0; g < n_ranks; ++g) counts_host[g] = base[g + 1] - base[g];
+        owner_counts(start, n_ranks, n, counts_host);
         return SPL_OK;
     }
     owner_rows_kernel<<<nblk(n), TILE, 0, st>>>(rows, n, (uint32_t)n_ranks, c->y[0].as<uint64_t>(), c->idx[0].as<uint32_t>());
@@ -978,54 +986,10 @@ int32_t spl_route_keys(spl_ctx *c, const void *cand_rows, int64_t n, int32_t n_r
     CKS(c, sort_pass(c, 0, 0, c->y[0].as<uint64_t>(), n, 0, nt, msz, st));  // stable: digit = owner; perm stays in idx[1]
     gather_keys_kernel<<<nblk(n), TILE, 0, st>>>(rows, c->idx[1].as<uint32_t>(), n, send_keys);
     ++c->launches;
-    std::vector<uint32_t> base(n_ranks + 1);
-    for (int g = 0; g <= n_ranks; ++g)
-        CK(c, cudaMemcpyAsync(&base[g], c->matrix2.as<uint32_t>() + (size_t)g * nt, 4, cudaMemcpyDeviceToHost, st));
+    std::vector<uint32_t> start;
+    CKS(c, read_owner_starts(c, nt, n_ranks + 1, start, st));
     CK(c, cudaStreamSynchronize(st));
-    c->d2h_bytes += 4 * (n_ranks + 1);
-    for (int g = 0; g < n_ranks; ++g) counts_host[g] = base[g + 1] - base[g];
-    return SPL_OK;
-}
-
-int32_t spl_dedup_flags(spl_ctx *c, const spl_key *keys, int64_t n, uint8_t *flags, void *stream) {
-    if (!c || n < 0 || n >= (1ll << 32)) return fail(c, SPL_E_INVALID, "spl_dedup_flags: bad arguments");
-    NO_LIVE_SOLVER(c, "spl_dedup_flags");
-    cudaStream_t st = (cudaStream_t)stream;
-    CK(c, enter_device(c));
-    if (n == 0) return SPL_OK;
-    CKS(c, zero_ctr(c, st));
-    CKS(c, ensure_table(c, (uint64_t)n, st));
-    uint64_t tag;
-    CKS(c, next_epoch(c, tag));
-    CK(c, c->cand_slot.ensure((size_t)n * 4, 0, st));
-    probe_list_kernel<IDENT_KEY><<<nblk(n), TILE, 0, st>>>(keys, n, c->table, c->nb, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
-    win_flags_kernel<<<nblk(n), TILE, 0, st>>>(c->cand_slot.as<uint32_t>(), c->table, n, flags);
-    c->launches += 2;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "spl_dedup_flags: probe overflow (table full)");
-    c->occupied += c->h_ctr->n_new;
-    return SPL_OK;
-}
-
-int32_t spl_compact_winners(spl_ctx *c, const void *cand_rows, int64_t n, const uint8_t *flags_partitioned, void *out_rows,
-                            int64_t *n_out, void *stream) {
-    if (!c || !n_out || n < 0 || n != c->route_n) return fail(c, SPL_E_STATE, "spl_compact_winners: must follow spl_route_keys on the same candidates");
-    cudaStream_t st = (cudaStream_t)stream;
-    CK(c, enter_device(c));
-    *n_out = 0;
-    if (n == 0) return SPL_OK;
-    CK(c, c->rtmp.ensure((size_t)n + 8, 0, st));
-    scatter_flags_kernel<<<nblk(n), TILE, 0, st>>>(flags_partitioned, c->idx[1].as<uint32_t>(), n, c->rtmp.as<uint8_t>());
-    const unsigned nt = nblk(n, TILE * 8);
-    CKS(c, zero_ctr(c, st));
-    CKS(c, prep_status(c, 0, nt, st));
-    compact_rows_kernel<<<nt, TILE, 0, st>>>(reinterpret_cast<const Rec *>(cand_rows), c->rtmp.as<uint8_t>(), n,
-                                              reinterpret_cast<Rec *>(out_rows), c->status[0].as<uint64_t>(), c->d_ctr, 0);
-    c->launches += 2;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    *n_out = (int64_t)c->h_ctr->n_emitted;
+    owner_counts(start, n_ranks, n, counts_host);
     return SPL_OK;
 }
 
@@ -1036,17 +1000,6 @@ int32_t spl_score_rows(spl_ctx *c, int32_t heuristic, int32_t noise, const void 
     CK(c, enter_device(c));
     if (n == 0) return SPL_OK;
     score_rows_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const Rec *>(rows), n, heuristic, noise, c->luts, scores, draws);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    return SPL_OK;
-}
-
-int32_t spl_move_rows(spl_ctx *c, const void *rows, const int64_t *idx, int64_t n, void *out_rows, int32_t scatter, void *stream) {
-    if (!c || n < 0) return fail(c, SPL_E_INVALID, "spl_move_rows: bad arguments");
-    cudaStream_t st = (cudaStream_t)stream;
-    CK(c, enter_device(c));
-    if (n == 0) return SPL_OK;
-    move_rows_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const Rec *>(rows), idx, n, reinterpret_cast<Rec *>(out_rows), scatter);
     ++c->launches;
     CK(c, cudaGetLastError());
     return SPL_OK;
@@ -2197,9 +2150,8 @@ static int ensure_rtable(spl_ctx *c, uint64_t need, cudaStream_t st) {
     return SPL_OK;
 }
 
-// count + materialise the successors of front[0..n) into c->rcand
-static int r_expand_all(spl_ctx *c, const RRec *front, int64_t n, int64_t rank_base, bool keys, int64_t *total_out,
-                        cudaStream_t st) {
+// count + scan of the successors of front[0..n): offsets in c->off, vis masks in c->rvmask, the count in *total (synchronises)
+static int r_count_scan(spl_ctx *c, const RRec *front, int64_t n, int64_t *total, cudaStream_t st) {
     const unsigned nt = nblk(n);
     CK(c, c->off.ensure((size_t)n * 4 + 4, 0, st));
     CK(c, c->rvmask.ensure((size_t)n * 4 + 4, 0, st));
@@ -2210,13 +2162,91 @@ static int r_expand_all(spl_ctx *c, const RRec *front, int64_t n, int64_t rank_b
     ++c->launches;
     CK(c, cudaGetLastError());
     CKS(c, read_ctr(c, st));
-    const int64_t total = (int64_t)c->h_ctr->total_cands;
-    *total_out = total;
+    *total = (int64_t)c->h_ctr->total_cands;
+    return SPL_OK;
+}
+
+// count + materialise the successors of front[0..n) into c->rcand
+static int r_expand_all(spl_ctx *c, const RRec *front, int64_t n, int64_t rank_base, int64_t *total_out, cudaStream_t st) {
+    CKS(c, r_count_scan(c, front, n, total_out, st));
+    const int64_t total = *total_out;
     if (total == 0) return SPL_OK;
     CK(c, c->rcand.ensure((size_t)total * 96, 0, st));
-    (void)keys;
-    r_expand_kernel<<<nt, TILE, 0, st>>>(front, n, c->rcfg.as<RConfigDev>(), c->off.as<uint32_t>(), c->rvmask.as<uint32_t>(),
-                                          rank_base, c->rcand.as<RRec>());
+    r_expand_kernel<<<nblk(n), TILE, 0, st>>>(front, n, c->rcfg.as<RConfigDev>(), c->off.as<uint32_t>(), c->rvmask.as<uint32_t>(),
+                                               rank_base, c->rcand.as<RRec>());
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    return SPL_OK;
+}
+
+// ---- row layer of the key-sharded driver, shared by speedrun (Rec, spl_*) and realistic (RRec, spl_r*) rows
+// Owner side of a key-sharded round: first-arrival insert of a received key list (index = arrival) into the speedrun
+// table (16-byte keys) or the realistic one (RKEY_WORDS-word keys), then one winner byte per key.
+static int dedup_flags(spl_ctx *c, bool realistic, const void *keys, int64_t n, uint8_t *flags, cudaStream_t st) {
+    CK(c, enter_device(c));
+    if (n == 0) return SPL_OK;
+    CKS(c, zero_ctr(c, st));
+    CKS(c, realistic ? ensure_rtable(c, (uint64_t)n, st) : ensure_table(c, (uint64_t)n, st));
+    uint64_t tag;
+    CKS(c, next_epoch(c, tag));
+    CK(c, c->cand_slot.ensure((size_t)n * 4, 0, st));
+    uint32_t *slot = c->cand_slot.as<uint32_t>();
+    if (realistic) {
+        CKS(c, zero_ctr(c, st));  // again after the table's growth, as rsolver_step does
+        r_probe_keys_kernel<<<nblk(n), TILE, 0, st>>>(static_cast<const uint64_t *>(keys), n, c->rtable, c->rnb, tag, slot, c->d_ctr);
+        win_flags_kernel<<<nblk(n), TILE, 0, st>>>(slot, c->rtable, n, flags);
+    } else {
+        probe_list_kernel<IDENT_KEY><<<nblk(n), TILE, 0, st>>>(static_cast<const spl_key *>(keys), n, c->table, c->nb, tag, slot, c->d_ctr);
+        win_flags_kernel<<<nblk(n), TILE, 0, st>>>(slot, c->table, n, flags);
+    }
+    c->launches += 2;
+    CK(c, cudaGetLastError());
+    CKS(c, read_ctr(c, st));
+    if (realistic) {
+        // the intended difference: counted before the error check, so that spl_rreset_visited clears a partial insert too
+        c->rocc += c->h_ctr->n_new;
+        if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "spl_rdedup_flags: probe overflow (realistic visited table full, %llu buckets)",
+                                         (unsigned long long)c->rnb);
+        return SPL_OK;
+    }
+    if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "spl_dedup_flags: probe overflow (table full)");
+    c->occupied += c->h_ctr->n_new;
+    return SPL_OK;
+}
+
+// Source side of a key-sharded round: winner bytes in the send order of the route call this follows (route_n candidates,
+// permutation perm; `what` is the SPL_E_STATE message) -> the winning rows in arrival order.
+template <typename R>
+static int compact_winners(spl_ctx *c, int64_t route_n, const uint32_t *perm, const char *what, const void *cand, int64_t n,
+                           const uint8_t *flags_partitioned, void *out, int64_t *n_out, void *stream) {
+    if (!c || !n_out || n < 0 || n != route_n) return fail(c, SPL_E_STATE, "%s", what);
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    *n_out = 0;
+    if (n == 0) return SPL_OK;
+    CK(c, c->rtmp.ensure((size_t)n + 8, 0, st));
+    scatter_flags_kernel<<<nblk(n), TILE, 0, st>>>(flags_partitioned, perm, n, c->rtmp.as<uint8_t>());
+    const unsigned nt = nblk(n, TILE * 8);
+    CKS(c, zero_ctr(c, st));
+    CKS(c, prep_status(c, 0, nt, st));
+    compact_rows_kernel<<<nt, TILE, 0, st>>>(reinterpret_cast<const R *>(cand), c->rtmp.as<uint8_t>(), n, reinterpret_cast<R *>(out),
+                                             c->status[0].as<uint64_t>(), c->d_ctr, 0);
+    c->launches += 2;
+    CK(c, cudaGetLastError());
+    CKS(c, read_ctr(c, st));
+    *n_out = (int64_t)c->h_ctr->n_emitted;
+    return SPL_OK;
+}
+
+// out[i] = rows[idx[i]] (scatter = 0) or out[idx[i]] = rows[i] (scatter = 1), rows of type R; `fn` names the entry point
+template <typename R>
+static int move_rows(spl_ctx *c, const char *fn, const void *rows, const int64_t *idx, int64_t n, void *out, int32_t scatter,
+                     void *stream) {
+    if (!c || n < 0 || (n && (!rows || !idx || !out))) return fail(c, SPL_E_INVALID, "%s: bad arguments", fn);
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    if (n == 0) return SPL_OK;
+    move_rows_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const R *>(rows), idx, n, reinterpret_cast<R *>(out), scatter);
     ++c->launches;
     CK(c, cudaGetLastError());
     return SPL_OK;
@@ -2253,7 +2283,7 @@ static int rsolver_step(spl_solver *s, spl_level_info *info, cudaStream_t st) {
     }
     int64_t total = 0, n_new = 0;
     CK(c, cudaEventRecord(c->ev[0], st));
-    CKS(c, r_expand_all(c, front, n, 0, true, &total, st));
+    CKS(c, r_expand_all(c, front, n, 0, &total, st));
     CK(c, cudaEventRecord(c->ev[1], st));
     info->expanded = n;
     info->generated = total;
@@ -2546,7 +2576,7 @@ int32_t spl_rexpand(spl_ctx *c, const spl_rconfig *cfg, const void *recs, int64_
     if (n == 0) return SPL_OK;
     CKS(c, upload_rconfig(c, cfg, st));
     int64_t total = 0;
-    CKS(c, r_expand_all(c, reinterpret_cast<const RRec *>(recs), n, 0, false, &total, st));
+    CKS(c, r_expand_all(c, reinterpret_cast<const RRec *>(recs), n, 0, &total, st));
     *n_out = total;
     if (total > cap) return fail(c, SPL_E_CAPACITY, "spl_rexpand: %lld successors, capacity %lld", (long long)total, (long long)cap);
     if (total) CK(c, cudaMemcpyAsync(out_recs, c->rcand.p, (size_t)total * 96, cudaMemcpyDeviceToDevice, st));
@@ -2648,7 +2678,8 @@ int32_t spl_rsolver_frontier(spl_solver *s, const void **recs, int64_t *n) {
     return SPL_OK;
 }
 
-// ---- realistic mode on the key-sharded driver: rows are 96-byte RRec records
+// ---- realistic mode on the key-sharded driver: rows are 96-byte RRec records (spl_dedup_flags, spl_compact_winners and
+// spl_move_rows sit beside their realistic twins)
 int32_t spl_rexpand_rows(spl_ctx *c, const spl_rconfig *cfg, const void *front, int64_t n, int64_t rank_base, void *out, int64_t cap,
                          int64_t *n_out, void *stream) {
     if (!c || !cfg || !n_out || n < 0 || n > (16ll << 20) || rank_base < 0) return fail(c, SPL_E_INVALID, "spl_rexpand_rows: bad arguments");
@@ -2657,21 +2688,12 @@ int32_t spl_rexpand_rows(spl_ctx *c, const spl_rconfig *cfg, const void *front, 
     *n_out = 0;
     if (n == 0) return SPL_OK;
     CKS(c, use_rconfig(c, cfg, st));
-    const unsigned nt = nblk(n);
-    CK(c, c->off.ensure((size_t)n * 4 + 4, 0, st));
-    CK(c, c->rvmask.ensure((size_t)n * 4 + 4, 0, st));
-    CKS(c, zero_ctr(c, st));
-    CKS(c, prep_status(c, 0, nt, st));
-    r_count_scan_kernel<<<nt, TILE, 0, st>>>(reinterpret_cast<const RRec *>(front), n, c->rcfg.as<RConfigDev>(), c->off.as<uint32_t>(),
-                                              c->rvmask.as<uint32_t>(), c->status[0].as<uint64_t>(), c->d_ctr, 0);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    const int64_t total = (int64_t)c->h_ctr->total_cands;
+    int64_t total = 0;
+    CKS(c, r_count_scan(c, reinterpret_cast<const RRec *>(front), n, &total, st));
     *n_out = total;
     if (total > cap) return fail(c, SPL_E_CAPACITY, "spl_rexpand_rows: %lld successors, capacity %lld", (long long)total, (long long)cap);
     if (total == 0) return SPL_OK;
-    r_expand_kernel<<<nt, TILE, 0, st>>>(reinterpret_cast<const RRec *>(front), n, c->rcfg.as<RConfigDev>(), c->off.as<uint32_t>(),
+    r_expand_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const RRec *>(front), n, c->rcfg.as<RConfigDev>(), c->off.as<uint32_t>(),
                                           c->rvmask.as<uint32_t>(), rank_base, reinterpret_cast<RRec *>(out));
     ++c->launches;
     CK(c, cudaGetLastError());
@@ -2706,72 +2728,47 @@ int32_t spl_rroute_keys(spl_ctx *c, const spl_rconfig *cfg, const void *cand, in
     r_gather_keys_kernel<<<nblk(n), TILE, 0, st>>>(c->rkeys.as<uint64_t>(), c->idx[1].as<uint32_t>(), n, send_keys, c->rperm.as<uint32_t>());
     ++c->launches;
     CK(c, cudaGetLastError());
-    // per-owner counts = differences of the digit-major scanned histogram at tile 0
-    std::vector<uint32_t> base(n_ranks + 1);
-    for (int g = 0; g <= n_ranks; ++g)
-        CK(c, cudaMemcpyAsync(&base[g], c->matrix2.as<uint32_t>() + (size_t)g * nt, 4, cudaMemcpyDeviceToHost, st));
-    c->d2h_bytes += 4 * (n_ranks + 1);
-    CKS(c, read_ctr(c, st));
+    std::vector<uint32_t> start;
+    CKS(c, read_owner_starts(c, nt, n_ranks + 1, start, st));
+    CKS(c, read_ctr(c, st));  // synchronises the reads of the starts too
     if (c->h_ctr->error == 4) return fail(c, SPL_E_INVALID, "a player saved 1024 gems or more: outside the packed identity key");
-    for (int g = 0; g < n_ranks; ++g) counts_host[g] = base[g + 1] - base[g];
+    owner_counts(start, n_ranks, n, counts_host);
     c->rroute_n = n;
     return SPL_OK;
+}
+
+int32_t spl_dedup_flags(spl_ctx *c, const spl_key *keys, int64_t n, uint8_t *flags, void *stream) {
+    if (!c || n < 0 || n >= (1ll << 32)) return fail(c, SPL_E_INVALID, "spl_dedup_flags: bad arguments");
+    NO_LIVE_SOLVER(c, "spl_dedup_flags");
+    return dedup_flags(c, false, keys, n, flags, (cudaStream_t)stream);
 }
 
 int32_t spl_rdedup_flags(spl_ctx *c, const uint64_t *keys, int64_t n, uint8_t *flags, void *stream) {
     if (!c || n < 0 || n >= (1ll << 32) || (n && (!keys || !flags))) return fail(c, SPL_E_INVALID, "spl_rdedup_flags: bad arguments");
     NO_LIVE_SOLVER(c, "spl_rdedup_flags");
-    cudaStream_t st = (cudaStream_t)stream;
-    CK(c, enter_device(c));
-    if (n == 0) return SPL_OK;
-    CKS(c, zero_ctr(c, st));
-    CKS(c, ensure_rtable(c, (uint64_t)n, st));
-    uint64_t tag;
-    CKS(c, next_epoch(c, tag));
-    CK(c, c->cand_slot.ensure((size_t)n * 4, 0, st));
-    CKS(c, zero_ctr(c, st));
-    r_probe_keys_kernel<<<nblk(n), TILE, 0, st>>>(keys, n, c->rtable, c->rnb, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
-    r_win_flags_kernel<<<nblk(n), TILE, 0, st>>>(c->cand_slot.as<uint32_t>(), c->rtable, n, flags);
-    c->launches += 2;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    c->rocc += c->h_ctr->n_new;  // counted before the error check, so that spl_rreset_visited clears a partial insert too
-    if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "spl_rdedup_flags: probe overflow (realistic visited table full, %llu buckets)",
-                                     (unsigned long long)c->rnb);
-    return SPL_OK;
+    return dedup_flags(c, true, keys, n, flags, (cudaStream_t)stream);
+}
+
+int32_t spl_compact_winners(spl_ctx *c, const void *cand_rows, int64_t n, const uint8_t *flags_partitioned, void *out_rows,
+                            int64_t *n_out, void *stream) {
+    return compact_winners<Rec>(c, c ? c->route_n : -1, c ? c->idx[1].as<uint32_t>() : nullptr,
+                                "spl_compact_winners: must follow spl_route_keys on the same candidates", cand_rows, n,
+                                flags_partitioned, out_rows, n_out, stream);
 }
 
 int32_t spl_rcompact_winners(spl_ctx *c, const void *cand, int64_t n, const uint8_t *flags_partitioned, void *out, int64_t *n_out,
                              void *stream) {
-    if (!c || !n_out || n < 0 || n != c->rroute_n)
-        return fail(c, SPL_E_STATE, "spl_rcompact_winners: must follow spl_rroute_keys on the same candidates");
-    cudaStream_t st = (cudaStream_t)stream;
-    CK(c, enter_device(c));
-    *n_out = 0;
-    if (n == 0) return SPL_OK;
-    CK(c, c->rtmp.ensure((size_t)n + 8, 0, st));
-    scatter_flags_kernel<<<nblk(n), TILE, 0, st>>>(flags_partitioned, c->rperm.as<uint32_t>(), n, c->rtmp.as<uint8_t>());
-    const unsigned nt = nblk(n, TILE * 8);
-    CKS(c, zero_ctr(c, st));
-    CKS(c, prep_status(c, 0, nt, st));
-    r_compact_kernel<<<nt, TILE, 0, st>>>(reinterpret_cast<const RRec *>(cand), c->rtmp.as<uint8_t>(), n, reinterpret_cast<RRec *>(out),
-                                          c->status[0].as<uint64_t>(), c->d_ctr, 0);
-    c->launches += 2;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    *n_out = (int64_t)c->h_ctr->n_emitted;
-    return SPL_OK;
+    return compact_winners<RRec>(c, c ? c->rroute_n : -1, c ? c->rperm.as<uint32_t>() : nullptr,
+                                 "spl_rcompact_winners: must follow spl_rroute_keys on the same candidates", cand, n,
+                                 flags_partitioned, out, n_out, stream);
+}
+
+int32_t spl_move_rows(spl_ctx *c, const void *rows, const int64_t *idx, int64_t n, void *out_rows, int32_t scatter, void *stream) {
+    return move_rows<Rec>(c, "spl_move_rows", rows, idx, n, out_rows, scatter, stream);
 }
 
 int32_t spl_rmove_rows(spl_ctx *c, const void *rows, const int64_t *idx, int64_t n, void *out, int32_t scatter, void *stream) {
-    if (!c || n < 0 || (n && (!rows || !idx || !out))) return fail(c, SPL_E_INVALID, "spl_rmove_rows: bad arguments");
-    cudaStream_t st = (cudaStream_t)stream;
-    CK(c, enter_device(c));
-    if (n == 0) return SPL_OK;
-    r_move_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const RRec *>(rows), idx, n, reinterpret_cast<RRec *>(out), scatter);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    return SPL_OK;
+    return move_rows<RRec>(c, "spl_rmove_rows", rows, idx, n, out, scatter, stream);
 }
 
 int32_t spl_rfirst_goal(spl_ctx *c, const spl_rconfig *cfg, const void *front, int64_t n, int64_t *rank_host, void *stream) {

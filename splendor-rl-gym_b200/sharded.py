@@ -5,23 +5,23 @@ parent links, same rank order after the beam cut (SURVEY.md 8e).
 
 Per level (G ranks; the queue is block-distributed by global rank: rank g holds a contiguous slice):
   1. goal test: local first rank with pts >= goal, all-reduce MIN                 (src/solver.py:443)
-  2. expand local parents (spl_expand); global arrival index t = exscan(counts) + local index
-  3. stable partition by owner (spl_owner_partition) and all-to-all of the 16-byte KEYS only;
+  2. expand local parents (spl_expand_rows); global arrival index t = exscan(counts) + local index
+  3. stable partition of the candidates' keys by owner (spl_route_keys) and all-to-all of the 16-byte KEYS only;
      the receive buffer, concatenated by source rank, is already in global arrival order
-  4. owner: first-arrival dedup against its slice of the visited set (spl_dedup)   (:447-450)
+  4. owner: first-arrival dedup against its slice of the visited set (spl_dedup_flags)   (:447-450)
   5. one winner byte per candidate travels back (reverse all-to-all); the SOURCE rank, which still
-     holds key/aux/link of its candidates in arrival order, compacts its winners -> the next
+     holds key/aux/link of its candidates in arrival order, compacts its winners (spl_compact_winners) -> the next
      queue is again block-distributed in global arrival order (pure BFS stops here)
-  6. beam: scores (spl_score); global radix select = the single-GPU passes with the 2048-bin
+  6. beam: scores (spl_score_rows); global radix select = the single-GPU passes with the 2048-bin
      histogram all-reduced between spl_dtopk_hist and spl_dtopk_pick; arrival-order tie quota
      split over ranks by an exclusive scan of local tie counts (stable) or key threshold (det)
   7. local cut + local rank sort (spl_dtopk_cut); global rank of every survivor = local index +
      counts against the other ranks' sorted sort-words (all-gather + spl_count_less); survivors
-     are sent to the rank that owns their global-rank block (all-to-all)          (:452-456)
+     are gathered (spl_move_rows) and sent to the rank that owns their global-rank block (all-to-all)  (:452-456)
 
 The compute primitives come from a `backend` object (CudaBackend below wraps the C ABI; RCudaBackend the realistic-mode
-calls that RShardedSolver runs the same levels with); the collectives go through torch.distributed (NCCL on GPUs, gloo
-in the CPU tests).
+calls spl_r*, with which RShardedSolver runs the same levels); the collectives go through torch.distributed (NCCL on
+GPUs, gloo in the CPU tests).
 """
 import ctypes as C
 
@@ -126,13 +126,58 @@ class Comm:
         return [o[:int(c)].to(t.device) for o, c in zip(outs, counts)]
 
 
-class _CutOps:
-    """The score-generic calls of the global beam cut (distributed radix select, local cut, global ranks): the same for
-    speedrun and realistic rows, since they see only scores and sort words."""
+class _Backend:
+    """What the speedrun and realistic backends share: the row layer of a key-sharded round (route keys, dedup flags,
+    compact winners, move rows) on rows of ROW_COLS and keys of KEY_COLS int64 columns through the entry points the
+    backend names, and the score-generic calls of the global beam cut (distributed radix select, local cut, global
+    ranks), which see only scores and sort words."""
+
+    ROW_COLS = KEY_COLS = None
+    ROUTE = DEDUP = COMPACT = MOVE = None  # C entry points (ctypes functions: class attributes, not bound methods)
+    _route_cfg = ()  # leading arguments of ROUTE after the context (the realistic config)
 
     def __init__(self, eng: Engine):
         self.eng = eng
         self.device = eng.tdev
+
+    # ---- row layer
+    def route_keys(self, cand, world):
+        """identity keys [m, KEY_COLS] of the candidates grouped by owner rank (arrival order inside a group) + per-owner
+        counts"""
+        m = cand.shape[0]
+        send = torch.empty((max(m, 1), self.KEY_COLS), dtype=torch.int64, device=self.device)
+        counts = (C.c_int64 * world)()
+        check(self.ROUTE(self.eng._h, *self._route_cfg, cand.data_ptr(), m, world, send.data_ptr(), counts, self.eng._stream()),
+              self.eng._h)
+        return send[:m], np.array(counts[:], dtype=np.int64)
+
+    def dedup_flags(self, keys):
+        """owner side: one winner byte per received key (first arrival of a never-seen state)"""
+        n = keys.shape[0]
+        flags = torch.empty(max(n, 1), dtype=torch.uint8, device=self.device)
+        check(self.DEDUP(self.eng._h, keys.data_ptr(), n, flags.data_ptr(), self.eng._stream()), self.eng._h)
+        return flags[:n]
+
+    def compact_winners(self, cand, flags_send_order):
+        """source side: the winning rows in arrival order"""
+        m = cand.shape[0]
+        out = torch.empty((max(m, 1), self.ROW_COLS), dtype=torch.int64, device=self.device)
+        k = C.c_int64()
+        check(self.COMPACT(self.eng._h, cand.data_ptr(), m, flags_send_order.data_ptr(), out.data_ptr(), C.byref(k),
+                           self.eng._stream()), self.eng._h)
+        return out[:k.value]
+
+    def scatter_into(self, dst, rows, pos):
+        """dst[pos[i]] = rows[i] (dst is an existing [n, ROW_COLS] int64 tensor)"""
+        check(self.MOVE(self.eng._h, rows.contiguous().data_ptr(), pos.contiguous().data_ptr(), pos.shape[0], dst.data_ptr(), 1,
+                        self.eng._stream()), self.eng._h)
+
+    def move_rows(self, rows, idx, n_out, scatter):
+        """gather (out[i] = rows[idx[i]]) or scatter (out[idx[i]] = rows[i])"""
+        out = torch.empty((max(n_out, 1), self.ROW_COLS), dtype=torch.int64, device=self.device)
+        check(self.MOVE(self.eng._h, rows.data_ptr(), idx.data_ptr(), idx.shape[0], out.data_ptr(), int(scatter),
+                        self.eng._stream()), self.eng._h)
+        return out[:n_out]
 
     # ---- distributed top-k passes
     def dtopk_begin(self, scores, keys):
@@ -182,8 +227,12 @@ class _CutOps:
                                  int(sorted_a), self.eng._stream()), self.eng._h)
 
 
-class CudaBackend(_CutOps):
-    """Compute primitives of one rank, all through the C ABI of libsplendor_b200.so."""
+class CudaBackend(_Backend):
+    """Compute primitives of one rank, all through the C ABI of libsplendor_b200.so: rows are the 32-byte speedrun records
+    {lo, hi, aux, link} as int64 [n, 4], keys the 128-bit (cards, gems) as int64 [n, 2]."""
+
+    ROW_COLS, KEY_COLS = 4, 2
+    ROUTE, DEDUP, COMPACT, MOVE = lib.spl_route_keys, lib.spl_dedup_flags, lib.spl_compact_winners, lib.spl_move_rows
 
     def reset_visited(self):
         self.eng.reset_visited()
@@ -204,7 +253,7 @@ class CudaBackend(_CutOps):
             out = torch.empty((cap, 4), dtype=torch.int64, device=self.device)
             m = C.c_int64()
             rc = lib.spl_expand_rows(self.eng._h, front.data_ptr(), n, rank_base, out.data_ptr(), cap, C.byref(m), self.eng._stream())
-            if rc == -6:
+            if rc == SPL_E_CAPACITY:
                 cap = m.value
                 continue
             check(rc, self.eng._h)
@@ -219,30 +268,6 @@ class CudaBackend(_CutOps):
             out[:m, 0] = self.eng.pyhash(cand[:, :2].contiguous())
         return out[:m]
 
-    def route_keys(self, cand, world):
-        """keys of the candidates grouped by owner rank (arrival order inside a group) + per-owner counts"""
-        m = cand.shape[0]
-        send = torch.empty((max(m, 1), 2), dtype=torch.int64, device=self.device)
-        counts = (C.c_int64 * world)()
-        check(lib.spl_route_keys(self.eng._h, cand.data_ptr(), m, world, send.data_ptr(), counts, self.eng._stream()), self.eng._h)
-        return send[:m], np.array(counts[:], dtype=np.int64)
-
-    def dedup_flags(self, keys):
-        """owner side: one winner byte per received key (first arrival of a never-seen key)"""
-        n = keys.shape[0]
-        flags = torch.empty(max(n, 1), dtype=torch.uint8, device=self.device)
-        check(lib.spl_dedup_flags(self.eng._h, keys.data_ptr(), n, flags.data_ptr(), self.eng._stream()), self.eng._h)
-        return flags[:n]
-
-    def compact_winners(self, cand, flags_send_order):
-        """source side: the winning rows in arrival order"""
-        m = cand.shape[0]
-        out = torch.empty((max(m, 1), 4), dtype=torch.int64, device=self.device)
-        k = C.c_int64()
-        check(lib.spl_compact_winners(self.eng._h, cand.data_ptr(), m, flags_send_order.data_ptr(), out.data_ptr(), C.byref(k),
-                                      self.eng._stream()), self.eng._h)
-        return out[:k.value]
-
     def owner_partition(self, keys, world):
         n = keys.shape[0]
         perm = torch.empty(max(n, 1), dtype=torch.int64, device=self.device)
@@ -251,29 +276,12 @@ class CudaBackend(_CutOps):
               self.eng._h)
         return perm[:n], np.array(counts[:], dtype=np.int64)
 
-    def dedup(self, keys):
-        aux = torch.zeros(keys.shape[0], dtype=torch.int64, device=self.device)
-        _, _, src = self.eng.dedup(keys.contiguous(), aux)
-        return src
-
     def score(self, heuristic, noise, rows, draws=None):
         n = rows.shape[0]
         out = torch.empty(n, dtype=torch.float64, device=self.device)
         check(lib.spl_score_rows(self.eng._h, heuristic_id(heuristic), NOISE_IDS[noise], rows.data_ptr(), n, out.data_ptr(),
                                  draws.data_ptr() if draws is not None else None, self.eng._stream()), self.eng._h)
         return out
-
-    def scatter_into(self, dst, rows, pos):
-        """dst[pos[i]] = rows[i] for 32-byte rows (dst is an existing [n, 4] int64 tensor)"""
-        check(lib.spl_move_rows(self.eng._h, rows.contiguous().data_ptr(), pos.contiguous().data_ptr(), pos.shape[0],
-                                dst.data_ptr(), 1, self.eng._stream()), self.eng._h)
-
-    def move_rows(self, rows, idx, n_out, scatter):
-        """gather (out[i] = rows[idx[i]]) or scatter (out[idx[i]] = rows[i]) of 32-byte rows"""
-        out = torch.empty((max(n_out, 1), 4), dtype=torch.int64, device=self.device)
-        check(lib.spl_move_rows(self.eng._h, rows.data_ptr(), idx.data_ptr(), idx.shape[0], out.data_ptr(), int(scatter),
-                                self.eng._stream()), self.eng._h)
-        return out[:n_out]
 
 
 class ShardedSolver(Stepper):
@@ -567,16 +575,20 @@ class ShardedSolver(Stepper):
         return out
 
 
-class RCudaBackend(_CutOps):
+class RCudaBackend(_Backend):
     """Compute primitives of one rank for realistic mode (MultiPlayerState, csrc/spl_realistic.cuh), with the method
     names of CudaBackend.  Rows are 96-byte records as int64 [n, 12]: players in columns 0-7, vis/cur in 8-9, link in
     10, spare in 11; keys are the 384-bit exact identity (spl_rpack) as int64 [n, 6].  Scores come from spl_rscore
     with the config's noise (`const` or `hash`); `root` is the record the search starts from (default: the config's
     new game)."""
 
+    ROW_COLS, KEY_COLS = 12, 6
+    ROUTE, DEDUP, COMPACT, MOVE = lib.spl_rroute_keys, lib.spl_rdedup_flags, lib.spl_rcompact_winners, lib.spl_rmove_rows
+
     def __init__(self, eng: Engine, rcfg, root=None):
         super().__init__(eng)
         self.rcfg = rcfg
+        self._route_cfg = (C.byref(rcfg),)
         self.noise = {v: k for k, v in NOISE_IDS.items()}[rcfg.noise]
         self.goal = rcfg.target_points
         self._fanout = 27.0  # successors per parent the next expand_rows allocates for
@@ -587,25 +599,22 @@ class RCudaBackend(_CutOps):
             root['link'] = (1 << 64) - 1
         self.root = np.ascontiguousarray(root).reshape(-1)[:1].copy()
 
-    def _call(self, rc):
-        check(rc, self.eng._h)
-
     def root_row(self):
         return torch.from_numpy(self.root.view(np.int64).reshape(1, 12).copy()).to(self.device)
 
     def reset_visited(self):
-        self._call(lib.spl_rreset_visited(self.eng._h, self.eng._stream()))
+        check(lib.spl_rreset_visited(self.eng._h, self.eng._stream()), self.eng._h)
 
     def visited_count(self):
         n = C.c_int64()
-        self._call(lib.spl_rvisited_count(self.eng._h, C.byref(n)))
+        check(lib.spl_rvisited_count(self.eng._h, C.byref(n)), self.eng._h)
         return n.value
 
     def first_goal(self, front, goal):
         """first queue index whose game is over (players[cur].pts >= the config's target), -1 if none"""
         r = C.c_int64()
-        self._call(lib.spl_rfirst_goal(self.eng._h, C.byref(self.rcfg), front.data_ptr(), front.shape[0], C.byref(r),
-                                       self.eng._stream()))
+        check(lib.spl_rfirst_goal(self.eng._h, C.byref(self.rcfg), front.data_ptr(), front.shape[0], C.byref(r),
+                                  self.eng._stream()), self.eng._h)
         return r.value
 
     def expand_rows(self, front, rank_base):
@@ -623,54 +632,17 @@ class RCudaBackend(_CutOps):
             if rc == SPL_E_CAPACITY:
                 cap = m.value
                 continue
-            self._call(rc)
+            check(rc, self.eng._h)
             if n:
                 self._fanout = min(27.0, 1.1 * m.value / n)
             return out[:m.value]
-
-    def route_keys(self, cand, world):
-        """identity keys [m, 6] of the candidates grouped by owner rank (arrival order inside a group) + per-owner counts"""
-        m = cand.shape[0]
-        send = torch.empty((max(m, 1), 6), dtype=torch.int64, device=self.device)
-        counts = (C.c_int64 * world)()
-        self._call(lib.spl_rroute_keys(self.eng._h, C.byref(self.rcfg), cand.data_ptr(), m, world, send.data_ptr(), counts,
-                                       self.eng._stream()))
-        return send[:m], np.array(counts[:], dtype=np.int64)
-
-    def dedup_flags(self, keys):
-        """owner side: one winner byte per received key (first arrival of a never-seen state)"""
-        n = keys.shape[0]
-        flags = torch.empty(max(n, 1), dtype=torch.uint8, device=self.device)
-        self._call(lib.spl_rdedup_flags(self.eng._h, keys.data_ptr(), n, flags.data_ptr(), self.eng._stream()))
-        return flags[:n]
-
-    def compact_winners(self, cand, flags_send_order):
-        """source side: the winning rows in arrival order"""
-        m = cand.shape[0]
-        out = torch.empty((max(m, 1), 12), dtype=torch.int64, device=self.device)
-        k = C.c_int64()
-        self._call(lib.spl_rcompact_winners(self.eng._h, cand.data_ptr(), m, flags_send_order.data_ptr(), out.data_ptr(),
-                                            C.byref(k), self.eng._stream()))
-        return out[:k.value]
 
     def score(self, heuristic, noise, rows, draws=None):
         """multi_competitive_heuristic of every row (the config's noise; `heuristic` is the reference's ignored name)"""
         n = rows.shape[0]
         out = torch.empty(n, dtype=torch.float64, device=self.device)
-        self._call(lib.spl_rscore(self.eng._h, C.byref(self.rcfg), rows.data_ptr(), n, out.data_ptr(), self.eng._stream()))
+        check(lib.spl_rscore(self.eng._h, C.byref(self.rcfg), rows.data_ptr(), n, out.data_ptr(), self.eng._stream()), self.eng._h)
         return out
-
-    def scatter_into(self, dst, rows, pos):
-        """dst[pos[i]] = rows[i] for 96-byte rows (dst is an existing [n, 12] int64 tensor)"""
-        self._call(lib.spl_rmove_rows(self.eng._h, rows.contiguous().data_ptr(), pos.contiguous().data_ptr(), pos.shape[0],
-                                      dst.data_ptr(), 1, self.eng._stream()))
-
-    def move_rows(self, rows, idx, n_out, scatter):
-        """gather (out[i] = rows[idx[i]]) or scatter (out[idx[i]] = rows[i]) of 96-byte rows"""
-        out = torch.empty((max(n_out, 1), 12), dtype=torch.int64, device=self.device)
-        self._call(lib.spl_rmove_rows(self.eng._h, rows.data_ptr(), idx.data_ptr(), idx.shape[0], out.data_ptr(), int(scatter),
-                                      self.eng._stream()))
-        return out[:n_out]
 
 
 class RShardedSolver(ShardedSolver):

@@ -1,5 +1,5 @@
-"""GPU tests (-m gpu) of realistic mode on the key-sharded driver: the spl_r* entry points of RCudaBackend against numpy
-and the CPU oracle on small hand-built inputs, RShardedSolver on one rank against oracle.RSolver level by level, and
+"""GPU tests (-m gpu) of realistic mode on the key-sharded driver: the spl_r* entry points of RCudaBackend (and, where the
+row layer is shared, the speedrun rows of CudaBackend) against numpy and the CPU oracle on small hand-built inputs, RShardedSolver on one rank against oracle.RSolver level by level, and
 MultiPlayerState.solve(shard=True) against the single-GPU search."""
 import ctypes as C
 
@@ -11,7 +11,7 @@ import oracle
 import splendor_rl_gym_b200 as S
 from splendor_rl_gym_b200._lib import SplendorB200Error, lib
 from splendor_rl_gym_b200.realistic import RConfig
-from splendor_rl_gym_b200.sharded import Comm, RCudaBackend, RShardedSolver
+from splendor_rl_gym_b200.sharded import Comm, CudaBackend, RCudaBackend, RShardedSolver
 
 pytestmark = pytest.mark.gpu
 
@@ -86,12 +86,55 @@ def test_rexpand_rows_links_with_rank_base(eng, sample):
     assert rc == -6 and m.value == len(got)
 
 
+@pytest.fixture(scope='module')
+def row_kinds(eng, sample):
+    """per row kind of the key-sharded driver: (backend factory, queues 0..9 of a beam search as device rows, identity keys
+    of device rows as host uint64 [n, KEY_COLS]).  The realistic queues are `sample`'s."""
+    cfg, _, lv, _, _ = sample
+    s = oracle.Solver(15, use_heuristic=True, heuristic_name='balanced', beam_width=2000)
+    for _ in range(9):
+        s.step()
+    slv = []
+    for i in range(10):
+        st, lk = s.level(i)
+        slv.append(torch.from_numpy(np.stack([st['lo'], st['hi'], st['aux'], lk], axis=1).view(np.int64).copy()).to(eng.tdev))
+    return {
+        'speedrun': (CudaBackend, slv, lambda rows: np.ascontiguousarray(rows[:, :2].cpu().numpy()).view(np.uint64)),
+        'realistic': (lambda e: RCudaBackend(e, cfg), [_rows(q, eng.tdev) for q in lv], lambda rows: eng.rpack(cfg, _recs(rows))),
+    }
+
+
+# The row-layer tests below check each row kind: speedrun rows through CudaBackend (spl_route_keys, spl_dedup_flags,
+# spl_compact_winners, spl_move_rows) and realistic rows through RCudaBackend (their spl_r* twins).
+ROW_KINDS = ('speedrun', 'realistic')
+
+
 @pytest.mark.parametrize('world', [1, 3, 8])
-def test_rroute_keys_groups_counts_stability(eng, sample, world):
-    cfg, _, _, _, dup = sample
-    be = RCudaBackend(eng, cfg)
-    send, counts = be.route_keys(_rows(dup, eng.tdev), world)
-    keys = eng.rpack(cfg, dup)
+def test_rroute_keys_groups_counts_stability(eng, row_kinds, world):
+    for kind in ROW_KINDS:
+        _route_keys_groups_counts_stability(eng, row_kinds, kind, world)
+
+
+def test_rdedup_flags_first_arrival_within_and_across_calls(eng, row_kinds):
+    for kind in ROW_KINDS:
+        _dedup_flags_first_arrival_within_and_across_calls(eng, row_kinds, kind)
+
+
+def test_rcompact_winners_order_and_state_error(eng, row_kinds):
+    for kind in ROW_KINDS:
+        _compact_winners_order_and_state_error(eng, row_kinds, kind)
+
+
+def test_rmove_rows_gather_scatter(eng, row_kinds):
+    for kind in ROW_KINDS:
+        _move_rows_gather_scatter(eng, row_kinds, kind)
+
+
+def _route_keys_groups_counts_stability(eng, row_kinds, kind, world):
+    make, lv, keys_of = row_kinds[kind]
+    dup = torch.cat([lv[7], lv[8][:50], lv[7]])  # each state of level 7 twice
+    send, counts = make(eng).route_keys(dup, world)
+    keys = keys_of(dup)
     send = send.cpu().numpy().view(np.uint64)
     assert counts.sum() == len(dup) and len(send) == len(dup)
     if world == 1:
@@ -115,11 +158,12 @@ def test_rroute_keys_groups_counts_stability(eng, sample, world):
         assert counts.min() > 0.5 * len(dup) / world
 
 
-def test_rdedup_flags_first_arrival_within_and_across_calls(eng, sample):
-    cfg, _, lv, _, dup = sample
-    be = RCudaBackend(eng, cfg)
+def _dedup_flags_first_arrival_within_and_across_calls(eng, row_kinds, kind):
+    make, lv, keys_of = row_kinds[kind]
+    be = make(eng)
     be.reset_visited()
-    keys = torch.from_numpy(eng.rpack(cfg, dup).view(np.int64).copy()).to(eng.tdev)
+    dup = torch.cat([lv[7], lv[8][:50], lv[7]])
+    keys = torch.from_numpy(keys_of(dup).view(np.int64).copy()).to(eng.tdev)
     f1 = be.dedup_flags(keys).cpu().numpy()
     seen, want = set(), []
     for k in keys.cpu().numpy():
@@ -128,8 +172,8 @@ def test_rdedup_flags_first_arrival_within_and_across_calls(eng, sample):
     assert (f1 == np.array(want)).all()
     assert be.visited_count() == len(seen)
     # second call: states of the first lose, new ones win on their first arrival
-    more = np.concatenate([lv[8][40:80], lv[9][:30], lv[9][:30]])
-    k2 = torch.from_numpy(eng.rpack(cfg, more).view(np.int64).copy()).to(eng.tdev)
+    more = torch.cat([lv[8][40:80], lv[9][:30], lv[9][:30]])
+    k2 = torch.from_numpy(keys_of(more).view(np.int64).copy()).to(eng.tdev)
     f2 = be.dedup_flags(k2).cpu().numpy()
     want2 = []
     for k in k2.cpu().numpy():
@@ -140,44 +184,52 @@ def test_rdedup_flags_first_arrival_within_and_across_calls(eng, sample):
     assert be.visited_count() == 0 and be.dedup_flags(keys).cpu().numpy().sum() == len(set(bytes(k) for k in keys.cpu().numpy()))
 
 
-def test_rcompact_winners_order_and_state_error(eng, sample):
-    cfg, _, _, distinct, _ = sample
-    be = RCudaBackend(eng, cfg)
-    cand = _rows(distinct, eng.tdev)
+def _compact_winners_order_and_state_error(eng, row_kinds, kind):
+    make, lv, keys_of = row_kinds[kind]
+    be = make(eng)
+    cand = torch.cat(lv[6:10])  # distinct states
     send, counts = be.route_keys(cand, 3)
-    keys = eng.rpack(cfg, distinct)
+    keys = keys_of(cand)
     where = {bytes(k): i for i, k in enumerate(keys)}
     src = np.array([where[bytes(k)] for k in send.cpu().numpy().view(np.uint64)])
     rng = np.random.default_rng(0)
-    flags = rng.integers(0, 2, len(distinct)).astype(np.uint8)
+    flags = rng.integers(0, 2, len(cand)).astype(np.uint8)
     got = be.compact_winners(cand, torch.from_numpy(flags).to(eng.tdev))
-    won = np.zeros(len(distinct), bool)
+    won = np.zeros(len(cand), bool)
     won[src[flags == 1]] = True
-    assert _recs(got).tobytes() == distinct[won].tobytes()
+    assert got.cpu().numpy().tobytes() == cand.cpu().numpy()[won].tobytes()
     with pytest.raises(SplendorB200Error) as e:  # not the candidates of the last route
         be.compact_winners(cand[:-1], torch.from_numpy(flags[:-1]).to(eng.tdev))
     assert e.value.code == -7
+    other_make, other_lv, _ = row_kinds[next(k for k in ROW_KINDS if k != kind)]
+    n = min(len(cand), len(torch.cat(other_lv[6:10])))
     fresh = S.Engine(0, table_slots=1 << 12)
     try:
         with pytest.raises(SplendorB200Error) as e:  # no route on this context yet
-            RCudaBackend(fresh, cfg).compact_winners(cand, torch.from_numpy(flags).to(eng.tdev))
+            make(fresh).compact_winners(cand, torch.from_numpy(flags).to(eng.tdev))
+        assert e.value.code == -7
+        # the other row kind's route on as many candidates is not a route of this kind
+        other_make(fresh).route_keys(torch.cat(other_lv[6:10])[:n], 3)
+        with pytest.raises(SplendorB200Error) as e:
+            make(fresh).compact_winners(cand[:n], torch.from_numpy(flags[:n]).to(eng.tdev))
         assert e.value.code == -7
     finally:
         fresh.close()
 
 
-def test_rmove_rows_gather_scatter(eng, sample):
-    cfg, _, _, distinct, _ = sample
-    be = RCudaBackend(eng, cfg)
-    rows = _rows(distinct, eng.tdev)
-    perm = torch.from_numpy(np.random.default_rng(1).permutation(len(distinct))).to(eng.tdev)
-    g = be.move_rows(rows, perm, len(distinct), False)
-    assert _recs(g).tobytes() == distinct[perm.cpu().numpy()].tobytes()
-    s = be.move_rows(g, perm, len(distinct), True)
-    assert _recs(s).tobytes() == distinct.tobytes()
+def _move_rows_gather_scatter(eng, row_kinds, kind):
+    make, lv, _ = row_kinds[kind]
+    be = make(eng)
+    rows = torch.cat(lv[6:10])
+    host = rows.cpu().numpy()
+    perm = torch.from_numpy(np.random.default_rng(1).permutation(len(rows))).to(eng.tdev)
+    g = be.move_rows(rows, perm, len(rows), False)
+    assert g.cpu().numpy().tobytes() == host[perm.cpu().numpy()].tobytes()
+    s = be.move_rows(g, perm, len(rows), True)
+    assert s.cpu().numpy().tobytes() == host.tobytes()
     dst = torch.zeros_like(rows)
     be.scatter_into(dst, g, perm)
-    assert _recs(dst).tobytes() == distinct.tobytes()
+    assert dst.cpu().numpy().tobytes() == host.tobytes()
 
 
 def test_rfirst_goal_vs_oracle_pts(eng, golden):
