@@ -37,7 +37,7 @@ struct GroupArgs;
 constexpr int NUM_CLS = 8;             // run classes; used: CLS_WARP (one warp per run), CLS_CTA (one CTA per run)
 constexpr int CLS_WARP = 6, CLS_CTA = 7;
 constexpr int M2_WARPS = TILE / 32;
-constexpr int BIG_DONE = 16;           // distinct card sets one equal-hash run of the CTA kernel may hold
+constexpr int BIG_DONE = 16;           // card sets of a run the CTA kernel remembers as done: it walks at most BIG_DONE + 1 per run
 constexpr int BIG_AT_BITS = 24;        // item offset inside a run, packed under the arrival index in the CTA kernel's table
 
 // card mask of a key as two words (90 bits)
@@ -743,7 +743,7 @@ __device__ __forceinline__ void warp_epilogue(const GroupArgs &A, WarpStage &W, 
 #define SPL_WARP_BATCH 8  // measured per beam-30M solve: 1: 290, 2: 267, 4: 257, 8: 254, 16: 268, 32: 262, 64: 276 ms
 #endif
 constexpr int WARP_BATCH = SPL_WARP_BATCH; // runs a warp of the warp kernel draws per ticket
-constexpr int MAX_SETS = 4;  // card sets under one sort key that the thread / warp kernels can tell apart
+constexpr int MAX_SETS = 4;  // card sets of a run the warp kernel remembers as done: it walks at most MAX_SETS + 1 per run
 constexpr int BSORT_MAX = 512;  // buy records of one run the warp kernel can put into arrival order itself
 struct WarpSmem {
     SmemTabs tabs;
@@ -1118,7 +1118,7 @@ __global__ void __launch_bounds__(TILE) m2_group_big_kernel(GroupArgs A) {
             __syncthreads();
             // pass 0: first arrival per gem hand among the candidates not in the visited set; the table word is
             // arrival index << 24 | offset of the producing item in the run (a run holds < 2^24 items: at most
-            // BIG_DONE card sets of <= 2898 parents and their predecessors' buy records; arrival indices are < 2^40)
+            // BIG_DONE + 1 card sets of <= 2898 parents and their predecessors' buy records; arrival indices are < 2^40)
             big_enumerate(A, S, s, e, M0, M1, [&](uint32_t rk, uint64_t t, uint32_t at) {
                 if (!((S.bm[rk >> 6] >> (rk & 63)) & 1))
                     atomicMin(reinterpret_cast<unsigned long long *>(&S.tbl[rk]), (unsigned long long)((t << BIG_AT_BITS) | at));

@@ -1433,7 +1433,7 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
                 (unsigned long long)c->nn);
     if (h.error == 3)
         return fail(c, SPL_E_CUDA, "level %d: more than %d card sets share one 30-bit sort key in a run of the warp kernel (or more than %d in one of the CTA kernel)",
-                    R.level, MAX_SETS, BIG_DONE);
+                    R.level, MAX_SETS + 1, BIG_DONE + 1);
     if (h.error)
         return fail(c, SPL_E_TABLE_FULL, "card-set table full during level %d (device error %u; %llu slots, max_node_bytes=%llu)", R.level,
                     h.error, (unsigned long long)c->nn, (unsigned long long)c->max_node_bytes);
