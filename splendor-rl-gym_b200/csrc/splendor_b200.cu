@@ -57,18 +57,87 @@ struct DevBuf {
     void swap(DevBuf &o) { std::swap(p, o.p); std::swap(cap, o.cap); }
 };
 
+static inline unsigned nblk(int64_t n, int per = TILE) { return (unsigned)((n + per - 1) / per); }
+
+// The key table is sized in slots (3 per 64-byte bucket); slot ids are u32 (bucket << 2 | slot), so at most 2^30 buckets.
+constexpr uint64_t MAX_BUCKETS = 1ull << 30;
+static uint64_t buckets_for(uint64_t slots) {
+    return std::min<uint64_t>(std::max<uint64_t>(slots / BUCKET_SLOTS, 16), MAX_BUCKETS);
+}
+
+// What differs between the three visited tables: their unit, how full they may get, and their rehash kernel.
+struct TableDesc {
+    uint64_t unit_bytes, unit_slots, max_units;  // a unit (bucket or card-set node): its bytes and its entry slots
+    double load;                                 // grow while entries + need > load * slots ...
+    uint64_t full_div;                           // ... and fail if then entries + need / full_div > slots - slots / 16
+    void (*rehash)(const void *from, uint64_t units, void *to, uint64_t to_units, Counters *ctr, cudaStream_t st);
+    const char *rehash_msg;                      // %llu: the new number of units
+    const char *full_msg;                        // %llu x 4: entries, need, slots, byte ceiling
+};
+static const TableDesc KEY_TABLE_DESC = {
+    64, BUCKET_SLOTS, MAX_BUCKETS, 0.7, 8,
+    [](const void *from, uint64_t units, void *to, uint64_t to_units, Counters *ctr, cudaStream_t st) {
+        rehash_kernel<<<nblk((int64_t)(units * BUCKET_SLOTS)), TILE, 0, st>>>(static_cast<const uint64_t *>(from), units,
+                                                                              static_cast<uint64_t *>(to), to_units, ctr);
+    },
+    "rehash into %llu buckets overflowed a probe sequence",
+    "visited table full: %llu occupied + %llu candidates vs %llu slots (max_table_bytes=%llu)"};
+static const TableDesc NODE_TABLE_DESC = {
+    NODE_WORDS * 8, 1, ~0ull, 0.6, 1,
+    [](const void *from, uint64_t units, void *to, uint64_t to_units, Counters *ctr, cudaStream_t st) {
+        m2_rehash_kernel<<<nblk((int64_t)units * 32), TILE, 0, st>>>(static_cast<const uint64_t *>(from), units,
+                                                                      static_cast<uint64_t *>(to), to_units, ctr);
+    },
+    "node rehash into %llu slots overflowed a probe sequence",
+    "card-set table full: %llu nodes + %llu new vs %llu slots (max_node_bytes=%llu)"};
+static const TableDesc REALISTIC_TABLE_DESC = {
+    64, 1, ~0ull, 0.6, 4,
+    [](const void *from, uint64_t units, void *to, uint64_t to_units, Counters *ctr, cudaStream_t st) {
+        r_rehash_kernel<<<nblk((int64_t)units), TILE, 0, st>>>(static_cast<const RBucket *>(from), units,
+                                                                static_cast<RBucket *>(to), to_units, ctr);
+    },
+    "realistic table rehash into %llu buckets overflowed a probe sequence",
+    "realistic visited table full: %llu states + %llu candidates vs %llu buckets (max_table_bytes=%llu)"};
+
+// A visited set on the device: an open-addressing table that grows by rehashing into one twice its size.  It counts
+// its own entries, those of an insert that failed part way included, so that clear() can skip a table that holds none.
+struct VisitTable {
+    const TableDesc &d;
+    void *p = nullptr;
+    uint64_t units = 0, max_bytes = 0, occ = 0;
+    explicit VisitTable(const TableDesc &desc) : d(desc) {}
+    ~VisitTable() { if (p) cudaFree(p); }
+    template <class T> T *as() const { return static_cast<T *>(p); }
+    uint64_t slots() const { return units * d.unit_slots; }
+    // a new, empty table of n units in place of the old one
+    cudaError_t alloc(uint64_t n, cudaStream_t st) {
+        if (p) cudaFree(p);
+        p = nullptr;
+        units = occ = 0;
+        cudaError_t e = cudaMalloc(&p, n * d.unit_bytes);
+        if (e != cudaSuccess) p = nullptr;
+        else e = cudaMemsetAsync(p, 0, n * d.unit_bytes, st);
+        if (e == cudaSuccess) units = n;
+        return e;
+    }
+    cudaError_t clear(cudaStream_t st) {
+        const cudaError_t e = occ ? cudaMemsetAsync(p, 0, units * d.unit_bytes, st) : cudaSuccess;
+        if (e == cudaSuccess) occ = 0;
+        return e;
+    }
+    int grow(spl_ctx *c, uint64_t need, cudaStream_t st);  // room for `need` more entries (if memory allows)
+};
+
 struct spl_ctx {
     int device = 0;
     std::string err;
-    // visited table
-    uint64_t *table = nullptr;
-    uint64_t cap = 0 /* slots = 3 * nb */, nb = 0 /* 64-byte buckets */, max_table_bytes = 0, occupied = 0;
+    // visited sets: the key table (BFS, the reference's hash identity, externally drawn noise and the stage operators),
+    // the card-set node table of the grouped level (spl_m2.cuh) and the realistic level's table (allocated on first use)
+    VisitTable key{KEY_TABLE_DESC}, nodes{NODE_TABLE_DESC}, rtab{REALISTIC_TABLE_DESC};
+    uint64_t occupied = 0;  // visited states: those of the last solve, plus what stage operators added to the key table
     uint32_t epoch = 0;
     uint64_t chunk_parents = 0;
     bool chunk_user = false;  // chunk_parents was set by the caller (spl_config), not the default
-    // card-set node table of the grouped level (spl_m2.cuh)
-    uint64_t *nodes = nullptr;
-    uint64_t nn = 0, node_occ = 0, max_node_bytes = 0;
     uint64_t link_budget = 0;          // device bytes a solver may hold in parent-link columns before it spills (0: no limit)
     uint64_t spilled_bytes = 0;        // link-column bytes moved to pinned host memory so far
     uint16_t *d_gemrank = nullptr;
@@ -97,8 +166,7 @@ struct spl_ctx {
     int64_t rroute_n = -1;     // candidates of the last spl_rroute_keys (its permutation lives in rperm)
     spl_rconfig rcfg_host{};   // what c->rcfg holds (valid when rcfg_have)
     bool rcfg_have = false;
-    RBucket *rtable = nullptr;  // realistic mode: exact-key visited table (64-byte buckets, one state each)
-    uint64_t rnb = 0, rocc = 0, rslots_hint = 0;
+    uint64_t rslots_hint = 0;  // spl_config.table_slots: the first size of the realistic table, in buckets
     std::vector<DevBuf *> pool_links;  // link columns of finished solves, reused by the next one
     cudaEvent_t ev[8]{};
     long long launches = 0, h2d_bytes = 0, d2h_bytes = 0;
@@ -146,7 +214,6 @@ static inline cudaError_t enter_device(spl_ctx *c) {
     if (e == cudaSuccess) cudaGetLastError();
     return e;
 }
-static inline unsigned nblk(int64_t n, int per = TILE) { return (unsigned)((n + per - 1) / per); }
 static inline int bitlen(uint64_t x) { return x ? 64 - __builtin_clzll(x) : 0; }
 
 extern "C" {
@@ -190,20 +257,6 @@ int32_t spl_host_buys(const uint8_t key[5], uint8_t out[90]) {
 }
 
 // ------------------------------------------------------------------ context
-// The table is sized in slots (3 per 64-byte bucket); slot ids are u32 (bucket << 2 | slot), so at most 2^30 buckets.
-constexpr uint64_t MAX_BUCKETS = 1ull << 30;
-static uint64_t buckets_for(uint64_t slots) {
-    return std::min<uint64_t>(std::max<uint64_t>(slots / BUCKET_SLOTS, 16), MAX_BUCKETS);
-}
-static int alloc_table(spl_ctx *c, uint64_t slots, cudaStream_t st) {
-    const uint64_t nb = buckets_for(slots);
-    CK(c, cudaMalloc(&c->table, nb * 64));
-    CK(c, cudaMemsetAsync(c->table, 0, nb * 64, st));
-    c->nb = nb;
-    c->cap = nb * BUCKET_SLOTS;
-    return SPL_OK;
-}
-
 int32_t spl_create(const spl_config *cfg, spl_ctx **out) {
     if (!cfg || !out) return fail(nullptr, SPL_E_INVALID, "spl_create: null argument");
     int ndev = 0;
@@ -234,7 +287,7 @@ int32_t spl_create(const spl_config *cfg, spl_ctx **out) {
     CKC(cudaSetDevice(c->device));
     size_t free_b = 0, total_b = 0;
     CKC(cudaMemGetInfo(&free_b, &total_b));
-    c->max_table_bytes = cfg->max_table_bytes ? cfg->max_table_bytes : (uint64_t)(free_b * 0.6);
+    c->key.max_bytes = c->rtab.max_bytes = cfg->max_table_bytes ? cfg->max_table_bytes : (uint64_t)(free_b * 0.6);
     c->chunk_user = cfg->chunk_parents != 0;
     c->chunk_parents = cfg->chunk_parents ? std::min<uint64_t>(cfg->chunk_parents, 16ull << 20) : (4ull << 20);
     c->chunk_parents = std::max<uint64_t>(c->chunk_parents, TILE);
@@ -284,22 +337,16 @@ int32_t spl_create(const spl_config *cfg, spl_ctx **out) {
     CKC(cudaMalloc(&c->d_dict2, sizeof(ScoreDict)));
     CKC(cudaMalloc(&c->d_dest, 3 * MAX_RANKS * 8));
     {
-        c->max_node_bytes = cfg->max_node_bytes ? cfg->max_node_bytes : (uint64_t)(free_b * 0.5);
+        c->nodes.max_bytes = cfg->max_node_bytes ? cfg->max_node_bytes : (uint64_t)(free_b * 0.5);
         uint64_t nn = cfg->node_slots ? cfg->node_slots : (1ull << 12);
-        nn = std::max<uint64_t>(std::min<uint64_t>(nn, c->max_node_bytes / (NODE_WORDS * 8)), 64);
-        CKC(cudaMalloc(&c->nodes, nn * NODE_WORDS * 8));
-        CKC(cudaMemset(c->nodes, 0, nn * NODE_WORDS * 8));
-        c->nn = nn;
+        nn = std::max<uint64_t>(std::min<uint64_t>(nn, c->nodes.max_bytes / (NODE_WORDS * 8)), 64);
+        CKC(c->nodes.alloc(nn, 0));
     }
     c->rslots_hint = cfg->table_slots;
     uint64_t slots = cfg->table_slots ? cfg->table_slots : (1ull << 22);
-    slots = std::min<uint64_t>(slots, c->max_table_bytes / 64 * BUCKET_SLOTS);
+    slots = std::min<uint64_t>(slots, c->key.max_bytes / 64 * BUCKET_SLOTS);
     slots = std::max<uint64_t>(slots, 1024);
-    if (alloc_table(c, slots, 0) != SPL_OK) {
-        g_create_error = c->err;
-        delete c;
-        return SPL_E_NOMEM;
-    }
+    CKC(c->key.alloc(buckets_for(slots), 0));
     CKC(cudaDeviceSynchronize());
 #undef CKC
     *out = c;
@@ -310,9 +357,9 @@ int32_t spl_destroy(spl_ctx *c) {
     if (!c) return SPL_OK;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    cudaFree(c->table); cudaFree(c->d_tabs); cudaFree(c->d_takes_idx); cudaFree(c->d_takes_edges);
+    cudaFree(c->d_tabs); cudaFree(c->d_takes_idx); cudaFree(c->d_takes_edges);
     cudaFree(c->d_lut); cudaFree(c->d_ctr); cudaFreeHost(c->h_ctr); cudaFree(c->d_sel); cudaFreeHost(c->h_sel);
-    cudaFree(c->rtable); cudaFree(c->d_hist); cudaFree(c->d_dict); cudaFree(c->d_dict2); cudaFree(c->d_dest); cudaFree(c->nodes); cudaFree(c->d_gemrank); cudaFree(c->d_rankgems);
+    cudaFree(c->d_hist); cudaFree(c->d_dict); cudaFree(c->d_dict2); cudaFree(c->d_dest); cudaFree(c->d_gemrank); cudaFree(c->d_rankgems);
     for (auto *b : c->pool_links) delete b;
     for (auto &ev : c->ev) if (ev) cudaEventDestroy(ev);
     delete c;
@@ -321,10 +368,9 @@ int32_t spl_destroy(spl_ctx *c) {
 
 static int reset_visited(spl_ctx *c, cudaStream_t st) {
     CK(c, enter_device(c));
-    CK(c, cudaMemsetAsync(c->table, 0, c->nb * 64, st));
-    if (c->node_occ) CK(c, cudaMemsetAsync(c->nodes, 0, c->nn * NODE_WORDS * 8, st));
+    CK(c, c->key.clear(st));
+    CK(c, c->nodes.clear(st));
     c->occupied = 0;
-    c->node_occ = 0;
     c->epoch = 0;
     return SPL_OK;
 }
@@ -414,17 +460,17 @@ static int prep_status(spl_ctx *c, int which, size_t ntiles, cudaStream_t st) {
     return SPL_OK;
 }
 
-// grow the visited table so that `need` more inserts keep the load factor <= 0.7 (if memory allows)
-static int ensure_table(spl_ctx *c, uint64_t need, cudaStream_t st) {
-    while ((double)(c->occupied + need) > 0.7 * (double)c->cap) {
-        uint64_t nnb = std::min<uint64_t>(c->nb * 2, MAX_BUCKETS);
-        if (nnb * 64 > c->max_table_bytes) nnb = c->max_table_bytes / 64;
-        if (nnb <= c->nb + c->nb / 8) break;  // cannot grow meaningfully
-        uint64_t *nt = nullptr;
-        cudaError_t e = cudaMalloc(&nt, nnb * 64);
+// grow so that `need` more entries keep the load factor (if memory allows)
+int VisitTable::grow(spl_ctx *c, uint64_t need, cudaStream_t st) {
+    while ((double)(occ + need) > d.load * (double)slots()) {
+        uint64_t nu = std::min<uint64_t>(units * 2, d.max_units);
+        if (nu * d.unit_bytes > max_bytes) nu = max_bytes / d.unit_bytes;
+        if (nu <= units + units / 8) break;  // cannot grow meaningfully
+        void *nt = nullptr;
+        cudaError_t e = cudaMalloc(&nt, nu * d.unit_bytes);
         if (e != cudaSuccess) { cudaGetLastError(); break; }
-        CK(c, cudaMemsetAsync(nt, 0, nnb * 64, st));
-        rehash_kernel<<<nblk((int64_t)c->cap), TILE, 0, st>>>(c->table, c->nb, nt, nnb, c->d_ctr);
+        CK(c, cudaMemsetAsync(nt, 0, nu * d.unit_bytes, st));
+        d.rehash(p, units, nt, nu, c->d_ctr, st);
         ++c->launches;
         CK(c, cudaGetLastError());
         unsigned int rehash_err = 0;  // read the flag now: callers zero the counters before their own launches
@@ -432,17 +478,15 @@ static int ensure_table(spl_ctx *c, uint64_t need, cudaStream_t st) {
         CK(c, cudaStreamSynchronize(st));
         if (rehash_err) {
             cudaFree(nt);
-            return fail(c, SPL_E_TABLE_FULL, "rehash into %llu buckets overflowed a probe sequence", (unsigned long long)nnb);
+            return fail(c, SPL_E_TABLE_FULL, d.rehash_msg, (unsigned long long)nu);
         }
-        cudaFree(c->table);
-        c->table = nt;
-        c->nb = nnb;
-        c->cap = nnb * BUCKET_SLOTS;
+        cudaFree(p);
+        p = nt;
+        units = nu;
     }
-    if (c->occupied + need / 8 > c->cap - c->cap / 16)
-        return fail(c, SPL_E_TABLE_FULL, "visited table full: %llu occupied + %llu candidates vs %llu slots (max_table_bytes=%llu)",
-                    (unsigned long long)c->occupied, (unsigned long long)need, (unsigned long long)c->cap,
-                    (unsigned long long)c->max_table_bytes);
+    if (occ + need / d.full_div > slots() - slots() / 16)
+        return fail(c, SPL_E_TABLE_FULL, d.full_msg, (unsigned long long)occ, (unsigned long long)need,
+                    (unsigned long long)slots(), (unsigned long long)max_bytes);
     return SPL_OK;
 }
 
@@ -803,14 +847,15 @@ int32_t spl_dedup(spl_ctx *c, const spl_key *ck, const uint64_t *ca, int64_t n, 
     *n_out = 0;
     if (n == 0) return SPL_OK;
     CKS(c, zero_ctr(c, st));
-    CKS(c, ensure_table(c, (uint64_t)n, st));
+    CKS(c, c->key.grow(c, (uint64_t)n, st));
     uint64_t tag;
     CKS(c, next_epoch(c, tag));
     CK(c, c->cand_slot.ensure((size_t)n * 4, 0, st));
-    probe_list_kernel<IDENT_KEY><<<nblk(n), TILE, 0, st>>>(ck, n, c->table, c->nb, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
+    probe_list_kernel<IDENT_KEY><<<nblk(n), TILE, 0, st>>>(ck, n, c->key.as<uint64_t>(), c->key.units, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
     ++c->launches;
     CK(c, cudaGetLastError());
     CKS(c, read_ctr(c, st));
+    c->key.occ += c->h_ctr->n_new;  // before the error check: a reset clears a partial insert too
     if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "spl_dedup: probe overflow (table full)");
     const int64_t n_new = (int64_t)c->h_ctr->n_new;
     c->occupied += n_new;
@@ -821,7 +866,7 @@ int32_t spl_dedup(spl_ctx *c, const spl_key *ck, const uint64_t *ca, int64_t n, 
     CKS(c, prep_status(c, 0, nt, st));
     CKS(c, reset_ticket(c, 0, st));
     resolve_kernel<SRC_LIST, false><<<nt, TILE, sizeof(ResolveSmem), st>>>(
-        nullptr, 0, c->d_tabs, c->d_takes_idx, c->d_takes_edges, nullptr, (uint32_t)n, c->table,
+        nullptr, 0, c->d_tabs, c->d_takes_idx, c->d_takes_edges, nullptr, (uint32_t)n, c->key.as<uint64_t>(),
         c->cand_slot.as<uint32_t>(), ck, ca, 0, 0, c->tmp_rec.as<Rec>(), nullptr, usrc, 0, 0, c->luts,
         c->status[0].as<uint64_t>(), c->d_ctr, 0);
     unpack_rec_kernel<<<nblk(n_new), TILE, 0, st>>>(c->tmp_rec.as<Rec>(), n_new, uk, ua, nullptr);
@@ -1238,10 +1283,19 @@ static int save_links(SolverBufs *s, int64_t n, bool realistic, bool with_ranks,
     return SPL_OK;
 }
 
+// The formulation of a solver's levels (DESIGN.md 3), and with it its visited table.
+enum LevelKind {
+    KEY_TABLE,  // expand + dedup against the key table, in chunks of parents
+    GROUPED,    // beam search on the card-set-grouped level (spl_m2.cuh), visited set in the node table
+    REALISTIC,  // realistic mode: materialised 96-byte successors, exact-key table
+};
+static const VisitTable &visited_table(const spl_ctx *c, LevelKind kind) {
+    return kind == KEY_TABLE ? c->key : kind == GROUPED ? c->nodes : c->rtab;
+}
+
 struct spl_solver : SolverBufs {
     int goal = 15, use_h = 0, heuristic = 0, tie = 0, noise = 0;
-    bool realistic = false;
-    bool grouped = false;  // beam search on the card-set-grouped level (spl_m2.cuh); otherwise the key-table level
+    LevelKind kind = KEY_TABLE;
     spl_rconfig rcfg{};
     // external-noise mode: the level is split in two calls (expand+dedup | score+cut)
     bool pending = false;
@@ -1255,45 +1309,14 @@ struct spl_solver : SolverBufs {
     explicit spl_solver(spl_ctx *ctx) : SolverBufs(ctx) {}
 };
 
+// What the expand + dedup half of a level leaves for the cut: n_uniq states in the first n_slots elements of s->uniq
+// (n_slots > n_uniq: the grouped level leaves unused slots) and, where scores were computed on the way, their range.
+struct LevelExpand {
+    int64_t n_uniq = 0, n_slots = 0, generated = 0;
+    uint64_t sk_min = ~0ull, sk_max = 0;
+};
+
 // ------------------------------------------------------------------ card-set-grouped level (spl_m2.cuh)
-// grow the node table so that `need` more card sets keep its load factor <= 0.6 (if memory allows)
-static int ensure_nodes(spl_ctx *c, uint64_t need, cudaStream_t st) {
-    while ((double)(c->node_occ + need) > 0.6 * (double)c->nn) {
-        uint64_t nnn = c->nn * 2;
-        if (nnn * NODE_WORDS * 8 > c->max_node_bytes) nnn = c->max_node_bytes / (NODE_WORDS * 8);
-        if (nnn <= c->nn + c->nn / 8) break;
-        uint64_t *nt = nullptr;
-        cudaError_t e = cudaMalloc(&nt, nnn * NODE_WORDS * 8);
-        if (e != cudaSuccess) { cudaGetLastError(); break; }
-        CK(c, cudaMemsetAsync(nt, 0, nnn * NODE_WORDS * 8, st));
-        m2_rehash_kernel<<<nblk((int64_t)c->nn * 32), TILE, 0, st>>>(c->nodes, c->nn, nt, nnn, c->d_ctr);
-        ++c->launches;
-        CK(c, cudaGetLastError());
-        unsigned int err = 0;
-        CK(c, cudaMemcpyAsync(&err, &c->d_ctr->error, 4, cudaMemcpyDeviceToHost, st));
-        CK(c, cudaStreamSynchronize(st));
-        if (err) { cudaFree(nt); return fail(c, SPL_E_TABLE_FULL, "node rehash into %llu slots overflowed a probe sequence", (unsigned long long)nnn); }
-        cudaFree(c->nodes);
-        c->nodes = nt;
-        c->nn = nnn;
-    }
-    if (c->node_occ + need > c->nn - c->nn / 16)
-        return fail(c, SPL_E_TABLE_FULL, "card-set table full: %llu nodes + %llu new vs %llu slots (max_node_bytes=%llu)",
-                    (unsigned long long)c->node_occ, (unsigned long long)need, (unsigned long long)c->nn,
-                    (unsigned long long)c->max_node_bytes);
-    return SPL_OK;
-}
-
-// the root's card set into the node table (the grouped level's visited set), with the counters zeroed
-static int add_grouped_root(spl_ctx *c, uint64_t lo, uint64_t hi, cudaStream_t st) {
-    m2_root_kernel<<<1, 1, 0, st>>>(c->nodes, c->nn, lo, hi, c->d_gemrank, c->d_ctr);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    c->node_occ = 1;
-    c->occupied = 1;
-    return SPL_OK;
-}
-
 // One-sweep stable LSD sort (spl_m2.cuh 2b) of k[*cur][0..n) by bits lo_bit .. lo_bit + nbits - 1, ping-ponging between
 // k[0] / k[1]; with a payload column (pl != nullptr) the pairs move together.  n < OS_MAX_ITEMS.
 static int onesweep_sort(spl_ctx *c, uint64_t *const k[2], uint32_t *const pl[2], int64_t n, int lo_bit, int nbits, int *cur, cudaStream_t st) {
@@ -1390,7 +1413,7 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
     CKS(c, read_ctr(c, st));
     const uint64_t n_runs = c->h_ctr->n_runs;
     // every run holds at least one card set; more than one only when two sets share the 30 sorted hash bits
-    CKS(c, ensure_nodes(c, n_runs + n_runs / 8 + 64, st));
+    CKS(c, c->nodes.grow(c, n_runs + n_runs / 8 + 64, st));
     CK(c, c->cls_list.ensure((size_t)n_runs * 8 + 16, 0, st));
     const size_t n_out = (size_t)R.out_base + (size_t)R.n_cands;
     CK(c, R.out->ensure(n_out * 32, (size_t)R.out_base * 32, st));
@@ -1401,7 +1424,7 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
     A.np = (uint32_t)R.np; A.rank_base = R.rank_base; A.grank = R.grank; A.unordered = R.unordered;
     A.warp_max = R.unordered ? std::min<uint32_t>(BIG_W, BSORT_MAX) : BIG_W;  // the warp kernel sorts at most BSORT_MAX records of a run itself
     A.tabs = c->d_tabs; A.takes_idx = c->d_takes_idx; A.takes_edges = c->d_takes_edges; A.gemrank = c->d_gemrank; A.rankgems = c->d_rankgems;
-    A.nodes = c->nodes; A.nn = c->nn; A.out = R.out->as<Rec>(); A.out_sk = c->sk.as<uint64_t>(); A.out_base = (uint64_t)R.out_base;
+    A.nodes = c->nodes.as<uint64_t>(); A.nn = c->nodes.units; A.out = R.out->as<Rec>(); A.out_sk = c->sk.as<uint64_t>(); A.out_base = (uint64_t)R.out_base;
     for (int k = 0; k < NUM_CLS; ++k) A.cls_list[k] = nullptr;
     A.cls_list[CLS_WARP] = c->cls_list.as<uint32_t>();
     A.cls_list[CLS_CTA] = c->cls_list.as<uint32_t>() + n_runs;
@@ -1429,15 +1452,15 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
         fprintf(stderr, "[grouped] L%d np=%lld items=%lld runs=%llu cls=%u/%u/%u new_nodes=%u winners=%llu | sort+runs %.2f prep %.2f thread %.2f warp %.2f cta %.2f ms | nodes %llu/%llu\n",
                 R.level, (long long)R.np, (long long)R.n_items, (unsigned long long)n_runs,
                 (unsigned)(n_runs - h.n_cls[CLS_WARP] - h.n_cls[CLS_CTA]), h.n_cls[CLS_WARP], h.n_cls[CLS_CTA], h.n_new_nodes,
-                (unsigned long long)h.n_emitted, t->sort, t->prep, t->thread, t->warp, t->cta, (unsigned long long)c->node_occ,
-                (unsigned long long)c->nn);
+                (unsigned long long)h.n_emitted, t->sort, t->prep, t->thread, t->warp, t->cta, (unsigned long long)c->nodes.occ,
+                (unsigned long long)c->nodes.units);
+    c->nodes.occ += h.n_new_nodes;  // before the error checks: a reset clears a partial insert too
     if (h.error == 3)
         return fail(c, SPL_E_CUDA, "level %d: more than %d card sets share one 30-bit sort key in a run of the warp kernel (or more than %d in one of the CTA kernel)",
                     R.level, MAX_SETS + 1, BIG_DONE + 1);
     if (h.error)
         return fail(c, SPL_E_TABLE_FULL, "card-set table full during level %d (device error %u; %llu slots, max_node_bytes=%llu)", R.level,
-                    h.error, (unsigned long long)c->nn, (unsigned long long)c->max_node_bytes);
-    c->node_occ += h.n_new_nodes;
+                    h.error, (unsigned long long)c->nodes.units, (unsigned long long)c->nodes.max_bytes);
     c->occupied += h.n_emitted;
     *n_new_out = (int64_t)h.n_emitted;
     return SPL_OK;
@@ -1445,9 +1468,9 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
 
 // expand + dedup (+ score) of the whole queue `front[0..n)` in rounds of parents; winners are appended to
 // s->uniq / c->sk in no particular order (their link words carry the arrival order)
-static int grouped_expand(spl_solver *s, const Rec *front, int64_t n, int64_t *n_uniq_out, int64_t *n_slots_out, int64_t *generated_out,
-                          uint64_t *sk_min_out, uint64_t *sk_max_out, float ms[6], cudaStream_t st) {
+static int grouped_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6], cudaStream_t st) {
     spl_ctx *c = s->c;
+    const Rec *front = s->front.as<Rec>();
     const int64_t chunk = c->chunk_user ? (int64_t)c->chunk_parents : (16ll << 20);
     int64_t n_uniq = 0, n_slots = 0, generated = 0;
     uint64_t sk_min = ~0ull, sk_max = 0;
@@ -1499,11 +1522,79 @@ static int grouped_expand(spl_solver *s, const Rec *front, int64_t n, int64_t *n
         ms[1] += t.thread + t.warp + t.cta;      // per-run dedup + emit + score (the dominant stage)
         ms[5] += t.warp;                         // ... of which the warp kernel
     }
-    *n_uniq_out = n_uniq;
-    *n_slots_out = n_slots;
-    *generated_out = generated;
-    *sk_min_out = sk_min;
-    *sk_max_out = sk_max;
+    *x = LevelExpand{n_uniq, n_slots, generated, sk_min, sk_max};
+    return SPL_OK;
+}
+
+// ------------------------------------------------------------------ solver create
+// The realistic table is allocated on first use, sized by the caller's table_slots.  A realistic search does not use
+// the key table: a large, empty one gives its memory back first.
+static int open_rtable(spl_ctx *c, cudaStream_t st) {
+    if (c->rtab.p) return SPL_OK;
+    if (c->key.occ == 0 && c->key.units > (1ull << 16)) CK(c, c->key.alloc(buckets_for(1ull << 12), st));
+    uint64_t nb = std::max<uint64_t>(c->rslots_hint ? c->rslots_hint : (1ull << 16), 1024);
+    nb = std::min<uint64_t>(nb, c->rtab.max_bytes / 64);
+    CK(c, c->rtab.alloc(nb, st));
+    return SPL_OK;
+}
+
+// What every solver create shares: clear the visited sets, upload the root record (`root_bytes`: a 32-byte Rec or a
+// 96-byte realistic record) and, on the card-set-sharded driver, its global rank 0; register the root in the visited
+// table of the level kind (trail = {self: None}); save the first link columns, synchronise and go live.  Without a
+// root (a sharded rank that does not own the root's card set) the queue starts empty.  On error `s` is deleted.
+template <class S>
+static int open_solver(S *s, LevelKind kind, const void *root, size_t root_bytes, bool sharded, const char *sync_msg, S **out) {
+    spl_ctx *c = s->c;
+    const cudaStream_t st = 0;
+    const int rc = [&]() -> int {
+        CKS(c, reset_visited(c, st));
+        if (root) {
+            const uint64_t zero = 0;
+            cudaError_t e = s->front.ensure(root_bytes, 0, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(s->front.p, root, root_bytes, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess && sharded) e = s->grank.ensure(8, 0, st);
+            if (e == cudaSuccess && sharded) e = cudaMemcpyAsync(s->grank.p, &zero, 8, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+            c->h2d_bytes += root_bytes + (sharded ? 8 : 0);
+            if (e != cudaSuccess) return fail(c, SPL_E_CUDA, "root upload: %s", cudaGetErrorString(e));
+            CKS(c, zero_ctr(c, st));
+            uint64_t tag = 0;
+            if (kind == KEY_TABLE) {
+                CKS(c, next_epoch(c, tag));
+                if (c->cand_slot.ensure(4, 0, st) != cudaSuccess) return fail(c, SPL_E_NOMEM, "cand_slot alloc");
+                const spl_key *k = s->front.template as<spl_key>();  // a Rec starts with its key
+                if (c->identity == IDENT_PYHASH)
+                    probe_list_kernel<IDENT_PYHASH><<<1, TILE, 0, st>>>(k, 1, c->key.as<uint64_t>(), c->key.units, tag,
+                                                                        c->cand_slot.as<uint32_t>(), c->d_ctr);
+                else
+                    probe_list_kernel<IDENT_KEY><<<1, TILE, 0, st>>>(k, 1, c->key.as<uint64_t>(), c->key.units, tag,
+                                                                     c->cand_slot.as<uint32_t>(), c->d_ctr);
+                c->key.occ = 1;
+            } else if (kind == GROUPED) {
+                const Rec *r = static_cast<const Rec *>(root);
+                m2_root_kernel<<<1, 1, 0, st>>>(c->nodes.as<uint64_t>(), c->nodes.units, r->lo, r->hi, c->d_gemrank, c->d_ctr);
+                c->nodes.occ = 1;
+            } else {
+                if (c->cand_slot.ensure(4, 0, st) != cudaSuccess) return fail(c, SPL_E_NOMEM, "realistic scratch alloc");
+                CKS(c, open_rtable(c, st));
+                CKS(c, c->rtab.grow(c, 1, st));
+                if (c->rtab.clear(st) != cudaSuccess) return fail(c, SPL_E_CUDA, "realistic table reset failed");  // forget the previous search
+                CKS(c, next_epoch(c, tag));
+                r_probe_kernel<<<1, TILE, 0, st>>>(s->front.template as<RRec>(), 1, c->rcfg.as<RConfigDev>(), c->rtab.as<RBucket>(),
+                                                    c->rtab.units, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
+                c->rtab.occ = 1;
+            }
+            ++c->launches;
+            CK(c, cudaGetLastError());
+            c->occupied = 1;
+        }
+        CKS(c, save_links(s, root ? 1 : 0, kind == REALISTIC, sharded, st));
+        if (cudaStreamSynchronize(st) != cudaSuccess) return fail(c, SPL_E_CUDA, "%s", sync_msg);
+        return SPL_OK;
+    }();
+    if (rc != SPL_OK) { delete s; return rc; }
+    s->activate();
+    *out = s;
     return SPL_OK;
 }
 
@@ -1543,34 +1634,15 @@ int32_t spl_gs_create(spl_ctx *c, int32_t rank, int32_t world, const spl_key *ro
     if (noise != SPL_NOISE_CONST && noise != SPL_NOISE_HASH) return fail(c, SPL_E_INVALID, "spl_gs_create: noise must be const or hash");
     NO_LIVE_SOLVER(c, "spl_gs_create");
     CK(c, enter_device(c));
-    cudaStream_t st = 0;
-    CKS(c, reset_visited(c, st));
     spl_gsolver *s = new spl_gsolver(c);
     s->rank = rank; s->world = world; s->goal = goal; s->heuristic = heuristic; s->beam = beam; s->noise = noise;
     s->keep_links = keep_links;
+    const Rec r{root_key->lo, root_key->hi & HI_KEY_MASK, root_aux, ~0ull};
     uint64_t m0, m1;
-    mask_words(root_key->lo, root_key->hi & HI_KEY_MASK, m0, m1);
-    int rc = SPL_OK;
-    if ((int)owner_of_mask(m0, m1, (uint32_t)world) == rank) {  // the root lives on the rank that owns its card set
-        Rec r{root_key->lo, root_key->hi & HI_KEY_MASK, root_aux, ~0ull};
-        uint64_t zero = 0;
-        cudaError_t e = s->front.ensure(32, 0, st);
-        if (e == cudaSuccess) e = s->grank.ensure(8, 0, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(s->front.p, &r, 32, cudaMemcpyHostToDevice, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(s->grank.p, &zero, 8, cudaMemcpyHostToDevice, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        c->h2d_bytes += 40;
-        if (e != cudaSuccess) rc = fail(c, SPL_E_CUDA, "root upload: %s", cudaGetErrorString(e));
-        if (rc == SPL_OK) rc = zero_ctr(c, st);
-        if (rc == SPL_OK) rc = add_grouped_root(c, r.lo, r.hi, st);
-        s->n_local = 1;
-    }
-    if (rc == SPL_OK) rc = save_links(s, s->n_local, false, true, st);
-    if (rc == SPL_OK && cudaStreamSynchronize(st) != cudaSuccess) rc = fail(c, SPL_E_CUDA, "spl_gs_create: sync failed");
-    if (rc != SPL_OK) { delete s; return rc; }
-    s->activate();
-    *out = s;
-    return SPL_OK;
+    mask_words(r.lo, r.hi, m0, m1);
+    const bool owner = (int)owner_of_mask(m0, m1, (uint32_t)world) == rank;  // the root lives on the rank that owns its card set
+    s->n_local = owner ? 1 : 0;
+    return open_solver(s, GROUPED, owner ? &r : nullptr, 32, true, "spl_gs_create: sync failed", out);
 }
 
 int32_t spl_gs_destroy(spl_gsolver *s) {
@@ -2025,52 +2097,6 @@ int32_t spl_gs_link_at(spl_gsolver *s, int32_t level, int64_t grank, int32_t *fo
 
 }  // extern "C"
 
-// ------------------------------------------------------------------ second half of a speedrun level
-// beam cut (src/solver.py:452-456) or plain BFS hand-over, then bookkeeping
-// n_uniq states in the first n_slots elements of s->uniq / c->sk (n_slots > n_uniq: the grouped level leaves unused slots)
-static int speedrun_cut(spl_solver *s, spl_level_info *info, int64_t n, int64_t n_uniq, uint64_t sk_min, uint64_t sk_max,
-                        cudaStream_t st, int64_t n_slots = -1) {
-    spl_ctx *c = s->c;
-    if (n_slots < 0) n_slots = n_uniq;
-    int64_t kept = n_uniq;
-    if (s->use_h && n_uniq > 0) {
-        int which = 0;
-        CK(c, cudaEventRecord(c->ev[4], st));
-        CutMode mode;
-        if (s->tie == SPL_TIE_KEY) mode.ties = TIES_KEY;
-        else if (s->grouped) mode = {TIES_LINK, 8 + bitlen((uint64_t)n)};  // unordered winners: arrival order is in their links
-        CKS(c, run_cut_sort(c, c->sk.as<uint64_t>(), s->uniq.as<Rec>(), n_slots, s->beam, sk_min, sk_max, mode, &which, &kept, st, n_uniq));
-        CK(c, cudaEventRecord(c->ev[5], st));
-        CK(c, s->front.ensure((size_t)kept * 32, 0, st));
-        gather_rec_kernel<<<nblk(kept), TILE, 0, st>>>(s->uniq.as<Rec>(), c->idx[which].as<uint32_t>(), kept, s->front.as<Rec>());
-        ++c->launches;
-        CK(c, cudaGetLastError());
-        CK(c, cudaEventRecord(c->ev[6], st));
-        CK(c, cudaStreamSynchronize(st));
-        float t;
-        cudaEventElapsedTime(&t, c->ev[4], c->ev[5]);
-        info->ms_select = t;  // select + cut + sort
-        cudaEventElapsedTime(&t, c->ev[5], c->ev[6]);
-        info->ms_sort = t;    // gather into rank order
-    } else if (kept > 0) {
-        s->front.swap(s->uniq);
-    }
-    info->kept = kept;
-    info->visited = (int64_t)c->occupied;
-    info->table_slots = s->grouped ? c->nn : c->cap;
-    if (kept == 0) {  // frontier exhausted: `puzzle` is the last dequeued state (src/solver.py:438,459);
-        s->ended = true;  // s->front still holds the level that was just expanded
-        s->goal_rank = n - 1;
-        info->ended = 1;
-        return SPL_OK;
-    }
-    s->n_front = kept;
-    s->level += 1;
-    CKS(c, save_links(s, s->n_front, s->realistic, false, st));
-    CK(c, cudaStreamSynchronize(st));
-    return SPL_OK;
-}
-
 // ------------------------------------------------------------------ realistic mode host side
 static int upload_rconfig(spl_ctx *c, const spl_rconfig *cfg, cudaStream_t st) {
     if (!cfg || cfg->num_players < 2 || cfg->num_players > 4 || cfg->gems_per_color < 1 || cfg->gems_per_color > 7)
@@ -2106,48 +2132,6 @@ static int upload_rconfig(spl_ctx *c, const spl_rconfig *cfg, cudaStream_t st) {
 static int use_rconfig(spl_ctx *c, const spl_rconfig *cfg, cudaStream_t st) {
     if (cfg && c->rcfg_have && memcmp(&c->rcfg_host, cfg, sizeof *cfg) == 0) return SPL_OK;
     return upload_rconfig(c, cfg, st);
-}
-
-// realistic mode's visited table: allocate / grow so that `need` more states keep the load factor <= 0.6
-static int ensure_rtable(spl_ctx *c, uint64_t need, cudaStream_t st) {
-    if (!c->rtable) {
-        // first use: the caller's table_slots sizes THIS table (a realistic search does not use the speedrun tables:
-        // give their memory back first if they were sized large)
-        if (c->occupied == 0 && c->nb > (1ull << 16)) {
-            cudaFree(c->table);
-            c->table = nullptr;
-            CKS(c, alloc_table(c, 1ull << 12, st));
-        }
-        uint64_t nb = std::max<uint64_t>(c->rslots_hint ? c->rslots_hint : (1ull << 16), 1024);
-        nb = std::min<uint64_t>(nb, c->max_table_bytes / 64);
-        CK(c, cudaMalloc(&c->rtable, nb * 64));
-        CK(c, cudaMemsetAsync(c->rtable, 0, nb * 64, st));
-        c->rnb = nb;
-        c->rocc = 0;
-    }
-    while ((double)(c->rocc + need) > 0.6 * (double)c->rnb) {
-        uint64_t nnb = c->rnb * 2;
-        if (nnb * 64 > c->max_table_bytes) nnb = c->max_table_bytes / 64;
-        if (nnb <= c->rnb + c->rnb / 8) break;
-        RBucket *nt = nullptr;
-        cudaError_t e = cudaMalloc(&nt, nnb * 64);
-        if (e != cudaSuccess) { cudaGetLastError(); break; }
-        CK(c, cudaMemsetAsync(nt, 0, nnb * 64, st));
-        r_rehash_kernel<<<nblk((int64_t)c->rnb), TILE, 0, st>>>(c->rtable, c->rnb, nt, nnb, c->d_ctr);
-        ++c->launches;
-        CK(c, cudaGetLastError());
-        unsigned int err = 0;
-        CK(c, cudaMemcpyAsync(&err, &c->d_ctr->error, 4, cudaMemcpyDeviceToHost, st));
-        CK(c, cudaStreamSynchronize(st));
-        if (err) { cudaFree(nt); return fail(c, SPL_E_TABLE_FULL, "realistic table rehash into %llu buckets overflowed a probe sequence", (unsigned long long)nnb); }
-        cudaFree(c->rtable);
-        c->rtable = nt;
-        c->rnb = nnb;
-    }
-    if (c->rocc + need / 4 > c->rnb - c->rnb / 16)
-        return fail(c, SPL_E_TABLE_FULL, "realistic visited table full: %llu states + %llu candidates vs %llu buckets (max_table_bytes=%llu)",
-                    (unsigned long long)c->rocc, (unsigned long long)need, (unsigned long long)c->rnb, (unsigned long long)c->max_table_bytes);
-    return SPL_OK;
 }
 
 // count + scan of the successors of front[0..n): offsets in c->off, vis masks in c->rvmask, the count in *total (synchronises)
@@ -2186,31 +2170,29 @@ static int dedup_flags(spl_ctx *c, bool realistic, const void *keys, int64_t n, 
     CK(c, enter_device(c));
     if (n == 0) return SPL_OK;
     CKS(c, zero_ctr(c, st));
-    CKS(c, realistic ? ensure_rtable(c, (uint64_t)n, st) : ensure_table(c, (uint64_t)n, st));
+    if (realistic) CKS(c, open_rtable(c, st));
+    VisitTable &t = realistic ? c->rtab : c->key;
+    CKS(c, t.grow(c, (uint64_t)n, st));
     uint64_t tag;
     CKS(c, next_epoch(c, tag));
     CK(c, c->cand_slot.ensure((size_t)n * 4, 0, st));
     uint32_t *slot = c->cand_slot.as<uint32_t>();
     if (realistic) {
-        CKS(c, zero_ctr(c, st));  // again after the table's growth, as rsolver_step does
-        r_probe_keys_kernel<<<nblk(n), TILE, 0, st>>>(static_cast<const uint64_t *>(keys), n, c->rtable, c->rnb, tag, slot, c->d_ctr);
-        win_flags_kernel<<<nblk(n), TILE, 0, st>>>(slot, c->rtable, n, flags);
+        CKS(c, zero_ctr(c, st));  // again after the table's growth, as realistic_expand does
+        r_probe_keys_kernel<<<nblk(n), TILE, 0, st>>>(static_cast<const uint64_t *>(keys), n, t.as<RBucket>(), t.units, tag, slot, c->d_ctr);
+        win_flags_kernel<<<nblk(n), TILE, 0, st>>>(slot, t.as<RBucket>(), n, flags);
     } else {
-        probe_list_kernel<IDENT_KEY><<<nblk(n), TILE, 0, st>>>(static_cast<const spl_key *>(keys), n, c->table, c->nb, tag, slot, c->d_ctr);
-        win_flags_kernel<<<nblk(n), TILE, 0, st>>>(slot, c->table, n, flags);
+        probe_list_kernel<IDENT_KEY><<<nblk(n), TILE, 0, st>>>(static_cast<const spl_key *>(keys), n, t.as<uint64_t>(), t.units, tag, slot, c->d_ctr);
+        win_flags_kernel<<<nblk(n), TILE, 0, st>>>(slot, t.as<uint64_t>(), n, flags);
     }
     c->launches += 2;
     CK(c, cudaGetLastError());
     CKS(c, read_ctr(c, st));
-    if (realistic) {
-        // the intended difference: counted before the error check, so that spl_rreset_visited clears a partial insert too
-        c->rocc += c->h_ctr->n_new;
-        if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "spl_rdedup_flags: probe overflow (realistic visited table full, %llu buckets)",
-                                         (unsigned long long)c->rnb);
-        return SPL_OK;
-    }
+    t.occ += c->h_ctr->n_new;  // before the error check: a reset clears a partial insert too
+    if (c->h_ctr->error && realistic)
+        return fail(c, SPL_E_TABLE_FULL, "spl_rdedup_flags: probe overflow (realistic visited table full, %llu buckets)", (unsigned long long)t.units);
     if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "spl_dedup_flags: probe overflow (table full)");
-    c->occupied += c->h_ctr->n_new;
+    if (!realistic) c->occupied += c->h_ctr->n_new;
     return SPL_OK;
 }
 
@@ -2252,237 +2234,14 @@ static int move_rows(spl_ctx *c, const char *fn, const void *rows, const int64_t
     return SPL_OK;
 }
 
-static int realistic_cut(spl_solver *s, spl_level_info *info, int64_t n, int64_t n_new, const uint8_t *draws, cudaStream_t st);
-
-static int rsolver_step(spl_solver *s, spl_level_info *info, cudaStream_t st) {
+// ------------------------------------------------------------------ expand + dedup of a level, by kind
+// Key-table level: chunks of parents, each expanded straight into probes of the key table, then the winners resolved
+// in arrival order into s->uniq (with on-device scores into c->sk).
+static int keytable_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6], cudaStream_t st) {
     spl_ctx *c = s->c;
-    memset(info, 0, sizeof *info);
-    info->level = s->level;
-    info->frontier = s->n_front;
-    info->goal_rank = -1;
-    const int64_t n = s->n_front;
-    const RRec *front = s->front.as<RRec>();
-    if (c->rcfg_dirty) {  // spl_rscore / spl_rexpand / spl_rmaxpts ran with their own GameConfig in between
-        CKS(c, upload_rconfig(c, &s->rcfg, st));
-        c->rcfg_dirty = false;
-    }
-    // game over on dequeue (src/solver.py:827-829)
-    CKS(c, zero_ctr(c, st));
-    r_goal_kernel<<<nblk(n), TILE, 0, st>>>(front, n, c->rcfg.as<RConfigDev>(), c->d_ctr);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    if (c->h_ctr->goal_rank != 0x7fffffffffffffffll) {
-        s->ended = true;
-        s->goal_rank = c->h_ctr->goal_rank;
-        info->ended = 1;
-        info->goal_rank = s->goal_rank;
-        info->visited = (int64_t)c->occupied;
-        info->table_slots = c->rnb;
-        return SPL_OK;
-    }
-    int64_t total = 0, n_new = 0;
-    CK(c, cudaEventRecord(c->ev[0], st));
-    CKS(c, r_expand_all(c, front, n, 0, &total, st));
-    CK(c, cudaEventRecord(c->ev[1], st));
-    info->expanded = n;
-    info->generated = total;
-    if (total >= 0xFFFFFFFFll) return fail(c, SPL_E_INVALID, "level produced %lld candidates (>= 2^32)", (long long)total);
-    if (total) {  // first-arrival dedup on the exact identity key (:840-843)
-        CKS(c, zero_ctr(c, st));
-        CKS(c, ensure_rtable(c, (uint64_t)total, st));
-        uint64_t tag;
-        CKS(c, next_epoch(c, tag));
-        CK(c, c->cand_slot.ensure((size_t)total * 4, 0, st));
-        CKS(c, zero_ctr(c, st));
-        r_probe_kernel<<<nblk(total), TILE, 0, st>>>(c->rcand.as<RRec>(), total, c->rcfg.as<RConfigDev>(), c->rtable, c->rnb, tag,
-                                                      c->cand_slot.as<uint32_t>(), c->d_ctr);
-        ++c->launches;
-        CK(c, cudaGetLastError());
-        CKS(c, read_ctr(c, st));
-        if (c->h_ctr->error == 4) return fail(c, SPL_E_INVALID, "a player saved 1024 gems or more: outside the packed identity key");
-        if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "visited table full during level %d", s->level);
-        n_new = (int64_t)c->h_ctr->n_new;
-        c->rocc += n_new;
-        c->occupied += n_new;
-    }
-    info->unique = n_new;
-    if (n_new) {
-        CK(c, c->ridx64.ensure((size_t)n_new * 8, 0, st));
-        const unsigned nt = nblk(total, TILE * 8);
-        CKS(c, prep_status(c, 0, nt, st));
-        CKS(c, reset_ticket(c, 0, st));
-        r_winners_kernel<<<nt, TILE, 0, st>>>(c->cand_slot.as<uint32_t>(), c->rtable, total, c->ridx64.as<int64_t>(),
-                                               c->status[0].as<uint64_t>(), c->d_ctr, 0);
-        CK(c, s->uniq.ensure((size_t)n_new * 96, 0, st));
-        r_gather_kernel<int64_t><<<nblk(n_new), TILE, 0, st>>>(c->rcand.as<RRec>(), c->ridx64.as<int64_t>(), n_new, s->uniq.as<RRec>());
-        c->launches += 2;
-        CK(c, cudaGetLastError());
-        if (s->rcfg.noise == SPL_NOISE_EXTERNAL) {  // wait for the host's randint draws
-            CK(c, cudaStreamSynchronize(st));
-            s->pending = true;
-            s->pend_n = n;
-            s->pend_uniq = n_new;
-            info->kept = -1;
-            info->visited = (int64_t)c->occupied;
-            info->table_slots = c->rnb;
-            s->pend_info = *info;
-            return SPL_OK;
-        }
-    }
-    return realistic_cut(s, info, n, n_new, nullptr, st);
-}
-
-static int realistic_cut(spl_solver *s, spl_level_info *info, int64_t n, int64_t n_new, const uint8_t *draws, cudaStream_t st) {
-    spl_ctx *c = s->c;
-    int64_t kept = 0;
-    if (n_new) {
-        // score + beam cut, ties by arrival order (:846)
-        CK(c, cudaEventRecord(c->ev[2], st));
-        CKS(c, zero_ctr(c, st));
-        CK(c, c->sk.ensure((size_t)n_new * 8, 0, st));
-        r_score_kernel<<<nblk(n_new), TILE, 0, st>>>(s->uniq.as<RRec>(), n_new, c->rcfg.as<RConfigDev>(), c->luts,
-                                                      c->sk.as<uint64_t>(), nullptr, c->d_ctr, draws);
-        ++c->launches;
-        CK(c, cudaGetLastError());
-        CKS(c, read_ctr(c, st));
-        const uint64_t smin = c->h_ctr->sk_min, smax = c->h_ctr->sk_max;
-        int which = 0;
-        CKS(c, run_cut_sort(c, c->sk.as<uint64_t>(), nullptr, n_new, s->beam, smin, smax, CutMode{}, &which, &kept, st));
-        if (s->level < 1000) {  // at the turn limit the queue just expanded stays in place (see below)
-            CK(c, s->front.ensure((size_t)kept * 96, 0, st));
-            r_gather_kernel<uint32_t><<<nblk(kept), TILE, 0, st>>>(s->uniq.as<RRec>(), c->idx[which].as<uint32_t>(), kept, s->front.as<RRec>());
-            ++c->launches;
-        }
-        CK(c, cudaGetLastError());
-        CK(c, cudaEventRecord(c->ev[3], st));
-        CK(c, cudaStreamSynchronize(st));
-        float t;
-        cudaEventElapsedTime(&t, c->ev[2], c->ev[3]);
-        info->ms_select = t;
-    }
-    info->kept = kept;
-    info->visited = (int64_t)c->occupied;
-    info->table_slots = c->rnb;
-    // queue exhausted, or the turn limit: the reference leaves its loop after the iteration with turn == 1000
-    // (src/solver.py:846-852), so `puzzle` is the last state dequeued from THAT queue and the path has 1001 states
-    if (kept == 0 || s->level >= 1000) {
-        s->ended = true;
-        s->goal_rank = n - 1;
-        info->ended = 1;
-        return SPL_OK;
-    }
-    s->n_front = kept;
-    s->level += 1;
-    CKS(c, save_links(s, s->n_front, s->realistic, false, st));
-    CK(c, cudaStreamSynchronize(st));
-    return SPL_OK;
-}
-
-extern "C" {
-
-int32_t spl_solver_create(spl_ctx *c, const spl_key *root_key, uint64_t root_aux, int32_t goal, int32_t use_h,
-                          int32_t heuristic, int64_t beam, int32_t tie, int32_t noise, int32_t keep_links,
-                          spl_solver **out) {
-    if (!c || !root_key || !out) return fail(c, SPL_E_INVALID, "spl_solver_create: null argument");
-    if (use_h && beam < 1) return fail(c, SPL_E_INVALID, "spl_solver_create: beam_width must be >= 1");
-    if (use_h && tie != SPL_TIE_STABLE && tie != SPL_TIE_KEY) return fail(c, SPL_E_INVALID, "spl_solver_create: unknown tie policy %d", tie);
-    if (noise < 0 || noise > SPL_NOISE_EXTERNAL) return fail(c, SPL_E_INVALID, "spl_solver_create: unknown noise policy %d", noise);
-    NO_LIVE_SOLVER(c, "spl_solver_create");
-    CK(c, enter_device(c));
-    cudaStream_t st = 0;
-    spl_solver *s = new spl_solver(c);
-    s->goal = goal; s->use_h = use_h; s->heuristic = heuristic; s->beam = beam; s->tie = tie;
-    s->noise = noise; s->keep_links = keep_links;
-    // beam search with on-device scoring runs on the card-set-grouped level; exhaustive BFS (queue order == arrival
-    // order), the reference's hash identity and externally drawn noise (arrival-ordered draws) on the key table
-    s->grouped = use_h && noise != SPL_NOISE_EXTERNAL && c->identity == IDENT_KEY && !getenv("SPL_NO_GROUPED");
-    int rc = reset_visited(c, st);
-    if (rc == SPL_OK) {
-        Rec r{root_key->lo, root_key->hi & HI_KEY_MASK, root_aux, ~0ull};
-        cudaError_t e = s->front.ensure(32, 0, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(s->front.p, &r, 32, cudaMemcpyHostToDevice, st);
-        c->h2d_bytes += 32;
-        if (e != cudaSuccess) rc = fail(c, SPL_E_CUDA, "root upload: %s", cudaGetErrorString(e));
-    }
-    if (rc == SPL_OK) rc = zero_ctr(c, st);
-    if (rc == SPL_OK) {  // trail = {self: None}
-        uint64_t tag;
-        rc = next_epoch(c, tag);
-        if (rc == SPL_OK) {
-            cudaError_t e = c->cand_slot.ensure(4, 0, st);
-            if (e != cudaSuccess) rc = fail(c, SPL_E_NOMEM, "cand_slot alloc");
-            else if (s->grouped) {
-                rc = add_grouped_root(c, root_key->lo, root_key->hi & HI_KEY_MASK, st);
-            } else {
-                if (c->identity == IDENT_PYHASH)
-                    probe_list_kernel<IDENT_PYHASH><<<1, TILE, 0, st>>>(reinterpret_cast<const spl_key *>(s->front.p), 1, c->table,
-                                                                        c->nb, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
-                else
-                    probe_list_kernel<IDENT_KEY><<<1, TILE, 0, st>>>(reinterpret_cast<const spl_key *>(s->front.p), 1, c->table,
-                                                                     c->nb, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
-                ++c->launches;
-                c->occupied = 1;
-            }
-        }
-    }
-    s->n_front = 1;
-    if (rc == SPL_OK) rc = save_links(s, s->n_front, false, false, st);
-    if (rc == SPL_OK && cudaStreamSynchronize(st) != cudaSuccess) rc = fail(c, SPL_E_CUDA, "solver create sync failed");
-    if (rc != SPL_OK) { delete s; return rc; }
-    s->activate();
-    *out = s;
-    return SPL_OK;
-}
-
-int32_t spl_solver_destroy(spl_solver *s) {
-    if (s) { cudaSetDevice(s->c->device); cudaDeviceSynchronize(); delete s; }
-    return SPL_OK;
-}
-
-int32_t spl_solver_step(spl_solver *s, spl_level_info *info, void *stream) {
-    if (!s || !info) return SPL_E_INVALID;
-    spl_ctx *c = s->c;
-    if (s->ended) return fail(c, SPL_E_STATE, "spl_solver_step: the search has already ended");
-    if (s->pending) return fail(c, SPL_E_STATE, "spl_solver_step: the previous level still waits for spl_solver_cut");
-    cudaStream_t st = (cudaStream_t)stream;
-    CK(c, enter_device(c));
-    if (s->realistic) return rsolver_step(s, info, st);
-    memset(info, 0, sizeof *info);
-    info->level = s->level;
-    info->frontier = s->n_front;
-    info->goal_rank = -1;
-    const int64_t n = s->n_front;
     const Rec *front = s->front.as<Rec>();
-    float ms[6] = {0, 0, 0, 0, 0, 0};  // count, expand, resolve, select, sort, (grouped level) warp kernel
-    // ---- goal test on the queue (src/solver.py:443-445): the first state in queue order with
-    // pts >= goal ends the search; the states before it would be expanded and discarded.
-    CKS(c, zero_ctr(c, st));
-    goal_kernel<<<nblk(n), TILE, 0, st>>>(front, n, s->goal, c->d_ctr);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    if (c->h_ctr->goal_rank != 0x7fffffffffffffffll) {
-        s->ended = true;
-        s->goal_rank = c->h_ctr->goal_rank;
-        info->ended = 1;
-        info->goal_rank = s->goal_rank;
-        info->visited = (int64_t)c->occupied;
-        info->table_slots = s->grouped ? c->nn : c->cap;
-        return SPL_OK;
-    }
-    // ---- expand + dedup by chunks of parents
     int64_t n_uniq = 0, generated = 0;
     uint64_t sk_min = ~0ull, sk_max = 0;
-    if (s->grouped) {
-        int64_t n_slots = 0;
-        CKS(c, grouped_expand(s, front, n, &n_uniq, &n_slots, &generated, &sk_min, &sk_max, ms, st));
-        info->expanded = n;
-        info->generated = generated;
-        info->unique = n_uniq;
-        info->ms_count = ms[0]; info->ms_expand = ms[1]; info->ms_resolve = ms[2]; info->ms_warp = ms[5];
-        return speedrun_cut(s, info, n, n_uniq, sk_min, sk_max, st, n_slots);
-    }
     for (int64_t p0 = 0; p0 < n; p0 += (int64_t)c->chunk_parents) {
         const int64_t np = std::min<int64_t>((int64_t)c->chunk_parents, n - p0);
         const unsigned nt = nblk(np);
@@ -2494,7 +2253,7 @@ int32_t spl_solver_step(spl_solver *s, spl_level_info *info, void *stream) {
         generated += (int64_t)total;
         if (total == 0) continue;
         if (total >= 0xFFFFFFFFull) return fail(c, SPL_E_INVALID, "chunk produced %llu candidates (>= 2^32)", (unsigned long long)total);
-        CKS(c, ensure_table(c, total, st));
+        CKS(c, c->key.grow(c, total, st));
         uint64_t tag;
         CKS(c, next_epoch(c, tag));
         CK(c, c->cand_slot.ensure((size_t)total * 4, 0, st));
@@ -2502,17 +2261,18 @@ int32_t spl_solver_step(spl_solver *s, spl_level_info *info, void *stream) {
         if (c->identity == IDENT_PYHASH)
             expand_kernel<MODE_PROBE, IDENT_PYHASH><<<nt, TILE, sizeof(ExpandSmem2), st>>>(
                 front + p0, np, c->d_tabs, c->d_takes_idx, c->d_takes_edges, c->off.as<uint32_t>(), (uint32_t)total,
-                c->table, c->nb, tag, c->cand_slot.as<uint32_t>(), nullptr, p0, c->d_ctr);
+                c->key.as<uint64_t>(), c->key.units, tag, c->cand_slot.as<uint32_t>(), nullptr, p0, c->d_ctr);
         else
             expand_kernel<MODE_PROBE, IDENT_KEY><<<nt, TILE, sizeof(ExpandSmem2), st>>>(
                 front + p0, np, c->d_tabs, c->d_takes_idx, c->d_takes_edges, c->off.as<uint32_t>(), (uint32_t)total,
-                c->table, c->nb, tag, c->cand_slot.as<uint32_t>(), nullptr, p0, c->d_ctr);
+                c->key.as<uint64_t>(), c->key.units, tag, c->cand_slot.as<uint32_t>(), nullptr, p0, c->d_ctr);
         ++c->launches;
         CK(c, cudaGetLastError());
         CK(c, cudaEventRecord(c->ev[1], st));
         CKS(c, read_ctr(c, st));
+        c->key.occ += c->h_ctr->n_new;  // before the error check: a reset clears a partial insert too
         if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "visited table full during level %d (slots=%llu, occupied=%llu)",
-                                         s->level, (unsigned long long)c->cap, (unsigned long long)c->occupied);
+                                         s->level, (unsigned long long)c->key.slots(), (unsigned long long)c->occupied);
         const int64_t n_new = (int64_t)c->h_ctr->n_new;
         c->occupied += n_new;
         if (n_new) {
@@ -2524,12 +2284,12 @@ int32_t spl_solver_step(spl_solver *s, spl_level_info *info, void *stream) {
             if (s->use_h && s->noise != SPL_NOISE_EXTERNAL)
                 resolve_kernel<SRC_PARENT, true><<<nt, TILE, sizeof(ResolveSmem), st>>>(
                     front + p0, np, c->d_tabs, c->d_takes_idx, c->d_takes_edges, c->off.as<uint32_t>(), (uint32_t)total,
-                    c->table, c->cand_slot.as<uint32_t>(), nullptr, nullptr, p0, (uint64_t)n_uniq, s->uniq.as<Rec>(),
+                    c->key.as<uint64_t>(), c->cand_slot.as<uint32_t>(), nullptr, nullptr, p0, (uint64_t)n_uniq, s->uniq.as<Rec>(),
                     c->sk.as<uint64_t>(), nullptr, s->heuristic, s->noise, c->luts, c->status[0].as<uint64_t>(), c->d_ctr, 0);
             else
                 resolve_kernel<SRC_PARENT, false><<<nt, TILE, sizeof(ResolveSmem), st>>>(
                     front + p0, np, c->d_tabs, c->d_takes_idx, c->d_takes_edges, c->off.as<uint32_t>(), (uint32_t)total,
-                    c->table, c->cand_slot.as<uint32_t>(), nullptr, nullptr, p0, (uint64_t)n_uniq, s->uniq.as<Rec>(),
+                    c->key.as<uint64_t>(), c->cand_slot.as<uint32_t>(), nullptr, nullptr, p0, (uint64_t)n_uniq, s->uniq.as<Rec>(),
                     nullptr, nullptr, s->heuristic, s->noise, c->luts, c->status[0].as<uint64_t>(), c->d_ctr, 0);
             ++c->launches;
             CK(c, cudaGetLastError());
@@ -2550,21 +2310,212 @@ int32_t spl_solver_step(spl_solver *s, spl_level_info *info, void *stream) {
         cudaEventElapsedTime(&t, c->ev[7], c->ev[1]);
         ms[1] += t;
     }
+    *x = LevelExpand{n_uniq, n_uniq, generated, sk_min, sk_max};
+    return SPL_OK;
+}
+
+// Realistic level: the successors materialised, first-arrival dedup on their exact identity key (src/solver.py:840-843),
+// the winners gathered in arrival order into s->uniq.
+static int realistic_expand(spl_solver *s, int64_t n, LevelExpand *x, cudaStream_t st) {
+    spl_ctx *c = s->c;
+    int64_t total = 0, n_new = 0;
+    CKS(c, r_expand_all(c, s->front.as<RRec>(), n, 0, &total, st));
+    if (total >= 0xFFFFFFFFll) return fail(c, SPL_E_INVALID, "level produced %lld candidates (>= 2^32)", (long long)total);
+    if (total) {
+        CKS(c, zero_ctr(c, st));
+        CKS(c, c->rtab.grow(c, (uint64_t)total, st));
+        uint64_t tag;
+        CKS(c, next_epoch(c, tag));
+        CK(c, c->cand_slot.ensure((size_t)total * 4, 0, st));
+        CKS(c, zero_ctr(c, st));
+        r_probe_kernel<<<nblk(total), TILE, 0, st>>>(c->rcand.as<RRec>(), total, c->rcfg.as<RConfigDev>(), c->rtab.as<RBucket>(),
+                                                      c->rtab.units, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CKS(c, read_ctr(c, st));
+        c->rtab.occ += c->h_ctr->n_new;  // before the error checks: a reset clears a partial insert too
+        if (c->h_ctr->error == 4) return fail(c, SPL_E_INVALID, "a player saved 1024 gems or more: outside the packed identity key");
+        if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "visited table full during level %d", s->level);
+        n_new = (int64_t)c->h_ctr->n_new;
+        c->occupied += n_new;
+    }
+    if (n_new) {
+        CK(c, c->ridx64.ensure((size_t)n_new * 8, 0, st));
+        const unsigned nt = nblk(total, TILE * 8);
+        CKS(c, prep_status(c, 0, nt, st));
+        CKS(c, reset_ticket(c, 0, st));
+        r_winners_kernel<<<nt, TILE, 0, st>>>(c->cand_slot.as<uint32_t>(), c->rtab.as<RBucket>(), total, c->ridx64.as<int64_t>(),
+                                               c->status[0].as<uint64_t>(), c->d_ctr, 0);
+        CK(c, s->uniq.ensure((size_t)n_new * 96, 0, st));
+        r_gather_kernel<int64_t><<<nblk(n_new), TILE, 0, st>>>(c->rcand.as<RRec>(), c->ridx64.as<int64_t>(), n_new, s->uniq.as<RRec>());
+        c->launches += 2;
+        CK(c, cudaGetLastError());
+    }
+    *x = LevelExpand{n_new, n_new, total, ~0ull, 0};
+    return SPL_OK;
+}
+
+// ------------------------------------------------------------------ second half of a level
+// Score (realistic level, or externally drawn noise: the key-table level scores as it resolves, the grouped level as it
+// deduplicates), beam cut (src/solver.py:452-456, :846) and gather of the queue in rank order, or the plain BFS
+// hand-over; then the bookkeeping.
+static int level_cut(spl_solver *s, spl_level_info *info, int64_t n, const LevelExpand &x, const uint8_t *draws, cudaStream_t st) {
+    spl_ctx *c = s->c;
+    const bool realistic = s->kind == REALISTIC;
+    // the reference leaves its realistic loop after the iteration with turn == 1000 (src/solver.py:846-852): `puzzle` is
+    // the last state dequeued from the queue just expanded, which stays in place, and the path has 1001 states
+    const bool turn_limit = realistic && s->level >= 1000;
+    int64_t kept = x.n_uniq;
+    if (s->use_h && kept > 0) {
+        uint64_t sk_min = x.sk_min, sk_max = x.sk_max;
+        CK(c, cudaEventRecord(c->ev[2], st));
+        if (realistic || draws) {
+            CKS(c, zero_ctr(c, st));
+            CK(c, c->sk.ensure((size_t)x.n_uniq * 8, 0, st));
+            if (realistic)
+                r_score_kernel<<<nblk(x.n_uniq), TILE, 0, st>>>(s->uniq.as<RRec>(), x.n_uniq, c->rcfg.as<RConfigDev>(), c->luts,
+                                                                 c->sk.as<uint64_t>(), nullptr, c->d_ctr, draws);
+            else
+                score_ext_kernel<<<nblk(x.n_uniq), TILE, 0, st>>>(s->uniq.as<Rec>(), draws, x.n_uniq, s->heuristic, c->luts,
+                                                                   c->sk.as<uint64_t>(), c->d_ctr);
+            ++c->launches;
+            CK(c, cudaGetLastError());
+            CKS(c, read_ctr(c, st));
+            sk_min = c->h_ctr->sk_min;
+            sk_max = c->h_ctr->sk_max;
+        }
+        CK(c, cudaEventRecord(c->ev[4], st));
+        CutMode mode;
+        if (s->tie == SPL_TIE_KEY) mode.ties = TIES_KEY;
+        else if (s->kind == GROUPED) mode = {TIES_LINK, 8 + bitlen((uint64_t)n)};  // unordered winners: arrival order is in their links
+        int which = 0;
+        CKS(c, run_cut_sort(c, c->sk.as<uint64_t>(), realistic ? nullptr : s->uniq.as<Rec>(), x.n_slots, s->beam, sk_min, sk_max,
+                            mode, &which, &kept, st, x.n_uniq));
+        CK(c, cudaEventRecord(c->ev[5], st));
+        if (!turn_limit) {
+            CK(c, s->front.ensure((size_t)kept * (realistic ? 96 : 32), 0, st));
+            if (realistic)
+                r_gather_kernel<uint32_t><<<nblk(kept), TILE, 0, st>>>(s->uniq.as<RRec>(), c->idx[which].as<uint32_t>(), kept, s->front.as<RRec>());
+            else
+                gather_rec_kernel<<<nblk(kept), TILE, 0, st>>>(s->uniq.as<Rec>(), c->idx[which].as<uint32_t>(), kept, s->front.as<Rec>());
+            ++c->launches;
+        }
+        CK(c, cudaGetLastError());
+        CK(c, cudaEventRecord(c->ev[6], st));
+        CK(c, cudaStreamSynchronize(st));
+        float t;
+        if (realistic) {
+            cudaEventElapsedTime(&t, c->ev[2], c->ev[6]);
+            info->ms_select = t;  // score + cut + gather
+        } else {
+            cudaEventElapsedTime(&t, c->ev[4], c->ev[5]);
+            info->ms_select = t;  // select + cut + sort
+            cudaEventElapsedTime(&t, c->ev[5], c->ev[6]);
+            info->ms_sort = t;    // gather into rank order
+        }
+    } else if (kept > 0) {
+        s->front.swap(s->uniq);
+    }
+    info->kept = kept;
+    info->visited = (int64_t)c->occupied;
+    info->table_slots = visited_table(c, s->kind).slots();
+    if (kept == 0 || turn_limit) {  // queue exhausted: `puzzle` is the last dequeued state (src/solver.py:438,459);
+        s->ended = true;            // s->front still holds the level that was just expanded
+        s->goal_rank = n - 1;
+        info->ended = 1;
+        return SPL_OK;
+    }
+    s->n_front = kept;
+    s->level += 1;
+    CKS(c, save_links(s, s->n_front, realistic, false, st));
+    CK(c, cudaStreamSynchronize(st));
+    return SPL_OK;
+}
+
+extern "C" {
+
+int32_t spl_solver_create(spl_ctx *c, const spl_key *root_key, uint64_t root_aux, int32_t goal, int32_t use_h,
+                          int32_t heuristic, int64_t beam, int32_t tie, int32_t noise, int32_t keep_links,
+                          spl_solver **out) {
+    if (!c || !root_key || !out) return fail(c, SPL_E_INVALID, "spl_solver_create: null argument");
+    if (use_h && beam < 1) return fail(c, SPL_E_INVALID, "spl_solver_create: beam_width must be >= 1");
+    if (use_h && tie != SPL_TIE_STABLE && tie != SPL_TIE_KEY) return fail(c, SPL_E_INVALID, "spl_solver_create: unknown tie policy %d", tie);
+    if (noise < 0 || noise > SPL_NOISE_EXTERNAL) return fail(c, SPL_E_INVALID, "spl_solver_create: unknown noise policy %d", noise);
+    NO_LIVE_SOLVER(c, "spl_solver_create");
+    CK(c, enter_device(c));
+    spl_solver *s = new spl_solver(c);
+    s->goal = goal; s->use_h = use_h; s->heuristic = heuristic; s->beam = beam; s->tie = tie;
+    s->noise = noise; s->keep_links = keep_links;
+    // beam search with on-device scoring runs on the card-set-grouped level; exhaustive BFS (queue order == arrival
+    // order), the reference's hash identity and externally drawn noise (arrival-ordered draws) on the key table
+    const bool grouped = use_h && noise != SPL_NOISE_EXTERNAL && c->identity == IDENT_KEY && !getenv("SPL_NO_GROUPED");
+    s->kind = grouped ? GROUPED : KEY_TABLE;
+    s->n_front = 1;
+    const Rec r{root_key->lo, root_key->hi & HI_KEY_MASK, root_aux, ~0ull};
+    return open_solver(s, s->kind, &r, 32, false, "solver create sync failed", out);
+}
+
+int32_t spl_solver_destroy(spl_solver *s) {
+    if (s) { cudaSetDevice(s->c->device); cudaDeviceSynchronize(); delete s; }
+    return SPL_OK;
+}
+
+int32_t spl_solver_step(spl_solver *s, spl_level_info *info, void *stream) {
+    if (!s || !info) return SPL_E_INVALID;
+    spl_ctx *c = s->c;
+    if (s->ended) return fail(c, SPL_E_STATE, "spl_solver_step: the search has already ended");
+    if (s->pending) return fail(c, SPL_E_STATE, "spl_solver_step: the previous level still waits for spl_solver_cut");
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c, enter_device(c));
+    memset(info, 0, sizeof *info);
+    info->level = s->level;
+    info->frontier = s->n_front;
+    info->goal_rank = -1;
+    const int64_t n = s->n_front;
+    const bool realistic = s->kind == REALISTIC;
+    if (realistic && c->rcfg_dirty) {  // spl_rscore / spl_rexpand / spl_rmaxpts ran with their own GameConfig in between
+        CKS(c, upload_rconfig(c, &s->rcfg, st));
+        c->rcfg_dirty = false;
+    }
+    // ---- goal test on the queue (src/solver.py:443-445; realistic mode: game over on dequeue, :827-829): the first
+    // state in queue order that has won ends the search; the states before it would be expanded and discarded.
+    CKS(c, zero_ctr(c, st));
+    if (realistic) r_goal_kernel<<<nblk(n), TILE, 0, st>>>(s->front.as<RRec>(), n, c->rcfg.as<RConfigDev>(), c->d_ctr);
+    else goal_kernel<<<nblk(n), TILE, 0, st>>>(s->front.as<Rec>(), n, s->goal, c->d_ctr);
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    CKS(c, read_ctr(c, st));
+    if (c->h_ctr->goal_rank != 0x7fffffffffffffffll) {
+        s->ended = true;
+        s->goal_rank = c->h_ctr->goal_rank;
+        info->ended = 1;
+        info->goal_rank = s->goal_rank;
+        info->visited = (int64_t)c->occupied;
+        info->table_slots = visited_table(c, s->kind).slots();
+        return SPL_OK;
+    }
+    // ---- expand + dedup
+    LevelExpand x;
+    float ms[6] = {0, 0, 0, 0, 0, 0};  // count, expand, resolve, select, sort, (grouped level) warp kernel
+    if (s->kind == KEY_TABLE) CKS(c, keytable_expand(s, n, &x, ms, st));
+    else if (s->kind == GROUPED) CKS(c, grouped_expand(s, n, &x, ms, st));
+    else CKS(c, realistic_expand(s, n, &x, st));
     info->expanded = n;
-    info->generated = generated;
-    info->unique = n_uniq;
-    info->ms_count = ms[0]; info->ms_expand = ms[1]; info->ms_resolve = ms[2];
-    if (s->use_h && s->noise == SPL_NOISE_EXTERNAL && n_uniq > 0) {  // wait for the host's randint draws
+    info->generated = x.generated;
+    info->unique = x.n_uniq;
+    info->ms_count = ms[0]; info->ms_expand = ms[1]; info->ms_resolve = ms[2]; info->ms_warp = ms[5];
+    if (s->use_h && s->noise == SPL_NOISE_EXTERNAL && x.n_uniq > 0) {  // wait for the host's randint draws
+        CK(c, cudaStreamSynchronize(st));
         s->pending = true;
         s->pend_n = n;
-        s->pend_uniq = n_uniq;
+        s->pend_uniq = x.n_uniq;
         info->kept = -1;
         info->visited = (int64_t)c->occupied;
-        info->table_slots = c->cap;
+        info->table_slots = visited_table(c, s->kind).slots();
         s->pend_info = *info;
         return SPL_OK;
     }
-    return speedrun_cut(s, info, n, n_uniq, sk_min, sk_max, st);
+    return level_cut(s, info, n, x, nullptr, st);
 }
 
 int32_t spl_rexpand(spl_ctx *c, const spl_rconfig *cfg, const void *recs, int64_t n, void *out_recs, int64_t cap,
@@ -2627,52 +2578,17 @@ int32_t spl_rsolver_create(spl_ctx *c, const spl_rconfig *cfg, const void *root_
     if (beam < 1) return fail(c, SPL_E_INVALID, "spl_rsolver_create: beam_width must be >= 1");
     NO_LIVE_SOLVER(c, "spl_rsolver_create");
     CK(c, enter_device(c));
-    cudaStream_t st = 0;
-    CKS(c, upload_rconfig(c, cfg, st));
+    CKS(c, upload_rconfig(c, cfg, 0));
     spl_solver *s = new spl_solver(c);
-    s->realistic = true; s->rcfg = *cfg; s->use_h = 1; s->beam = beam; s->keep_links = keep_links;
+    s->kind = REALISTIC; s->rcfg = *cfg; s->use_h = 1; s->noise = cfg->noise; s->beam = beam; s->keep_links = keep_links;
     s->goal = cfg->target_points;
+    s->n_front = 1;
     c->rcfg_dirty = false;
-    int rc = reset_visited(c, st);
-    if (rc == SPL_OK) {
-        cudaError_t e = s->front.ensure(96, 0, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(s->front.p, root_rec_host, 96, cudaMemcpyHostToDevice, st);
-        c->h2d_bytes += 96;
-        if (e != cudaSuccess) rc = fail(c, SPL_E_CUDA, "root upload: %s", cudaGetErrorString(e));
-    }
-    if (rc == SPL_OK) {  // trail = {self: None}: register the root's identity key
-        s->n_front = 1;
-        cudaError_t e = c->rcand.ensure(96, 0, st);
-        if (e == cudaSuccess) e = c->cand_slot.ensure(4, 0, st);
-        if (e != cudaSuccess) rc = fail(c, SPL_E_NOMEM, "realistic scratch alloc");
-    }
-    if (rc == SPL_OK) rc = zero_ctr(c, st);
-    if (rc == SPL_OK) rc = ensure_rtable(c, 1, st);
-    if (rc == SPL_OK && c->rocc) {  // forget the previous search
-        if (cudaMemsetAsync(c->rtable, 0, c->rnb * 64, st) != cudaSuccess) rc = fail(c, SPL_E_CUDA, "realistic table reset failed");
-        c->rocc = 0;
-    }
-    if (rc == SPL_OK) {
-        uint64_t tag;
-        rc = next_epoch(c, tag);
-        if (rc == SPL_OK) {
-            r_probe_kernel<<<1, TILE, 0, st>>>(s->front.as<RRec>(), 1, c->rcfg.as<RConfigDev>(), c->rtable, c->rnb, tag,
-                                                c->cand_slot.as<uint32_t>(), c->d_ctr);
-            ++c->launches;
-            c->rocc = 1;
-            c->occupied = 1;
-        }
-    }
-    if (rc == SPL_OK) rc = save_links(s, s->n_front, true, false, st);
-    if (rc == SPL_OK && cudaStreamSynchronize(st) != cudaSuccess) rc = fail(c, SPL_E_CUDA, "rsolver create sync failed");
-    if (rc != SPL_OK) { delete s; return rc; }
-    s->activate();
-    *out = s;
-    return SPL_OK;
+    return open_solver(s, REALISTIC, root_rec_host, 96, false, "rsolver create sync failed", out);
 }
 
 int32_t spl_rsolver_frontier(spl_solver *s, const void **recs, int64_t *n) {
-    if (!s || !recs || !n || !s->realistic) return SPL_E_INVALID;
+    if (!s || !recs || !n || s->kind != REALISTIC) return SPL_E_INVALID;
     *recs = s->front.p;
     *n = s->n_front;
     return SPL_OK;
@@ -2794,14 +2710,13 @@ int32_t spl_rreset_visited(spl_ctx *c, void *stream) {
     // the speedrun table is cleared too, as spl_rsolver_create does: both tables share the epoch counter, which can only
     // restart at 0 once neither holds a tag (every spl_rdedup_flags call takes one epoch; TAG_MAX bounds them per search)
     CKS(c, reset_visited(c, st));
-    if (c->rtable && c->rocc) CK(c, cudaMemsetAsync(c->rtable, 0, c->rnb * 64, st));
-    c->rocc = 0;
+    CK(c, c->rtab.clear(st));
     return SPL_OK;
 }
 
 int32_t spl_rvisited_count(spl_ctx *c, int64_t *n_host) {
     if (!c || !n_host) return SPL_E_INVALID;
-    *n_host = (int64_t)c->rocc;
+    *n_host = (int64_t)c->rtab.occ;
     return SPL_OK;
 }
 
@@ -2814,15 +2729,9 @@ int32_t spl_solver_cut(spl_solver *s, const uint8_t *draws, int64_t n_draws, spl
     CK(c, enter_device(c));
     *info = s->pend_info;
     s->pending = false;
-    if (s->realistic) return realistic_cut(s, info, s->pend_n, s->pend_uniq, draws, st);
-    CKS(c, zero_ctr(c, st));
-    CK(c, c->sk.ensure((size_t)s->pend_uniq * 8, 0, st));
-    score_ext_kernel<<<nblk(s->pend_uniq), TILE, 0, st>>>(s->uniq.as<Rec>(), draws, s->pend_uniq, s->heuristic, c->luts,
-                                                            c->sk.as<uint64_t>(), c->d_ctr);
-    ++c->launches;
-    CK(c, cudaGetLastError());
-    CKS(c, read_ctr(c, st));
-    return speedrun_cut(s, info, s->pend_n, s->pend_uniq, c->h_ctr->sk_min, c->h_ctr->sk_max, st);
+    LevelExpand x;
+    x.n_uniq = x.n_slots = s->pend_uniq;
+    return level_cut(s, info, s->pend_n, x, draws, st);
 }
 
 int32_t spl_solver_frontier(spl_solver *s, const spl_key **keys, const uint64_t **aux, const uint64_t **link, int64_t *n) {
