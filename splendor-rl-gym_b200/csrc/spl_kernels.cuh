@@ -54,10 +54,9 @@ __device__ __forceinline__ void load_tabs(SmemTabs &s, const DevTables *__restri
     for (int i = threadIdx.x; i < SPL_NUM_CARDS; i += blockDim.x) s.card[i] = g->card[i];
 }
 
-// buys mask (key layout) and take-table entry of one parent: State.__iter__ :360-369, :381
-__device__ __forceinline__ void derive_parent(const SmemTabs &s, const uint32_t *__restrict__ takes_idx, uint64_t lo,
-                                              uint64_t hi, uint64_t aux, uint64_t &bm_lo, uint64_t &bm_hi,
-                                              uint32_t &nb, uint32_t &tk) {
+// buys mask (key layout) of one parent: State.__iter__ :360-369
+__device__ __forceinline__ void buy_mask(const SmemTabs &s, uint64_t lo, uint64_t hi, uint64_t aux, uint64_t &bm_lo,
+                                         uint64_t &bm_hi) {
     const uint32_t g = (uint32_t)(lo & GEM_MASK);
     bm_lo = ~lo;
     bm_hi = ~hi & HI_KEY_MASK;
@@ -68,8 +67,14 @@ __device__ __forceinline__ void derive_parent(const SmemTabs &s, const uint32_t 
         bm_lo &= s.buy_lo[c][v];
         bm_hi &= s.buy_hi[c][v];
     }
+}
+// buys mask and take-table entry of one parent: State.__iter__ :360-369, :381
+__device__ __forceinline__ void derive_parent(const SmemTabs &s, const uint32_t *__restrict__ takes_idx, uint64_t lo,
+                                              uint64_t hi, uint64_t aux, uint64_t &bm_lo, uint64_t &bm_hi,
+                                              uint32_t &nb, uint32_t &tk) {
+    buy_mask(s, lo, hi, aux, bm_lo, bm_hi);
     nb = __popcll(bm_lo) + __popcll(bm_hi);
-    tk = __ldg(takes_idx + g);
+    tk = __ldg(takes_idx + (uint32_t)(lo & GEM_MASK));
 }
 
 __device__ __forceinline__ int nth_set_bit64(uint64_t m, int n) {
@@ -317,6 +322,25 @@ __device__ __forceinline__ uint32_t buy_gems(const SmemTabs &s, uint64_t lo, uin
     }
     return ng;
 }
+// owns card `pos` (key bit) from now on
+__device__ __forceinline__ void set_key_bit(uint64_t &lo, uint64_t &hi, int pos) {
+    if (pos < 64) lo |= 1ull << pos; else hi |= 1ull << (pos - 64);
+}
+// key and aux of the successor that buys card `pos` (State.buy_card :338-355): new gems, the card, saved gems,
+// points and bonus
+__device__ __forceinline__ void buy_child(const SmemTabs &s, uint64_t lo, uint64_t hi, uint64_t aux, int pos, uint64_t &clo,
+                                          uint64_t &chi, uint64_t &caux) {
+    uint32_t saved, cd;
+    const uint32_t ng = buy_gems(s, lo, aux, pos, saved, cd);
+    clo = (lo & ~GEM_MASK) | ng;
+    chi = hi;
+    set_key_bit(clo, chi, pos);
+    caux = aux + saved + ((uint64_t)((cd >> 15) & 7) << 16) + (1ull << (24 + 5 * ((cd >> 18) & 7)));
+}
+// ordinal of that successor in list(iter(parent)): the buys come first, in ascending card order
+__device__ __forceinline__ uint32_t buy_ordinal(uint64_t bm_lo, uint64_t bm_hi, int pos) {
+    return pos < 64 ? __popcll(bm_lo & ((1ull << pos) - 1)) : __popcll(bm_lo) + __popcll(bm_hi & ((1ull << (pos - 64)) - 1));
+}
 
 constexpr int BUY_WIN = 4096;  // buy-list window (entries) staged in shared memory
 
@@ -415,17 +439,13 @@ __global__ void __launch_bounds__(TILE) expand_kernel(const Rec *__restrict__ fr
         for (uint32_t i = tid; i < nbw; i += TILE) {
             const uint32_t ent = S.blist[i], j = ent >> 7;
             const int pos = ent & 127;
-            const uint64_t lo = S.lo[j], aux = S.aux[j];
-            uint32_t saved, cd;
-            const uint32_t ng = buy_gems(S.tabs, lo, aux, pos, saved, cd);
-            uint64_t klo = (lo & ~GEM_MASK) | ng, khi = S.hi[j];
-            if (pos < 64) klo |= 1ull << pos; else khi |= 1ull << (pos - 64);
+            uint64_t klo, khi, caux;
+            buy_child(S.tabs, S.lo[j], S.hi[j], S.aux[j], pos, klo, khi, caux);
             const uint32_t ord = w0 + i - S.prefb[j];
             const uint32_t tt = c0 + S.pref[j] + ord;
             if (MODE == MODE_PROBE) {
                 cand_slot[tt] = probe_ident<IDENT>(table, cap, tag, klo, khi, ~(uint64_t)tt, n_new, &ctr->error);
             } else {
-                const uint64_t caux = aux + saved + ((uint64_t)((cd >> 15) & 7) << 16) + (1ull << (24 + 5 * ((cd >> 18) & 7)));
                 Rec r{klo, khi, caux, ((uint64_t)(rank_base + p0 + j) << 8) | ord};
                 st_rec(cand_out + tt, r);
             }

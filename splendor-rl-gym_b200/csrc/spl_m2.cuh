@@ -8,12 +8,13 @@
 //
 //   visited set  = open-addressed table of 384-byte NODES, one per card set that was ever generated:
 //                  {90-bit card mask, 2898-bit bitmap over the gem hands}  (`trail` membership = one bit)
-//   one level    = 1. m2_count / m2_buys : per-parent fan-out; card buys are written out as 32-byte
-//                     records (they change the card set); gem takes are NOT materialised
-//                  2. LSD radix sort of {parents, buy records} by the hash of their (target) card set
+//   one level    = 1. m2_count / m2_buys : per-parent fan-out; every card buy (it changes the card set) becomes
+//                     one 8-byte sort item {target card-set hash, parent, card}; gem takes are NOT materialised
+//                  2. LSD radix sort of {parents, buys} by the hash of their (target) card set
 //                  3. m2_runs : boundaries of equal-hash runs + candidate-weight prefix
 //                  4. m2_group_small / m2_group_big : one warp / one CTA per run loads the node, replays
-//                     the takes of the run's parents and the run's buy records against an ON-CHIP table
+//                     the takes of the run's parents and the run's buys (rebuilt from their parents' records)
+//                     against an ON-CHIP table
 //                     (min arrival index per gem hand, src/solver.py:447-450 first arrival wins), emits the
 //                     winners with their scores and sets their bits.  No global atomics per candidate,
 //                     no second visit to the table.
@@ -39,6 +40,13 @@ constexpr int CLS_WARP = 6, CLS_CTA = 7;
 constexpr int M2_WARPS = TILE / 32;
 constexpr int BIG_DONE = 16;           // card sets of a run the CTA kernel remembers as done: it walks at most BIG_DONE + 1 per run
 constexpr int BIG_AT_BITS = 24;        // item offset inside a run, packed under the arrival index in the CTA kernel's table
+// Item id (low 32 bits of a sort item) of a round on one GPU: parent p of the round is id p, the buy of card `pos` (key
+// bit) by parent p is ITEM_BUY | p << 7 | pos.  The buy is not stored anywhere else: the dedup kernels rebuild it from
+// the parent's record (load_buy).  Every parent id (< np) is below every buy id.  Rounds of the card-set-sharded driver
+// number their received buy records np + i instead.
+constexpr int ITEM_PARENT_BITS = 24;   // parents of one round: at most 2^24 (splendor_b200.cu clamps chunk_parents to it)
+constexpr uint32_t ITEM_BUY = 1u << 31;
+__device__ __forceinline__ uint32_t buy_item_id(uint32_t p, int pos) { return ITEM_BUY | p << 7 | (uint32_t)pos; }
 
 // card mask of a key as two words (90 bits)
 __device__ __host__ __forceinline__ void mask_words(uint64_t lo, uint64_t hi, uint64_t &m0, uint64_t &m1) {
@@ -150,11 +158,11 @@ __global__ void __launch_bounds__(TILE) m2_count_kernel(const Rec *__restrict__ 
     if (p < np) boff[p] = (uint32_t)(s_base + excl);
 }
 
-// card buys of the round's parents (src/solver.py:369-374, State.buy_card :338-355) as 32-byte records
-// {child key, child aux, link = parent rank << 8 | ordinal}; also their items (sort key + item id)
+// card buys of the round's parents (src/solver.py:369-374) as items: high half of the hash of the child's card set
+// (the parent's plus card `pos`) << 32 | buy_item_id(parent, pos), at np + boff[parent] + ordinal
 struct BuySmem {
     SmemTabs tabs;
-    uint64_t lo[TILE], hi[TILE], aux[TILE];
+    uint64_t lo[TILE], hi[TILE];
     uint32_t prefb[TILE + 1];
     uint16_t blist[BUY_WIN];
     uint32_t warp_sums[TILE / 32 + 1];
@@ -162,8 +170,7 @@ struct BuySmem {
 __global__ void __launch_bounds__(TILE) m2_buys_kernel(const Rec *__restrict__ front, int64_t np,
                                                        const DevTables *__restrict__ tabs,
                                                        const uint32_t *__restrict__ takes_idx,
-                                                       const uint32_t *__restrict__ boff, int64_t rank_base,
-                                                       Rec *__restrict__ brec, uint64_t *__restrict__ iv) {
+                                                       const uint32_t *__restrict__ boff, uint64_t *__restrict__ iv) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     BuySmem &S = *reinterpret_cast<BuySmem *>(smem_raw);
     const unsigned tid = threadIdx.x;
@@ -177,7 +184,7 @@ __global__ void __launch_bounds__(TILE) m2_buys_kernel(const Rec *__restrict__ f
         Rec r;
         ld_rec(front + p, r);
         derive_parent(S.tabs, takes_idx, r.lo, r.hi, r.aux, bm_lo, bm_hi, nb, tk);
-        S.lo[tid] = r.lo; S.hi[tid] = r.hi; S.aux[tid] = r.aux;
+        S.lo[tid] = r.lo; S.hi[tid] = r.hi;
     }
     uint32_t total_buys;
     const uint32_t prefb = block_excl_scan(nb, S.warp_sums, total_buys);
@@ -207,19 +214,11 @@ __global__ void __launch_bounds__(TILE) m2_buys_kernel(const Rec *__restrict__ f
         for (uint32_t i = tid; i < nbw; i += TILE) {
             const uint32_t ent = S.blist[i], j = ent >> 7;
             const int pos = ent & 127;
-            const uint64_t lo = S.lo[j], aux = S.aux[j];
-            uint32_t saved, cd;
-            const uint32_t ng = buy_gems(S.tabs, lo, aux, pos, saved, cd);
-            uint64_t klo = (lo & ~GEM_MASK) | ng, khi = S.hi[j];
-            if (pos < 64) klo |= 1ull << pos; else khi |= 1ull << (pos - 64);
-            const uint32_t ord = w0 + i - S.prefb[j];
-            const uint64_t caux = aux + saved + ((uint64_t)((cd >> 15) & 7) << 16) + (1ull << (24 + 5 * ((cd >> 18) & 7)));
-            const uint64_t g = (uint64_t)b0 + w0 + i;  // == boff[parent] + ord
-            Rec r{klo, khi, caux, ((uint64_t)(rank_base + p0 + j) << 8) | ord};
-            st_rec(brec + g, r);
-            uint64_t m0, m1;
+            uint64_t klo = S.lo[j], khi = S.hi[j], m0, m1;
+            set_key_bit(klo, khi, pos);
             mask_words(klo, khi, m0, m1);
-            iv[np + g] = (mask_hash(m0, m1) & 0xFFFFFFFF00000000ull) | (uint64_t)(np + g);
+            const uint64_t g = (uint64_t)b0 + w0 + i;  // == boff[parent] + ordinal
+            iv[np + g] = (mask_hash(m0, m1) & 0xFFFFFFFF00000000ull) | buy_item_id((uint32_t)(p0 + j), pos);
         }
     }
 }
@@ -528,8 +527,8 @@ __global__ void __launch_bounds__(TILE) m2_runs_kernel(const uint64_t *__restric
 // ------------------------------------------------------------------ 4. per-run dedup
 struct GroupArgs {
     const Rec *front;              // the round's parents (rank order)
-    const Rec *brec;               // the round's buy records
-    const uint64_t *iv;            // sorted items: hash half << 32 | item id (id < np: parent, else np + buy index)
+    const Rec *brec;               // the buy records the round received (card-set-sharded driver; one GPU: none)
+    const uint64_t *iv;            // sorted items: hash half << 32 | item id (id < np: parent; else a buy, see ITEM_BUY)
     const uint32_t *run_start, *run_wpre;
     uint32_t np;
     int64_t rank_base;             // global rank of parent 0 of the round (when the parents' ranks are contiguous) ...
@@ -565,6 +564,35 @@ struct GroupArgs {
 __device__ __forceinline__ uint32_t item_id(const GroupArgs &A, uint32_t i) { return (uint32_t)A.iv[i]; }
 __device__ __forceinline__ uint64_t parent_rank(const GroupArgs &A, uint32_t id) {
     return A.grank ? A.grank[id] : (uint64_t)(A.rank_base + id);
+}
+// the buy record {child key, child aux, link = parent rank << 8 | ordinal} of item id `id` (>= np): as received
+// (UNORDERED), or rebuilt from the record of the parent and the card named in the id
+template <bool UNORDERED>
+__device__ __forceinline__ void load_buy(const GroupArgs &A, const SmemTabs &tabs, uint32_t id, Rec &b) {
+    if (UNORDERED) {
+        ld_rec(A.brec + (id - A.np), b);
+        return;
+    }
+    const uint32_t p = (id >> 7) & ((1u << ITEM_PARENT_BITS) - 1);
+    const int pos = id & 127;
+    Rec par;
+    ld_rec(A.front + p, par);
+    buy_child(tabs, par.lo, par.hi, par.aux, pos, b.lo, b.hi, b.aux);
+    uint64_t bl, bh;
+    buy_mask(tabs, par.lo, par.hi, par.aux, bl, bh);
+    b.link = (uint64_t)(A.rank_base + p) << 8 | buy_ordinal(bl, bh, pos);
+}
+// only the key words {lo, hi} of buy item `id` (the thread kernel's first look at a run)
+template <bool UNORDERED>
+__device__ __forceinline__ void load_buy_key(const GroupArgs &A, const SmemTabs &tabs, uint32_t id, uint64_t &lo, uint64_t &hi) {
+    if (UNORDERED) {
+        ld_cg_u64x2(reinterpret_cast<const uint64_t *>(A.brec + (id - A.np)), lo, hi);
+        return;
+    }
+    Rec b;
+    load_buy<false>(A, tabs, id, b);
+    lo = b.lo;
+    hi = b.hi;
 }
 
 // per-warp winner staging: records are collected in shared memory and written out 17..48 at a time behind one
@@ -704,22 +732,14 @@ __device__ __forceinline__ void take_steps(const GroupArgs &A, WarpStage &W, uin
         bm_step(A, W, bm, act, false, g, (pgr << 8) | (pnb + q), (plo & ~GEM_MASK) | g, phi, paux);
     }
 }
-// item `i` of the sorted list -> record, parent fan-out, card-set words
-__device__ __forceinline__ void load_item(const GroupArgs &A, const SmemTabs &tabs, uint32_t i, Rec &it, bool &isP, uint32_t &nb,
-                                          uint32_t &tk, uint64_t &grank, uint64_t &m0, uint64_t &m1) {
+// parent item `i` of the sorted list -> record, fan-out, rank, card-set words
+__device__ __forceinline__ void load_parent_item(const GroupArgs &A, const SmemTabs &tabs, uint32_t i, Rec &it, uint32_t &nb,
+                                                 uint32_t &tk, uint64_t &grank, uint64_t &m0, uint64_t &m1) {
     const uint32_t id = item_id(A, i);
-    isP = id < A.np;
-    nb = tk = 0;
-    grank = 0;
-    if (isP) {
-        ld_rec(A.front + id, it);
-        uint64_t bl, bh;
-        derive_parent(tabs, A.takes_idx, it.lo, it.hi, it.aux, bl, bh, nb, tk);
-        grank = parent_rank(A, id);
-    } else {
-        ld_rec(A.brec + (id - A.np), it);
-        grank = it.link >> 8;  // rank of the generating parent
-    }
+    ld_rec(A.front + id, it);
+    uint64_t bl, bh;
+    derive_parent(tabs, A.takes_idx, it.lo, it.hi, it.aux, bl, bh, nb, tk);
+    grank = parent_rank(A, id);
     mask_words(it.lo, it.hi, m0, m1);
 }
 __device__ __forceinline__ void warp_epilogue(const GroupArgs &A, WarpStage &W, uint32_t n_fresh) {
@@ -824,8 +844,9 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
             uint64_t M0 = 0, M1 = 0;
             if (lane == 0) {
                 const uint32_t id = item_id(A, lead);
-                const Rec *src = id < A.np ? A.front + id : A.brec + (id - A.np);
-                mask_words(src->lo, src->hi, M0, M1);
+                Rec src;
+                if (id < A.np) ld_rec(A.front + id, src); else load_buy<UNORDERED>(A, S.tabs, id, src);
+                mask_words(src.lo, src.hi, M0, M1);
             }
             M0 = __shfl_sync(0xffffffffu, M0, 0); M1 = __shfl_sync(0xffffffffu, M1, 0);
             uint64_t *N = node_open(A, M0, M1, bm, n_fresh);
@@ -838,9 +859,8 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
             for (;;) {
                 if (!pmask && pnext < pe) {  // refill the parent window
                     const bool valid = pnext + lane < pe;
-                    bool p_;
                     uint64_t m0 = 0, m1 = 0;
-                    if (valid) load_item(A, S.tabs, pnext + lane, it, p_, nb, tk, grank, m0, m1);
+                    if (valid) load_parent_item(A, S.tabs, pnext + lane, it, nb, tk, grank, m0, m1);
                     const bool ok = valid && m0 == M0 && m1 == M1;
                     bool other = valid && !ok;  // a card set not walked yet?
 #pragma unroll
@@ -856,7 +876,7 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
                     uint64_t m0 = 0, m1 = 0;
                     if (valid) {
                         const uint32_t at = resort ? pe + (uint32_t)(bs[bnext - pe + lane] & 1023u) : bnext + lane;
-                        ld_rec(A.brec + (item_id(A, at) - A.np), bt);
+                        load_buy<UNORDERED>(A, S.tabs, item_id(A, at), bt);
                         mask_words(bt.lo, bt.hi, m0, m1);
                         brank = bt.link >> 8;
                     }
@@ -929,6 +949,11 @@ template <bool UNORDERED>
 __global__ void __launch_bounds__(TILE) m2_group_tiny_kernel(GroupArgs A, uint32_t n_runs) {
     __shared__ uint32_t warp_sums[TILE / 32 + 1];
     __shared__ uint64_t s_base;
+    __shared__ SmemTabs tabs;  // the buys are rebuilt from their parents (one GPU)
+    if (!UNORDERED) {
+        load_tabs(tabs, A.tabs);
+        __syncthreads();
+    }
     const unsigned lane = threadIdx.x & 31;
     const uint32_t r = blockIdx.x * TILE + threadIdx.x;
     int cls = -1;  // -1 none, 0 handled here, CLS_WARP / CLS_CTA queued
@@ -945,7 +970,7 @@ __global__ void __launch_bounds__(TILE) m2_group_tiny_kernel(GroupArgs A, uint32
         else cls = wgt <= A.warp_max ? CLS_WARP : CLS_CTA;
         if (cls == 0) {
             uint64_t lo0, hi0, M0, M1;
-            ld_cg_u64x2(reinterpret_cast<const uint64_t *>(A.brec + (id0 - A.np)), lo0, hi0);
+            load_buy_key<UNORDERED>(A, tabs, id0, lo0, hi0);
             mask_words(lo0, hi0, M0, M1);
             uint32_t gp[TINY_ITEMS / 2];  // gem hands, two per word
 #pragma unroll
@@ -956,7 +981,7 @@ __global__ void __launch_bounds__(TILE) m2_group_tiny_kernel(GroupArgs A, uint32
             for (int j = 1; j < TINY_ITEMS; ++j) {
                 if (j < (int)cnt) {
                     uint64_t lo, hi, m0, m1;
-                    ld_cg_u64x2(reinterpret_cast<const uint64_t *>(A.brec + (item_id(A, s + j) - A.np)), lo, hi);
+                    load_buy_key<UNORDERED>(A, tabs, item_id(A, s + j), lo, hi);
                     mask_words(lo, hi, m0, m1);
                     same = same && m0 == M0 && m1 == M1;
                     gp[j >> 1] |= (uint32_t)(lo & GEM_MASK) << (16 * (j & 1));
@@ -1011,7 +1036,7 @@ __global__ void __launch_bounds__(TILE) m2_group_tiny_kernel(GroupArgs A, uint32
     for (uint32_t m = winmask; m; m &= m - 1) {
         const int j = __ffs(m) - 1;
         Rec it;
-        ld_rec(A.brec + (item_id(A, s + j) - A.np), it);
+        load_buy<UNORDERED>(A, tabs, item_id(A, s + j), it);
         st_rec(A.out + pos, it);
         const uint64_t k = flip_f64((uint64_t)__double_as_longlong(score_state(A.h, A.noise_mode, it.lo, it.hi & HI_KEY_MASK, it.aux, A.L)));
         A.out_sk[pos] = k;
@@ -1047,13 +1072,13 @@ struct BigSmem {
 // enumerate the candidates of the items of run [s, e) whose card set is (M0, M1): f(rank, t, item offset in the run)
 // (spreading the takes of a batch of items evenly over the threads was measured: slower, the extra barriers cost more
 // than the serial take loops)
-template <class F>
+template <bool UNORDERED, class F>
 __device__ __forceinline__ void big_enumerate(const GroupArgs &A, BigSmem &S, uint32_t s, uint32_t e, uint64_t M0, uint64_t M1, F &&f) {
     for (uint32_t i = s + threadIdx.x; i < e; i += TILE) {
         const uint32_t id = item_id(A, i);
         Rec it;
         const bool isP = id < A.np;
-        if (isP) ld_rec(A.front + id, it); else ld_rec(A.brec + (id - A.np), it);
+        if (isP) ld_rec(A.front + id, it); else load_buy<UNORDERED>(A, S.tabs, id, it);
         uint64_t m0, m1;
         mask_words(it.lo, it.hi, m0, m1);
         if (m0 != M0 || m1 != M1) {  // another card set with the same sort key: remember the first one not done yet
@@ -1075,6 +1100,7 @@ __device__ __forceinline__ void big_enumerate(const GroupArgs &A, BigSmem &S, ui
     }
 }
 
+template <bool UNORDERED>
 __global__ void __launch_bounds__(TILE) m2_group_big_kernel(GroupArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     BigSmem &S = *reinterpret_cast<BigSmem *>(smem_raw);
@@ -1102,8 +1128,9 @@ __global__ void __launch_bounds__(TILE) m2_group_big_kernel(GroupArgs A) {
             __syncthreads();
             if (tid == 0) {
                 const uint32_t id = item_id(A, lead);
-                const Rec *src = id < A.np ? A.front + id : A.brec + (id - A.np);
-                mask_words(src->lo, src->hi, S.m0, S.m1);
+                Rec src;
+                if (id < A.np) ld_rec(A.front + id, src); else load_buy<UNORDERED>(A, S.tabs, id, src);
+                mask_words(src.lo, src.hi, S.m0, S.m1);
                 bool fresh;
                 S.node = node_find_or_create(A.nodes, A.nn, S.m0, S.m1, fresh, &A.ctr->error);
                 S.fresh = fresh;
@@ -1119,7 +1146,7 @@ __global__ void __launch_bounds__(TILE) m2_group_big_kernel(GroupArgs A) {
             // pass 0: first arrival per gem hand among the candidates not in the visited set; the table word is
             // arrival index << 24 | offset of the producing item in the run (a run holds < 2^24 items: at most
             // BIG_DONE + 1 card sets of <= 2898 parents and their predecessors' buy records; arrival indices are < 2^40)
-            big_enumerate(A, S, s, e, M0, M1, [&](uint32_t rk, uint64_t t, uint32_t at) {
+            big_enumerate<UNORDERED>(A, S, s, e, M0, M1, [&](uint32_t rk, uint64_t t, uint32_t at) {
                 if (!((S.bm[rk >> 6] >> (rk & 63)) & 1))
                     atomicMin(reinterpret_cast<unsigned long long *>(&S.tbl[rk]), (unsigned long long)((t << BIG_AT_BITS) | at));
             });
@@ -1141,7 +1168,7 @@ __global__ void __launch_bounds__(TILE) m2_group_big_kernel(GroupArgs A) {
                     ld_rec(A.front + id, o);
                     o.lo = (o.lo & ~GEM_MASK) | __ldg(A.rankgems + rk);
                 } else {
-                    ld_rec(A.brec + (id - A.np), o);
+                    load_buy<UNORDERED>(A, S.tabs, id, o);
                 }
                 o.link = v >> BIG_AT_BITS;
                 st_rec(A.out + pos, o);

@@ -19,6 +19,11 @@
 
 using namespace spl;
 
+// parents per round of a level (spl_config.chunk_parents is clamped to it); a grouped round numbers its parents in the
+// ITEM_PARENT_BITS of a buy's sort item
+constexpr uint64_t MAX_CHUNK_PARENTS = 16ull << 20;
+static_assert(MAX_CHUNK_PARENTS <= (1ull << ITEM_PARENT_BITS), "a round's parent index must fit the item of its buys");
+
 static std::string g_create_error;
 
 struct DevBuf {
@@ -142,7 +147,7 @@ struct spl_ctx {
     uint64_t spilled_bytes = 0;        // link-column bytes moved to pinned host memory so far
     uint16_t *d_gemrank = nullptr;
     uint16_t *d_rankgems = nullptr;   // inverse of d_gemrank
-    DevBuf brec, ntk8, boff2, run_start, run_wpre, cls_list;
+    DevBuf ntk8, boff2, run_start, run_wpre, cls_list;
     // constant tables
     DevTables *d_tabs = nullptr;
     uint32_t *d_takes_idx = nullptr;
@@ -289,7 +294,7 @@ int32_t spl_create(const spl_config *cfg, spl_ctx **out) {
     CKC(cudaMemGetInfo(&free_b, &total_b));
     c->key.max_bytes = c->rtab.max_bytes = cfg->max_table_bytes ? cfg->max_table_bytes : (uint64_t)(free_b * 0.6);
     c->chunk_user = cfg->chunk_parents != 0;
-    c->chunk_parents = cfg->chunk_parents ? std::min<uint64_t>(cfg->chunk_parents, 16ull << 20) : (4ull << 20);
+    c->chunk_parents = cfg->chunk_parents ? std::min<uint64_t>(cfg->chunk_parents, MAX_CHUNK_PARENTS) : (4ull << 20);
     c->chunk_parents = std::max<uint64_t>(c->chunk_parents, TILE);
     const HostTables &T = host_tables();
     CKC(cudaMalloc(&c->d_tabs, sizeof(DevTables)));
@@ -330,7 +335,8 @@ int32_t spl_create(const spl_config *cfg, spl_ctx **out) {
     CKC(cudaFuncSetAttribute(m2_buys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BuySmem)));
     CKC(cudaFuncSetAttribute(m2_group_warp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)offsetof(WarpSmem, bsort)));
     CKC(cudaFuncSetAttribute(m2_group_warp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(WarpSmem)));
-    CKC(cudaFuncSetAttribute(m2_group_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BigSmem)));
+    CKC(cudaFuncSetAttribute(m2_group_big_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BigSmem)));
+    CKC(cudaFuncSetAttribute(m2_group_big_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BigSmem)));
     CKC(cudaFuncSetAttribute(os_scatter_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)offsetof(OsSmem, stage_p)));
     CKC(cudaFuncSetAttribute(os_scatter_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(OsSmem)));
     CKC(cudaFuncSetAttribute(gs_buys_route_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RouteSmem)));
@@ -1380,7 +1386,7 @@ static int sort_items(spl_ctx *c, int64_t n_items, int *cur, cudaStream_t st) {
 // One round of a grouped level after its fan-out, the same on one GPU and on the card-set-sharded driver.
 struct GroupRound {
     const Rec *front = nullptr;      // the round's parents
-    const Rec *brec = nullptr;       // the buy records: the round's own (one GPU) or those this rank received (sharded)
+    const Rec *brec = nullptr;       // the buy records this rank received (sharded; one GPU: rebuilt from front)
     int64_t np = 0, n_items = 0;     // parents; items packed in c->y[0], the parents' first
     uint64_t n_cands = 0;            // candidates (gem takes + buy records): the most winners the round can have
     int64_t rank_base = 0;           // queue rank of front[0] (one GPU) ...
@@ -1437,7 +1443,8 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
     if (R.unordered) m2_group_warp_kernel<true><<<148 * SPL_WARP_CTAS, TILE, sizeof(WarpSmem), st>>>(A);
     else m2_group_warp_kernel<false><<<148 * SPL_WARP_CTAS, TILE, offsetof(WarpSmem, bsort), st>>>(A);  // no sort area
     CK(c, cudaEventRecord(c->ev[5], st));
-    m2_group_big_kernel<<<148 * 5, TILE, sizeof(BigSmem), st>>>(A);
+    if (R.unordered) m2_group_big_kernel<true><<<148 * 5, TILE, sizeof(BigSmem), st>>>(A);
+    else m2_group_big_kernel<false><<<148 * 5, TILE, sizeof(BigSmem), st>>>(A);
     c->launches += 3;
     CK(c, cudaGetLastError());
     CK(c, cudaEventRecord(c->ev[6], st));
@@ -1471,7 +1478,7 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
 static int grouped_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6], cudaStream_t st) {
     spl_ctx *c = s->c;
     const Rec *front = s->front.as<Rec>();
-    const int64_t chunk = c->chunk_user ? (int64_t)c->chunk_parents : (16ll << 20);
+    const int64_t chunk = c->chunk_user ? (int64_t)c->chunk_parents : (int64_t)MAX_CHUNK_PARENTS;
     int64_t n_uniq = 0, n_slots = 0, generated = 0;
     uint64_t sk_min = ~0ull, sk_max = 0;
     for (int64_t p0 = 0; p0 < n; p0 += chunk) {
@@ -1482,8 +1489,8 @@ static int grouped_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6],
         CK(c, cudaEventRecord(c->ev[0], st));
         CK(c, c->boff2.ensure((size_t)np * 4 + 4, 0, st));
         CK(c, c->ntk8.ensure((size_t)np + 8, 0, st));
-        // items of the round = parents + buy records (packed: hash half << 32 | item id); the array is sized for the
-        // parents first and grown (contents kept) once the buys are counted
+        // items of the round = parents + buys (packed: hash half << 32 | item id); the array is sized for the parents
+        // first and grown (contents kept) once the buys are counted
         CK(c, c->y[0].ensure((size_t)np * 8 + 8, 0, st));
         CKS(c, prep_status(c, 0, nt, st));
         m2_count_kernel<<<nt, TILE, 0, st>>>(front + p0, np, c->d_tabs, c->d_takes_idx, c->boff2.as<uint32_t>(),
@@ -1499,15 +1506,14 @@ static int grouped_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6],
             return fail(c, SPL_E_INVALID, "round produced %llu candidates (>= 2^32): lower spl_config.chunk_parents", (unsigned long long)total);
         CK(c, c->y[0].ensure((size_t)n_items * 8 + 8, (size_t)np * 8, st));
         CK(c, c->y[1].ensure((size_t)n_items * 8 + 8, 0, st));
-        CK(c, c->brec.ensure((size_t)n_buys * 32 + 32, 0, st));
         if (n_buys) {
-            m2_buys_kernel<<<nt, TILE, sizeof(BuySmem), st>>>(front + p0, np, c->d_tabs, c->d_takes_idx, c->boff2.as<uint32_t>(), p0,
-                                                               c->brec.as<Rec>(), c->y[0].as<uint64_t>());
+            m2_buys_kernel<<<nt, TILE, sizeof(BuySmem), st>>>(front + p0, np, c->d_tabs, c->d_takes_idx, c->boff2.as<uint32_t>(),
+                                                               c->y[0].as<uint64_t>());
             ++c->launches;
             CK(c, cudaGetLastError());
         }
         GroupRound R;
-        R.front = front + p0; R.brec = c->brec.as<Rec>(); R.np = np; R.n_items = n_items; R.n_cands = total; R.rank_base = p0;
+        R.front = front + p0; R.np = np; R.n_items = n_items; R.n_cands = total; R.rank_base = p0;
         R.out = &s->uniq; R.out_base = n_slots; R.heuristic = s->heuristic; R.noise = s->noise; R.level = s->level;
         int64_t n_new = 0;
         RoundTimes t;
@@ -1517,7 +1523,7 @@ static int grouped_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6],
         n_slots += n_new;  // dense output
         float t_count;
         cudaEventElapsedTime(&t_count, c->ev[0], c->ev[1]);
-        ms[0] += t_count;                        // fan-out + buy records
+        ms[0] += t_count;                        // fan-out + buy items
         ms[2] += t.sort;                         // item sort + runs (grouping)
         ms[1] += t.thread + t.warp + t.cta;      // per-run dedup + emit + score (the dominant stage)
         ms[5] += t.warp;                         // ... of which the warp kernel
