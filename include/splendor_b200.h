@@ -249,6 +249,14 @@ int32_t spl_count_less(spl_ctx *ctx, int32_t words, int32_t inclusive, const uin
 int32_t spl_solver_create(spl_ctx *ctx, const spl_key *root_key_host, uint64_t root_aux_host,
                           int32_t goal_pts, int32_t use_heuristic, int32_t heuristic, int64_t beam_width,
                           int32_t tie_policy, int32_t noise, int32_t keep_links, spl_solver **out);
+/* The same solve from a level-0 queue of n_rows >= 1 packed rows {lo, hi, aux, link} (32 bytes each, HOST memory) in
+ * rank order; the link words are ignored.  Every row is registered as visited (trail = {row: None for row in rows}),
+ * and spl_solver_path ends at the rank of the row the goal descends from.  spl_solver_create is this call with its
+ * root as the only row.  SPL_E_INVALID, naming the row, for an illegal gem hand (a colour above 7 or more than 10
+ * gems), a key bit at or above 105, or two rows with the same key. */
+int32_t spl_solver_create_queue(spl_ctx *ctx, const void *rows_host, int64_t n_rows, int32_t goal_pts,
+                                int32_t use_heuristic, int32_t heuristic, int64_t beam_width, int32_t tie_policy,
+                                int32_t noise, int32_t keep_links, spl_solver **out);
 int32_t spl_solver_destroy(spl_solver *s);
 /* one `while queue` iteration; returns SPL_OK and fills *info_host; info->ended tells the caller to stop */
 int32_t spl_solver_step(spl_solver *s, spl_level_info *info_host, void *stream);

@@ -49,7 +49,7 @@ def lib():
         L.orc_expand.argtypes = [C.c_void_p, C.c_void_p]
         L.orc_score.argtypes = [C.c_void_p, C.c_int, C.c_int]
         L.orc_score.restype = C.c_double
-        L.orc_solver_new.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int]
+        L.orc_solver_new.argtypes = [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int]
         L.orc_solver_new.restype = C.c_void_p
         L.orc_solver_free.argtypes = [C.c_void_p]
         L.orc_solver_set_identity.argtypes = [C.c_void_p, C.c_int]
@@ -153,14 +153,20 @@ def score(states: np.ndarray, heuristic: str, noise: str = 'const') -> np.ndarra
 
 
 class Solver:
-    """Level stepper over the oracle's restatement of State.solve (src/solver.py:390-464)."""
+    """Level stepper over the oracle's restatement of State.solve (src/solver.py:390-464).  `root`: the packed
+    state(s) of level 0 in rank order (fields lo, hi, aux; others ignored), each registered as visited."""
 
     def __init__(self, goal_pts=15, *, use_heuristic=False, heuristic_name='simple', beam_width=300_000,
                  policy='stable', noise='const', root=None, identity='key'):
         if root is None:
             root = pack_state((), (0,) * 5, (0,) * 5, 0, 0)
-        self._root = np.ascontiguousarray(root)
-        self._h = lib().orc_solver_new(self._root.ctypes.data, goal_pts, int(use_heuristic),
+        root = np.asarray(root).reshape(-1)
+        if len(root) < 1:
+            raise ValueError('the level-0 queue needs at least one state')
+        self._root = np.zeros(len(root), STATE_DTYPE)
+        for f in ('lo', 'hi', 'aux'):
+            self._root[f] = root[f]
+        self._h = lib().orc_solver_new(self._root.ctypes.data, len(self._root), goal_pts, int(use_heuristic),
                                        HEURISTIC_IDS.get(heuristic_name, 0), beam_width,
                                        POLICY_IDS[policy], NOISE_IDS[noise])
         if identity != 'key':  # 'pyhash': dedup on the reference's own 64-bit hash((cards, gems))

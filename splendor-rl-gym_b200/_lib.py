@@ -98,6 +98,7 @@ def _load():
         'spl_rreset_visited': (i32, [vp, vp]),
         'spl_rvisited_count': (i32, [vp, C.POINTER(i64)]),
         'spl_solver_create': (i32, [vp, C.POINTER(Key), u64, i32, i32, i32, i64, i32, i32, i32, C.POINTER(vp)]),
+        'spl_solver_create_queue': (i32, [vp, vp, i64, i32, i32, i32, i64, i32, i32, i32, C.POINTER(vp)]),
         'spl_solver_destroy': (i32, [vp]),
         'spl_solver_step': (i32, [vp, C.POINTER(LevelInfo), vp]),
         'spl_solver_cut': (i32, [vp, vp, i64, C.POINTER(LevelInfo), vp]),

@@ -458,8 +458,9 @@ __global__ void __launch_bounds__(TILE) expand_kernel(const Rec *__restrict__ fr
     }
 }
 
-// probe/insert of a materialised candidate list (stage operator spl_dedup; multi-GPU owner side)
-template <int IDENT>
+// probe/insert of a materialised candidate list (stage operator spl_dedup; multi-GPU owner side); key t is
+// keys[t * STRIDE] (STRIDE = 2: the keys of 32-byte records, as a solver's level-0 queue holds them)
+template <int IDENT, int STRIDE = 1>
 __global__ void __launch_bounds__(TILE) probe_list_kernel(const spl_key *__restrict__ keys, int64_t n,
                                                           uint64_t *__restrict__ table, uint64_t cap, uint64_t tag,
                                                           uint32_t *__restrict__ cand_slot, Counters *ctr) {
@@ -467,7 +468,7 @@ __global__ void __launch_bounds__(TILE) probe_list_kernel(const spl_key *__restr
     uint32_t n_new = 0;
     if (t < n) {
         uint64_t a, b;
-        ld_cg_u64x2(reinterpret_cast<const uint64_t *>(keys + t), a, b);
+        ld_cg_u64x2(reinterpret_cast<const uint64_t *>(keys + t * STRIDE), a, b);
         cand_slot[t] = probe_ident<IDENT>(table, cap, tag, a, b & HI_KEY_MASK, ~(uint64_t)t, n_new, &ctr->error);
     }
 #pragma unroll

@@ -84,9 +84,13 @@ __device__ __forceinline__ bool node_bit(const uint64_t *N, uint32_t r) {
     return (w >> (r & 63)) & 1;
 }
 
-// trail = {root: None} (src/solver.py:426)
-__global__ void m2_root_kernel(uint64_t *nodes, uint64_t nn, uint64_t lo, uint64_t hi, const uint16_t *__restrict__ gemrank,
-                               Counters *ctr) {
+// trail = {row: None for row in rows} (src/solver.py:426): one thread per row of the level-0 queue.  The host has
+// checked that every row has a legal gem hand and that no two rows share a key.
+__global__ void m2_root_kernel(uint64_t *nodes, uint64_t nn, const Rec *__restrict__ rows, int64_t n,
+                               const uint16_t *__restrict__ gemrank, Counters *ctr) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const uint64_t lo = rows[t].lo, hi = rows[t].hi;
     uint64_t m0, m1;
     mask_words(lo, hi, m0, m1);
     bool fresh;

@@ -1544,42 +1544,48 @@ static int open_rtable(spl_ctx *c, cudaStream_t st) {
     return SPL_OK;
 }
 
-// What every solver create shares: clear the visited sets, upload the root record (`root_bytes`: a 32-byte Rec or a
-// 96-byte realistic record) and, on the card-set-sharded driver, its global rank 0; register the root in the visited
-// table of the level kind (trail = {self: None}); save the first link columns, synchronise and go live.  Without a
-// root (a sharded rank that does not own the root's card set) the queue starts empty.  On error `s` is deleted.
+// What every solver create shares: clear the visited sets, upload the n level-0 rows (`row_bytes` each: a 32-byte Rec
+// or a 96-byte realistic record) and, on the card-set-sharded driver, the root's global rank 0; register the rows in
+// the visited table of the level kind (trail = {row: None for row in rows}); save the first link columns, synchronise
+// and go live.  With n = 0 (a sharded rank that does not own the root's card set) the queue starts empty.  Realistic
+// mode and the sharded driver start from one root (n <= 1).  On error `s` is deleted.
 template <class S>
-static int open_solver(S *s, LevelKind kind, const void *root, size_t root_bytes, bool sharded, const char *sync_msg, S **out) {
+static int open_solver(S *s, LevelKind kind, const void *rows, int64_t n, size_t row_bytes, bool sharded, const char *sync_msg,
+                       S **out) {
     spl_ctx *c = s->c;
     const cudaStream_t st = 0;
     const int rc = [&]() -> int {
         CKS(c, reset_visited(c, st));
-        if (root) {
+        if (n) {
             const uint64_t zero = 0;
-            cudaError_t e = s->front.ensure(root_bytes, 0, st);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(s->front.p, root, root_bytes, cudaMemcpyHostToDevice, st);
+            const size_t bytes = (size_t)n * row_bytes;
+            cudaError_t e = s->front.ensure(bytes, 0, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(s->front.p, rows, bytes, cudaMemcpyHostToDevice, st);
             if (e == cudaSuccess && sharded) e = s->grank.ensure(8, 0, st);
             if (e == cudaSuccess && sharded) e = cudaMemcpyAsync(s->grank.p, &zero, 8, cudaMemcpyHostToDevice, st);
             if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-            c->h2d_bytes += root_bytes + (sharded ? 8 : 0);
+            c->h2d_bytes += bytes + (sharded ? 8 : 0);
             if (e != cudaSuccess) return fail(c, SPL_E_CUDA, "root upload: %s", cudaGetErrorString(e));
             CKS(c, zero_ctr(c, st));
             uint64_t tag = 0;
             if (kind == KEY_TABLE) {
+                CKS(c, c->key.grow(c, (uint64_t)n, st));
                 CKS(c, next_epoch(c, tag));
-                if (c->cand_slot.ensure(4, 0, st) != cudaSuccess) return fail(c, SPL_E_NOMEM, "cand_slot alloc");
+                if (c->cand_slot.ensure((size_t)n * 4, 0, st) != cudaSuccess) return fail(c, SPL_E_NOMEM, "cand_slot alloc");
                 const spl_key *k = s->front.template as<spl_key>();  // a Rec starts with its key
+                constexpr int REC_KEYS = sizeof(Rec) / sizeof(spl_key);
                 if (c->identity == IDENT_PYHASH)
-                    probe_list_kernel<IDENT_PYHASH><<<1, TILE, 0, st>>>(k, 1, c->key.as<uint64_t>(), c->key.units, tag,
-                                                                        c->cand_slot.as<uint32_t>(), c->d_ctr);
+                    probe_list_kernel<IDENT_PYHASH, REC_KEYS><<<nblk(n), TILE, 0, st>>>(k, n, c->key.as<uint64_t>(), c->key.units, tag,
+                                                                              c->cand_slot.as<uint32_t>(), c->d_ctr);
                 else
-                    probe_list_kernel<IDENT_KEY><<<1, TILE, 0, st>>>(k, 1, c->key.as<uint64_t>(), c->key.units, tag,
-                                                                     c->cand_slot.as<uint32_t>(), c->d_ctr);
-                c->key.occ = 1;
+                    probe_list_kernel<IDENT_KEY, REC_KEYS><<<nblk(n), TILE, 0, st>>>(k, n, c->key.as<uint64_t>(), c->key.units, tag,
+                                                                           c->cand_slot.as<uint32_t>(), c->d_ctr);
+                c->key.occ = (uint64_t)n;
             } else if (kind == GROUPED) {
-                const Rec *r = static_cast<const Rec *>(root);
-                m2_root_kernel<<<1, 1, 0, st>>>(c->nodes.as<uint64_t>(), c->nodes.units, r->lo, r->hi, c->d_gemrank, c->d_ctr);
-                c->nodes.occ = 1;
+                CKS(c, c->nodes.grow(c, (uint64_t)n, st));
+                m2_root_kernel<<<nblk(n), TILE, 0, st>>>(c->nodes.as<uint64_t>(), c->nodes.units, s->front.template as<Rec>(), n,
+                                                         c->d_gemrank, c->d_ctr);
+                c->nodes.occ = (uint64_t)n;  // card sets registered, at most: only the table's load factor reads it
             } else {
                 if (c->cand_slot.ensure(4, 0, st) != cudaSuccess) return fail(c, SPL_E_NOMEM, "realistic scratch alloc");
                 CKS(c, open_rtable(c, st));
@@ -1592,9 +1598,9 @@ static int open_solver(S *s, LevelKind kind, const void *root, size_t root_bytes
             }
             ++c->launches;
             CK(c, cudaGetLastError());
-            c->occupied = 1;
+            c->occupied = (uint64_t)n;
         }
-        CKS(c, save_links(s, root ? 1 : 0, kind == REALISTIC, sharded, st));
+        CKS(c, save_links(s, n, kind == REALISTIC, sharded, st));
         if (cudaStreamSynchronize(st) != cudaSuccess) return fail(c, SPL_E_CUDA, "%s", sync_msg);
         return SPL_OK;
     }();
@@ -1648,7 +1654,7 @@ int32_t spl_gs_create(spl_ctx *c, int32_t rank, int32_t world, const spl_key *ro
     mask_words(r.lo, r.hi, m0, m1);
     const bool owner = (int)owner_of_mask(m0, m1, (uint32_t)world) == rank;  // the root lives on the rank that owns its card set
     s->n_local = owner ? 1 : 0;
-    return open_solver(s, GROUPED, owner ? &r : nullptr, 32, true, "spl_gs_create: sync failed", out);
+    return open_solver(s, GROUPED, &r, owner ? 1 : 0, 32, true, "spl_gs_create: sync failed", out);
 }
 
 int32_t spl_gs_destroy(spl_gsolver *s) {
@@ -2438,16 +2444,32 @@ static int level_cut(spl_solver *s, spl_level_info *info, int64_t n, const Level
     return SPL_OK;
 }
 
-extern "C" {
-
-int32_t spl_solver_create(spl_ctx *c, const spl_key *root_key, uint64_t root_aux, int32_t goal, int32_t use_h,
-                          int32_t heuristic, int64_t beam, int32_t tie, int32_t noise, int32_t keep_links,
-                          spl_solver **out) {
-    if (!c || !root_key || !out) return fail(c, SPL_E_INVALID, "spl_solver_create: null argument");
-    if (use_h && beam < 1) return fail(c, SPL_E_INVALID, "spl_solver_create: beam_width must be >= 1");
-    if (use_h && tie != SPL_TIE_STABLE && tie != SPL_TIE_KEY) return fail(c, SPL_E_INVALID, "spl_solver_create: unknown tie policy %d", tie);
-    if (noise < 0 || noise > SPL_NOISE_EXTERNAL) return fail(c, SPL_E_INVALID, "spl_solver_create: unknown noise policy %d", noise);
-    NO_LIVE_SOLVER(c, "spl_solver_create");
+// The speedrun solver's create from a level-0 queue rows[0..n) (links ~0), checked on the host before any kernel sees
+// a row: a gem hand without a rank indexes past a node's bitmap, a key bit at or above 105 is outside the card set,
+// and a second row with the same key would be a state registered twice.
+static int create_solver(spl_ctx *c, const char *fn, const Rec *rows, int64_t n, int32_t goal, int32_t use_h,
+                         int32_t heuristic, int64_t beam, int32_t tie, int32_t noise, int32_t keep_links, spl_solver **out) {
+    if (use_h && beam < 1) return fail(c, SPL_E_INVALID, "%s: beam_width must be >= 1", fn);
+    if (use_h && tie != SPL_TIE_STABLE && tie != SPL_TIE_KEY) return fail(c, SPL_E_INVALID, "%s: unknown tie policy %d", fn, tie);
+    if (noise < 0 || noise > SPL_NOISE_EXTERNAL) return fail(c, SPL_E_INVALID, "%s: unknown noise policy %d", fn, noise);
+    const HostTables &T = host_tables();
+    for (int64_t i = 0; i < n; ++i) {
+        if (T.gemrank[rows[i].lo & GEM_MASK] == 0xFFFF)
+            return fail(c, SPL_E_INVALID, "%s: row %lld has an illegal gem hand (0x%llx)", fn, (long long)i,
+                        (unsigned long long)(rows[i].lo & GEM_MASK));
+        if (rows[i].hi & ~HI_KEY_MASK)
+            return fail(c, SPL_E_INVALID, "%s: row %lld has a key bit at or above 105", fn, (long long)i);
+    }
+    if (n > 1) {
+        std::vector<int64_t> ord(n);
+        for (int64_t i = 0; i < n; ++i) ord[i] = i;
+        const auto key_less = [&](int64_t a, int64_t b) { return rows[a].hi != rows[b].hi ? rows[a].hi < rows[b].hi : rows[a].lo < rows[b].lo; };
+        std::sort(ord.begin(), ord.end(), [&](int64_t a, int64_t b) { return key_less(a, b) || (!key_less(b, a) && a < b); });
+        for (int64_t i = 1; i < n; ++i)
+            if (!key_less(ord[i - 1], ord[i]))
+                return fail(c, SPL_E_INVALID, "%s: row %lld has the same key as row %lld", fn, (long long)ord[i], (long long)ord[i - 1]);
+    }
+    if (c->active) return fail(c, SPL_E_STATE, "%s: a solver is open on this context (destroy it first)", fn);
     CK(c, enter_device(c));
     spl_solver *s = new spl_solver(c);
     s->goal = goal; s->use_h = use_h; s->heuristic = heuristic; s->beam = beam; s->tie = tie;
@@ -2456,9 +2478,28 @@ int32_t spl_solver_create(spl_ctx *c, const spl_key *root_key, uint64_t root_aux
     // order), the reference's hash identity and externally drawn noise (arrival-ordered draws) on the key table
     const bool grouped = use_h && noise != SPL_NOISE_EXTERNAL && c->identity == IDENT_KEY && !getenv("SPL_NO_GROUPED");
     s->kind = grouped ? GROUPED : KEY_TABLE;
-    s->n_front = 1;
+    s->n_front = n;
+    return open_solver(s, s->kind, rows, n, 32, false, "solver create sync failed", out);
+}
+
+extern "C" {
+
+int32_t spl_solver_create(spl_ctx *c, const spl_key *root_key, uint64_t root_aux, int32_t goal, int32_t use_h,
+                          int32_t heuristic, int64_t beam, int32_t tie, int32_t noise, int32_t keep_links,
+                          spl_solver **out) {
+    if (!c || !root_key || !out) return fail(c, SPL_E_INVALID, "spl_solver_create: null argument");
     const Rec r{root_key->lo, root_key->hi & HI_KEY_MASK, root_aux, ~0ull};
-    return open_solver(s, s->kind, &r, 32, false, "solver create sync failed", out);
+    return create_solver(c, "spl_solver_create", &r, 1, goal, use_h, heuristic, beam, tie, noise, keep_links, out);
+}
+
+int32_t spl_solver_create_queue(spl_ctx *c, const void *rows_host, int64_t n_rows, int32_t goal, int32_t use_h,
+                                int32_t heuristic, int64_t beam, int32_t tie, int32_t noise, int32_t keep_links,
+                                spl_solver **out) {
+    if (!c || !rows_host || !out || n_rows < 1) return fail(c, SPL_E_INVALID, "spl_solver_create_queue: bad arguments (n_rows >= 1)");
+    std::vector<Rec> rows((size_t)n_rows);
+    memcpy(rows.data(), rows_host, (size_t)n_rows * sizeof(Rec));
+    for (Rec &r : rows) r.link = ~0ull;
+    return create_solver(c, "spl_solver_create_queue", rows.data(), n_rows, goal, use_h, heuristic, beam, tie, noise, keep_links, out);
 }
 
 int32_t spl_solver_destroy(spl_solver *s) {
@@ -2590,7 +2631,7 @@ int32_t spl_rsolver_create(spl_ctx *c, const spl_rconfig *cfg, const void *root_
     s->goal = cfg->target_points;
     s->n_front = 1;
     c->rcfg_dirty = false;
-    return open_solver(s, REALISTIC, root_rec_host, 96, false, "rsolver create sync failed", out);
+    return open_solver(s, REALISTIC, root_rec_host, 1, 96, false, "rsolver create sync failed", out);
 }
 
 int32_t spl_rsolver_frontier(spl_solver *s, const void **recs, int64_t *n) {

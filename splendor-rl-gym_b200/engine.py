@@ -284,10 +284,13 @@ class Engine:
 
     # -------------------------------------------------------------- fused solver
     def solver(self, root_key: int, root_aux: int, goal_pts: int, use_heuristic: bool, heuristic: str, beam_width: int,
-               tie: str = 'stable', noise: str = 'const', keep_links: bool = True, identity: str = 'key') -> 'LevelSolver':
+               tie: str = 'stable', noise: str = 'const', keep_links: bool = True, identity: str = 'key',
+               queue: np.ndarray = None) -> 'LevelSolver':
+        """With `queue` (an array of 32-byte rows {lo, hi, aux, link} in rank order; links ignored) the solve starts
+        from that level-0 queue instead of the one state (root_key, root_aux), which are then ignored."""
         self.set_identity(identity)
         return LevelSolver(self, root_key, root_aux, goal_pts, use_heuristic, heuristic, beam_width, tie, noise,
-                           keep_links)
+                           keep_links, queue)
 
 
 class Stepper:
@@ -305,13 +308,19 @@ class LevelSolver(Stepper):
     """spl_solver_*: one object per solve(); step() == one `while queue` iteration (src/solver.py:434-457)."""
 
     def __init__(self, eng: Engine, root_key, root_aux, goal_pts, use_heuristic, heuristic, beam_width, tie, noise,
-                 keep_links):
+                 keep_links, queue=None):
         self.eng = eng
-        k = Key(root_key & M64, root_key >> 64)
         h = C.c_void_p()
-        check(lib.spl_solver_create(eng._h, C.byref(k), root_aux, goal_pts, int(bool(use_heuristic)),
-                                    heuristic_id(heuristic), beam_width, TIE_IDS[tie], NOISE_IDS[noise],
-                                    int(keep_links), C.byref(h)), eng._h)
+        args = (goal_pts, int(bool(use_heuristic)), heuristic_id(heuristic), beam_width, TIE_IDS[tie], NOISE_IDS[noise],
+                int(keep_links), C.byref(h))
+        if queue is None:
+            k = Key(root_key & M64, root_key >> 64)
+            check(lib.spl_solver_create(eng._h, C.byref(k), root_aux, *args), eng._h)
+        else:
+            rows = np.ascontiguousarray(queue)
+            if rows.dtype.itemsize != 32:
+                raise ValueError(f'queue rows must be 32 bytes {{lo, hi, aux, link}}, not {rows.dtype}')
+            check(lib.spl_solver_create_queue(eng._h, rows.ctypes.data, len(rows), *args), eng._h)
         self._h = h
         self.infos = []
         self.ended = False

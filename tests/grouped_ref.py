@@ -14,6 +14,9 @@ MIX_INV = pow(MIX, -1, 1 << 64)
 SORT_SHIFT = 34           # items are ordered, and runs cut, by the top 30 bits of the card-set hash (ITEM_KEY_LO)
 TINY_ITEMS = 16           # buy-only runs of at most this many records of one card set: thread kernel
 WARP_MAX_UNORDERED = 512  # candidates of a run above which the card-set-sharded round uses the CTA kernel
+WARP_MAX_ORDERED = 1024   # BIG_W: the same threshold on the single-GPU round
+SORT_ITEMS_WARP = 512     # items one warp of the item sort owns (SORT_ITEMS = 16 per thread)
+SORT_TILE = 4096          # items one CTA of the item sort owns
 INJECT_ORD0 = 192         # ordinals of injected records: above the largest real fan-out (190)
 MAX_SCORES = 2048         # distinct scores one level may hold in the score dictionary of the card-set-sharded cut
 
@@ -87,6 +90,81 @@ def records(rows) -> np.ndarray:
     for i, r in enumerate(rows):
         out[i] = r
     return out
+
+
+# ---------------------------------------------------------------- level-0 queues (spl_solver_create_queue)
+def card_set(cards) -> tuple:
+    """(m0, m1) of a list of card indices 0..89"""
+    m = 0
+    for c in cards:
+        assert 0 <= c < 90
+        m |= 1 << c
+    return m & M64, m >> 64
+
+
+def cards_of(m0: int, m1: int) -> list:
+    m = m0 | m1 << 64
+    return [c for c in range(90) if m >> c & 1]
+
+
+def make_row(m0: int, m1: int, gems, bonus=(0,) * 5, pts: int = 0, saved: int = 0) -> tuple:
+    """A queue row {key, aux, link 0}.  Asserts what spl_solver_create_queue rejects (an illegal hand, a key bit at or
+    above 105) and the packed ranges of aux."""
+    assert legal_hand(gems), gems
+    assert 0 <= m0 <= M64 and 0 <= m1 < 1 << 26
+    assert len(bonus) == 5 and all(0 <= b < 32 for b in bonus) and 0 <= pts < 256 and 0 <= saved < 1 << 16
+    key = (m0 | m1 << 64) << 15
+    for i, g in enumerate(gems):
+        key |= g << (3 * i)
+    assert key < 1 << 105
+    aux = saved | pts << 16
+    for i, b in enumerate(bonus):
+        aux |= b << (24 + 5 * i)
+    return key & M64, key >> 64, aux, 0
+
+
+def queue_of(rows) -> np.ndarray:
+    """rows in rank order as one level-0 queue; asserts that no two rows share a key (the create rejects that)"""
+    q = records(rows)
+    assert len({(int(a), int(b)) for a, b in zip(q['lo'], q['hi'])}) == len(q), 'two rows with the same key'
+    return q
+
+
+_COST = None
+
+
+def card_cost(c: int) -> tuple:
+    """the gems of each colour card c costs (from the oracle's buy table: the least value of each colour that buys it)"""
+    global _COST
+    if _COST is None:
+        _COST = np.zeros((90, 5), np.int64)
+        for col in range(5):
+            for v in range(7, -1, -1):
+                key = [7] * 5
+                key[col] = v
+                _COST[oracle.buys(key), col] = v
+    return tuple(int(x) for x in _COST[c])
+
+
+def buyer(m0: int, m1: int, c: int, gems, bonus=None, pts: int = 0, saved: int = 0) -> tuple:
+    """The row T \\ {c} of target card set T = (m0, m1) with hand `gems`; by default its bonus is the cost of c, so it
+    can afford c without paying gems and its buy of c is the state (T, gems)."""
+    m = m0 | m1 << 64
+    assert m >> c & 1, 'the card must be in the target set'
+    m &= ~(1 << c)
+    return make_row(m & M64, m >> 64, gems, card_cost(c) if bonus is None else bonus, pts, saved)
+
+
+def filler(m0: int, m1: int) -> tuple:
+    """A row of card set (m0, m1) with no bonus and no gems: no card is affordable, 15 gem takes; one item of a round"""
+    return make_row(m0, m1, (0,) * 5)
+
+
+def buys_of(queue, cands):
+    """the buy successors (card set differs from the parent's) of `cands` = expand_queue(queue)[0], in arrival order"""
+    par = (cands['link'] >> np.uint64(8)).astype(np.int64)
+    same = (cands['lo'] >> np.uint64(15) == queue['lo'][par] >> np.uint64(15)) & (cands['hi'] == queue['hi'][par])
+    return cands[~same]
 
 
 def random_hand(rng) -> tuple:

@@ -111,3 +111,51 @@ def test_run_prediction_counts_classes():
     assert runs[7] == (G.WARP, 1, 17, 17) and runs[8] == (G.CTA, 3, 513, 513)
     m0, m1 = G.card_words_np(G.records(recs)['lo'], G.records(recs)['hi'])
     assert [int(h) for h in G.hash_np(m0, m1)] == [G.hash_key(a, b) for a, b in zip(m0.tolist(), m1.tolist())]
+
+
+def test_queue_builder_rejects_what_the_create_rejects():
+    """make_row / queue_of refuse the rows spl_solver_create_queue refuses: an illegal hand, a key bit >= 105, a key twice"""
+    m = G.card_set([0, 48, 49, 89])
+    with pytest.raises(AssertionError):
+        G.make_row(*m, (3, 3, 3, 2, 0))          # 11 gems
+    with pytest.raises(AssertionError):
+        G.make_row(*m, (8, 0, 0, 0, 0))          # a colour above 7
+    with pytest.raises(AssertionError):
+        G.make_row(m[0], 1 << 26, (0,) * 5)      # key bit 105
+    with pytest.raises(AssertionError):
+        G.queue_of([G.make_row(*m, (1,) * 5), G.filler(5, 0), G.make_row(*m, (1,) * 5, (7,) * 5)])  # one key twice
+    with pytest.raises(AssertionError):
+        G.buyer(*G.card_set([1, 2]), 3, (0,) * 5)  # the card is not in the target set
+
+
+def test_buyer_and_filler_rows():
+    """a buyer of T buys its missing card into (T, hand) without paying gems; a filler has no buys and 15 takes"""
+    T = G.card_set([0, 17, 48, 49, 89])
+    q = G.queue_of([G.buyer(*T, c, (1, 1, 1, 0, 0)) for c in G.cards_of(*T)] + [G.filler(*G.card_set([3, 70]))])
+    cands, ntk = G.expand_queue(q)
+    buys = G.buys_of(q, cands)
+    assert ntk[-1] == 15 and not (buys['link'] >> np.uint64(8) == np.uint64(len(q) - 1)).any()
+    want = G.make_row(*T, (1, 1, 1, 0, 0))
+    into_T = buys[(buys['lo'] == np.uint64(want[0])) & (buys['hi'] == np.uint64(want[1]))]
+    assert [int(x) >> 8 for x in into_T['link']] == list(range(5))
+
+
+def test_oracle_queue_start_reproduces_the_reference_level():
+    """oracle.Solver started from a constructed queue (several rows, all visited) equals G.ref_level level by level"""
+    rng = np.random.default_rng(4)
+    T = G.card_set([0, 30, 48, 49, 89])
+    rows = [G.buyer(*T, c, g) for c in G.cards_of(*T) for g in ((1, 1, 1, 0, 0), (0, 0, 0, 0, 0))]
+    rows += [G.filler(int(rng.integers(1, 1 << 62)), int(rng.integers(0, 1 << 26))) for _ in range(20)]
+    q = G.queue_of(rows)
+    orc = oracle.Solver(255, use_heuristic=True, heuristic_name='aggressive', beam_width=10 ** 7, root=q)
+    try:
+        st, _ = orc.level(0)
+        assert np.array_equal(st['lo'], q['lo']) and np.array_equal(st['aux'], q['aux'])
+        visited = {(int(a), int(b)) for a, b in zip(q['lo'], q['hi'])}
+        for lv in range(2):
+            q, unique = G.ref_level(q, visited, None, 'aggressive')
+            info = orc.step()
+            assert unique == info['unique'] and len(visited) == info['visited']
+            assert np.array_equal(q, _queue(*orc.level(lv + 1)))
+    finally:
+        orc.close()
