@@ -362,6 +362,39 @@ int32_t spl_rsolver_create(spl_ctx *ctx, const spl_rconfig *cfg, const void *roo
                            int32_t keep_links, spl_solver **out);
 int32_t spl_rsolver_frontier(spl_solver *s, const void **recs_dev, int64_t *n_host);
 
+/* ---- batched realistic search (realistic.py: solve_many) -------------------------------------------------------------
+ * n_games independent MultiPlayerState.solve() searches advance in lockstep on one GPU: each spl_solver_step is one level
+ * of every game still running, at a number of kernel launches that does not depend on n_games.  Game g has its own
+ * rules, market (cfgs[g]), root record (root_recs_host[g], 96 bytes) and beam width (beams[g] >= 1); noise must be
+ * SPL_NOISE_CONST or SPL_NOISE_HASH (SPL_E_INVALID otherwise: the draws of 'mt' depend on the other games).  Every level
+ * of game g equals spl_rsolver's level for that game alone: the same records in the same rank order (link words carry
+ * ranks inside the game), the same counters, goal rank and line.  A state of one game never merges with a state of
+ * another: the visited identity is (game, exact key).  A game leaves the batch when its goal is dequeued, its queue
+ * runs out or it reaches the 1000-turn limit; the batch ends when every game has.  spl_solver_step fills the aggregate
+ * counters over the games of the level (frontier, generated, unique, kept: sums; visited: the batch's table; goal_rank
+ * -1; ended when every game has) with ms_count = goal test + count, ms_expand = expand, ms_resolve = probe + winners,
+ * ms_select = score, ms_sort = the segmented cut.  A level above 2^32 - 1 candidates fails with SPL_E_INVALID; a full
+ * visited table or device memory fails with SPL_E_TABLE_FULL / SPL_E_NOMEM, and the context stays usable once the
+ * solver is destroyed.  Destroy with spl_solver_destroy; spl_solver_path does not apply (use spl_rbatch_lines). */
+typedef struct {
+    int64_t level;      /* the last level the game took part in */
+    int64_t frontier;   /* its queue length at the top of that level */
+    int64_t generated, unique, kept, visited;  /* as spl_level_info, for this game alone */
+    int64_t goal_rank;  /* rank of its first finished state in that queue, or -1 */
+    int32_t ended;      /* 1 once the game has ended (its counters no longer change) */
+    int32_t pad;
+} spl_rgame_info;
+int32_t spl_rbatch_create(spl_ctx *ctx, const spl_rconfig *cfgs, const void *root_recs_host, const int64_t *beams,
+                          int32_t n_games, int32_t keep_links, spl_solver **out);
+/* the per-game counters after the last spl_solver_step (n_games must be the batch's) */
+int32_t spl_rbatch_games(spl_solver *s, spl_rgame_info *out_host, int32_t n_games);
+/* game `game`'s queue (its records in rank order, device memory of the solver); empty once the game has ended */
+int32_t spl_rbatch_frontier(spl_solver *s, int32_t game, const void **recs_dev, int64_t *n_host);
+/* after the batch has ended (keep_links = 1): every game's line, root first.  plies_host[g] = moves of game g; its
+ * plies_host[g] + 1 records go to recs_host[g * cap ...].  SPL_E_CAPACITY (plies_host filled) when a line needs more
+ * than cap records.  The lines are rebuilt on the device from the link columns, one thread per game. */
+int32_t spl_rbatch_lines(spl_solver *s, void *recs_host, int64_t cap, int32_t *plies_host);
+
 /* ---- realistic mode on the key-sharded driver (sharded.py: RCudaBackend + RShardedSolver) ---------------------------
  * MultiPlayerState.solve(shard=True) / --realistic --shard: the level loop of :820-852 over a queue spread block-cyclically
  * across ranks, with the same per-level steps as spl_expand_rows .. spl_move_rows above.  Every level holds the same

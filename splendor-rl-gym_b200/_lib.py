@@ -42,6 +42,15 @@ class LevelInfo(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class RGameInfo(C.Structure):
+    _fields_ = [('level', C.c_int64), ('frontier', C.c_int64), ('generated', C.c_int64), ('unique', C.c_int64),
+                ('kept', C.c_int64), ('visited', C.c_int64), ('goal_rank', C.c_int64), ('ended', C.c_int32),
+                ('pad', C.c_int32)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_ if k != 'pad'}
+
+
 def _load():
     if not LIB_PATH.exists():
         raise ImportError(
@@ -89,6 +98,10 @@ def _load():
         'spl_rpack': (i32, [vp, vp, vp, i64, vp, vp]),
         'spl_rsolver_create': (i32, [vp, vp, vp, i64, i32, C.POINTER(vp)]),
         'spl_rsolver_frontier': (i32, [vp, C.POINTER(vp), C.POINTER(i64)]),
+        'spl_rbatch_create': (i32, [vp, vp, vp, vp, i32, i32, C.POINTER(vp)]),
+        'spl_rbatch_games': (i32, [vp, vp, i32]),
+        'spl_rbatch_frontier': (i32, [vp, i32, C.POINTER(vp), C.POINTER(i64)]),
+        'spl_rbatch_lines': (i32, [vp, vp, i64, vp]),
         'spl_rexpand_rows': (i32, [vp, vp, vp, i64, i64, vp, i64, C.POINTER(i64), vp]),
         'spl_rroute_keys': (i32, [vp, vp, vp, i64, i32, vp, vp, vp]),
         'spl_rdedup_flags': (i32, [vp, vp, i64, vp, vp]),

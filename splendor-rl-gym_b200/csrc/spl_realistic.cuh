@@ -609,4 +609,291 @@ __global__ void __launch_bounds__(TILE) move_rows_kernel(const R *__restrict__ r
     }
 }
 
+// ------------------------------------------------------------------ batched search (spl_rbatch_*): B games in lockstep
+// Every per-record array of a batch level is game-major: game g owns the index range seg[g] .. seg[g + 1] (seg[0] = 0,
+// seg[B] = n; a game that has ended owns an empty range), and inside it the records keep the order the single-game
+// solver gives them.  Link words carry the parent's rank inside its game, so each game's segment of the queue is
+// byte-identical to spl_rsolver's queue.  cfg[g] is game g's RConfigDev.
+//
+// The batch's visited table holds (game, exact key) entries: RBucket.pad is the game, and the game is mixed into the
+// bucket hash, so that B games sharing a root (every 2-player game starts from the same key) do not share a probe run.
+__device__ __forceinline__ int rb_game_of(const int64_t *__restrict__ seg, int n_games, int64_t i) {
+    int lo = 0, hi = n_games;  // seg[lo] <= i < seg[hi]
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (__ldg(seg + mid) <= i) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+// ctr[g] += v, one atomic per run of lanes of a warp that share a game (every lane calls it; g < 0: nothing to add)
+__device__ __forceinline__ void rb_warp_add(unsigned long long *ctr, int g, uint32_t v) {
+    const unsigned peers = __match_any_sync(0xffffffffu, g);
+    const uint32_t sum = __reduce_add_sync(peers, v);
+    if (g >= 0 && sum && (int)(threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(ctr + g, (unsigned long long)sum);
+}
+__device__ __forceinline__ uint64_t rb_key_hash(const uint64_t key[RKEY_WORDS], uint32_t game) {
+    return mix64(r_key_hash(key), 0x9E3779B97F4A7C15ull * ((uint64_t)game + 1));
+}
+
+// r_probe with the game as part of the identity
+__device__ __forceinline__ uint32_t rb_probe(RBucket *__restrict__ table, uint64_t nb, uint64_t tag, const uint64_t key[RKEY_WORDS],
+                                             uint32_t game, uint32_t tinv, uint32_t &n_new, unsigned int *error) {
+    uint64_t b = __umul64hi(rb_key_hash(key, game), nb);
+    for (int probes = 0; probes < MAX_PROBE; ++probes) {
+        RBucket *B = table + b;
+        unsigned long long c = *reinterpret_cast<volatile unsigned long long *>(&B->ctrl);
+        if (c == 0) {
+            c = atomicCAS(&B->ctrl, 0ull, (unsigned long long)(tag << 8 | 1));
+            if (c == 0) {
+#pragma unroll
+                for (int i = 0; i < RKEY_WORDS; ++i) B->key[i] = key[i];
+                B->pad = game;
+                __threadfence();
+                atomicExch(&B->ctrl, (unsigned long long)(tag << 8 | 3));
+                ++n_new;
+                atomicMax(&B->tinv, tinv);
+                return (uint32_t)b;
+            }
+        }
+        while ((c & 3) == 1) c = *reinterpret_cast<volatile unsigned long long *>(&B->ctrl);
+        __threadfence();
+        bool same = *reinterpret_cast<volatile unsigned int *>(&B->pad) == game;
+#pragma unroll
+        for (int i = 0; i < RKEY_WORDS; ++i) same &= *reinterpret_cast<volatile uint64_t *>(&B->key[i]) == key[i];
+        if (same) {
+            if ((c >> 8) != tag) return R_DEAD;
+            if (*reinterpret_cast<volatile unsigned int *>(&B->tinv) > tinv) return R_DEAD;
+            atomicMax(&B->tinv, tinv);
+            return (uint32_t)b;
+        }
+        if (++b == nb) b = 0;
+    }
+    atomicExch(error, 1u);
+    return R_DEAD;
+}
+__global__ void __launch_bounds__(TILE) rb_rehash_kernel(const RBucket *__restrict__ old_table, uint64_t old_nb,
+                                                         RBucket *__restrict__ table, uint64_t nb, Counters *ctr) {
+    const uint64_t i = (uint64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i >= old_nb || old_table[i].ctrl == 0) return;
+    uint64_t key[RKEY_WORDS];
+#pragma unroll
+    for (int k = 0; k < RKEY_WORDS; ++k) key[k] = old_table[i].key[k];
+    const uint32_t game = old_table[i].pad;
+    uint64_t b = __umul64hi(rb_key_hash(key, game), nb);
+    for (int probes = 0; probes < MAX_PROBE; ++probes) {
+        if (atomicCAS(&table[b].ctrl, 0ull, old_table[i].ctrl) == 0) {
+#pragma unroll
+            for (int k = 0; k < RKEY_WORDS; ++k) table[b].key[k] = key[k];
+            table[b].pad = game;
+            return;
+        }
+        if (++b == nb) b = 0;
+    }
+    atomicExch(&ctr->error, 1u);
+}
+
+// goal test on dequeue (:827-829), per game: goal[g] = first rank inside game g whose game is over
+__global__ void __launch_bounds__(TILE) rb_goal_kernel(const RRec *__restrict__ front, int64_t n, const int64_t *__restrict__ seg,
+                                                       int n_games, const RConfigDev *__restrict__ cfg, long long *__restrict__ goal) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i >= n) return;
+    const int g = rb_game_of(seg, n_games, i);
+    const RPlayer p = front[i].p[front[i].cur];
+    if (r_pts(cfg[g], p) >= cfg[g].target) atomicMin(goal + g, (long long)(i - seg[g]));
+}
+
+// r_count_scan_kernel over the batch queue; the parents of a game whose goal was found this level get no successors.
+// cands[g] += successors of game g.
+__global__ void __launch_bounds__(TILE) rb_count_scan_kernel(const RRec *__restrict__ front, int64_t n, const int64_t *__restrict__ seg,
+                                                             int n_games, const RConfigDev *__restrict__ cfg,
+                                                             const long long *__restrict__ goal, uint32_t *__restrict__ off,
+                                                             uint32_t *__restrict__ vmask, uint64_t *status, Counters *ctr, int ticket_id,
+                                                             unsigned long long *cands) {
+    __shared__ uint32_t warp_sums[TILE / 32 + 1];
+    __shared__ uint32_t s_tile;
+    __shared__ uint64_t s_base;
+    if (threadIdx.x == 0) s_tile = atomicAdd(&ctr->ticket[ticket_id], 1u);
+    __syncthreads();
+    const uint32_t tile = s_tile;
+    const int64_t p = (int64_t)tile * TILE + threadIdx.x;
+    uint32_t cnt = 0, m = 0;
+    int g = -1;
+    if (p < n) {
+        g = rb_game_of(seg, n_games, p);
+        if (goal[g] == 0x7fffffffffffffffll) {
+            RRec s;
+            ld_rec(front + p, s);
+            int bonus[NCOL], pts;
+            r_derive(cfg[g], s.p[s.cur], bonus, pts);
+            m = r_valid_mask(cfg[g], s, bonus);
+            cnt = __popc(m);
+        }
+        vmask[p] = m;
+    }
+    rb_warp_add(cands, g, cnt);
+    uint32_t total;
+    const uint32_t excl = block_excl_scan(cnt, warp_sums, total);
+    if (threadIdx.x < 32) {
+        const uint64_t e = lookback_exclusive(status, tile, total, 0);
+        if (threadIdx.x == 0) {
+            s_base = e;
+            if ((int64_t)(tile + 1) * TILE >= n) ctr->total_cands = e + total;
+        }
+    }
+    __syncthreads();
+    if (p < n) off[p] = (uint32_t)(s_base + excl);
+}
+
+// r_expand_kernel over the batch queue: link = rank of the parent inside its game << 8 | ordinal; cand_game[t] = game
+__global__ void __launch_bounds__(TILE) rb_expand_kernel(const RRec *__restrict__ front, int64_t n, const int64_t *__restrict__ seg,
+                                                         int n_games, const RConfigDev *__restrict__ cfg,
+                                                         const uint32_t *__restrict__ off, const uint32_t *__restrict__ vmask,
+                                                         RRec *__restrict__ cand, uint32_t *__restrict__ cand_game) {
+    const int64_t p = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (p >= n) return;
+    uint32_t m = vmask[p], ord = 0;
+    if (!m) return;
+    const int g = rb_game_of(seg, n_games, p);
+    RRec s;
+    ld_rec(front + p, s);
+    int bonus[NCOL], pts;
+    r_derive(cfg[g], s.p[s.cur], bonus, pts);
+    uint64_t t = off[p];
+    const uint64_t rank = (uint64_t)(p - seg[g]);
+    while (m) {
+        const int slot = __ffs(m) - 1;
+        m &= m - 1;
+        RRec o;
+        r_make_child(cfg[g], s, bonus, slot, o);
+        o.link = (rank << 8) | ord;
+        o.spare = 0;
+        st_rec(cand + t, o);
+        cand_game[t] = (uint32_t)g;
+        ++t;
+        ++ord;
+    }
+}
+
+// exact-key probe / insert of the batch's candidates, (game, key) identity; n_new[g] += new states of game g
+__global__ void __launch_bounds__(TILE) rb_probe_kernel(const RRec *__restrict__ cand, const uint32_t *__restrict__ cand_game, int64_t n,
+                                                        const RConfigDev *__restrict__ cfg, RBucket *__restrict__ table, uint64_t nb,
+                                                        uint64_t tag, uint32_t *__restrict__ cand_slot, Counters *ctr,
+                                                        unsigned long long *n_new_game) {
+    const int64_t t = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    uint32_t n_new = 0;
+    int g = -1;
+    if (t < n) {
+        g = (int)cand_game[t];
+        RRec s;
+        ld_rec(cand + t, s);
+        uint64_t key[RKEY_WORDS];
+        if (!r_pack_key(cfg[g], s, key)) atomicExch(&ctr->error, 4u);
+        cand_slot[t] = rb_probe(table, nb, tag, key, (uint32_t)g, ~(uint32_t)t, n_new, &ctr->error);
+    }
+    rb_warp_add(n_new_game, g, n_new);
+#pragma unroll
+    for (int d = 16; d; d >>= 1) n_new += __shfl_xor_sync(0xffffffffu, n_new, d);
+    if ((threadIdx.x & 31) == 0 && n_new) atomicAdd(&ctr->n_new, (unsigned long long)n_new);
+}
+
+// the winners' records and games, in arrival order
+__global__ void __launch_bounds__(TILE) rb_gather_kernel(const RRec *__restrict__ src, const uint32_t *__restrict__ src_game,
+                                                         const int64_t *__restrict__ idx, int64_t n, RRec *__restrict__ dst,
+                                                         uint32_t *__restrict__ dst_game) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i < n) {
+        const int64_t j = idx[i];
+        RRec r;
+        ld_rec(src + j, r);
+        st_rec(dst + i, r);
+        dst_game[i] = src_game[j];
+    }
+}
+
+// sort pairs of the beam cut: y[i] = ~flip_f64(score) (ascending y = descending score), slot[i] = i; score key range
+// in ctr->sk_min / sk_max
+__global__ void __launch_bounds__(TILE) rb_score_kernel(const RRec *__restrict__ recs, const uint32_t *__restrict__ games, int64_t n,
+                                                        const RConfigDev *__restrict__ cfg, ScoreLuts L, uint64_t *__restrict__ y,
+                                                        uint32_t *__restrict__ slot, Counters *ctr) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    uint64_t kmin = ~0ull, kmax = 0;
+    if (i < n) {
+        RRec s;
+        ld_rec(recs + i, s);
+        const uint64_t k = flip_f64((uint64_t)__double_as_longlong(r_score(cfg[games[i]], s, L)));
+        y[i] = ~k;
+        slot[i] = (uint32_t)i;
+        kmin = kmax = k;
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) {
+        kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, d));
+        kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, d));
+    }
+    if ((threadIdx.x & 31) == 0 && kmin <= kmax) {
+        atomicMin(&ctr->sk_min, (unsigned long long)kmin);
+        atomicMax(&ctr->sk_max, (unsigned long long)kmax);
+    }
+}
+// sort word of the second (game) pass: the game of each pair, in the score order the first pass left
+__global__ void __launch_bounds__(TILE) rb_game_words_kernel(const uint32_t *__restrict__ slot, const uint32_t *__restrict__ games,
+                                                             int64_t n, uint64_t *__restrict__ y) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i < n) y[i] = games[slot[i]];
+}
+// segmented cut: the pairs are in (game, score desc, arrival) order; pair i is rank i - useg[g] of game g and is kept
+// at kseg[g] + rank when that rank is below kseg[g + 1] - kseg[g] = min(beam_g, unique_g)
+__global__ void __launch_bounds__(TILE) rb_cut_kernel(const RRec *__restrict__ uniq, const uint32_t *__restrict__ games,
+                                                      const uint32_t *__restrict__ slot, int64_t n, const int64_t *__restrict__ useg,
+                                                      const int64_t *__restrict__ kseg, RRec *__restrict__ front) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t j = slot[i];
+    const int g = (int)games[j];
+    const int64_t r = i - useg[g];
+    if (r < kseg[g + 1] - kseg[g]) {
+        RRec rec;
+        ld_rec(uniq + j, rec);
+        st_rec(front + kseg[g] + r, rec);
+    }
+}
+
+// out[i] = col[at[i]]: the link words of the games' path states at one level
+__global__ void __launch_bounds__(TILE) rb_pick_kernel(const uint64_t *__restrict__ col, const int64_t *__restrict__ at, int64_t n,
+                                                       uint64_t *__restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    if (i < n) out[i] = col[at[i]];
+}
+
+// every game's line, one thread per game: out[g][0] = root, out[g][p + 1] = successor ords[g][p] of out[g][p]
+// (the reference's list(iter(state))[ordinal]) for p < plies[g]
+__global__ void __launch_bounds__(TILE) rb_line_kernel(const RRec *__restrict__ roots, const RConfigDev *__restrict__ cfg, int n_games,
+                                                       const int32_t *__restrict__ plies, const uint8_t *__restrict__ ords,
+                                                       int max_plies, RRec *__restrict__ out, Counters *ctr) {
+    const int g = blockIdx.x * TILE + threadIdx.x;
+    if (g >= n_games) return;
+    const RConfigDev &C = cfg[g];
+    RRec s;
+    ld_rec(roots + g, s);
+    RRec *line = out + (int64_t)g * (max_plies + 1);
+    st_rec(line, s);
+    for (int p = 0; p < plies[g]; ++p) {
+        int bonus[NCOL], pts;
+        r_derive(C, s.p[s.cur], bonus, pts);
+        uint32_t m = r_valid_mask(C, s, bonus);
+        const int ord = ords[(int64_t)g * max_plies + p];
+        if (ord >= __popc(m)) {
+            atomicExch(&ctr->error, 1u);
+            return;
+        }
+        for (int k = 0; k < ord; ++k) m &= m - 1;
+        RRec o;
+        r_make_child(C, s, bonus, __ffs(m) - 1, o);
+        o.link = (uint64_t)ord;
+        o.spare = 0;
+        st_rec(line + p + 1, o);
+        s = o;
+    }
+}
+
 }  // namespace spl

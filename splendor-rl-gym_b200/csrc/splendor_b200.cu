@@ -8,7 +8,9 @@
 #include <string.h>
 
 #include <algorithm>
+#include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "spl_kernels.cuh"
@@ -103,6 +105,14 @@ static const TableDesc REALISTIC_TABLE_DESC = {
     },
     "realistic table rehash into %llu buckets overflowed a probe sequence",
     "realistic visited table full: %llu states + %llu candidates vs %llu buckets (max_table_bytes=%llu)"};
+static const TableDesc RBATCH_TABLE_DESC = {
+    64, 1, ~0ull, 0.6, 4,
+    [](const void *from, uint64_t units, void *to, uint64_t to_units, Counters *ctr, cudaStream_t st) {
+        rb_rehash_kernel<<<nblk((int64_t)units), TILE, 0, st>>>(static_cast<const RBucket *>(from), units,
+                                                                 static_cast<RBucket *>(to), to_units, ctr);
+    },
+    "batch table rehash into %llu buckets overflowed a probe sequence",
+    "batch visited table full: %llu states + %llu candidates vs %llu buckets (max_table_bytes=%llu)"};
 
 // A visited set on the device: an open-addressing table that grows by rehashing into one twice its size.  It counts
 // its own entries, those of an insert that failed part way included, so that clear() can skip a table that holds none.
@@ -137,8 +147,9 @@ struct spl_ctx {
     int device = 0;
     std::string err;
     // visited sets: the key table (BFS, the reference's hash identity, externally drawn noise and the stage operators),
-    // the card-set node table of the grouped level (spl_m2.cuh) and the realistic level's table (allocated on first use)
-    VisitTable key{KEY_TABLE_DESC}, nodes{NODE_TABLE_DESC}, rtab{REALISTIC_TABLE_DESC};
+    // the card-set node table of the grouped level (spl_m2.cuh), the realistic level's table and the batched realistic
+    // level's (game, key) table (both allocated on first use)
+    VisitTable key{KEY_TABLE_DESC}, nodes{NODE_TABLE_DESC}, rtab{REALISTIC_TABLE_DESC}, rbtab{RBATCH_TABLE_DESC};
     uint64_t occupied = 0;  // visited states: those of the last solve, plus what stage operators added to the key table
     uint32_t epoch = 0;
     uint64_t chunk_parents = 0;
@@ -292,7 +303,7 @@ int32_t spl_create(const spl_config *cfg, spl_ctx **out) {
     CKC(cudaSetDevice(c->device));
     size_t free_b = 0, total_b = 0;
     CKC(cudaMemGetInfo(&free_b, &total_b));
-    c->key.max_bytes = c->rtab.max_bytes = cfg->max_table_bytes ? cfg->max_table_bytes : (uint64_t)(free_b * 0.6);
+    c->key.max_bytes = c->rtab.max_bytes = c->rbtab.max_bytes = cfg->max_table_bytes ? cfg->max_table_bytes : (uint64_t)(free_b * 0.6);
     c->chunk_user = cfg->chunk_parents != 0;
     c->chunk_parents = cfg->chunk_parents ? std::min<uint64_t>(cfg->chunk_parents, MAX_CHUNK_PARENTS) : (4ull << 20);
     c->chunk_parents = std::max<uint64_t>(c->chunk_parents, TILE);
@@ -1294,10 +1305,23 @@ enum LevelKind {
     KEY_TABLE,  // expand + dedup against the key table, in chunks of parents
     GROUPED,    // beam search on the card-set-grouped level (spl_m2.cuh), visited set in the node table
     REALISTIC,  // realistic mode: materialised 96-byte successors, exact-key table
+    REALISTIC_BATCH,  // realistic mode, many games in lockstep: game-major queues, (game, exact key) table
 };
 static const VisitTable &visited_table(const spl_ctx *c, LevelKind kind) {
-    return kind == KEY_TABLE ? c->key : kind == GROUPED ? c->nodes : c->rtab;
+    return kind == KEY_TABLE ? c->key : kind == GROUPED ? c->nodes : kind == REALISTIC ? c->rtab : c->rbtab;
 }
+
+// What a batched realistic solver keeps beside the common queue buffers (spl_rbatch_*, spl_realistic.cuh): the games'
+// configs and roots, the queue's game-major offsets (on the device for the kernels, on the host per level for the line
+// walk), the per-game counters, and the game column of the candidates and of the winners.
+struct RBatch {
+    int B = 0;
+    std::vector<int64_t> beam;
+    std::vector<spl_rgame_info> info;          // per game: the counters of the last level it took part in
+    std::vector<int64_t> final_rank;           // per ended game: rank of its last state in the queue of info.level
+    std::vector<std::vector<int64_t>> seg_at;  // per level: the queue offsets of the games (B + 1)
+    DevBuf cfg, roots, seg, gctr, cand_game, uniq_game, scratch, lines;
+};
 
 struct spl_solver : SolverBufs {
     int goal = 15, use_h = 0, heuristic = 0, tie = 0, noise = 0;
@@ -1312,6 +1336,7 @@ struct spl_solver : SolverBufs {
     int level = 0;
     bool ended = false;
     int64_t goal_rank = -1;
+    std::unique_ptr<RBatch> rb;  // REALISTIC_BATCH only
     explicit spl_solver(spl_ctx *ctx) : SolverBufs(ctx) {}
 };
 
@@ -1533,22 +1558,24 @@ static int grouped_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6],
 }
 
 // ------------------------------------------------------------------ solver create
-// The realistic table is allocated on first use, sized by the caller's table_slots.  A realistic search does not use
-// the key table: a large, empty one gives its memory back first.
-static int open_rtable(spl_ctx *c, cudaStream_t st) {
-    if (c->rtab.p) return SPL_OK;
+// The realistic tables (rtab, or rbtab of the batched search) are allocated on first use, sized by the caller's
+// table_slots.  A realistic search does not use the key table: a large, empty one gives its memory back first.
+static int open_rtable(spl_ctx *c, cudaStream_t st, VisitTable &t) {
+    if (t.p) return SPL_OK;
     if (c->key.occ == 0 && c->key.units > (1ull << 16)) CK(c, c->key.alloc(buckets_for(1ull << 12), st));
     uint64_t nb = std::max<uint64_t>(c->rslots_hint ? c->rslots_hint : (1ull << 16), 1024);
-    nb = std::min<uint64_t>(nb, c->rtab.max_bytes / 64);
-    CK(c, c->rtab.alloc(nb, st));
+    nb = std::min<uint64_t>(nb, t.max_bytes / 64);
+    CK(c, t.alloc(nb, st));
     return SPL_OK;
 }
+static int open_rtable(spl_ctx *c, cudaStream_t st) { return open_rtable(c, st, c->rtab); }
 
 // What every solver create shares: clear the visited sets, upload the n level-0 rows (`row_bytes` each: a 32-byte Rec
 // or a 96-byte realistic record) and, on the card-set-sharded driver, the root's global rank 0; register the rows in
 // the visited table of the level kind (trail = {row: None for row in rows}); save the first link columns, synchronise
 // and go live.  With n = 0 (a sharded rank that does not own the root's card set) the queue starts empty.  Realistic
-// mode and the sharded driver start from one root (n <= 1).  On error `s` is deleted.
+// mode and the sharded driver start from one root (n <= 1), the batched realistic search from one root per game.  On
+// error `s` is deleted.
 template <class S>
 static int open_solver(S *s, LevelKind kind, const void *rows, int64_t n, size_t row_bytes, bool sharded, const char *sync_msg,
                        S **out) {
@@ -1586,7 +1613,7 @@ static int open_solver(S *s, LevelKind kind, const void *rows, int64_t n, size_t
                 m2_root_kernel<<<nblk(n), TILE, 0, st>>>(c->nodes.as<uint64_t>(), c->nodes.units, s->front.template as<Rec>(), n,
                                                          c->d_gemrank, c->d_ctr);
                 c->nodes.occ = (uint64_t)n;  // card sets registered, at most: only the table's load factor reads it
-            } else {
+            } else if (kind == REALISTIC) {
                 if (c->cand_slot.ensure(4, 0, st) != cudaSuccess) return fail(c, SPL_E_NOMEM, "realistic scratch alloc");
                 CKS(c, open_rtable(c, st));
                 CKS(c, c->rtab.grow(c, 1, st));
@@ -1595,12 +1622,25 @@ static int open_solver(S *s, LevelKind kind, const void *rows, int64_t n, size_t
                 r_probe_kernel<<<1, TILE, 0, st>>>(s->front.template as<RRec>(), 1, c->rcfg.as<RConfigDev>(), c->rtab.as<RBucket>(),
                                                     c->rtab.units, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
                 c->rtab.occ = 1;
+            } else if constexpr (std::is_same_v<S, spl_solver>) {  // REALISTIC_BATCH: one root per game, rb->cand_game = 0 .. n - 1
+                if (c->cand_slot.ensure((size_t)n * 4, 0, st) != cudaSuccess) return fail(c, SPL_E_NOMEM, "batch scratch alloc");
+                CKS(c, open_rtable(c, st, c->rbtab));
+                CKS(c, c->rbtab.grow(c, (uint64_t)n, st));
+                if (c->rbtab.clear(st) != cudaSuccess) return fail(c, SPL_E_CUDA, "batch table reset failed");
+                CKS(c, next_epoch(c, tag));
+                CKS(c, zero_ctr(c, st));  // after the table's growth
+                RBatch &R = *s->rb;
+                rb_probe_kernel<<<nblk(n), TILE, 0, st>>>(s->front.template as<RRec>(), R.cand_game.as<uint32_t>(), n,
+                                                          R.cfg.as<RConfigDev>(), c->rbtab.as<RBucket>(), c->rbtab.units, tag,
+                                                          c->cand_slot.as<uint32_t>(), c->d_ctr,
+                                                          R.gctr.as<unsigned long long>() + 2 * R.B);
+                c->rbtab.occ = (uint64_t)n;
             }
             ++c->launches;
             CK(c, cudaGetLastError());
             c->occupied = (uint64_t)n;
         }
-        CKS(c, save_links(s, n, kind == REALISTIC, sharded, st));
+        CKS(c, save_links(s, n, kind == REALISTIC || kind == REALISTIC_BATCH, sharded, st));
         if (cudaStreamSynchronize(st) != cudaSuccess) return fail(c, SPL_E_CUDA, "%s", sync_msg);
         return SPL_OK;
     }();
@@ -2110,11 +2150,11 @@ int32_t spl_gs_link_at(spl_gsolver *s, int32_t level, int64_t grank, int32_t *fo
 }  // extern "C"
 
 // ------------------------------------------------------------------ realistic mode host side
-static int upload_rconfig(spl_ctx *c, const spl_rconfig *cfg, cudaStream_t st) {
+// the kernels' form of a config (checked)
+static int make_rconfig(spl_ctx *c, const spl_rconfig *cfg, RConfigDev &h) {
     if (!cfg || cfg->num_players < 2 || cfg->num_players > 4 || cfg->gems_per_color < 1 || cfg->gems_per_color > 7)
         return fail(c, SPL_E_INVALID, "realistic config: num_players must be 2..4 and gems_per_color 1..7");
     const HostTables &T = host_tables();
-    RConfigDev h;
     memset(&h, 0, sizeof h);
     h.P = cfg->num_players; h.target = cfg->target_points; h.gpc = cfg->gems_per_color; h.noise = cfg->noise;
     for (int t = 0; t < 3; ++t) {
@@ -2130,6 +2170,11 @@ static int upload_rconfig(spl_ctx *c, const spl_rconfig *cfg, cudaStream_t st) {
         else { h.col_hi[T.card_bonus[i]] |= 1u << (i - 64); h.pt_hi[T.card_pt[i]] |= 1u << (i - 64); h.tier_hi[t] |= 1u << (i - 64); }
         h.card[i] = T.dev.card[i];
     }
+    return SPL_OK;
+}
+static int upload_rconfig(spl_ctx *c, const spl_rconfig *cfg, cudaStream_t st) {
+    RConfigDev h;
+    CKS(c, make_rconfig(c, cfg, h));
     CK(c, c->rcfg.ensure(sizeof h, 0, st));
     c->rcfg_dirty = true;
     c->rcfg_have = false;
@@ -2367,6 +2412,190 @@ static int realistic_expand(spl_solver *s, int64_t n, LevelExpand *x, cudaStream
     return SPL_OK;
 }
 
+// ------------------------------------------------------------------ batched realistic level (spl_rbatch_*)
+// One level of every game still running, a fixed sequence of launches whatever the number of games: goal test + count
+// (per-game goal ranks and successor counts), expand, probe of (game, key), winners in arrival order, score, then the
+// segmented beam cut -- a stable sort of the winners by score, a stable pass by game, and a gather of the first
+// min(beam_g, unique_g) pairs of every game's run into the next queue.  The host reads the per-game counters twice
+// (after the count and after the probe) and uploads the next queue's offsets once.
+static int rbatch_step(spl_solver *s, spl_level_info *info, cudaStream_t st) {
+    spl_ctx *c = s->c;
+    RBatch &R = *s->rb;
+    const int B = R.B;
+    const int64_t n = s->n_front;
+    const std::vector<int64_t> &seg = R.seg_at.back();
+    long long *goal = R.gctr.as<long long>();
+    unsigned long long *cands = R.gctr.as<unsigned long long>() + B, *n_new_g = cands + B;
+    std::vector<int64_t> g_host(3 * (size_t)B, 0);  // goal | cands | n_new per game
+    for (int g = 0; g < B; ++g) g_host[g] = 0x7fffffffffffffffll;
+    // ---- goal test + successor count
+    CK(c, cudaEventRecord(c->ev[0], st));
+    CK(c, cudaMemcpyAsync(R.gctr.p, g_host.data(), g_host.size() * 8, cudaMemcpyHostToDevice, st));
+    CKS(c, zero_ctr(c, st));
+    const unsigned nt = nblk(n);
+    CK(c, c->off.ensure((size_t)n * 4 + 4, 0, st));
+    CK(c, c->rvmask.ensure((size_t)n * 4 + 4, 0, st));
+    CKS(c, prep_status(c, 0, nt, st));
+    const RConfigDev *cfg = R.cfg.as<RConfigDev>();
+    const int64_t *dseg = R.seg.as<int64_t>();
+    rb_goal_kernel<<<nt, TILE, 0, st>>>(s->front.as<RRec>(), n, dseg, B, cfg, goal);
+    rb_count_scan_kernel<<<nt, TILE, 0, st>>>(s->front.as<RRec>(), n, dseg, B, cfg, goal, c->off.as<uint32_t>(), c->rvmask.as<uint32_t>(),
+                                               c->status[0].as<uint64_t>(), c->d_ctr, 0, cands);
+    c->launches += 2;
+    CK(c, cudaGetLastError());
+    CK(c, cudaMemcpyAsync(g_host.data(), R.gctr.p, (size_t)B * 16, cudaMemcpyDeviceToHost, st));
+    CKS(c, read_ctr(c, st));
+    c->d2h_bytes += B * 16;
+    CK(c, cudaEventRecord(c->ev[1], st));
+    const int64_t total = (int64_t)c->h_ctr->total_cands;
+    if (total >= 0xFFFFFFFFll) return fail(c, SPL_E_INVALID, "batch level produced %lld candidates (>= 2^32)", (long long)total);
+    // ---- expand + (game, key) dedup + winners in arrival order
+    int64_t n_uniq = 0;
+    if (total) {
+        CK(c, c->rcand.ensure((size_t)total * 96, 0, st));
+        CK(c, R.cand_game.ensure((size_t)total * 4, 0, st));
+        rb_expand_kernel<<<nt, TILE, 0, st>>>(s->front.as<RRec>(), n, dseg, B, cfg, c->off.as<uint32_t>(), c->rvmask.as<uint32_t>(),
+                                               c->rcand.as<RRec>(), R.cand_game.as<uint32_t>());
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CK(c, cudaEventRecord(c->ev[2], st));
+        CKS(c, zero_ctr(c, st));
+        CKS(c, c->rbtab.grow(c, (uint64_t)total, st));
+        uint64_t tag;
+        CKS(c, next_epoch(c, tag));
+        CK(c, c->cand_slot.ensure((size_t)total * 4, 0, st));
+        CKS(c, zero_ctr(c, st));
+        rb_probe_kernel<<<nblk(total), TILE, 0, st>>>(c->rcand.as<RRec>(), R.cand_game.as<uint32_t>(), total, cfg, c->rbtab.as<RBucket>(),
+                                                       c->rbtab.units, tag, c->cand_slot.as<uint32_t>(), c->d_ctr, n_new_g);
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CK(c, cudaMemcpyAsync(g_host.data() + 2 * B, n_new_g, (size_t)B * 8, cudaMemcpyDeviceToHost, st));
+        CKS(c, read_ctr(c, st));
+        c->d2h_bytes += B * 8;
+        c->rbtab.occ += c->h_ctr->n_new;  // before the error checks: a reset clears a partial insert too
+        if (c->h_ctr->error == 4) return fail(c, SPL_E_INVALID, "a player saved 1024 gems or more: outside the packed identity key");
+        if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "batch visited table full during level %d", s->level);
+        n_uniq = (int64_t)c->h_ctr->n_new;
+        c->occupied += n_uniq;
+        if (n_uniq) {
+            CK(c, c->ridx64.ensure((size_t)n_uniq * 8, 0, st));
+            const unsigned wt = nblk(total, TILE * 8);
+            CKS(c, prep_status(c, 0, wt, st));
+            CKS(c, reset_ticket(c, 0, st));
+            r_winners_kernel<<<wt, TILE, 0, st>>>(c->cand_slot.as<uint32_t>(), c->rbtab.as<RBucket>(), total, c->ridx64.as<int64_t>(),
+                                                   c->status[0].as<uint64_t>(), c->d_ctr, 0);
+            CK(c, s->uniq.ensure((size_t)n_uniq * 96, 0, st));
+            CK(c, R.uniq_game.ensure((size_t)n_uniq * 4, 0, st));
+            rb_gather_kernel<<<nblk(n_uniq), TILE, 0, st>>>(c->rcand.as<RRec>(), R.cand_game.as<uint32_t>(), c->ridx64.as<int64_t>(), n_uniq,
+                                                             s->uniq.as<RRec>(), R.uniq_game.as<uint32_t>());
+            c->launches += 2;
+            CK(c, cudaGetLastError());
+        }
+    } else {
+        CK(c, cudaEventRecord(c->ev[2], st));
+    }
+    CK(c, cudaEventRecord(c->ev[3], st));
+    // ---- per-game bookkeeping: who ends at this level, and the offsets of the winners' and of the next queue's runs
+    // (the reference leaves its loop after the iteration with turn == 1000, src/solver.py:846-852)
+    const bool turn_limit = s->level >= 1000;
+    std::vector<int64_t> kseg(B + 1, 0), useg(B + 1, 0);
+    bool all_ended = true;
+    for (int g = 0; g < B; ++g) {
+        const int64_t ng = seg[g + 1] - seg[g];
+        int64_t kept = 0;
+        useg[g + 1] = useg[g];
+        if (ng > 0) {
+            spl_rgame_info &I = R.info[g];
+            const int64_t uniq = (int64_t)g_host[2 * B + g];
+            I.level = s->level;
+            I.frontier = ng;
+            I.goal_rank = -1;
+            if (g_host[g] != 0x7fffffffffffffffll) {  // goal dequeued: nothing of this level is expanded
+                I.generated = I.unique = I.kept = 0;
+                I.goal_rank = R.final_rank[g] = g_host[g];
+                I.ended = 1;
+            } else {
+                I.generated = g_host[B + g];
+                I.unique = uniq;
+                I.visited += uniq;
+                I.kept = std::min(uniq, R.beam[g]);
+                if (I.kept == 0 || turn_limit) {  // queue exhausted / turn limit: the last state dequeued ends the game
+                    I.ended = 1;
+                    R.final_rank[g] = ng - 1;
+                } else {
+                    kept = I.kept;
+                    all_ended = false;
+                }
+            }
+            useg[g + 1] += uniq;
+        }
+        kseg[g + 1] = kseg[g] + kept;
+    }
+    if (useg[B] != n_uniq) return fail(c, SPL_E_CUDA, "internal: %lld winners, %lld counted per game", (long long)n_uniq, (long long)useg[B]);
+    const int64_t n_kept = kseg[B];
+    // ---- score + segmented cut into the next queue
+    if (n_kept) {
+        for (int b = 0; b < 2; ++b) {
+            CK(c, c->y[b].ensure((size_t)n_uniq * 8 + 8, 0, st));
+            CK(c, c->idx[b].ensure((size_t)n_uniq * 4 + 4, 0, st));
+        }
+        CKS(c, zero_ctr(c, st));
+        rb_score_kernel<<<nblk(n_uniq), TILE, 0, st>>>(s->uniq.as<RRec>(), R.uniq_game.as<uint32_t>(), n_uniq, cfg, c->luts,
+                                                        c->y[0].as<uint64_t>(), c->idx[0].as<uint32_t>(), c->d_ctr);
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CKS(c, read_ctr(c, st));
+        CK(c, cudaEventRecord(c->ev[4], st));
+        // every score key lies between sk_min and sk_max, so the y words differ only in the low bits where those two do
+        int cur = 0;
+        CKS(c, sort_pairs(c, n_uniq, bitlen(c->h_ctr->sk_min ^ c->h_ctr->sk_max), &cur, st));
+        if (B > 1) {
+            rb_game_words_kernel<<<nblk(n_uniq), TILE, 0, st>>>(c->idx[cur].as<uint32_t>(), R.uniq_game.as<uint32_t>(), n_uniq,
+                                                                 c->y[cur].as<uint64_t>());
+            ++c->launches;
+            CKS(c, sort_pairs(c, n_uniq, bitlen((uint64_t)B - 1), &cur, st));
+        }
+        std::vector<int64_t> segs(kseg);  // the next queue's offsets, then the winners'
+        segs.insert(segs.end(), useg.begin(), useg.end());
+        CK(c, cudaMemcpyAsync(R.seg.p, segs.data(), segs.size() * 8, cudaMemcpyHostToDevice, st));
+        c->h2d_bytes += segs.size() * 8;
+        CK(c, s->front.ensure((size_t)n_kept * 96, 0, st));
+        rb_cut_kernel<<<nblk(n_uniq), TILE, 0, st>>>(s->uniq.as<RRec>(), R.uniq_game.as<uint32_t>(), c->idx[cur].as<uint32_t>(), n_uniq,
+                                                      R.seg.as<int64_t>() + (B + 1), R.seg.as<int64_t>(), s->front.as<RRec>());
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CK(c, cudaStreamSynchronize(st));  // segs is a local
+    } else {
+        CK(c, cudaEventRecord(c->ev[4], st));
+    }
+    CK(c, cudaEventRecord(c->ev[5], st));
+    CK(c, cudaEventSynchronize(c->ev[5]));
+    float t;
+    cudaEventElapsedTime(&t, c->ev[0], c->ev[1]); info->ms_count = t;
+    cudaEventElapsedTime(&t, c->ev[1], c->ev[2]); info->ms_expand = t;
+    cudaEventElapsedTime(&t, c->ev[2], c->ev[3]); info->ms_resolve = t;
+    cudaEventElapsedTime(&t, c->ev[3], c->ev[4]); info->ms_select = t;
+    cudaEventElapsedTime(&t, c->ev[4], c->ev[5]); info->ms_sort = t;
+    info->expanded = n;
+    info->generated = total;
+    info->unique = n_uniq;
+    for (int g = 0; g < B; ++g)
+        if (seg[g + 1] > seg[g]) info->kept += R.info[g].kept;
+    info->visited = (int64_t)c->occupied;
+    info->table_slots = c->rbtab.slots();
+    if (all_ended) {
+        s->ended = true;
+        info->ended = 1;
+        return SPL_OK;
+    }
+    s->n_front = n_kept;
+    s->level += 1;
+    R.seg_at.push_back(kseg);
+    CKS(c, save_links(s, n_kept, true, false, st));
+    CK(c, cudaStreamSynchronize(st));
+    return SPL_OK;
+}
+
 // ------------------------------------------------------------------ second half of a level
 // Score (realistic level, or externally drawn noise: the key-table level scores as it resolves, the grouped level as it
 // deduplicates), beam cut (src/solver.py:452-456, :846) and gather of the queue in rank order, or the plain BFS
@@ -2518,6 +2747,7 @@ int32_t spl_solver_step(spl_solver *s, spl_level_info *info, void *stream) {
     info->level = s->level;
     info->frontier = s->n_front;
     info->goal_rank = -1;
+    if (s->kind == REALISTIC_BATCH) return rbatch_step(s, info, st);
     const int64_t n = s->n_front;
     const bool realistic = s->kind == REALISTIC;
     if (realistic && c->rcfg_dirty) {  // spl_rscore / spl_rexpand / spl_rmaxpts ran with their own GameConfig in between
@@ -2638,6 +2868,145 @@ int32_t spl_rsolver_frontier(spl_solver *s, const void **recs, int64_t *n) {
     if (!s || !recs || !n || s->kind != REALISTIC) return SPL_E_INVALID;
     *recs = s->front.p;
     *n = s->n_front;
+    return SPL_OK;
+}
+
+// ---- batched realistic search
+constexpr int32_t MAX_BATCH_GAMES = 1 << 16;
+
+int32_t spl_rbatch_create(spl_ctx *c, const spl_rconfig *cfgs, const void *root_recs_host, const int64_t *beams, int32_t n_games,
+                          int32_t keep_links, spl_solver **out) {
+    if (!c || !cfgs || !root_recs_host || !beams || !out) return fail(c, SPL_E_INVALID, "spl_rbatch_create: null argument");
+    if (n_games < 1 || n_games > MAX_BATCH_GAMES) return fail(c, SPL_E_INVALID, "spl_rbatch_create: n_games must be 1..%d", MAX_BATCH_GAMES);
+    std::vector<RConfigDev> dev((size_t)n_games);
+    for (int g = 0; g < n_games; ++g) {
+        if (beams[g] < 1) return fail(c, SPL_E_INVALID, "spl_rbatch_create: game %d: beam_width must be >= 1", g);
+        if (cfgs[g].noise != SPL_NOISE_CONST && cfgs[g].noise != SPL_NOISE_HASH)
+            return fail(c, SPL_E_INVALID, "spl_rbatch_create: game %d: noise must be const or hash (mt draws depend on the other games)", g);
+        CKS(c, make_rconfig(c, cfgs + g, dev[g]));
+    }
+    NO_LIVE_SOLVER(c, "spl_rbatch_create");
+    CK(c, enter_device(c));
+    spl_solver *s = new spl_solver(c);
+    s->kind = REALISTIC_BATCH; s->use_h = 1; s->keep_links = keep_links; s->n_front = n_games;
+    s->rb = std::make_unique<RBatch>();
+    RBatch &R = *s->rb;
+    R.B = n_games;
+    R.beam.assign(beams, beams + n_games);
+    R.info.assign((size_t)n_games, spl_rgame_info{});
+    for (auto &I : R.info) { I.visited = 1; I.goal_rank = -1; }
+    R.final_rank.assign((size_t)n_games, 0);
+    std::vector<int64_t> seg((size_t)n_games + 1);
+    std::vector<uint32_t> iota((size_t)n_games);
+    for (int g = 0; g <= n_games; ++g) seg[g] = g;
+    for (int g = 0; g < n_games; ++g) iota[g] = (uint32_t)g;
+    R.seg_at.push_back(seg);
+    const size_t B = (size_t)n_games;
+    const cudaError_t e = [&]() -> cudaError_t {
+        cudaError_t r = R.cfg.ensure(B * sizeof(RConfigDev), 0, 0);
+        if (r == cudaSuccess) r = R.roots.ensure(B * 96, 0, 0);
+        if (r == cudaSuccess) r = R.seg.ensure((2 * B + 2) * 8, 0, 0);
+        if (r == cudaSuccess) r = R.gctr.ensure(3 * B * 8, 0, 0);
+        if (r == cudaSuccess) r = R.cand_game.ensure(B * 4, 0, 0);
+        if (r == cudaSuccess) r = cudaMemcpyAsync(R.cfg.p, dev.data(), B * sizeof(RConfigDev), cudaMemcpyHostToDevice, 0);
+        if (r == cudaSuccess) r = cudaMemcpyAsync(R.roots.p, root_recs_host, B * 96, cudaMemcpyHostToDevice, 0);
+        if (r == cudaSuccess) r = cudaMemcpyAsync(R.seg.p, seg.data(), (B + 1) * 8, cudaMemcpyHostToDevice, 0);
+        if (r == cudaSuccess) r = cudaMemsetAsync(R.gctr.p, 0, 3 * B * 8, 0);
+        if (r == cudaSuccess) r = cudaMemcpyAsync(R.cand_game.p, iota.data(), B * 4, cudaMemcpyHostToDevice, 0);
+        if (r == cudaSuccess) r = cudaStreamSynchronize(0);
+        return r;
+    }();
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        delete s;
+        return fail(c, e == cudaErrorMemoryAllocation ? SPL_E_NOMEM : SPL_E_CUDA, "spl_rbatch_create: %s", cudaGetErrorString(e));
+    }
+    c->h2d_bytes += B * (sizeof(RConfigDev) + 96 + 8 + 4) + 8;
+    return open_solver(s, REALISTIC_BATCH, root_recs_host, n_games, 96, false, "rbatch create sync failed", out);
+}
+
+int32_t spl_rbatch_games(spl_solver *s, spl_rgame_info *out_host, int32_t n_games) {
+    if (!s || !out_host || s->kind != REALISTIC_BATCH) return SPL_E_INVALID;
+    if (n_games != s->rb->B) return fail(s->c, SPL_E_INVALID, "spl_rbatch_games: the batch has %d games", s->rb->B);
+    memcpy(out_host, s->rb->info.data(), sizeof(spl_rgame_info) * (size_t)n_games);
+    return SPL_OK;
+}
+
+int32_t spl_rbatch_frontier(spl_solver *s, int32_t game, const void **recs_dev, int64_t *n_host) {
+    if (!s || !recs_dev || !n_host || s->kind != REALISTIC_BATCH) return SPL_E_INVALID;
+    if (game < 0 || game >= s->rb->B) return fail(s->c, SPL_E_INVALID, "spl_rbatch_frontier: no game %d", game);
+    const std::vector<int64_t> &seg = s->rb->seg_at.back();
+    const bool live = !s->ended;  // the last level's queue was expanded and replaced by nothing
+    *recs_dev = static_cast<const char *>(s->front.p) + seg[game] * 96;
+    *n_host = live ? seg[game + 1] - seg[game] : 0;
+    return SPL_OK;
+}
+
+// Walk every game's line back through the link columns, one batched read per level (a spilled column is read where it
+// lies, on the host), then rebuild the records forward from the roots on the device.
+int32_t spl_rbatch_lines(spl_solver *s, void *recs_host, int64_t cap, int32_t *plies_host) {
+    if (!s || !recs_host || !plies_host || s->kind != REALISTIC_BATCH) return SPL_E_INVALID;
+    spl_ctx *c = s->c;
+    RBatch &R = *s->rb;
+    if (!s->ended) return fail(c, SPL_E_STATE, "spl_rbatch_lines: the batch has not ended");
+    if (!s->keep_links) return fail(c, SPL_E_STATE, "spl_rbatch_lines: solver was created with keep_links = 0");
+    CK(c, enter_device(c));
+    const int B = R.B;
+    int max_plies = 0;
+    for (int g = 0; g < B; ++g) {
+        plies_host[g] = (int32_t)R.info[g].level;
+        max_plies = std::max(max_plies, plies_host[g]);
+    }
+    if (max_plies + 1 > cap) return fail(c, SPL_E_CAPACITY, "spl_rbatch_lines: a line needs %d records", max_plies + 1);
+    const cudaStream_t st = 0;
+    std::vector<int64_t> rank(R.final_rank), at;
+    std::vector<int> who;
+    std::vector<uint64_t> link;
+    std::vector<uint8_t> ords((size_t)B * std::max(max_plies, 1), 0);
+    for (int l = max_plies; l >= 1; --l) {
+        at.clear();
+        who.clear();
+        for (int g = 0; g < B; ++g)
+            if (plies_host[g] >= l) { who.push_back(g); at.push_back(R.seg_at[l][g] + rank[g]); }
+        const int64_t m = (int64_t)at.size();
+        link.resize(at.size());
+        if (s->links.host[l]) {
+            for (int64_t k = 0; k < m; ++k) link[k] = s->links.host[l][at[k]];
+        } else {
+            CK(c, R.scratch.ensure((size_t)m * 16, 0, st));
+            int64_t *d_at = R.scratch.as<int64_t>();
+            CK(c, cudaMemcpyAsync(d_at, at.data(), (size_t)m * 8, cudaMemcpyHostToDevice, st));
+            rb_pick_kernel<<<nblk(m), TILE, 0, st>>>(s->links.dev[l]->as<uint64_t>(), d_at, m, reinterpret_cast<uint64_t *>(d_at + m));
+            ++c->launches;
+            CK(c, cudaGetLastError());
+            CK(c, cudaMemcpyAsync(link.data(), d_at + m, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
+            CK(c, cudaStreamSynchronize(st));
+            c->h2d_bytes += m * 8;
+            c->d2h_bytes += m * 8;
+        }
+        for (int64_t k = 0; k < m; ++k) {
+            const int g = who[k];
+            ords[(size_t)g * max_plies + (l - 1)] = (uint8_t)(link[k] & 0xff);
+            rank[g] = (int64_t)(link[k] >> 8);
+        }
+    }
+    const size_t line_recs = (size_t)max_plies + 1;
+    CK(c, R.scratch.ensure(ords.size() + (size_t)B * 4 + 16, 0, st));
+    CK(c, R.lines.ensure((size_t)B * line_recs * 96, 0, st));
+    int32_t *d_plies = R.scratch.as<int32_t>();
+    uint8_t *d_ords = reinterpret_cast<uint8_t *>(d_plies + B);
+    CK(c, cudaMemcpyAsync(d_plies, plies_host, (size_t)B * 4, cudaMemcpyHostToDevice, st));
+    CK(c, cudaMemcpyAsync(d_ords, ords.data(), ords.size(), cudaMemcpyHostToDevice, st));
+    CKS(c, zero_ctr(c, st));
+    rb_line_kernel<<<nblk(B), TILE, 0, st>>>(R.roots.as<RRec>(), R.cfg.as<RConfigDev>(), B, d_plies, d_ords, max_plies,
+                                              R.lines.as<RRec>(), c->d_ctr);
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    CK(c, cudaMemcpy2DAsync(recs_host, (size_t)cap * 96, R.lines.p, line_recs * 96, line_recs * 96, (size_t)B, cudaMemcpyDeviceToHost, st));
+    CKS(c, read_ctr(c, st));
+    c->h2d_bytes += (int64_t)(B * 4 + ords.size());
+    c->d2h_bytes += (int64_t)(B * line_recs * 96);
+    if (c->h_ctr->error) return fail(c, SPL_E_CUDA, "internal: a link ordinal names no successor");
     return SPL_OK;
 }
 
@@ -2795,6 +3164,7 @@ int32_t spl_solver_frontier(spl_solver *s, const spl_key **keys, const uint64_t 
 int32_t spl_solver_path(spl_solver *s, int64_t *ranks, int32_t *ordinals, int32_t cap, int32_t *n_moves) {
     if (!s || !ranks || !ordinals || !n_moves) return SPL_E_INVALID;
     spl_ctx *c = s->c;
+    if (s->kind == REALISTIC_BATCH) return fail(c, SPL_E_INVALID, "spl_solver_path: a batched solver's lines come from spl_rbatch_lines");
     if (!s->ended) return fail(c, SPL_E_STATE, "spl_solver_path: the search has not ended");
     if (!s->keep_links) return fail(c, SPL_E_STATE, "spl_solver_path: solver was created with keep_links = 0");
     const int L = s->level;  // level index of the final state

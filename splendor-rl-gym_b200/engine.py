@@ -7,7 +7,7 @@ import ctypes as C
 import numpy as np
 import torch
 
-from ._lib import Config, Key, LevelInfo, check, lib
+from ._lib import Config, Key, LevelInfo, RGameInfo, check, lib
 
 HEURISTIC_IDS = {'simple': 0, 'balanced': 1, 'aggressive': 2, 'efficiency': 3, 'competitive': 1}
 TIE_IDS = {'stable': 0, 'det': 1, 'key': 1, 'det_ordered': 2}
@@ -282,6 +282,10 @@ class Engine:
     def rsolver(self, rcfg, root_rec_np: np.ndarray, beam_width: int, keep_links: bool = True) -> 'RLevelSolver':
         return RLevelSolver(self, rcfg, root_rec_np, beam_width, keep_links)
 
+    def rbatch_solver(self, rcfgs, roots_np: np.ndarray, beams, keep_links: bool = True) -> 'RBatchSolver':
+        """spl_rbatch_create: len(rcfgs) realistic-mode games searched in lockstep (root record and beam width per game)."""
+        return RBatchSolver(self, rcfgs, roots_np, beams, keep_links)
+
     # -------------------------------------------------------------- fused solver
     def solver(self, root_key: int, root_aux: int, goal_pts: int, use_heuristic: bool, heuristic: str, beam_width: int,
                tie: str = 'stable', noise: str = 'const', keep_links: bool = True, identity: str = 'key',
@@ -414,3 +418,67 @@ class RLevelSolver(LevelSolver):
             return np.zeros(0, self._dtype)
         t = torch.as_tensor(_DevArray(p.value, (n.value, 96), '|u1'), device=self.eng.tdev)
         return t.cpu().numpy().reshape(-1).view(self._dtype).copy()
+
+
+class RBatchSolver(Stepper):
+    """spl_rbatch_create + spl_solver_step: B MultiPlayerState.solve() searches in lockstep (realistic.solve_many)."""
+
+    def __init__(self, eng: Engine, rcfgs, roots_np, beams, keep_links=True):
+        self.eng = eng
+        self.n_games = len(rcfgs)
+        roots = np.ascontiguousarray(roots_np).reshape(-1)
+        if len(roots) != self.n_games or len(beams) != self.n_games:
+            raise ValueError(f'{self.n_games} configs, {len(roots)} roots and {len(beams)} beam widths')
+        cfgs = (type(rcfgs[0]) * self.n_games)(*rcfgs)
+        bw = np.ascontiguousarray(beams, dtype=np.int64)
+        h = C.c_void_p()
+        check(lib.spl_rbatch_create(eng._h, cfgs, roots.ctypes.data, bw.ctypes.data, self.n_games, int(keep_links),
+                                    C.byref(h)), eng._h)
+        self._h = h
+        self._dtype = roots.dtype
+        self.infos = []
+        self.ended = False
+
+    def step(self) -> dict:
+        """One level of every running game: the aggregate counters (spl_level_info) plus 'games', the per-game
+        counters (a game's dict stops changing once it has ended)."""
+        li = LevelInfo()
+        check(lib.spl_solver_step(self._h, C.byref(li), self.eng._stream()), self.eng._h)
+        d = li.as_dict()
+        d['games'] = self.games()
+        self.infos.append(d)
+        self.ended = bool(li.ended)
+        return d
+
+    def games(self) -> list:
+        out = (RGameInfo * self.n_games)()
+        check(lib.spl_rbatch_games(self._h, out, self.n_games), self.eng._h)
+        return [g.as_dict() for g in out]
+
+    def frontier(self, game: int) -> np.ndarray:
+        """game `game`'s current queue as host records (96 B each); empty once the game has ended"""
+        p, n = C.c_void_p(), C.c_int64()
+        check(lib.spl_rbatch_frontier(self._h, int(game), C.byref(p), C.byref(n)), self.eng._h)
+        if n.value == 0:
+            return np.zeros(0, self._dtype)
+        t = torch.as_tensor(_DevArray(p.value, (n.value, 96), '|u1'), device=self.eng.tdev)
+        return t.cpu().numpy().reshape(-1).view(self._dtype).copy()
+
+    def lines(self) -> list:
+        """every game's line as host records, root first (spl_rbatch_lines)"""
+        plies = (C.c_int32 * self.n_games)()
+        cap = max((g['level'] for g in self.games()), default=0) + 1
+        recs = np.zeros(self.n_games * cap, self._dtype)
+        check(lib.spl_rbatch_lines(self._h, recs.ctypes.data, cap, plies), self.eng._h)
+        return [recs[g * cap:g * cap + plies[g] + 1] for g in range(self.n_games)]
+
+    def close(self):
+        if getattr(self, '_h', None):
+            lib.spl_solver_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

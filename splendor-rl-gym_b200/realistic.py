@@ -2,7 +2,7 @@
 MultiPlayerState surface (src/solver.py:25-200, 471-860) driven by the CUDA library.
 
 `MultiPlayerState.solve()` -> spl_rsolver_* (with `shard=True`: RShardedSolver over the ranks of the process group,
-sharded.py) ; `__iter__` -> spl_rexpand on one record; the
+sharded.py) ; `solve_many()` -> spl_rbatch_* (many games in lockstep on one GPU) ; `__iter__` -> spl_rexpand on one record; the
 competitive heuristic -> spl_rscore.  The card market order (optionally shuffled with Python's
 `random.Random(seed)` exactly as CardMarket.from_full_deck does) is computed here on the host and
 handed to the kernels as an input table.  The reference draws tie-break noise from the unseeded
@@ -10,6 +10,7 @@ global RNG; here `randint` is the declared constant 50 (`noise='const'`) and sco
 arrival order, which is what the reference's stable `sorted(..., reverse=True)` does.
 """
 import ctypes as C
+import numbers
 import random
 from dataclasses import dataclass
 
@@ -364,3 +365,44 @@ class MultiPlayerState:
         finally:
             sol.close()
         return ordinals
+
+
+def solve_many(roots, *, beam_width=20_000, noise: str = 'const', device: int | None = None, engine: Engine | None = None,
+               stats: list | None = None) -> list[list[MultiPlayerState]]:
+    """`root.solve(beam_width=..., noise=..., verbose=False)` for every root of `roots`, searched together on one GPU:
+    the games advance one level at a time in lockstep, each with its own rules, market and beam width (`beam_width` is
+    one int or one per game), and each returns exactly the line its own solve() returns.  noise is 'const' or 'hash'
+    ('mt' draws depend on the other games).  With `stats`, one dict per level is appended: the aggregate counters and
+    'games', the per-game counters."""
+    from .solver import _engine
+    roots = list(roots)
+    if not roots:
+        raise ValueError('solve_many needs at least one game')
+    for r in roots:
+        if r.config.infinite_resources:
+            raise ValueError('solve_many: a root with infinite_resources=True follows the speedrun rules; use State.solve')
+    if noise not in ('const', 'hash'):
+        raise ValueError(f"solve_many supports noise 'const' and 'hash', not {noise!r}: 'mt' draws depend on the other games")
+    beams = [beam_width] * len(roots) if isinstance(beam_width, numbers.Integral) else list(beam_width)
+    if len(beams) != len(roots):
+        raise ValueError(f'solve_many: {len(beams)} beam widths for {len(roots)} games')
+    if any(int(b) < 1 for b in beams):
+        raise ValueError('solve_many: every beam width must be >= 1')
+    eng = engine or _engine(device)
+    sol = eng.rbatch_solver([r.rconfig(noise) for r in roots], np.concatenate([r.record() for r in roots]),
+                            [int(b) for b in beams])
+    try:
+        while not sol.ended:
+            info = sol.step()
+            if stats is not None:
+                stats.append(info)
+        lines = sol.lines()
+    finally:
+        sol.close()
+    out = []
+    for root, recs in zip(roots, lines):
+        path = [root]
+        for rec in recs[1:]:
+            path.append(path[-1]._child_from_record(rec))
+        out.append(path)
+    return out
