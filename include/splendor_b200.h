@@ -395,6 +395,37 @@ int32_t spl_rbatch_frontier(spl_solver *s, int32_t game, const void **recs_dev, 
  * than cap records.  The lines are rebuilt on the device from the link columns, one thread per game. */
 int32_t spl_rbatch_lines(spl_solver *s, void *recs_host, int64_t cap, int32_t *plies_host);
 
+/* ---- batched speedrun search (solver.py: State.solve_many) --------------------------------------------------------
+ * n_games independent State.solve() searches advance in lockstep on one GPU: each spl_solver_step is one level of every
+ * game still running, at a number of kernel launches that does not depend on n_games.  Game g starts from the 32-byte
+ * row root_rows_host[g] = {lo, hi, aux, link} (link ignored) and has its own goal (goals[g]), search kind
+ * (use_heuristic[g]: 0 = exhaustive BFS, every unique state in arrival order) and, for beam search, heuristic
+ * (heuristics[g], as spl_solver_create's) and beam width (beams[g] >= 1).  tie_policy (SPL_TIE_STABLE or SPL_TIE_KEY)
+ * and noise (SPL_NOISE_CONST or SPL_NOISE_HASH: externally drawn noise would depend on the other games) hold for the
+ * whole batch.  Every root is checked as spl_solver_create_queue checks its rows (illegal gem hand, key bit at or
+ * above 105); equal roots in different games are separate games.  A bad root, beam, tie policy or noise fails with
+ * SPL_E_INVALID, naming the game.  Every level of game g equals spl_solver_create's level for that game alone: the
+ * same rows in the same rank order (link words carry ranks inside the game), the same counters, goal rank and line.
+ * A state of one game never merges with a state of another: the visited identity is (game, key).  A game leaves the
+ * batch when a state of its queue meets its goal or its queue runs out (there is no turn limit, as in State.solve);
+ * the batch ends when every game has.  spl_solver_step fills the aggregate counters as for spl_rbatch_create, with
+ * ms_select = score and ms_sort = the key passes ('det') and the segmented cut.  A level above 2^32 - 1 candidates
+ * fails with SPL_E_INVALID; a full visited table or device memory fails with SPL_E_TABLE_FULL / SPL_E_NOMEM, and the
+ * context stays usable once the solver is destroyed.  Destroy with spl_solver_destroy; spl_solver_path does not apply
+ * (use spl_sbatch_lines).  Link columns spill past spl_set_link_budget as a single solve's do. */
+int32_t spl_sbatch_create(spl_ctx *ctx, const void *root_rows_host /* n_games x {lo, hi, aux, link} */, const int32_t *goals,
+                          const int32_t *use_heuristic, const int32_t *heuristics, const int64_t *beams, int32_t n_games,
+                          int32_t tie_policy, int32_t noise, int32_t keep_links, spl_solver **out);
+/* the per-game counters after the last spl_solver_step (n_games must be the batch's) */
+int32_t spl_sbatch_games(spl_solver *s, spl_rgame_info *out_host, int32_t n_games);
+/* game `game`'s queue as 32-byte rows {lo, hi, aux, link} in rank order (device memory of the solver; link = parent
+ * rank inside the game << 8 | ordinal); empty once the game has ended */
+int32_t spl_sbatch_frontier(spl_solver *s, int32_t game, const void **rows_dev, int64_t *n_host);
+/* after the batch has ended (keep_links = 1): every game's line, root first, as 32-byte rows (link = the ordinal that
+ * leads to the row, ~0 for the root).  plies_host[g] = moves of game g; its plies_host[g] + 1 rows go to
+ * rows_host[g * cap ...].  SPL_E_CAPACITY (plies_host filled) when a line needs more than cap rows. */
+int32_t spl_sbatch_lines(spl_solver *s, void *rows_host, int64_t cap, int32_t *plies_host);
+
 /* ---- realistic mode on the key-sharded driver (sharded.py: RCudaBackend + RShardedSolver) ---------------------------
  * MultiPlayerState.solve(shard=True) / --realistic --shard: the level loop of :820-852 over a queue spread block-cyclically
  * across ranks, with the same per-level steps as spl_expand_rows .. spl_move_rows above.  Every level holds the same

@@ -102,6 +102,10 @@ def _load():
         'spl_rbatch_games': (i32, [vp, vp, i32]),
         'spl_rbatch_frontier': (i32, [vp, i32, C.POINTER(vp), C.POINTER(i64)]),
         'spl_rbatch_lines': (i32, [vp, vp, i64, vp]),
+        'spl_sbatch_create': (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, C.POINTER(vp)]),
+        'spl_sbatch_games': (i32, [vp, vp, i32]),
+        'spl_sbatch_frontier': (i32, [vp, i32, C.POINTER(vp), C.POINTER(i64)]),
+        'spl_sbatch_lines': (i32, [vp, vp, i64, vp]),
         'spl_rexpand_rows': (i32, [vp, vp, vp, i64, i64, vp, i64, C.POINTER(i64), vp]),
         'spl_rroute_keys': (i32, [vp, vp, vp, i64, i32, vp, vp, vp]),
         'spl_rdedup_flags': (i32, [vp, vp, i64, vp, vp]),

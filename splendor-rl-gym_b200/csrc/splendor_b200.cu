@@ -17,6 +17,7 @@
 #include "spl_m2.cuh"
 #include "spl_shard.cuh"
 #include "spl_realistic.cuh"
+#include "spl_sbatch.cuh"
 #include "spl_tables.cuh"
 
 using namespace spl;
@@ -113,6 +114,15 @@ static const TableDesc RBATCH_TABLE_DESC = {
     },
     "batch table rehash into %llu buckets overflowed a probe sequence",
     "batch visited table full: %llu states + %llu candidates vs %llu buckets (max_table_bytes=%llu)"};
+// bucket ids are u32 with R_DEAD = 2^32 - 1 reserved: at most 2^32 - 1 buckets (128 GiB)
+static const TableDesc SBATCH_TABLE_DESC = {
+    32, 1, 0xFFFFFFFFull, 0.6, 4,
+    [](const void *from, uint64_t units, void *to, uint64_t to_units, Counters *ctr, cudaStream_t st) {
+        sb_rehash_kernel<<<nblk((int64_t)units), TILE, 0, st>>>(static_cast<const SBucket *>(from), units,
+                                                                 static_cast<SBucket *>(to), to_units, ctr);
+    },
+    "speedrun batch table rehash into %llu buckets overflowed a probe sequence",
+    "speedrun batch visited table full: %llu states + %llu candidates vs %llu buckets (max_table_bytes=%llu)"};
 
 // A visited set on the device: an open-addressing table that grows by rehashing into one twice its size.  It counts
 // its own entries, those of an insert that failed part way included, so that clear() can skip a table that holds none.
@@ -147,9 +157,10 @@ struct spl_ctx {
     int device = 0;
     std::string err;
     // visited sets: the key table (BFS, the reference's hash identity, externally drawn noise and the stage operators),
-    // the card-set node table of the grouped level (spl_m2.cuh), the realistic level's table and the batched realistic
-    // level's (game, key) table (both allocated on first use)
-    VisitTable key{KEY_TABLE_DESC}, nodes{NODE_TABLE_DESC}, rtab{REALISTIC_TABLE_DESC}, rbtab{RBATCH_TABLE_DESC};
+    // the card-set node table of the grouped level (spl_m2.cuh), the realistic level's table and the (game, key) tables
+    // of the batched realistic and speedrun levels (all three allocated on first use)
+    VisitTable key{KEY_TABLE_DESC}, nodes{NODE_TABLE_DESC}, rtab{REALISTIC_TABLE_DESC}, rbtab{RBATCH_TABLE_DESC},
+        sbtab{SBATCH_TABLE_DESC};
     uint64_t occupied = 0;  // visited states: those of the last solve, plus what stage operators added to the key table
     uint32_t epoch = 0;
     uint64_t chunk_parents = 0;
@@ -303,7 +314,7 @@ int32_t spl_create(const spl_config *cfg, spl_ctx **out) {
     CKC(cudaSetDevice(c->device));
     size_t free_b = 0, total_b = 0;
     CKC(cudaMemGetInfo(&free_b, &total_b));
-    c->key.max_bytes = c->rtab.max_bytes = c->rbtab.max_bytes = cfg->max_table_bytes ? cfg->max_table_bytes : (uint64_t)(free_b * 0.6);
+    c->key.max_bytes = c->rtab.max_bytes = c->rbtab.max_bytes = c->sbtab.max_bytes = cfg->max_table_bytes ? cfg->max_table_bytes : (uint64_t)(free_b * 0.6);
     c->chunk_user = cfg->chunk_parents != 0;
     c->chunk_parents = cfg->chunk_parents ? std::min<uint64_t>(cfg->chunk_parents, MAX_CHUNK_PARENTS) : (4ull << 20);
     c->chunk_parents = std::max<uint64_t>(c->chunk_parents, TILE);
@@ -1306,14 +1317,17 @@ enum LevelKind {
     GROUPED,    // beam search on the card-set-grouped level (spl_m2.cuh), visited set in the node table
     REALISTIC,  // realistic mode: materialised 96-byte successors, exact-key table
     REALISTIC_BATCH,  // realistic mode, many games in lockstep: game-major queues, (game, exact key) table
+    SPEEDRUN_BATCH,   // speedrun mode, many games in lockstep: game-major 32-byte queues, (game, key) table (spl_sbatch.cuh)
 };
 static const VisitTable &visited_table(const spl_ctx *c, LevelKind kind) {
-    return kind == KEY_TABLE ? c->key : kind == GROUPED ? c->nodes : kind == REALISTIC ? c->rtab : c->rbtab;
+    return kind == KEY_TABLE ? c->key : kind == GROUPED ? c->nodes : kind == REALISTIC ? c->rtab
+         : kind == REALISTIC_BATCH ? c->rbtab : c->sbtab;
 }
 
-// What a batched realistic solver keeps beside the common queue buffers (spl_rbatch_*, spl_realistic.cuh): the games'
-// configs and roots, the queue's game-major offsets (on the device for the kernels, on the host per level for the line
-// walk), the per-game counters, and the game column of the candidates and of the winners.
+// What a batched solver keeps beside the common queue buffers (spl_rbatch_*, spl_realistic.cuh; spl_sbatch_*,
+// spl_sbatch.cuh): the games' configs (RConfigDev or SGame) and roots, the queue's game-major offsets (on the device for
+// the kernels, on the host per level for the line walk), the per-game counters, and the game column of the candidates
+// and of the winners.
 struct RBatch {
     int B = 0;
     std::vector<int64_t> beam;
@@ -1336,7 +1350,7 @@ struct spl_solver : SolverBufs {
     int level = 0;
     bool ended = false;
     int64_t goal_rank = -1;
-    std::unique_ptr<RBatch> rb;  // REALISTIC_BATCH only
+    std::unique_ptr<RBatch> rb;  // REALISTIC_BATCH and SPEEDRUN_BATCH only
     explicit spl_solver(spl_ctx *ctx) : SolverBufs(ctx) {}
 };
 
@@ -1558,13 +1572,13 @@ static int grouped_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6],
 }
 
 // ------------------------------------------------------------------ solver create
-// The realistic tables (rtab, or rbtab of the batched search) are allocated on first use, sized by the caller's
-// table_slots.  A realistic search does not use the key table: a large, empty one gives its memory back first.
+// The realistic tables and the batch tables (rtab, rbtab, sbtab) are allocated on first use, sized by the caller's
+// table_slots.  They do not use the key table: a large, empty one gives its memory back first.
 static int open_rtable(spl_ctx *c, cudaStream_t st, VisitTable &t) {
     if (t.p) return SPL_OK;
     if (c->key.occ == 0 && c->key.units > (1ull << 16)) CK(c, c->key.alloc(buckets_for(1ull << 12), st));
     uint64_t nb = std::max<uint64_t>(c->rslots_hint ? c->rslots_hint : (1ull << 16), 1024);
-    nb = std::min<uint64_t>(nb, t.max_bytes / 64);
+    nb = std::min<uint64_t>(nb, t.max_bytes / t.d.unit_bytes);
     CK(c, t.alloc(nb, st));
     return SPL_OK;
 }
@@ -1622,19 +1636,25 @@ static int open_solver(S *s, LevelKind kind, const void *rows, int64_t n, size_t
                 r_probe_kernel<<<1, TILE, 0, st>>>(s->front.template as<RRec>(), 1, c->rcfg.as<RConfigDev>(), c->rtab.as<RBucket>(),
                                                     c->rtab.units, tag, c->cand_slot.as<uint32_t>(), c->d_ctr);
                 c->rtab.occ = 1;
-            } else if constexpr (std::is_same_v<S, spl_solver>) {  // REALISTIC_BATCH: one root per game, rb->cand_game = 0 .. n - 1
+            } else if constexpr (std::is_same_v<S, spl_solver>) {  // the batches: one root per game, rb->cand_game = 0 .. n - 1
+                VisitTable &t = kind == REALISTIC_BATCH ? c->rbtab : c->sbtab;
                 if (c->cand_slot.ensure((size_t)n * 4, 0, st) != cudaSuccess) return fail(c, SPL_E_NOMEM, "batch scratch alloc");
-                CKS(c, open_rtable(c, st, c->rbtab));
-                CKS(c, c->rbtab.grow(c, (uint64_t)n, st));
-                if (c->rbtab.clear(st) != cudaSuccess) return fail(c, SPL_E_CUDA, "batch table reset failed");
+                CKS(c, open_rtable(c, st, t));
+                CKS(c, t.grow(c, (uint64_t)n, st));
+                if (t.clear(st) != cudaSuccess) return fail(c, SPL_E_CUDA, "batch table reset failed");
                 CKS(c, next_epoch(c, tag));
                 CKS(c, zero_ctr(c, st));  // after the table's growth
                 RBatch &R = *s->rb;
-                rb_probe_kernel<<<nblk(n), TILE, 0, st>>>(s->front.template as<RRec>(), R.cand_game.as<uint32_t>(), n,
-                                                          R.cfg.as<RConfigDev>(), c->rbtab.as<RBucket>(), c->rbtab.units, tag,
-                                                          c->cand_slot.as<uint32_t>(), c->d_ctr,
-                                                          R.gctr.as<unsigned long long>() + 2 * R.B);
-                c->rbtab.occ = (uint64_t)n;
+                unsigned long long *n_new_game = R.gctr.as<unsigned long long>() + 2 * R.B;
+                if (kind == REALISTIC_BATCH)
+                    rb_probe_kernel<<<nblk(n), TILE, 0, st>>>(s->front.template as<RRec>(), R.cand_game.as<uint32_t>(), n,
+                                                              R.cfg.as<RConfigDev>(), t.as<RBucket>(), t.units, tag,
+                                                              c->cand_slot.as<uint32_t>(), c->d_ctr, n_new_game);
+                else
+                    sb_probe_kernel<<<nblk(n), TILE, 0, st>>>(s->front.template as<Rec>(), R.cand_game.as<uint32_t>(), n,
+                                                              t.as<SBucket>(), t.units, tag, c->cand_slot.as<uint32_t>(), c->d_ctr,
+                                                              n_new_game);
+                t.occ = (uint64_t)n;
             }
             ++c->launches;
             CK(c, cudaGetLastError());
@@ -2412,6 +2432,129 @@ static int realistic_expand(spl_solver *s, int64_t n, LevelExpand *x, cudaStream
     return SPL_OK;
 }
 
+// ------------------------------------------------------------------ batched levels (spl_rbatch_*, spl_sbatch_*)
+// What the two batch kinds share after their expand + dedup: the per-game bookkeeping, the segmented beam cut and the
+// end of the level.
+//
+// Who ends at this level, and the offsets of the winners' runs (useg) and of the next queue's (kseg).  g_host holds per
+// game its goal rank (LLONG_MAX: none) | successors | new states.  A game ends when its goal is dequeued, when its queue
+// runs out, or at the turn limit (realistic mode: the reference leaves its loop after the iteration with turn == 1000,
+// src/solver.py:846-852; the speedrun solver has none).
+static int batch_bookkeeping(spl_solver *s, const std::vector<int64_t> &g_host, int64_t n_uniq, bool turn_limit,
+                             std::vector<int64_t> &kseg, std::vector<int64_t> &useg, bool *all_ended) {
+    RBatch &R = *s->rb;
+    const int B = R.B;
+    const std::vector<int64_t> &seg = R.seg_at.back();
+    kseg.assign(B + 1, 0);
+    useg.assign(B + 1, 0);
+    *all_ended = true;
+    for (int g = 0; g < B; ++g) {
+        const int64_t ng = seg[g + 1] - seg[g];
+        int64_t kept = 0;
+        useg[g + 1] = useg[g];
+        if (ng > 0) {
+            spl_rgame_info &I = R.info[g];
+            const int64_t uniq = (int64_t)g_host[2 * B + g];
+            I.level = s->level;
+            I.frontier = ng;
+            I.goal_rank = -1;
+            if (g_host[g] != 0x7fffffffffffffffll) {  // goal dequeued: nothing of this level is expanded
+                I.generated = I.unique = I.kept = 0;
+                I.goal_rank = R.final_rank[g] = g_host[g];
+                I.ended = 1;
+            } else {
+                I.generated = g_host[B + g];
+                I.unique = uniq;
+                I.visited += uniq;
+                I.kept = std::min(uniq, R.beam[g]);
+                if (I.kept == 0 || turn_limit) {  // queue exhausted / turn limit: the last state dequeued ends the game
+                    I.ended = 1;
+                    R.final_rank[g] = ng - 1;
+                } else {
+                    kept = I.kept;
+                    *all_ended = false;
+                }
+            }
+            useg[g + 1] += uniq;
+        }
+        kseg[g + 1] = kseg[g] + kept;
+    }
+    if (useg[B] != n_uniq)
+        return fail(s->c, SPL_E_CUDA, "internal: %lld winners, %lld counted per game", (long long)n_uniq, (long long)useg[B]);
+    return SPL_OK;
+}
+
+// The segmented beam cut: c->y[*cur] / c->idx[*cur] hold the n winners' score sort words (ascending = best first) in a
+// stable order, score_bits the low bits in which they differ, rb->uniq_game the winners' games.  One stable sort by
+// score, a stable pass by game, then a gather of the first min(beam_g, unique_g) pairs of every game's run into the
+// next queue (kseg: its offsets, useg: the winners').  Row: the queue's rows, 96-byte RRec or 32-byte Rec.
+template <class Row>
+static int segmented_cut(spl_solver *s, int64_t n, int score_bits, const std::vector<int64_t> &kseg, const std::vector<int64_t> &useg,
+                         int *cur, cudaStream_t st) {
+    spl_ctx *c = s->c;
+    RBatch &R = *s->rb;
+    const int B = R.B;
+    CKS(c, sort_pairs(c, n, score_bits, cur, st));
+    if (B > 1) {
+        rb_game_words_kernel<<<nblk(n), TILE, 0, st>>>(c->idx[*cur].as<uint32_t>(), R.uniq_game.as<uint32_t>(), n,
+                                                        c->y[*cur].as<uint64_t>());
+        ++c->launches;
+        CKS(c, sort_pairs(c, n, bitlen((uint64_t)B - 1), cur, st));
+    }
+    std::vector<int64_t> segs(kseg);  // the next queue's offsets, then the winners'
+    segs.insert(segs.end(), useg.begin(), useg.end());
+    CK(c, cudaMemcpyAsync(R.seg.p, segs.data(), segs.size() * 8, cudaMemcpyHostToDevice, st));
+    c->h2d_bytes += segs.size() * 8;
+    CK(c, s->front.ensure((size_t)kseg[B] * sizeof(Row), 0, st));
+    const int64_t *useg_dev = R.seg.as<int64_t>() + (B + 1), *kseg_dev = R.seg.as<int64_t>();
+    if constexpr (std::is_same_v<Row, RRec>)
+        rb_cut_kernel<<<nblk(n), TILE, 0, st>>>(s->uniq.as<RRec>(), R.uniq_game.as<uint32_t>(), c->idx[*cur].as<uint32_t>(), n,
+                                                 useg_dev, kseg_dev, s->front.as<RRec>());
+    else
+        sb_cut_kernel<<<nblk(n), TILE, 0, st>>>(s->uniq.as<Rec>(), R.uniq_game.as<uint32_t>(), c->idx[*cur].as<uint32_t>(), n,
+                                                 useg_dev, kseg_dev, s->front.as<Rec>());
+    ++c->launches;
+    CK(c, cudaGetLastError());
+    CK(c, cudaStreamSynchronize(st));  // segs is a local
+    return SPL_OK;
+}
+
+// The end of a batch level: the phase times (events 0..5: count | expand | resolve | select | sort), the aggregate
+// counters, and either the end of the batch or the next queue's offsets and link column.
+static int batch_finish(spl_solver *s, spl_level_info *info, int64_t n, int64_t total, int64_t n_uniq, const std::vector<int64_t> &kseg,
+                        bool all_ended, const VisitTable &table, bool realistic, cudaStream_t st) {
+    spl_ctx *c = s->c;
+    RBatch &R = *s->rb;
+    const int B = R.B;
+    const std::vector<int64_t> &seg = R.seg_at.back();
+    CK(c, cudaEventRecord(c->ev[5], st));
+    CK(c, cudaEventSynchronize(c->ev[5]));
+    float t;
+    cudaEventElapsedTime(&t, c->ev[0], c->ev[1]); info->ms_count = t;
+    cudaEventElapsedTime(&t, c->ev[1], c->ev[2]); info->ms_expand = t;
+    cudaEventElapsedTime(&t, c->ev[2], c->ev[3]); info->ms_resolve = t;
+    cudaEventElapsedTime(&t, c->ev[3], c->ev[4]); info->ms_select = t;
+    cudaEventElapsedTime(&t, c->ev[4], c->ev[5]); info->ms_sort = t;
+    info->expanded = n;
+    info->generated = total;
+    info->unique = n_uniq;
+    for (int g = 0; g < B; ++g)
+        if (seg[g + 1] > seg[g]) info->kept += R.info[g].kept;
+    info->visited = (int64_t)c->occupied;
+    info->table_slots = table.slots();
+    if (all_ended) {
+        s->ended = true;
+        info->ended = 1;
+        return SPL_OK;
+    }
+    s->n_front = kseg[B];
+    s->level += 1;
+    R.seg_at.push_back(kseg);
+    CKS(c, save_links(s, s->n_front, realistic, false, st));
+    CK(c, cudaStreamSynchronize(st));
+    return SPL_OK;
+}
+
 // ------------------------------------------------------------------ batched realistic level (spl_rbatch_*)
 // One level of every game still running, a fixed sequence of launches whatever the number of games: goal test + count
 // (per-game goal ranks and successor counts), expand, probe of (game, key), winners in arrival order, score, then the
@@ -2423,7 +2566,6 @@ static int rbatch_step(spl_solver *s, spl_level_info *info, cudaStream_t st) {
     RBatch &R = *s->rb;
     const int B = R.B;
     const int64_t n = s->n_front;
-    const std::vector<int64_t> &seg = R.seg_at.back();
     long long *goal = R.gctr.as<long long>();
     unsigned long long *cands = R.gctr.as<unsigned long long>() + B, *n_new_g = cands + B;
     std::vector<int64_t> g_host(3 * (size_t)B, 0);  // goal | cands | n_new per game
@@ -2495,46 +2637,12 @@ static int rbatch_step(spl_solver *s, spl_level_info *info, cudaStream_t st) {
         CK(c, cudaEventRecord(c->ev[2], st));
     }
     CK(c, cudaEventRecord(c->ev[3], st));
-    // ---- per-game bookkeeping: who ends at this level, and the offsets of the winners' and of the next queue's runs
-    // (the reference leaves its loop after the iteration with turn == 1000, src/solver.py:846-852)
-    const bool turn_limit = s->level >= 1000;
-    std::vector<int64_t> kseg(B + 1, 0), useg(B + 1, 0);
-    bool all_ended = true;
-    for (int g = 0; g < B; ++g) {
-        const int64_t ng = seg[g + 1] - seg[g];
-        int64_t kept = 0;
-        useg[g + 1] = useg[g];
-        if (ng > 0) {
-            spl_rgame_info &I = R.info[g];
-            const int64_t uniq = (int64_t)g_host[2 * B + g];
-            I.level = s->level;
-            I.frontier = ng;
-            I.goal_rank = -1;
-            if (g_host[g] != 0x7fffffffffffffffll) {  // goal dequeued: nothing of this level is expanded
-                I.generated = I.unique = I.kept = 0;
-                I.goal_rank = R.final_rank[g] = g_host[g];
-                I.ended = 1;
-            } else {
-                I.generated = g_host[B + g];
-                I.unique = uniq;
-                I.visited += uniq;
-                I.kept = std::min(uniq, R.beam[g]);
-                if (I.kept == 0 || turn_limit) {  // queue exhausted / turn limit: the last state dequeued ends the game
-                    I.ended = 1;
-                    R.final_rank[g] = ng - 1;
-                } else {
-                    kept = I.kept;
-                    all_ended = false;
-                }
-            }
-            useg[g + 1] += uniq;
-        }
-        kseg[g + 1] = kseg[g] + kept;
-    }
-    if (useg[B] != n_uniq) return fail(c, SPL_E_CUDA, "internal: %lld winners, %lld counted per game", (long long)n_uniq, (long long)useg[B]);
-    const int64_t n_kept = kseg[B];
+    // ---- per-game bookkeeping
+    std::vector<int64_t> kseg, useg;
+    bool all_ended;
+    CKS(c, batch_bookkeeping(s, g_host, n_uniq, s->level >= 1000, kseg, useg, &all_ended));
     // ---- score + segmented cut into the next queue
-    if (n_kept) {
+    if (kseg[B]) {
         for (int b = 0; b < 2; ++b) {
             CK(c, c->y[b].ensure((size_t)n_uniq * 8 + 8, 0, st));
             CK(c, c->idx[b].ensure((size_t)n_uniq * 4 + 4, 0, st));
@@ -2548,52 +2656,136 @@ static int rbatch_step(spl_solver *s, spl_level_info *info, cudaStream_t st) {
         CK(c, cudaEventRecord(c->ev[4], st));
         // every score key lies between sk_min and sk_max, so the y words differ only in the low bits where those two do
         int cur = 0;
-        CKS(c, sort_pairs(c, n_uniq, bitlen(c->h_ctr->sk_min ^ c->h_ctr->sk_max), &cur, st));
-        if (B > 1) {
-            rb_game_words_kernel<<<nblk(n_uniq), TILE, 0, st>>>(c->idx[cur].as<uint32_t>(), R.uniq_game.as<uint32_t>(), n_uniq,
-                                                                 c->y[cur].as<uint64_t>());
-            ++c->launches;
-            CKS(c, sort_pairs(c, n_uniq, bitlen((uint64_t)B - 1), &cur, st));
-        }
-        std::vector<int64_t> segs(kseg);  // the next queue's offsets, then the winners'
-        segs.insert(segs.end(), useg.begin(), useg.end());
-        CK(c, cudaMemcpyAsync(R.seg.p, segs.data(), segs.size() * 8, cudaMemcpyHostToDevice, st));
-        c->h2d_bytes += segs.size() * 8;
-        CK(c, s->front.ensure((size_t)n_kept * 96, 0, st));
-        rb_cut_kernel<<<nblk(n_uniq), TILE, 0, st>>>(s->uniq.as<RRec>(), R.uniq_game.as<uint32_t>(), c->idx[cur].as<uint32_t>(), n_uniq,
-                                                      R.seg.as<int64_t>() + (B + 1), R.seg.as<int64_t>(), s->front.as<RRec>());
-        ++c->launches;
-        CK(c, cudaGetLastError());
-        CK(c, cudaStreamSynchronize(st));  // segs is a local
+        CKS(c, segmented_cut<RRec>(s, n_uniq, bitlen(c->h_ctr->sk_min ^ c->h_ctr->sk_max), kseg, useg, &cur, st));
     } else {
         CK(c, cudaEventRecord(c->ev[4], st));
     }
-    CK(c, cudaEventRecord(c->ev[5], st));
-    CK(c, cudaEventSynchronize(c->ev[5]));
-    float t;
-    cudaEventElapsedTime(&t, c->ev[0], c->ev[1]); info->ms_count = t;
-    cudaEventElapsedTime(&t, c->ev[1], c->ev[2]); info->ms_expand = t;
-    cudaEventElapsedTime(&t, c->ev[2], c->ev[3]); info->ms_resolve = t;
-    cudaEventElapsedTime(&t, c->ev[3], c->ev[4]); info->ms_select = t;
-    cudaEventElapsedTime(&t, c->ev[4], c->ev[5]); info->ms_sort = t;
-    info->expanded = n;
-    info->generated = total;
-    info->unique = n_uniq;
-    for (int g = 0; g < B; ++g)
-        if (seg[g + 1] > seg[g]) info->kept += R.info[g].kept;
-    info->visited = (int64_t)c->occupied;
-    info->table_slots = c->rbtab.slots();
-    if (all_ended) {
-        s->ended = true;
-        info->ended = 1;
-        return SPL_OK;
+    return batch_finish(s, info, n, total, n_uniq, kseg, all_ended, c->rbtab, true, st);
+}
+
+// ------------------------------------------------------------------ batched speedrun level (spl_sbatch_*, spl_sbatch.cuh)
+// rbatch_step's sequence over 32-byte rows: goal test + count, expand, probe of (game, key), winners in arrival order,
+// score, then -- for the 'det' policy -- stable passes by the inverted key (larger keys first among equal scores), and
+// the segmented cut.  A game of exhaustive BFS scores 0 and keeps all its unique states (its beam is unbounded), so the
+// stable passes leave them in arrival order, which is its queue order in State.solve.
+static int sbatch_step(spl_solver *s, spl_level_info *info, cudaStream_t st) {
+    spl_ctx *c = s->c;
+    RBatch &R = *s->rb;
+    const int B = R.B;
+    const int64_t n = s->n_front;
+    long long *goal = R.gctr.as<long long>();
+    unsigned long long *cands = R.gctr.as<unsigned long long>() + B, *n_new_g = cands + B;
+    std::vector<int64_t> g_host(3 * (size_t)B, 0);  // goal | cands | n_new per game
+    for (int g = 0; g < B; ++g) g_host[g] = 0x7fffffffffffffffll;
+    // ---- goal test + successor count
+    CK(c, cudaEventRecord(c->ev[0], st));
+    CK(c, cudaMemcpyAsync(R.gctr.p, g_host.data(), g_host.size() * 8, cudaMemcpyHostToDevice, st));
+    CKS(c, zero_ctr(c, st));
+    const unsigned nt = nblk(n);
+    CK(c, c->off.ensure((size_t)n * 4 + 4, 0, st));
+    CKS(c, prep_status(c, 0, nt, st));
+    const SGame *gm = R.cfg.as<SGame>();
+    const int64_t *dseg = R.seg.as<int64_t>();
+    sb_goal_kernel<<<nt, TILE, 0, st>>>(s->front.as<Rec>(), n, dseg, B, gm, goal);
+    sb_count_scan_kernel<<<nt, TILE, 0, st>>>(s->front.as<Rec>(), n, dseg, B, goal, c->d_tabs, c->d_takes_idx, c->off.as<uint32_t>(),
+                                               c->status[0].as<uint64_t>(), c->d_ctr, 0, cands);
+    c->launches += 2;
+    CK(c, cudaGetLastError());
+    CK(c, cudaMemcpyAsync(g_host.data(), R.gctr.p, (size_t)B * 16, cudaMemcpyDeviceToHost, st));
+    CKS(c, read_ctr(c, st));
+    c->d2h_bytes += B * 16;
+    CK(c, cudaEventRecord(c->ev[1], st));
+    const int64_t total = (int64_t)c->h_ctr->total_cands;
+    if (total >= 0xFFFFFFFFll) return fail(c, SPL_E_INVALID, "batch level produced %lld candidates (>= 2^32)", (long long)total);
+    // ---- expand + (game, key) dedup + winners in arrival order
+    int64_t n_uniq = 0;
+    if (total) {
+        CK(c, c->tmp_rec.ensure((size_t)total * 32, 0, st));
+        CK(c, R.cand_game.ensure((size_t)total * 4, 0, st));
+        sb_expand_kernel<<<nt, TILE, 0, st>>>(s->front.as<Rec>(), n, dseg, B, goal, c->d_tabs, c->d_takes_idx, c->d_takes_edges,
+                                               c->off.as<uint32_t>(), c->tmp_rec.as<Rec>(), R.cand_game.as<uint32_t>());
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CK(c, cudaEventRecord(c->ev[2], st));
+        CKS(c, zero_ctr(c, st));
+        CKS(c, c->sbtab.grow(c, (uint64_t)total, st));
+        uint64_t tag;
+        CKS(c, next_epoch(c, tag));
+        CK(c, c->cand_slot.ensure((size_t)total * 4, 0, st));
+        CKS(c, zero_ctr(c, st));
+        sb_probe_kernel<<<nblk(total), TILE, 0, st>>>(c->tmp_rec.as<Rec>(), R.cand_game.as<uint32_t>(), total, c->sbtab.as<SBucket>(),
+                                                       c->sbtab.units, tag, c->cand_slot.as<uint32_t>(), c->d_ctr, n_new_g);
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CK(c, cudaMemcpyAsync(g_host.data() + 2 * B, n_new_g, (size_t)B * 8, cudaMemcpyDeviceToHost, st));
+        CKS(c, read_ctr(c, st));
+        c->d2h_bytes += B * 8;
+        c->sbtab.occ += c->h_ctr->n_new;  // before the error check: a reset clears a partial insert too
+        if (c->h_ctr->error) return fail(c, SPL_E_TABLE_FULL, "batch visited table full during level %d", s->level);
+        n_uniq = (int64_t)c->h_ctr->n_new;
+        c->occupied += n_uniq;
+        if (n_uniq) {
+            CK(c, c->ridx64.ensure((size_t)n_uniq * 8, 0, st));
+            const unsigned wt = nblk(total, TILE * 8);
+            CKS(c, prep_status(c, 0, wt, st));
+            CKS(c, reset_ticket(c, 0, st));
+            sb_winners_kernel<<<wt, TILE, 0, st>>>(c->cand_slot.as<uint32_t>(), c->sbtab.as<SBucket>(), total, c->ridx64.as<int64_t>(),
+                                                    c->status[0].as<uint64_t>(), c->d_ctr, 0);
+            CK(c, s->uniq.ensure((size_t)n_uniq * 32, 0, st));
+            CK(c, R.uniq_game.ensure((size_t)n_uniq * 4, 0, st));
+            sb_gather_kernel<<<nblk(n_uniq), TILE, 0, st>>>(c->tmp_rec.as<Rec>(), R.cand_game.as<uint32_t>(), c->ridx64.as<int64_t>(), n_uniq,
+                                                             s->uniq.as<Rec>(), R.uniq_game.as<uint32_t>());
+            c->launches += 2;
+            CK(c, cudaGetLastError());
+        }
+    } else {
+        CK(c, cudaEventRecord(c->ev[2], st));
     }
-    s->n_front = n_kept;
-    s->level += 1;
-    R.seg_at.push_back(kseg);
-    CKS(c, save_links(s, n_kept, true, false, st));
-    CK(c, cudaStreamSynchronize(st));
-    return SPL_OK;
+    CK(c, cudaEventRecord(c->ev[3], st));
+    // ---- per-game bookkeeping
+    std::vector<int64_t> kseg, useg;
+    bool all_ended;
+    CKS(c, batch_bookkeeping(s, g_host, n_uniq, false, kseg, useg, &all_ended));
+    // ---- score (+ key passes) + segmented cut into the next queue
+    if (kseg[B]) {
+        const bool by_key = s->tie == SPL_TIE_KEY;
+        for (int b = 0; b < 2; ++b) {
+            CK(c, c->y[b].ensure((size_t)n_uniq * 8 + 8, 0, st));
+            CK(c, c->idx[b].ensure((size_t)n_uniq * 4 + 4, 0, st));
+        }
+        if (by_key) CK(c, c->sk.ensure((size_t)n_uniq * 8, 0, st));
+        CKS(c, zero_ctr(c, st));
+        uint64_t *score_words = by_key ? c->sk.as<uint64_t>() : c->y[0].as<uint64_t>();  // by key: the key passes come first
+        sb_score_kernel<<<nblk(n_uniq), TILE, 0, st>>>(s->uniq.as<Rec>(), R.uniq_game.as<uint32_t>(), n_uniq, gm, s->noise, c->luts,
+                                                        score_words, c->idx[0].as<uint32_t>(), c->d_ctr);
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CKS(c, read_ctr(c, st));
+        CK(c, cudaEventRecord(c->ev[4], st));
+        // the beam games' score keys lie between sk_min and sk_max (none: a level of BFS games only, every word 0)
+        const uint64_t kmin = c->h_ctr->sk_min, kmax = c->h_ctr->sk_max;
+        int cur = 0;
+        if (by_key && kmin <= kmax) {  // least significant first: ~key.lo, ~key.hi over the bits that vary, then the score words
+            const uint64_t *rows = s->uniq.as<uint64_t>();
+            const int key_bits[2] = {bitlen(c->h_ctr->key_or[0] ^ c->h_ctr->key_and[0]),
+                                     bitlen(c->h_ctr->key_or[1] ^ c->h_ctr->key_and[1])};
+            for (int w = 0; w < 2; ++w) {
+                if (!key_bits[w]) continue;
+                sb_words_kernel<<<nblk(n_uniq), TILE, 0, st>>>(c->idx[cur].as<uint32_t>(), n_uniq, rows + w, 4, ~0ull,
+                                                                R.uniq_game.as<uint32_t>(), gm, c->y[cur].as<uint64_t>());
+                ++c->launches;
+                CKS(c, sort_pairs(c, n_uniq, key_bits[w], &cur, st));
+            }
+            sb_words_kernel<<<nblk(n_uniq), TILE, 0, st>>>(c->idx[cur].as<uint32_t>(), n_uniq, score_words, 1, 0,
+                                                            R.uniq_game.as<uint32_t>(), gm, c->y[cur].as<uint64_t>());
+            ++c->launches;
+            CK(c, cudaGetLastError());
+        }
+        CKS(c, segmented_cut<Rec>(s, n_uniq, kmin <= kmax ? bitlen(kmin ^ kmax) : 0, kseg, useg, &cur, st));
+    } else {
+        CK(c, cudaEventRecord(c->ev[4], st));
+    }
+    return batch_finish(s, info, n, total, n_uniq, kseg, all_ended, c->sbtab, false, st);
 }
 
 // ------------------------------------------------------------------ second half of a level
@@ -2673,22 +2865,29 @@ static int level_cut(spl_solver *s, spl_level_info *info, int64_t n, const Level
     return SPL_OK;
 }
 
-// The speedrun solver's create from a level-0 queue rows[0..n) (links ~0), checked on the host before any kernel sees
-// a row: a gem hand without a rank indexes past a node's bitmap, a key bit at or above 105 is outside the card set,
-// and a second row with the same key would be a state registered twice.
+// The row checks of every speedrun create, on the host before any kernel sees a row: a gem hand without a rank indexes
+// past a node's bitmap, and a key bit at or above 105 is outside the card set.  `what` names a row in the message
+// ("row" of a queue, "game" of a batch).
+static int check_rows(spl_ctx *c, const char *fn, const char *what, const Rec *rows, int64_t n) {
+    const HostTables &T = host_tables();
+    for (int64_t i = 0; i < n; ++i) {
+        if (T.gemrank[rows[i].lo & GEM_MASK] == 0xFFFF)
+            return fail(c, SPL_E_INVALID, "%s: %s %lld has an illegal gem hand (0x%llx)", fn, what, (long long)i,
+                        (unsigned long long)(rows[i].lo & GEM_MASK));
+        if (rows[i].hi & ~HI_KEY_MASK)
+            return fail(c, SPL_E_INVALID, "%s: %s %lld has a key bit at or above 105", fn, what, (long long)i);
+    }
+    return SPL_OK;
+}
+
+// The speedrun solver's create from a level-0 queue rows[0..n) (links ~0), checked on the host (check_rows; a second
+// row with the same key would be a state registered twice).
 static int create_solver(spl_ctx *c, const char *fn, const Rec *rows, int64_t n, int32_t goal, int32_t use_h,
                          int32_t heuristic, int64_t beam, int32_t tie, int32_t noise, int32_t keep_links, spl_solver **out) {
     if (use_h && beam < 1) return fail(c, SPL_E_INVALID, "%s: beam_width must be >= 1", fn);
     if (use_h && tie != SPL_TIE_STABLE && tie != SPL_TIE_KEY) return fail(c, SPL_E_INVALID, "%s: unknown tie policy %d", fn, tie);
     if (noise < 0 || noise > SPL_NOISE_EXTERNAL) return fail(c, SPL_E_INVALID, "%s: unknown noise policy %d", fn, noise);
-    const HostTables &T = host_tables();
-    for (int64_t i = 0; i < n; ++i) {
-        if (T.gemrank[rows[i].lo & GEM_MASK] == 0xFFFF)
-            return fail(c, SPL_E_INVALID, "%s: row %lld has an illegal gem hand (0x%llx)", fn, (long long)i,
-                        (unsigned long long)(rows[i].lo & GEM_MASK));
-        if (rows[i].hi & ~HI_KEY_MASK)
-            return fail(c, SPL_E_INVALID, "%s: row %lld has a key bit at or above 105", fn, (long long)i);
-    }
+    CKS(c, check_rows(c, fn, "row", rows, n));
     if (n > 1) {
         std::vector<int64_t> ord(n);
         for (int64_t i = 0; i < n; ++i) ord[i] = i;
@@ -2748,6 +2947,7 @@ int32_t spl_solver_step(spl_solver *s, spl_level_info *info, void *stream) {
     info->frontier = s->n_front;
     info->goal_rank = -1;
     if (s->kind == REALISTIC_BATCH) return rbatch_step(s, info, st);
+    if (s->kind == SPEEDRUN_BATCH) return sbatch_step(s, info, st);
     const int64_t n = s->n_front;
     const bool realistic = s->kind == REALISTIC;
     if (realistic && c->rcfg_dirty) {  // spl_rscore / spl_rexpand / spl_rmaxpts ran with their own GameConfig in between
@@ -2871,24 +3071,21 @@ int32_t spl_rsolver_frontier(spl_solver *s, const void **recs, int64_t *n) {
     return SPL_OK;
 }
 
-// ---- batched realistic search
+// ---- batched searches (spl_rbatch_*, spl_sbatch_*)
 constexpr int32_t MAX_BATCH_GAMES = 1 << 16;
 
-int32_t spl_rbatch_create(spl_ctx *c, const spl_rconfig *cfgs, const void *root_recs_host, const int64_t *beams, int32_t n_games,
-                          int32_t keep_links, spl_solver **out) {
-    if (!c || !cfgs || !root_recs_host || !beams || !out) return fail(c, SPL_E_INVALID, "spl_rbatch_create: null argument");
-    if (n_games < 1 || n_games > MAX_BATCH_GAMES) return fail(c, SPL_E_INVALID, "spl_rbatch_create: n_games must be 1..%d", MAX_BATCH_GAMES);
-    std::vector<RConfigDev> dev((size_t)n_games);
-    for (int g = 0; g < n_games; ++g) {
-        if (beams[g] < 1) return fail(c, SPL_E_INVALID, "spl_rbatch_create: game %d: beam_width must be >= 1", g);
-        if (cfgs[g].noise != SPL_NOISE_CONST && cfgs[g].noise != SPL_NOISE_HASH)
-            return fail(c, SPL_E_INVALID, "spl_rbatch_create: game %d: noise must be const or hash (mt draws depend on the other games)", g);
-        CKS(c, make_rconfig(c, cfgs + g, dev[g]));
-    }
-    NO_LIVE_SOLVER(c, "spl_rbatch_create");
+}  // extern "C"
+
+// What both batch creates share once their arguments are checked: a solver of `kind` with the per-game bookkeeping,
+// and on the device the games' configs (cfg_bytes each: RConfigDev or SGame), their roots (row_bytes each), the level-0
+// offsets 0 .. B, the per-game counters and the roots' games 0 .. B - 1; then open_solver.
+static int open_batch(spl_ctx *c, LevelKind kind, const void *cfgs, size_t cfg_bytes, const void *roots, size_t row_bytes,
+                      const int64_t *beams, int32_t n_games, int32_t keep_links, const char *fn, spl_solver **out, int tie = 0,
+                      int noise = 0) {
+    if (c->active) return fail(c, SPL_E_STATE, "%s: a solver is open on this context (destroy it first)", fn);
     CK(c, enter_device(c));
     spl_solver *s = new spl_solver(c);
-    s->kind = REALISTIC_BATCH; s->use_h = 1; s->keep_links = keep_links; s->n_front = n_games;
+    s->kind = kind; s->use_h = 1; s->keep_links = keep_links; s->n_front = n_games; s->tie = tie; s->noise = noise;
     s->rb = std::make_unique<RBatch>();
     RBatch &R = *s->rb;
     R.B = n_games;
@@ -2903,13 +3100,13 @@ int32_t spl_rbatch_create(spl_ctx *c, const spl_rconfig *cfgs, const void *root_
     R.seg_at.push_back(seg);
     const size_t B = (size_t)n_games;
     const cudaError_t e = [&]() -> cudaError_t {
-        cudaError_t r = R.cfg.ensure(B * sizeof(RConfigDev), 0, 0);
-        if (r == cudaSuccess) r = R.roots.ensure(B * 96, 0, 0);
+        cudaError_t r = R.cfg.ensure(B * cfg_bytes, 0, 0);
+        if (r == cudaSuccess) r = R.roots.ensure(B * row_bytes, 0, 0);
         if (r == cudaSuccess) r = R.seg.ensure((2 * B + 2) * 8, 0, 0);
         if (r == cudaSuccess) r = R.gctr.ensure(3 * B * 8, 0, 0);
         if (r == cudaSuccess) r = R.cand_game.ensure(B * 4, 0, 0);
-        if (r == cudaSuccess) r = cudaMemcpyAsync(R.cfg.p, dev.data(), B * sizeof(RConfigDev), cudaMemcpyHostToDevice, 0);
-        if (r == cudaSuccess) r = cudaMemcpyAsync(R.roots.p, root_recs_host, B * 96, cudaMemcpyHostToDevice, 0);
+        if (r == cudaSuccess) r = cudaMemcpyAsync(R.cfg.p, cfgs, B * cfg_bytes, cudaMemcpyHostToDevice, 0);
+        if (r == cudaSuccess) r = cudaMemcpyAsync(R.roots.p, roots, B * row_bytes, cudaMemcpyHostToDevice, 0);
         if (r == cudaSuccess) r = cudaMemcpyAsync(R.seg.p, seg.data(), (B + 1) * 8, cudaMemcpyHostToDevice, 0);
         if (r == cudaSuccess) r = cudaMemsetAsync(R.gctr.p, 0, 3 * B * 8, 0);
         if (r == cudaSuccess) r = cudaMemcpyAsync(R.cand_game.p, iota.data(), B * 4, cudaMemcpyHostToDevice, 0);
@@ -2919,37 +3116,40 @@ int32_t spl_rbatch_create(spl_ctx *c, const spl_rconfig *cfgs, const void *root_
     if (e != cudaSuccess) {
         cudaGetLastError();
         delete s;
-        return fail(c, e == cudaErrorMemoryAllocation ? SPL_E_NOMEM : SPL_E_CUDA, "spl_rbatch_create: %s", cudaGetErrorString(e));
+        return fail(c, e == cudaErrorMemoryAllocation ? SPL_E_NOMEM : SPL_E_CUDA, "%s: %s", fn, cudaGetErrorString(e));
     }
-    c->h2d_bytes += B * (sizeof(RConfigDev) + 96 + 8 + 4) + 8;
-    return open_solver(s, REALISTIC_BATCH, root_recs_host, n_games, 96, false, "rbatch create sync failed", out);
+    c->h2d_bytes += B * (cfg_bytes + row_bytes + 8 + 4) + 8;
+    return open_solver(s, kind, roots, n_games, row_bytes, false, "batch create sync failed", out);
 }
 
-int32_t spl_rbatch_games(spl_solver *s, spl_rgame_info *out_host, int32_t n_games) {
-    if (!s || !out_host || s->kind != REALISTIC_BATCH) return SPL_E_INVALID;
-    if (n_games != s->rb->B) return fail(s->c, SPL_E_INVALID, "spl_rbatch_games: the batch has %d games", s->rb->B);
+static int batch_games(spl_solver *s, LevelKind kind, const char *fn, spl_rgame_info *out_host, int32_t n_games) {
+    if (!s || !out_host || s->kind != kind) return SPL_E_INVALID;
+    if (n_games != s->rb->B) return fail(s->c, SPL_E_INVALID, "%s: the batch has %d games", fn, s->rb->B);
     memcpy(out_host, s->rb->info.data(), sizeof(spl_rgame_info) * (size_t)n_games);
     return SPL_OK;
 }
 
-int32_t spl_rbatch_frontier(spl_solver *s, int32_t game, const void **recs_dev, int64_t *n_host) {
-    if (!s || !recs_dev || !n_host || s->kind != REALISTIC_BATCH) return SPL_E_INVALID;
-    if (game < 0 || game >= s->rb->B) return fail(s->c, SPL_E_INVALID, "spl_rbatch_frontier: no game %d", game);
+static int batch_frontier(spl_solver *s, LevelKind kind, size_t row_bytes, const char *fn, int32_t game, const void **rows_dev,
+                          int64_t *n_host) {
+    if (!s || !rows_dev || !n_host || s->kind != kind) return SPL_E_INVALID;
+    if (game < 0 || game >= s->rb->B) return fail(s->c, SPL_E_INVALID, "%s: no game %d", fn, game);
     const std::vector<int64_t> &seg = s->rb->seg_at.back();
     const bool live = !s->ended;  // the last level's queue was expanded and replaced by nothing
-    *recs_dev = static_cast<const char *>(s->front.p) + seg[game] * 96;
+    *rows_dev = static_cast<const char *>(s->front.p) + seg[game] * row_bytes;
     *n_host = live ? seg[game + 1] - seg[game] : 0;
     return SPL_OK;
 }
 
 // Walk every game's line back through the link columns, one batched read per level (a spilled column is read where it
-// lies, on the host), then rebuild the records forward from the roots on the device.
-int32_t spl_rbatch_lines(spl_solver *s, void *recs_host, int64_t cap, int32_t *plies_host) {
-    if (!s || !recs_host || !plies_host || s->kind != REALISTIC_BATCH) return SPL_E_INVALID;
+// lies, on the host), then rebuild the rows forward from the roots on the device, one thread per game.  Row: RRec
+// (rb_line_kernel) or Rec (sb_line_kernel).
+template <class Row>
+static int batch_lines(spl_solver *s, LevelKind kind, const char *fn, void *rows_host, int64_t cap, int32_t *plies_host) {
+    if (!s || !rows_host || !plies_host || s->kind != kind) return SPL_E_INVALID;
     spl_ctx *c = s->c;
     RBatch &R = *s->rb;
-    if (!s->ended) return fail(c, SPL_E_STATE, "spl_rbatch_lines: the batch has not ended");
-    if (!s->keep_links) return fail(c, SPL_E_STATE, "spl_rbatch_lines: solver was created with keep_links = 0");
+    if (!s->ended) return fail(c, SPL_E_STATE, "%s: the batch has not ended", fn);
+    if (!s->keep_links) return fail(c, SPL_E_STATE, "%s: solver was created with keep_links = 0", fn);
     CK(c, enter_device(c));
     const int B = R.B;
     int max_plies = 0;
@@ -2957,7 +3157,7 @@ int32_t spl_rbatch_lines(spl_solver *s, void *recs_host, int64_t cap, int32_t *p
         plies_host[g] = (int32_t)R.info[g].level;
         max_plies = std::max(max_plies, plies_host[g]);
     }
-    if (max_plies + 1 > cap) return fail(c, SPL_E_CAPACITY, "spl_rbatch_lines: a line needs %d records", max_plies + 1);
+    if (max_plies + 1 > cap) return fail(c, SPL_E_CAPACITY, "%s: a line needs %d records", fn, max_plies + 1);
     const cudaStream_t st = 0;
     std::vector<int64_t> rank(R.final_rank), at;
     std::vector<int> who;
@@ -2992,22 +3192,94 @@ int32_t spl_rbatch_lines(spl_solver *s, void *recs_host, int64_t cap, int32_t *p
     }
     const size_t line_recs = (size_t)max_plies + 1;
     CK(c, R.scratch.ensure(ords.size() + (size_t)B * 4 + 16, 0, st));
-    CK(c, R.lines.ensure((size_t)B * line_recs * 96, 0, st));
+    CK(c, R.lines.ensure((size_t)B * line_recs * sizeof(Row), 0, st));
     int32_t *d_plies = R.scratch.as<int32_t>();
     uint8_t *d_ords = reinterpret_cast<uint8_t *>(d_plies + B);
     CK(c, cudaMemcpyAsync(d_plies, plies_host, (size_t)B * 4, cudaMemcpyHostToDevice, st));
     CK(c, cudaMemcpyAsync(d_ords, ords.data(), ords.size(), cudaMemcpyHostToDevice, st));
     CKS(c, zero_ctr(c, st));
-    rb_line_kernel<<<nblk(B), TILE, 0, st>>>(R.roots.as<RRec>(), R.cfg.as<RConfigDev>(), B, d_plies, d_ords, max_plies,
-                                              R.lines.as<RRec>(), c->d_ctr);
+    if constexpr (std::is_same_v<Row, RRec>)
+        rb_line_kernel<<<nblk(B), TILE, 0, st>>>(R.roots.as<RRec>(), R.cfg.as<RConfigDev>(), B, d_plies, d_ords, max_plies,
+                                                  R.lines.as<RRec>(), c->d_ctr);
+    else
+        sb_line_kernel<<<nblk(B), TILE, 0, st>>>(R.roots.as<Rec>(), B, d_plies, d_ords, max_plies, c->d_tabs, c->d_takes_idx,
+                                                  c->d_takes_edges, R.lines.as<Rec>(), c->d_ctr);
     ++c->launches;
     CK(c, cudaGetLastError());
-    CK(c, cudaMemcpy2DAsync(recs_host, (size_t)cap * 96, R.lines.p, line_recs * 96, line_recs * 96, (size_t)B, cudaMemcpyDeviceToHost, st));
+    CK(c, cudaMemcpy2DAsync(rows_host, (size_t)cap * sizeof(Row), R.lines.p, line_recs * sizeof(Row), line_recs * sizeof(Row), (size_t)B,
+                            cudaMemcpyDeviceToHost, st));
     CKS(c, read_ctr(c, st));
     c->h2d_bytes += (int64_t)(B * 4 + ords.size());
-    c->d2h_bytes += (int64_t)(B * line_recs * 96);
+    c->d2h_bytes += (int64_t)(B * line_recs * sizeof(Row));
     if (c->h_ctr->error) return fail(c, SPL_E_CUDA, "internal: a link ordinal names no successor");
     return SPL_OK;
+}
+
+extern "C" {
+
+int32_t spl_rbatch_create(spl_ctx *c, const spl_rconfig *cfgs, const void *root_recs_host, const int64_t *beams, int32_t n_games,
+                          int32_t keep_links, spl_solver **out) {
+    if (!c || !cfgs || !root_recs_host || !beams || !out) return fail(c, SPL_E_INVALID, "spl_rbatch_create: null argument");
+    if (n_games < 1 || n_games > MAX_BATCH_GAMES) return fail(c, SPL_E_INVALID, "spl_rbatch_create: n_games must be 1..%d", MAX_BATCH_GAMES);
+    std::vector<RConfigDev> dev((size_t)n_games);
+    for (int g = 0; g < n_games; ++g) {
+        if (beams[g] < 1) return fail(c, SPL_E_INVALID, "spl_rbatch_create: game %d: beam_width must be >= 1", g);
+        if (cfgs[g].noise != SPL_NOISE_CONST && cfgs[g].noise != SPL_NOISE_HASH)
+            return fail(c, SPL_E_INVALID, "spl_rbatch_create: game %d: noise must be const or hash (mt draws depend on the other games)", g);
+        CKS(c, make_rconfig(c, cfgs + g, dev[g]));
+    }
+    return open_batch(c, REALISTIC_BATCH, dev.data(), sizeof(RConfigDev), root_recs_host, 96, beams, n_games, keep_links,
+                      "spl_rbatch_create", out);
+}
+
+int32_t spl_rbatch_games(spl_solver *s, spl_rgame_info *out_host, int32_t n_games) {
+    return batch_games(s, REALISTIC_BATCH, "spl_rbatch_games", out_host, n_games);
+}
+
+int32_t spl_rbatch_frontier(spl_solver *s, int32_t game, const void **recs_dev, int64_t *n_host) {
+    return batch_frontier(s, REALISTIC_BATCH, 96, "spl_rbatch_frontier", game, recs_dev, n_host);
+}
+
+int32_t spl_rbatch_lines(spl_solver *s, void *recs_host, int64_t cap, int32_t *plies_host) {
+    return batch_lines<RRec>(s, REALISTIC_BATCH, "spl_rbatch_lines", recs_host, cap, plies_host);
+}
+
+// ---- batched speedrun search
+int32_t spl_sbatch_create(spl_ctx *c, const void *root_rows_host, const int32_t *goals, const int32_t *use_heuristic,
+                          const int32_t *heuristics, const int64_t *beams, int32_t n_games, int32_t tie_policy, int32_t noise,
+                          int32_t keep_links, spl_solver **out) {
+    if (!c || !root_rows_host || !goals || !use_heuristic || !heuristics || !beams || !out)
+        return fail(c, SPL_E_INVALID, "spl_sbatch_create: null argument");
+    if (n_games < 1 || n_games > MAX_BATCH_GAMES) return fail(c, SPL_E_INVALID, "spl_sbatch_create: n_games must be 1..%d", MAX_BATCH_GAMES);
+    if (tie_policy != SPL_TIE_STABLE && tie_policy != SPL_TIE_KEY)
+        return fail(c, SPL_E_INVALID, "spl_sbatch_create: tie policy must be stable or key, not %d", tie_policy);
+    if (noise != SPL_NOISE_CONST && noise != SPL_NOISE_HASH)
+        return fail(c, SPL_E_INVALID, "spl_sbatch_create: noise must be const or hash, not %d (external draws depend on the other games)", noise);
+    std::vector<Rec> rows((size_t)n_games);
+    memcpy(rows.data(), root_rows_host, rows.size() * sizeof(Rec));
+    std::vector<SGame> games((size_t)n_games);
+    std::vector<int64_t> beam((size_t)n_games);
+    CKS(c, check_rows(c, "spl_sbatch_create", "game", rows.data(), n_games));
+    for (int g = 0; g < n_games; ++g) {
+        if (beams[g] < 1) return fail(c, SPL_E_INVALID, "spl_sbatch_create: game %d: beam_width must be >= 1", g);
+        rows[g].link = ~0ull;
+        games[g] = SGame{goals[g], use_heuristic[g] ? 1 : 0, heuristics[g], 0};
+        beam[g] = use_heuristic[g] ? beams[g] : INT64_MAX;  // BFS keeps every unique state
+    }
+    return open_batch(c, SPEEDRUN_BATCH, games.data(), sizeof(SGame), rows.data(), 32, beam.data(), n_games, keep_links,
+                      "spl_sbatch_create", out, tie_policy, noise);
+}
+
+int32_t spl_sbatch_games(spl_solver *s, spl_rgame_info *out_host, int32_t n_games) {
+    return batch_games(s, SPEEDRUN_BATCH, "spl_sbatch_games", out_host, n_games);
+}
+
+int32_t spl_sbatch_frontier(spl_solver *s, int32_t game, const void **rows_dev, int64_t *n_host) {
+    return batch_frontier(s, SPEEDRUN_BATCH, 32, "spl_sbatch_frontier", game, rows_dev, n_host);
+}
+
+int32_t spl_sbatch_lines(spl_solver *s, void *rows_host, int64_t cap, int32_t *plies_host) {
+    return batch_lines<Rec>(s, SPEEDRUN_BATCH, "spl_sbatch_lines", rows_host, cap, plies_host);
 }
 
 // ---- realistic mode on the key-sharded driver: rows are 96-byte RRec records (spl_dedup_flags, spl_compact_winners and
@@ -3165,6 +3437,7 @@ int32_t spl_solver_path(spl_solver *s, int64_t *ranks, int32_t *ordinals, int32_
     if (!s || !ranks || !ordinals || !n_moves) return SPL_E_INVALID;
     spl_ctx *c = s->c;
     if (s->kind == REALISTIC_BATCH) return fail(c, SPL_E_INVALID, "spl_solver_path: a batched solver's lines come from spl_rbatch_lines");
+    if (s->kind == SPEEDRUN_BATCH) return fail(c, SPL_E_INVALID, "spl_solver_path: a batched solver's lines come from spl_sbatch_lines");
     if (!s->ended) return fail(c, SPL_E_STATE, "spl_solver_path: the search has not ended");
     if (!s->keep_links) return fail(c, SPL_E_STATE, "spl_solver_path: solver was created with keep_links = 0");
     const int L = s->level;  // level index of the final state

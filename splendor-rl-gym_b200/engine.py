@@ -286,6 +286,12 @@ class Engine:
         """spl_rbatch_create: len(rcfgs) realistic-mode games searched in lockstep (root record and beam width per game)."""
         return RBatchSolver(self, rcfgs, roots_np, beams, keep_links)
 
+    def sbatch_solver(self, roots_np: np.ndarray, goals, use_heuristic, heuristics, beams, tie: str = 'stable',
+                      noise: str = 'const', keep_links: bool = True) -> 'SBatchSolver':
+        """spl_sbatch_create: len(roots_np) speedrun games searched in lockstep.  roots_np: 32-byte rows {lo, hi, aux,
+        link} (an [n, 4] uint64 array); goals, use_heuristic, heuristics (names or ids) and beams: one per game."""
+        return SBatchSolver(self, roots_np, goals, use_heuristic, heuristics, beams, tie, noise, keep_links)
+
     # -------------------------------------------------------------- fused solver
     def solver(self, root_key: int, root_aux: int, goal_pts: int, use_heuristic: bool, heuristic: str, beam_width: int,
                tie: str = 'stable', noise: str = 'const', keep_links: bool = True, identity: str = 'key',
@@ -471,6 +477,73 @@ class RBatchSolver(Stepper):
         recs = np.zeros(self.n_games * cap, self._dtype)
         check(lib.spl_rbatch_lines(self._h, recs.ctypes.data, cap, plies), self.eng._h)
         return [recs[g * cap:g * cap + plies[g] + 1] for g in range(self.n_games)]
+
+    def close(self):
+        if getattr(self, '_h', None):
+            lib.spl_solver_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class SBatchSolver(Stepper):
+    """spl_sbatch_create + spl_solver_step: B State.solve() searches in lockstep (State.solve_many)."""
+
+    def __init__(self, eng: Engine, roots_np, goals, use_heuristic, heuristics, beams, tie='stable', noise='const',
+                 keep_links=True):
+        self.eng = eng
+        roots = np.ascontiguousarray(roots_np, dtype=np.uint64).reshape(-1, 4)
+        self.n_games = len(roots)
+        cols = [goals, use_heuristic, heuristics, beams]
+        if any(len(x) != self.n_games for x in cols):
+            raise ValueError(f'{self.n_games} roots, but {[len(x) for x in cols]} goals / kinds / heuristics / beam widths')
+        ids = [h if isinstance(h, int) else heuristic_id(h) for h in heuristics]
+        g = np.ascontiguousarray(goals, dtype=np.int32)
+        u = np.ascontiguousarray([int(bool(x)) for x in use_heuristic], dtype=np.int32)
+        h = np.ascontiguousarray(ids, dtype=np.int32)
+        bw = np.ascontiguousarray(beams, dtype=np.int64)
+        hd = C.c_void_p()
+        check(lib.spl_sbatch_create(eng._h, roots.ctypes.data, g.ctypes.data, u.ctypes.data, h.ctypes.data, bw.ctypes.data,
+                                    self.n_games, TIE_IDS[tie], NOISE_IDS[noise], int(keep_links), C.byref(hd)), eng._h)
+        self._h = hd
+        self.infos = []
+        self.ended = False
+
+    def step(self) -> dict:
+        """One level of every running game: the aggregate counters (spl_level_info) plus 'games', the per-game
+        counters (a game's dict stops changing once it has ended)."""
+        li = LevelInfo()
+        check(lib.spl_solver_step(self._h, C.byref(li), self.eng._stream()), self.eng._h)
+        d = li.as_dict()
+        d['games'] = self.games()
+        self.infos.append(d)
+        self.ended = bool(li.ended)
+        return d
+
+    def games(self) -> list:
+        out = (RGameInfo * self.n_games)()
+        check(lib.spl_sbatch_games(self._h, out, self.n_games), self.eng._h)
+        return [g.as_dict() for g in out]
+
+    def frontier(self, game: int) -> np.ndarray:
+        """game `game`'s current queue as host rows [n, 4] uint64 (lo, hi, aux, link); empty once the game has ended"""
+        p, n = C.c_void_p(), C.c_int64()
+        check(lib.spl_sbatch_frontier(self._h, int(game), C.byref(p), C.byref(n)), self.eng._h)
+        if n.value == 0:
+            return np.zeros((0, 4), np.uint64)
+        return torch.as_tensor(_DevArray(p.value, (n.value, 4)), device=self.eng.tdev).cpu().numpy().view(np.uint64)
+
+    def lines(self) -> list:
+        """every game's line as host rows [plies + 1, 4] uint64, root first (spl_sbatch_lines)"""
+        plies = (C.c_int32 * self.n_games)()
+        cap = max((g['level'] for g in self.games()), default=0) + 1
+        rows = np.zeros((self.n_games * cap, 4), np.uint64)
+        check(lib.spl_sbatch_lines(self._h, rows.ctypes.data, cap, plies), self.eng._h)
+        return [rows[g * cap:g * cap + plies[g] + 1] for g in range(self.n_games)]
 
     def close(self):
         if getattr(self, '_h', None):

@@ -3,6 +3,7 @@
 
 What runs where
   * `State.solve()`      -> spl_solver_* (expand + dedup + score + top-k kernels, one level per step)
+  * `State.solve_many()` -> spl_sbatch_* (many searches in lockstep on one GPU, lines rebuilt on the device)
   * `State.__iter__()`   -> spl_expand on a batch of one
   * `HEURISTICS[name]()` -> spl_score on a batch of one
   * path reconstruction  -> spl_solver_path (parent ranks + ordinals), replayed through `__iter__`
@@ -27,10 +28,13 @@ import torch
 
 from .cardparser import CardIndices, get_deck
 from .color import COLOR_NUM
-from .engine import Engine, heuristic_id, pack_aux, pack_key, unpack_record, _i64
+from .engine import M64, Engine, heuristic_id, pack_aux, pack_key, unpack_record, _i64
 from .gems import MAX_GEMS, Gems, increase_bonus, subtract_with_bonus
 
 deck = get_deck()
+
+#: most games in one State.solve_many batch (spl_sbatch_create's limit)
+MAX_BATCH_GAMES = 1 << 16
 
 #: module-level policy defaults (overridable per solve() call)
 DEFAULT_TIE_POLICY = 'stable'
@@ -259,6 +263,78 @@ class State:
         for o in ordinals:
             path.append(path[-1]._successors(eng)[o])
         return path
+
+    @classmethod
+    def solve_many(
+        cls,
+        roots,
+        goal_pts=15,
+        *,
+        use_heuristic=False,
+        heuristic_name='simple',
+        beam_width=300_000,
+        tie_policy: str | None = None,
+        noise: str | None = None,
+        device: int | None = None,
+        engine: Engine | None = None,
+        stats: list | None = None,
+    ) -> list[list['State']]:
+        """`root.solve(goal_pts=..., use_heuristic=..., heuristic_name=..., beam_width=..., tie_policy=..., noise=...,
+        verbose=False)` for every root of `roots`, searched together on one GPU: the games advance one level at a time
+        in lockstep, and each returns exactly the line its own solve() returns.
+
+        `goal_pts`, `use_heuristic`, `heuristic_name` and `beam_width` are one value or one per root; `tie_policy`
+        ('stable' | 'det') and `noise` ('const' | 'hash': 'mt' draws would depend on the other games) hold for the
+        whole batch.  Equal roots are separate games.  Nothing is printed.  With `stats`, one dict per level is
+        appended: the aggregate counters and 'games', the per-game counters.  Every argument is checked before the
+        GPU is used."""
+        roots = list(roots)
+        if not roots:
+            raise ValueError('solve_many needs at least one root')
+        n = len(roots)
+        if n > MAX_BATCH_GAMES:
+            raise ValueError(f'solve_many: {n} roots, at most {MAX_BATCH_GAMES} in one batch')
+
+        def per_game(value, name):
+            if np.ndim(value) == 0:  # one value (str, int, bool, numpy scalar) for every root
+                return [value] * n
+            values = list(value)
+            if len(values) != n:
+                raise ValueError(f'solve_many: {len(values)} values of {name} for {n} roots')
+            return values
+
+        goals = [int(g) for g in per_game(goal_pts, 'goal_pts')]
+        kinds = [bool(u) for u in per_game(use_heuristic, 'use_heuristic')]
+        names = per_game(heuristic_name, 'heuristic_name')
+        beams = [int(b) for b in per_game(beam_width, 'beam_width')]
+        if any(b < 1 for b in beams):
+            raise ValueError('solve_many: every beam width must be >= 1')
+        tie_policy = tie_policy or DEFAULT_TIE_POLICY
+        noise = noise or DEFAULT_NOISE
+        if tie_policy not in ('stable', 'det'):
+            raise ValueError(f"solve_many supports tie_policy 'stable' and 'det', not {tie_policy!r}")
+        if noise not in ('const', 'hash'):
+            raise ValueError(f"solve_many supports noise 'const' and 'hash', not {noise!r}: 'mt' draws depend on the other games")
+        rows = np.zeros((n, 4), np.uint64)
+        for g, r in enumerate(roots):
+            if len(r.gems) != COLOR_NUM or any(not 0 <= x <= MAX_GEMS for x in r.gems) or sum(r.gems) > 10:
+                raise ValueError(f'solve_many: root {g} has an illegal gem hand {r.gems!r}')
+            if any(not 0 <= c < len(deck) for c in r.cards):
+                raise ValueError(f'solve_many: root {g} holds a card index outside 0..{len(deck) - 1}')
+            k, a = r.record()
+            rows[g] = (k & M64, k >> 64, a, M64)
+        eng = engine or _engine(device)
+        sol = eng.sbatch_solver(rows, goals, kinds, [heuristic_id(h) for h in names], beams, tie_policy, noise)
+        try:
+            while not sol.ended:
+                info = sol.step()
+                if stats is not None:
+                    stats.append(info)
+            lines = sol.lines()
+        finally:
+            sol.close()
+        return [[root] + [State.from_record(int(lo), int(hi), int(aux)) for lo, hi, aux, _ in line[1:]]
+                for root, line in zip(roots, lines)]
 
 
 def _print_progress(sol, turn: int, max_pts: int, goal_pts: int) -> int:
