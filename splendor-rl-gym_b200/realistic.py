@@ -374,10 +374,12 @@ def solve_many(roots, *, beam_width=20_000, noise: str = 'const', device: int | 
     one int or one per game), and each returns exactly the line its own solve() returns.  noise is 'const' or 'hash'
     ('mt' draws depend on the other games).  With `stats`, one dict per level is appended: the aggregate counters and
     'games', the per-game counters."""
-    from .solver import _engine
+    from .solver import MAX_BATCH_GAMES, _engine
     roots = list(roots)
     if not roots:
         raise ValueError('solve_many needs at least one game')
+    if len(roots) > MAX_BATCH_GAMES:
+        raise ValueError(f'solve_many: {len(roots)} roots, at most {MAX_BATCH_GAMES} in one batch')
     for r in roots:
         if r.config.infinite_resources:
             raise ValueError('solve_many: a root with infinite_resources=True follows the speedrun rules; use State.solve')

@@ -31,6 +31,12 @@ def test_solve_many_argument_errors(roots, kw, match):
         S.solve_many(roots, **kw)
 
 
+def test_too_many_roots():
+    """The 65 536-game ceiling is checked before any config or record is packed."""
+    with pytest.raises(ValueError, match='at most 65536'):
+        S.solve_many([_game()] * ((1 << 16) + 1))
+
+
 def test_rgame_info_layout():
     """int64 level, frontier, generated, unique, kept, visited, goal_rank; int32 ended, pad"""
     assert C.sizeof(RGameInfo) == 64 and RGameInfo.ended.offset == 56
