@@ -2076,6 +2076,7 @@ int32_t spl_gs_rank_sort(spl_gsolver *s, const uint64_t *y_dev, int64_t n, int32
     cudaStream_t st = (cudaStream_t)stream;
     CK(c, enter_device(c));
     if (n == 0) return SPL_OK;
+    if (n >= OS_MAX_ITEMS) return fail(c, SPL_E_INVALID, "spl_gs_rank_sort: %lld sort words (limit 2^30 per rank)", (long long)n);
     // y[] / idx[] of the context hold the local survivors (spl_gs_cut): work in separate buffers
     CK(c, c->kl[0].ensure((size_t)n * 8 + 8, 0, st));
     CK(c, c->kl[1].ensure((size_t)n * 8 + 8, 0, st));
@@ -2085,7 +2086,6 @@ int32_t spl_gs_rank_sort(spl_gsolver *s, const uint64_t *y_dev, int64_t n, int32
     gs_iota_kernel<<<nblk(n), TILE, 0, st>>>(c->kh[0].as<uint32_t>(), n);
     ++c->launches;
     int cur = 0;
-    if (n >= OS_MAX_ITEMS) return fail(c, SPL_E_INVALID, "spl_gs_rank_sort: %lld sort words (limit 2^30 per rank)", (long long)n);
     {
         uint64_t *const k[2] = {c->kl[0].as<uint64_t>(), c->kl[1].as<uint64_t>()};
         uint32_t *const pl[2] = {c->kh[0].as<uint32_t>(), c->kh[1].as<uint32_t>()};

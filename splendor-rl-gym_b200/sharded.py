@@ -104,6 +104,18 @@ class Comm:
             dist.all_reduce(t, op=op)
         return t
 
+    def all_gather(self, t):
+        """all_gather of a 1-D device tensor of the same length on every rank -> [world, len] on t's device"""
+        if not self.on:
+            return t.reshape(1, -1)
+        if self.stage:
+            out = torch.empty((self.world, t.shape[0]), dtype=t.dtype)
+            dist.all_gather(list(out.unbind(0)), t.cpu())
+            return out.to(t.device)
+        out = torch.empty((self.world, t.shape[0]), dtype=t.dtype, device=t.device)
+        dist.all_gather_into_tensor(out, t.reshape(1, -1))
+        return out
+
     def all_to_all_rows(self, send, send_counts, recv_counts):
         """variable all-to-all of rows (dim 0); send is grouped by destination rank"""
         if not self.on:
@@ -853,17 +865,13 @@ class GroupedShardedSolver(Stepper):
         # 3. global beam threshold from the merged score dictionaries
         dp, nbytes = C.c_void_p(), C.c_int64()
         check(lib.spl_gs_dict(self._h, C.byref(dp), C.byref(nbytes), self._st()), eng._h)
-        local = self._dev(dp.value, (nbytes.value,), '|u1')
-        if comm.on:
-            alld = torch.empty((G, nbytes.value), dtype=torch.uint8, device=dev)
-            dist.all_gather_into_tensor(alld, local.reshape(1, -1))
-        else:
-            alld = local.reshape(1, -1)
+        alld = comm.all_gather(self._dev(dp.value, (nbytes.value,), '|u1'))
         need = C.c_int32()
         rc = lib.spl_gs_threshold(self._h, alld.data_ptr(), self.beam, u_total, C.byref(need), self._st())
         if rc == -6:  # SPL_E_CAPACITY
             raise DictionaryOverflow(f'level {self.level}: more than 2048 distinct scores')
         check(rc, eng._h)
+        info['tie_split'] = need.value
         if need.value:  # split the ties of the threshold score by arrival order
             lt = C.c_int32()
             check(lib.spl_gs_tie_begin(self._h, C.byref(lt), self._st()), eng._h)
@@ -900,9 +908,7 @@ class GroupedShardedSolver(Stepper):
             m = min(S, k_local)
             pick = (torch.arange(m, dtype=torch.int64, device=dev) * (k_local - 1)) // max(m - 1, 1)  # exact integer positions
             smp[:m] = y[pick]
-        alls = torch.empty((G, S), dtype=torch.int64, device=dev)
-        dist.all_gather_into_tensor(alls, smp.reshape(1, -1))
-        alls = np.sort(alls.cpu().numpy().reshape(-1))
+        alls = np.sort(comm.all_gather(smp).cpu().numpy().reshape(-1))
         alls = alls[alls != I64_MAX]
         if len(alls):
             spl = [int(alls[min(len(alls) - 1, (g * len(alls)) // G)]) for g in range(1, G)]

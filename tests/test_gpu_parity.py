@@ -319,7 +319,8 @@ def test_verbose_output_matches_reference_format(capsys):
                                  (255, False, 'simple', 0, 'stable', 'const', 6, 3000, 'pyhash')])
 def test_sharded_solver_world1_vs_oracle(eng, cfg):
     """The sharded driver (routing, winner bytes, pass-wise select, global ranks) on a single rank, with the
-    real CUDA backend, must reproduce the oracle level by level (the 2-rank logic is covered on gloo)."""
+    real CUDA backend, must reproduce the oracle level by level (2 and 3 ranks: on gloo with a CPU stand-in for the
+    kernels in test_sharded_gloo.py, with the real kernels on one GPU in test_gpu_sharded_ranks.py)."""
     from splendor_rl_gym_b200.sharded import Comm, CudaBackend, ShardedSolver
     goal, use_h, hname, beam, tie, noise, max_levels, block = cfg[:8]
     identity = cfg[8] if len(cfg) > 8 else 'key'  # 'pyhash': routing + visited set on the reference's State.hash (8(f).3)
@@ -349,7 +350,7 @@ def test_sharded_solver_world1_vs_oracle(eng, cfg):
 def test_grouped_sharded_solver_world1_vs_oracle(eng, hname, beam, rounds):
     """The card-set-sharded driver (spl_gs_*: routed buy records, order-agnostic per-run dedup, merged score dictionary,
     arrival-order tie select, sample-sort ranks) on a single rank must reproduce the oracle level by level, with one and
-    with many rounds per level (2+ ranks: tools/sharded_check.py --grouped under torchrun)."""
+    with many rounds per level (2 to 8 ranks on one GPU: test_gpu_sharded_ranks.py)."""
     from splendor_rl_gym_b200.sharded import Comm, GroupedShardedSolver
     sol = GroupedShardedSolver(eng, Comm(eng.tdev), 0, 0, 15, hname, beam, 'const', round_parents=rounds)
     orc = oracle.Solver(15, use_heuristic=True, heuristic_name=hname, beam_width=beam, policy='stable', noise='const')
