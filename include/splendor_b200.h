@@ -65,6 +65,44 @@ enum {
  * unknown names map to SIMPLE on the host side, as HEURISTICS.get(name, simple) does (:429). */
 enum { SPL_H_SIMPLE = 0, SPL_H_BALANCED = 1, SPL_H_AGGRESSIVE = 2, SPL_H_EFFICIENCY = 3 };
 
+/* User-declared formula heuristics (spl_add_formula).  A formula is a left-to-right sum of 1..8 terms, each
+ * coef * x1 ** e1 [* x2 ** e2 [* x3 ** e3]], plus the randint(1, 100) * 0.01 noise term of the built-ins:
+ *     t_i   = ((coef_i * x_i1 ** e_i1) * x_i2 ** e_i2) * x_i3 ** e_i3
+ *     score = ((t_0 + t_1) + t_2) ... + randint(1, 100) * 0.01
+ * with x ** e == libm pow((double)x, e) and every * and + separately rounded, as CPython evaluates the same
+ * expression.  Each x is a feature of the packed state record, over a bounded domain: */
+enum {
+    SPL_F_PTS = 0,        /* aux pts,                       0..255   */
+    SPL_F_SAVED = 1,      /* aux saved,                     0..65535 */
+    SPL_F_CARDS = 2,      /* len(cards),                    0..90    */
+    SPL_F_GEMS = 3,       /* sum(gems),                     0..35    */
+    SPL_F_BONUS = 4,      /* sum(bonus),                    0..155   */
+    SPL_F_RESOURCES = 5,  /* sum(gems) + 2 * sum(bonus),    0..345   */
+    SPL_F_COLORS = 6,     /* bonus colours that are not 0,  0..5     */
+    SPL_F_GEM0 = 7,       /* gems[c] = SPL_F_GEM0 + c,      0..7     (c = White, Blue, Green, Red, Black) */
+    SPL_F_BONUS0 = 12,    /* bonus[c] = SPL_F_BONUS0 + c,   0..31    */
+    SPL_F_COUNT = 17
+};
+enum { SPL_FORMULA_MAX_TERMS = 8, SPL_FORMULA_MAX_FACTORS = 3 };
+/* Formula ids: SPL_H_FORMULA_BASE + k for the k-th formula registered on a context; valid on that context only.
+ * At most SPL_MAX_FORMULAS formulas per context, whose power tables (8 bytes per domain value of every distinct
+ * (feature, exponent) pair, shared between the formulas) take at most SPL_FORMULA_TABLE_BYTES of device memory. */
+enum { SPL_H_FORMULA_BASE = 256, SPL_MAX_FORMULAS = 4096 };
+#define SPL_FORMULA_TABLE_BYTES (256ull << 20)
+
+typedef struct {
+    double coef;          /* finite */
+    int32_t n_factors;    /* 1..SPL_FORMULA_MAX_FACTORS */
+    int32_t feature[SPL_FORMULA_MAX_FACTORS];  /* SPL_F_* */
+    double exponent[SPL_FORMULA_MAX_FACTORS];  /* finite, >= 0 */
+} spl_formula_term;
+
+typedef struct {
+    int32_t n_terms;      /* 1..SPL_FORMULA_MAX_TERMS */
+    int32_t reserved;
+    spl_formula_term term[SPL_FORMULA_MAX_TERMS];
+} spl_formula;
+
 /* noise policy for the `randint(1,100)*0.01` term (src/solver.py:215,247,260,284), SURVEY.md 8a-N */
 enum {
     SPL_NOISE_CONST = 0,    /* randint -> 50 */
@@ -179,6 +217,19 @@ int32_t spl_expand(spl_ctx *ctx, const spl_key *keys_dev, const uint64_t *aux_de
 int32_t spl_dedup(spl_ctx *ctx, const spl_key *cand_keys_dev, const uint64_t *cand_aux_dev, int64_t n,
                   spl_key *uniq_keys_dev, uint64_t *uniq_aux_dev, int64_t *uniq_src_dev,
                   int64_t *n_out_host, void *stream);
+
+/* Registers a formula heuristic on the context and returns its id (SPL_H_FORMULA_BASE + k) in *id_host.  The formula
+ * is validated (SPL_E_INVALID): features in range, 1..8 terms of 1..3 factors, finite coefficients, finite exponents
+ * >= 0, and a largest possible |t_0| + ... + |t_n| over the feature domains that is a finite double, so that no score
+ * is inf or NaN.  The power table of every (feature, exponent) pair not seen before on this context is built with host
+ * libm pow and uploaded.  SPL_E_CAPACITY past SPL_MAX_FORMULAS formulas or SPL_FORMULA_TABLE_BYTES of tables; the
+ * context stays usable.  Synchronous; the tables are freed with the context.
+ *
+ * Every entry point that takes a heuristic (spl_score, spl_score_rows, spl_solver_create[_queue], spl_sbatch_create,
+ * spl_gs_create) accepts these ids.  An id in SPL_H_FORMULA_BASE .. SPL_H_FORMULA_BASE + SPL_MAX_FORMULAS - 1 that
+ * is not registered on the context fails with SPL_E_INVALID; any other id that is not a built-in scores as
+ * SPL_H_SIMPLE. */
+int32_t spl_add_formula(spl_ctx *ctx, const spl_formula *formula_host, int32_t *id_host);
 
 /* HEURISTICS[name](state) for a batch (src/solver.py:210-286), bit-exact IEEE doubles. */
 int32_t spl_score(spl_ctx *ctx, int32_t heuristic, int32_t noise, const spl_key *keys_dev,

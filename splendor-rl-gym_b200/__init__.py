@@ -11,10 +11,11 @@ from .buys import get_buys, load_buys, possible_buys  # noqa: F401
 from .cardparser import Card, get_deck, sort_cards  # noqa: F401
 from .color import COLOR_NUM, Color  # noqa: F401
 from .engine import Engine, LevelSolver  # noqa: F401
+from .formula import Formula  # noqa: F401
 from .gems import MAX_GEMS, get_takes, increase_bonus, subtract_with_bonus, take_gems  # noqa: F401
 from .realistic import CardMarket, GameConfig, GemPool, MultiPlayerState, PlayerState, solve_many  # noqa: F401
 from .solver import HEURISTICS, State  # noqa: F401
 
-__all__ = ['State', 'HEURISTICS', 'GameConfig', 'GemPool', 'CardMarket', 'PlayerState', 'MultiPlayerState', 'solve_many', 'Engine', 'LevelSolver', 'Card', 'Color', 'COLOR_NUM', 'MAX_GEMS', 'get_deck',
+__all__ = ['State', 'HEURISTICS', 'Formula', 'GameConfig', 'GemPool', 'CardMarket', 'PlayerState', 'MultiPlayerState', 'solve_many', 'Engine', 'LevelSolver', 'Card', 'Color', 'COLOR_NUM', 'MAX_GEMS', 'get_deck',
            'get_takes', 'get_buys', 'possible_buys', 'load_buys', 'take_gems', 'subtract_with_bonus',
            'increase_bonus', 'sort_cards', 'SplendorB200Error']

@@ -32,6 +32,14 @@ class Config(C.Structure):
                 ('max_node_bytes', C.c_uint64)]
 
 
+class FormulaTerm(C.Structure):
+    _fields_ = [('coef', C.c_double), ('n_factors', C.c_int32), ('feature', C.c_int32 * 3), ('exponent', C.c_double * 3)]
+
+
+class Formula(C.Structure):  # spl_formula
+    _fields_ = [('n_terms', C.c_int32), ('reserved', C.c_int32), ('term', FormulaTerm * 8)]
+
+
 class LevelInfo(C.Structure):
     _fields_ = [('level', C.c_int32), ('ended', C.c_int32), ('frontier', C.c_int64), ('expanded', C.c_int64),
                 ('generated', C.c_int64), ('unique', C.c_int64), ('kept', C.c_int64), ('goal_rank', C.c_int64),
@@ -76,6 +84,7 @@ def _load():
         'spl_transfer_bytes': (i32, [vp, C.POINTER(i64), C.POINTER(i64)]),
         'spl_expand': (i32, [vp, vp, vp, i64, vp, vp, vp, i64, C.POINTER(i64), vp]),
         'spl_dedup': (i32, [vp, vp, vp, i64, vp, vp, vp, C.POINTER(i64), vp]),
+        'spl_add_formula': (i32, [vp, C.POINTER(Formula), C.POINTER(i32)]),
         'spl_score': (i32, [vp, i32, i32, vp, vp, i64, vp, vp]),
         'spl_topk': (i32, [vp, vp, vp, i64, i64, i32, vp, C.POINTER(i64), vp]),
         'spl_owner_partition': (i32, [vp, vp, i64, i32, vp, vp, vp]),

@@ -36,6 +36,25 @@ struct DevTables {
     uint32_t card[SPL_NUM_CARDS];  // packed cost|pt|bonus (deck_table.h)
 };
 
+// A registered formula heuristic (spl_add_formula) as the device reads it; the context's formulas sit in one table,
+// id SPL_H_FORMULA_BASE + k at index k, which the kernels that can score formulas take as their last parameter (so the
+// parameters of the built-in kernels keep their layout).  Every factor points at the power table of its (feature,
+// exponent) pair, pw[x] = pow(x, exponent) over the feature's whole domain.
+struct FormFactor {
+    const double *pw;
+    int32_t feat;  // SPL_F_*
+    int32_t pad;
+};
+struct FormTerm {
+    double coef;
+    int32_t nf, pad;
+    FormFactor f[SPL_FORMULA_MAX_FACTORS];
+};
+struct FormDev {
+    int32_t nt, pad[3];
+    FormTerm t[SPL_FORMULA_MAX_TERMS];
+};
+
 struct ScoreLuts {  // x ** e for every integer argument the heuristics can see (src/solver.py:210-286)
     const double *pts;    // [4][256]   pts ** {2.5, 2.8, 3.2, 2.0}
     const double *saved;  // [4][65536] saved ** {0.4, 0.5, 0.3, 0.7}

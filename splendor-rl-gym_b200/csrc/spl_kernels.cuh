@@ -5,7 +5,8 @@
 //                         probe/insert (MODE_PROBE) or materialising candidates (MODE_LIST)
 //   probe_list_kernel     visited-table probe/insert of a materialised candidate list
 //   resolve_kernel<SRC>   first-arrival winner resolution + ordered emission (+ scoring)
-//   score_kernel          heuristics on a batch
+//   score_kernel<FORM>    heuristics on a batch (FORM: formula heuristics too, spl_add_formula)
+//   score_rec_kernel      a formula heuristic on records: grouped rounds and external noise of formula searches
 //   sel_* / cut_kernel    radix select of the beam threshold + arrival-order cut
 //   sort_* / gather       stable LSD radix sort into rank order
 //
@@ -524,11 +525,61 @@ __device__ __forceinline__ double score_state(int h, int noise_mode, uint64_t lo
     return __dadd_rn(acc, noise);
 }
 
+// A formula heuristic (spl_add_formula) on the same packed record and with the same noise as score_state: every pow
+// from the formula's host-built tables, every * and + separately rounded, in the order of the Python expression
+// coef * x1 ** e1 * x2 ** e2 ... (left to right), then t_0 + t_1 + ... + noise (left to right).
+__device__ __forceinline__ uint32_t formula_feature(int f, uint64_t lo, uint64_t hi, uint64_t aux) {
+    const uint32_t g = (uint32_t)(lo & GEM_MASK);
+    if (f >= SPL_F_BONUS0) return (uint32_t)((aux >> (24 + 5 * (f - SPL_F_BONUS0))) & 31);
+    if (f >= SPL_F_GEM0) return (g >> (3 * (f - SPL_F_GEM0))) & 7;
+    switch (f) {
+        case SPL_F_PTS: return (uint32_t)((aux >> 16) & 0xff);
+        case SPL_F_SAVED: return (uint32_t)(aux & 0xffff);
+        case SPL_F_CARDS: return __popcll(lo >> 15) + __popcll(hi & HI_KEY_MASK);
+        default: break;
+    }
+    uint32_t sum_g = 0, sum_b = 0, nnz = 0;
+#pragma unroll
+    for (int c = 0; c < NCOL; ++c) {
+        sum_g += (g >> (3 * c)) & 7;
+        const uint32_t b = (uint32_t)((aux >> (24 + 5 * c)) & 31);
+        sum_b += b;
+        nnz += b > 0;
+    }
+    return f == SPL_F_GEMS ? sum_g : f == SPL_F_BONUS ? sum_b : f == SPL_F_RESOURCES ? sum_g + 2 * sum_b : nnz;
+}
+__device__ __forceinline__ double score_formula(const FormDev *__restrict__ F, int noise_mode, uint64_t lo, uint64_t hi,
+                                                uint64_t aux, int r_ext) {
+    const int r = noise_mode == 1 ? 1 + (int)(mix64(lo, hi) % 100ull) : noise_mode == 2 ? r_ext : 50;
+    const int nt = __ldg(&F->nt);
+    double acc = 0.0;
+    for (int i = 0; i < nt; ++i) {
+        const FormTerm &T = F->t[i];
+        double t = __ldg(&T.coef);
+        const int nf = __ldg(&T.nf);
+        for (int j = 0; j < nf; ++j) {
+            const double *pw = (const double *)__ldg((const unsigned long long *)&T.f[j].pw);
+            t = __dmul_rn(t, __ldg(pw + formula_feature(__ldg(&T.f[j].feat), lo, hi, aux)));
+        }
+        acc = i ? __dadd_rn(acc, t) : t;
+    }
+    return __dadd_rn(acc, __dmul_rn((double)r, 0.01));
+}
+// FORM: h may be a formula id (SPL_H_FORMULA_BASE + k, the k-th of the context's formulas `forms`).  The instantiations
+// with FORM = false are score_state itself, so the built-in heuristics' kernels carry no formula code.
+template <bool FORM>
+__device__ __forceinline__ double score_any(int h, int noise_mode, uint64_t lo, uint64_t hi, uint64_t aux,
+                                            const ScoreLuts &L, const FormDev *forms, int r_ext = 50) {
+    if (FORM && h >= SPL_H_FORMULA_BASE) return score_formula(forms + (h - SPL_H_FORMULA_BASE), noise_mode, lo, hi, aux, r_ext);
+    return score_state(h, noise_mode, lo, hi, aux, L, r_ext);
+}
+
+template <bool FORM>
 __global__ void __launch_bounds__(TILE) score_kernel(const spl_key *__restrict__ keys, const uint64_t *__restrict__ aux,
                                                      int64_t n, int h, int noise_mode, ScoreLuts L,
-                                                     double *__restrict__ out) {
+                                                     double *__restrict__ out, const FormDev *__restrict__ forms) {
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
-    if (i < n) out[i] = score_state(h, noise_mode, keys[i].lo, keys[i].hi & HI_KEY_MASK, aux[i], L);
+    if (i < n) out[i] = score_any<FORM>(h, noise_mode, keys[i].lo, keys[i].hi & HI_KEY_MASK, aux[i], L, forms);
 }
 
 // ------------------------------------------------------------------ resolve + ordered emission
@@ -548,7 +599,7 @@ struct ResolveSmem {
 // Pass 1 finds the winners (table slot still holds ~t of the first arrival); look-back turns the
 // per-tile winner counts into global output ranks; pass 2 re-derives each winner from its
 // parent (no second gather) and writes it, with its score, in arrival order.
-template <int SRC, bool SCORE>
+template <int SRC, bool SCORE, bool FORM = false>
 __global__ void __launch_bounds__(TILE) resolve_kernel(const Rec *__restrict__ front, int64_t n_par,
                                                        const DevTables *__restrict__ tabs,
                                                        const uint32_t *__restrict__ takes_idx,
@@ -561,7 +612,7 @@ __global__ void __launch_bounds__(TILE) resolve_kernel(const Rec *__restrict__ f
                                                        uint64_t out_base, Rec *__restrict__ out,
                                                        uint64_t *__restrict__ out_sk, int64_t *__restrict__ out_src,
                                                        int h, int noise_mode, ScoreLuts L, uint64_t *status,
-                                                       Counters *ctr, int ticket_id) {
+                                                       Counters *ctr, int ticket_id, const FormDev *__restrict__ forms = nullptr) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     ResolveSmem &S = *reinterpret_cast<ResolveSmem *>(smem_raw);
     if (SRC == SRC_PARENT) load_tabs(S.E.tabs, tabs);
@@ -646,7 +697,7 @@ __global__ void __launch_bounds__(TILE) resolve_kernel(const Rec *__restrict__ f
         }
         st_rec(out + pos, r);
         if (SCORE) {
-            const double sc = score_state(h, noise_mode, r.lo, r.hi, r.aux, L);
+            const double sc = score_any<FORM>(h, noise_mode, r.lo, r.hi, r.aux, L, forms);
             const uint64_t k = flip_f64((uint64_t)__double_as_longlong(sc));
             out_sk[pos] = k;
             kmin = min(kmin, k);
@@ -1405,14 +1456,42 @@ __global__ void __launch_bounds__(TILE) score_ext_kernel(const Rec *__restrict__
     }
 }
 
+// formula heuristic F on rows[0..n): flip_f64 score keys and their range (ctr->sk_min / sk_max); noise_mode, or the i-th
+// draw when draws != null.  The winners of a grouped round of a formula search (its dedup kernels emit no scores), and
+// the externally drawn noise of a formula search on the key table.
+__global__ void __launch_bounds__(TILE) score_rec_kernel(const Rec *__restrict__ rows, const uint8_t *__restrict__ draws,
+                                                         int64_t n, const FormDev *__restrict__ F, int noise_mode,
+                                                         uint64_t *__restrict__ sk, Counters *ctr) {
+    const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
+    uint64_t kmin = ~0ull, kmax = 0;
+    if (i < n) {
+        Rec r;
+        ld_rec(rows + i, r);
+        const double sc = score_formula(F, draws ? 2 : noise_mode, r.lo, r.hi & HI_KEY_MASK, r.aux, draws ? draws[i] : 50);
+        const uint64_t k = flip_f64((uint64_t)__double_as_longlong(sc));
+        sk[i] = k;
+        kmin = kmax = k;
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) {
+        kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, d));
+        kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, d));
+    }
+    if ((threadIdx.x & 31) == 0 && kmin <= kmax) {
+        atomicMin(&ctr->sk_min, (unsigned long long)kmin);
+        atomicMax(&ctr->sk_max, (unsigned long long)kmax);
+    }
+}
+
+template <bool FORM>
 __global__ void __launch_bounds__(TILE) score_rows_kernel(const Rec *__restrict__ rows, int64_t n, int h, int noise_mode,
                                                           ScoreLuts L, double *__restrict__ out,
-                                                          const uint8_t *__restrict__ draws) {
+                                                          const uint8_t *__restrict__ draws, const FormDev *__restrict__ forms) {
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
     if (i < n) {
         Rec r;
         ld_rec(rows + i, r);
-        out[i] = score_state(h, noise_mode, r.lo, r.hi & HI_KEY_MASK, r.aux, L, draws ? draws[i] : 50);
+        out[i] = score_any<FORM>(h, noise_mode, r.lo, r.hi & HI_KEY_MASK, r.aux, L, forms, draws ? draws[i] : 50);
     }
 }
 

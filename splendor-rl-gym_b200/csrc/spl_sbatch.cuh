@@ -16,7 +16,7 @@ namespace spl {
 struct SGame {
     int32_t goal;       // points that end the game when a state with them is dequeued
     int32_t use_h;      // 0: exhaustive BFS (every unique state, arrival order), 1: beam search
-    int32_t heuristic;  // score_state's h
+    int32_t heuristic;  // score_any's h
     int32_t pad;
 };
 
@@ -239,9 +239,11 @@ __global__ void __launch_bounds__(TILE) sb_gather_kernel(const Rec *__restrict__
 // game's heuristic and `noise`), or 0 for a game of exhaustive BFS, whose arrival order the stable passes then keep;
 // slot[i] = i.  ctr->sk_min / sk_max: the range of flip_f64(score); ctr->key_or / key_and: which key bits vary (the
 // 'det' policy's key passes).  Both over the beam games only.
+template <bool FORM>  // some game of the batch scores with a formula
 __global__ void __launch_bounds__(TILE) sb_score_kernel(const Rec *__restrict__ recs, const uint32_t *__restrict__ games, int64_t n,
                                                         const SGame *__restrict__ gm, int noise_mode, ScoreLuts L,
-                                                        uint64_t *__restrict__ y, uint32_t *__restrict__ slot, Counters *ctr) {
+                                                        uint64_t *__restrict__ y, uint32_t *__restrict__ slot, Counters *ctr,
+                                                        const FormDev *__restrict__ forms) {
     const int64_t i = (int64_t)blockIdx.x * TILE + threadIdx.x;
     uint64_t kmin = ~0ull, kmax = 0, or_lo = 0, or_hi = 0, and_lo = ~0ull, and_hi = ~0ull;
     if (i < n) {
@@ -250,7 +252,7 @@ __global__ void __launch_bounds__(TILE) sb_score_kernel(const Rec *__restrict__ 
         const SGame G = gm[games[i]];
         uint64_t w = 0;
         if (G.use_h) {
-            const uint64_t k = flip_f64((uint64_t)__double_as_longlong(score_state(G.heuristic, noise_mode, r.lo, r.hi & HI_KEY_MASK, r.aux, L)));
+            const uint64_t k = flip_f64((uint64_t)__double_as_longlong(score_any<FORM>(G.heuristic, noise_mode, r.lo, r.hi & HI_KEY_MASK, r.aux, L, forms)));
             w = ~k;
             kmin = kmax = k;
             or_lo = and_lo = r.lo;

@@ -176,6 +176,12 @@ struct spl_ctx {
     uint16_t *d_takes_edges = nullptr;
     double *d_lut = nullptr;
     ScoreLuts luts{};
+    // formula heuristics (spl_add_formula): device formula table (allocated with the first formula) and one
+    // power table per distinct (feature, exponent bits) pair
+    FormDev *d_forms = nullptr;
+    int n_forms = 0;
+    std::vector<std::pair<std::pair<int, uint64_t>, double *>> pow_tabs;
+    uint64_t pow_bytes = 0;
     // scalars
     Counters *d_ctr = nullptr, *h_ctr = nullptr;
     SelState *d_sel = nullptr, *h_sel = nullptr;
@@ -233,6 +239,16 @@ static int fail(spl_ctx *c, int code, const char *fmt, ...) {
         int s_ = (expr);          \
         if (s_ != SPL_OK) return s_; \
     } while (0)
+
+// heuristic ids: a formula id (SPL_H_FORMULA_BASE + k) must name a formula registered on the context; every other id
+// keeps its meaning (built-ins, and the fallback to simple for the rest)
+static inline bool is_formula_id(int32_t h) { return h >= SPL_H_FORMULA_BASE && h < SPL_H_FORMULA_BASE + SPL_MAX_FORMULAS; }
+static int check_heuristic(spl_ctx *c, const char *fn, int32_t h) {
+    if (is_formula_id(h) && h - SPL_H_FORMULA_BASE >= c->n_forms)
+        return fail(c, SPL_E_INVALID, "%s: heuristic %d is a formula id that is not registered on this context (%d formulas)", fn,
+                    h, c->n_forms);
+    return SPL_OK;
+}
 
 // every entry point: select the context's device and drop any stale non-sticky error another library left in this
 // thread's runtime state (the launch checks below read cudaGetLastError, which would otherwise report it as ours)
@@ -388,6 +404,8 @@ int32_t spl_destroy(spl_ctx *c) {
     cudaFree(c->d_tabs); cudaFree(c->d_takes_idx); cudaFree(c->d_takes_edges);
     cudaFree(c->d_lut); cudaFree(c->d_ctr); cudaFreeHost(c->h_ctr); cudaFree(c->d_sel); cudaFreeHost(c->h_sel);
     cudaFree(c->d_hist); cudaFree(c->d_dict); cudaFree(c->d_dict2); cudaFree(c->d_dest); cudaFree(c->d_gemrank); cudaFree(c->d_rankgems);
+    cudaFree(c->d_forms);
+    for (auto &t : c->pow_tabs) cudaFree(t.second);
     for (auto *b : c->pool_links) delete b;
     for (auto &ev : c->ev) if (ev) cudaEventDestroy(ev);
     delete c;
@@ -904,13 +922,76 @@ int32_t spl_dedup(spl_ctx *c, const spl_key *ck, const uint64_t *ca, int64_t n, 
     return SPL_OK;
 }
 
+int32_t spl_add_formula(spl_ctx *c, const spl_formula *f, int32_t *id) {
+    if (!c || !f || !id) return fail(c, SPL_E_INVALID, "spl_add_formula: null argument");
+    if (const char *why = formula_error(*f)) return fail(c, SPL_E_INVALID, "spl_add_formula: %s", why);
+    if (c->n_forms >= SPL_MAX_FORMULAS)
+        return fail(c, SPL_E_CAPACITY, "spl_add_formula: a context holds at most %d formulas", (int)SPL_MAX_FORMULAS);
+    // the (feature, exponent) pairs without a table yet; -0.0 + 0.0 == +0.0 keys both zeros alike
+    const auto pair_of = [](int feat, double e) {
+        const double z = e + 0.0;
+        uint64_t bits;
+        memcpy(&bits, &z, 8);
+        return std::make_pair(feat, bits);
+    };
+    const auto find = [&](const std::pair<int, uint64_t> &k) -> double * {
+        for (auto &t : c->pow_tabs)
+            if (t.first == k) return t.second;
+        return nullptr;
+    };
+    std::vector<std::pair<int, uint64_t>> fresh;
+    uint64_t fresh_bytes = 0;
+    for (int i = 0; i < f->n_terms; ++i)
+        for (int j = 0; j < f->term[i].n_factors; ++j) {
+            const auto k = pair_of(f->term[i].feature[j], f->term[i].exponent[j]);
+            if (find(k) || std::find(fresh.begin(), fresh.end(), k) != fresh.end()) continue;
+            fresh.push_back(k);
+            fresh_bytes += 8ull * (formula_feature_max(k.first) + 1);
+        }
+    if (c->pow_bytes + fresh_bytes > SPL_FORMULA_TABLE_BYTES)
+        return fail(c, SPL_E_CAPACITY, "spl_add_formula: the power tables of a context take at most %llu bytes (%llu in use, %llu more needed)",
+                    (unsigned long long)SPL_FORMULA_TABLE_BYTES, (unsigned long long)c->pow_bytes, (unsigned long long)fresh_bytes);
+    CK(c, enter_device(c));
+    if (!c->d_forms) {
+        CK(c, cudaMalloc(&c->d_forms, sizeof(FormDev) * SPL_MAX_FORMULAS));
+    }
+    for (const auto &k : fresh) {
+        double e;
+        memcpy(&e, &k.second, 8);
+        const std::vector<double> t = formula_pow_table(k.first, e);
+        double *d = nullptr;
+        CK(c, cudaMalloc(&d, t.size() * 8));
+        c->pow_tabs.emplace_back(k, d);
+        c->pow_bytes += t.size() * 8;
+        CK(c, cudaMemcpy(d, t.data(), t.size() * 8, cudaMemcpyHostToDevice));
+        c->h2d_bytes += (long long)t.size() * 8;
+    }
+    FormDev F{};
+    F.nt = f->n_terms;
+    for (int i = 0; i < f->n_terms; ++i) {
+        F.t[i].coef = f->term[i].coef;
+        F.t[i].nf = f->term[i].n_factors;
+        for (int j = 0; j < f->term[i].n_factors; ++j) {
+            F.t[i].f[j].feat = f->term[i].feature[j];
+            F.t[i].f[j].pw = find(pair_of(f->term[i].feature[j], f->term[i].exponent[j]));
+        }
+    }
+    CK(c, cudaMemcpy(c->d_forms + c->n_forms, &F, sizeof F, cudaMemcpyHostToDevice));
+    CK(c, cudaStreamSynchronize(nullptr));  // the pageable copies have landed before any later launch reads them
+    c->h2d_bytes += (long long)sizeof F;
+    *id = SPL_H_FORMULA_BASE + c->n_forms++;
+    return SPL_OK;
+}
+
 int32_t spl_score(spl_ctx *c, int32_t heuristic, int32_t noise, const spl_key *keys, const uint64_t *aux, int64_t n,
                   double *scores, void *stream) {
     if (!c || n < 0) return fail(c, SPL_E_INVALID, "spl_score: bad arguments");
+    CKS(c, check_heuristic(c, "spl_score", heuristic));
     cudaStream_t st = (cudaStream_t)stream;
     CK(c, enter_device(c));
     if (n == 0) return SPL_OK;
-    score_kernel<<<nblk(n), TILE, 0, st>>>(keys, aux, n, heuristic, noise, c->luts, scores);
+    if (is_formula_id(heuristic)) score_kernel<true><<<nblk(n), TILE, 0, st>>>(keys, aux, n, heuristic, noise, c->luts, scores, c->d_forms);
+    else score_kernel<false><<<nblk(n), TILE, 0, st>>>(keys, aux, n, heuristic, noise, c->luts, scores, nullptr);
     ++c->launches;
     CK(c, cudaGetLastError());
     return SPL_OK;
@@ -1069,10 +1150,16 @@ int32_t spl_route_keys(spl_ctx *c, const void *cand_rows, int64_t n, int32_t n_r
 int32_t spl_score_rows(spl_ctx *c, int32_t heuristic, int32_t noise, const void *rows, int64_t n, double *scores,
                        const uint8_t *draws, void *stream) {
     if (!c || n < 0 || (noise == SPL_NOISE_EXTERNAL && !draws)) return fail(c, SPL_E_INVALID, "spl_score_rows: bad arguments");
+    CKS(c, check_heuristic(c, "spl_score_rows", heuristic));
     cudaStream_t st = (cudaStream_t)stream;
     CK(c, enter_device(c));
     if (n == 0) return SPL_OK;
-    score_rows_kernel<<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const Rec *>(rows), n, heuristic, noise, c->luts, scores, draws);
+    if (is_formula_id(heuristic))
+        score_rows_kernel<true><<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const Rec *>(rows), n, heuristic, noise, c->luts, scores, draws,
+                                                          c->d_forms);
+    else
+        score_rows_kernel<false><<<nblk(n), TILE, 0, st>>>(reinterpret_cast<const Rec *>(rows), n, heuristic, noise, c->luts, scores, draws,
+                                                           nullptr);
     ++c->launches;
     CK(c, cudaGetLastError());
     return SPL_OK;
@@ -1339,6 +1426,7 @@ struct RBatch {
 
 struct spl_solver : SolverBufs {
     int goal = 15, use_h = 0, heuristic = 0, tie = 0, noise = 0;
+    bool form = false;  // batch: some beam game scores with a formula (sb_score_kernel<true>)
     LevelKind kind = KEY_TABLE;
     spl_rconfig rcfg{};
     // external-noise mode: the level is split in two calls (expand+dedup | score+cut)
@@ -1435,7 +1523,9 @@ struct GroupRound {
     int64_t out_base = 0;
     int heuristic = 0, noise = 0, level = 0;
 };
-struct RoundTimes { float sort, prep, thread, warp, cta; };  // CUDA-event ms: item sort + runs, node table + buffers, the kernels
+struct RoundTimes { float sort, prep, thread, warp, cta; };
+
+  // CUDA-event ms: item sort + runs, node table + buffers, the kernels
 
 // Sort the round's items by card-set hash, find the runs of equal key, then deduplicate every run against the node
 // table: thread kernel over all runs, then the warp kernel and the CTA kernel over the runs each one queued.  The caller
@@ -1507,6 +1597,21 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
     if (h.error)
         return fail(c, SPL_E_TABLE_FULL, "card-set table full during level %d (device error %u; %llu slots, max_node_bytes=%llu)", R.level,
                     h.error, (unsigned long long)c->nodes.units, (unsigned long long)c->nodes.max_bytes);
+    // A formula search runs the dedup kernels unchanged: they score its winners as they score an unknown id, with
+    // `simple`, and this pass replaces those score keys and their range by the formula's (the caller reads sk_min /
+    // sk_max from h_ctr).  The formula evaluator inside the register-bound warp and CTA kernels would spill.
+    if (is_formula_id(R.heuristic) && h.n_emitted) {
+        const unsigned long long range0[2] = {~0ull, 0ull};
+        static_assert(offsetof(Counters, sk_max) == offsetof(Counters, sk_min) + 8, "sk_min, sk_max adjacent");
+        CK(c, cudaMemcpyAsync(&c->d_ctr->sk_min, range0, sizeof range0, cudaMemcpyHostToDevice, st));
+        c->h2d_bytes += sizeof range0;
+        score_rec_kernel<<<nblk((int64_t)h.n_emitted), TILE, 0, st>>>(R.out->as<Rec>() + R.out_base, nullptr, (int64_t)h.n_emitted,
+                                                                      c->d_forms + (R.heuristic - SPL_H_FORMULA_BASE), R.noise,
+                                                                      c->sk.as<uint64_t>() + R.out_base, c->d_ctr);
+        ++c->launches;
+        CK(c, cudaGetLastError());
+        CKS(c, read_ctr(c, st));
+    }
     c->occupied += h.n_emitted;
     *n_new_out = (int64_t)h.n_emitted;
     return SPL_OK;
@@ -1704,6 +1809,7 @@ int32_t spl_gs_create(spl_ctx *c, int32_t rank, int32_t world, const spl_key *ro
     if (!c || !root_key || !out || world < 1 || world > MAX_RANKS || rank < 0 || rank >= world || beam < 1)
         return fail(c, SPL_E_INVALID, "spl_gs_create: bad arguments (1 <= world <= %d)", MAX_RANKS);
     if (noise != SPL_NOISE_CONST && noise != SPL_NOISE_HASH) return fail(c, SPL_E_INVALID, "spl_gs_create: noise must be const or hash");
+    CKS(c, check_heuristic(c, "spl_gs_create", heuristic));
     NO_LIVE_SOLVER(c, "spl_gs_create");
     CK(c, enter_device(c));
     spl_gsolver *s = new spl_gsolver(c);
@@ -2358,7 +2464,12 @@ static int keytable_expand(spl_solver *s, int64_t n, LevelExpand *x, float ms[6]
             CKS(c, prep_status(c, 0, nt, st));
             CKS(c, reset_ticket(c, 0, st));
             CK(c, cudaEventRecord(c->ev[2], st));
-            if (s->use_h && s->noise != SPL_NOISE_EXTERNAL)
+            if (s->use_h && s->noise != SPL_NOISE_EXTERNAL && is_formula_id(s->heuristic))
+                resolve_kernel<SRC_PARENT, true, true><<<nt, TILE, sizeof(ResolveSmem), st>>>(
+                    front + p0, np, c->d_tabs, c->d_takes_idx, c->d_takes_edges, c->off.as<uint32_t>(), (uint32_t)total,
+                    c->key.as<uint64_t>(), c->cand_slot.as<uint32_t>(), nullptr, nullptr, p0, (uint64_t)n_uniq, s->uniq.as<Rec>(),
+                    c->sk.as<uint64_t>(), nullptr, s->heuristic, s->noise, c->luts, c->status[0].as<uint64_t>(), c->d_ctr, 0, c->d_forms);
+            else if (s->use_h && s->noise != SPL_NOISE_EXTERNAL)
                 resolve_kernel<SRC_PARENT, true><<<nt, TILE, sizeof(ResolveSmem), st>>>(
                     front + p0, np, c->d_tabs, c->d_takes_idx, c->d_takes_edges, c->off.as<uint32_t>(), (uint32_t)total,
                     c->key.as<uint64_t>(), c->cand_slot.as<uint32_t>(), nullptr, nullptr, p0, (uint64_t)n_uniq, s->uniq.as<Rec>(),
@@ -2756,8 +2867,12 @@ static int sbatch_step(spl_solver *s, spl_level_info *info, cudaStream_t st) {
         if (by_key) CK(c, c->sk.ensure((size_t)n_uniq * 8, 0, st));
         CKS(c, zero_ctr(c, st));
         uint64_t *score_words = by_key ? c->sk.as<uint64_t>() : c->y[0].as<uint64_t>();  // by key: the key passes come first
-        sb_score_kernel<<<nblk(n_uniq), TILE, 0, st>>>(s->uniq.as<Rec>(), R.uniq_game.as<uint32_t>(), n_uniq, gm, s->noise, c->luts,
-                                                        score_words, c->idx[0].as<uint32_t>(), c->d_ctr);
+        if (s->form)
+            sb_score_kernel<true><<<nblk(n_uniq), TILE, 0, st>>>(s->uniq.as<Rec>(), R.uniq_game.as<uint32_t>(), n_uniq, gm, s->noise,
+                                                                  c->luts, score_words, c->idx[0].as<uint32_t>(), c->d_ctr, c->d_forms);
+        else
+            sb_score_kernel<false><<<nblk(n_uniq), TILE, 0, st>>>(s->uniq.as<Rec>(), R.uniq_game.as<uint32_t>(), n_uniq, gm, s->noise,
+                                                                   c->luts, score_words, c->idx[0].as<uint32_t>(), c->d_ctr, nullptr);
         ++c->launches;
         CK(c, cudaGetLastError());
         CKS(c, read_ctr(c, st));
@@ -2808,6 +2923,10 @@ static int level_cut(spl_solver *s, spl_level_info *info, int64_t n, const Level
             if (realistic)
                 r_score_kernel<<<nblk(x.n_uniq), TILE, 0, st>>>(s->uniq.as<RRec>(), x.n_uniq, c->rcfg.as<RConfigDev>(), c->luts,
                                                                  c->sk.as<uint64_t>(), nullptr, c->d_ctr, draws);
+            else if (is_formula_id(s->heuristic))
+                score_rec_kernel<<<nblk(x.n_uniq), TILE, 0, st>>>(s->uniq.as<Rec>(), draws, x.n_uniq,
+                                                                   c->d_forms + (s->heuristic - SPL_H_FORMULA_BASE), SPL_NOISE_EXTERNAL,
+                                                                   c->sk.as<uint64_t>(), c->d_ctr);
             else
                 score_ext_kernel<<<nblk(x.n_uniq), TILE, 0, st>>>(s->uniq.as<Rec>(), draws, x.n_uniq, s->heuristic, c->luts,
                                                                    c->sk.as<uint64_t>(), c->d_ctr);
@@ -2887,6 +3006,7 @@ static int create_solver(spl_ctx *c, const char *fn, const Rec *rows, int64_t n,
     if (use_h && beam < 1) return fail(c, SPL_E_INVALID, "%s: beam_width must be >= 1", fn);
     if (use_h && tie != SPL_TIE_STABLE && tie != SPL_TIE_KEY) return fail(c, SPL_E_INVALID, "%s: unknown tie policy %d", fn, tie);
     if (noise < 0 || noise > SPL_NOISE_EXTERNAL) return fail(c, SPL_E_INVALID, "%s: unknown noise policy %d", fn, noise);
+    CKS(c, check_heuristic(c, fn, heuristic));
     CKS(c, check_rows(c, fn, "row", rows, n));
     if (n > 1) {
         std::vector<int64_t> ord(n);
@@ -3260,14 +3380,19 @@ int32_t spl_sbatch_create(spl_ctx *c, const void *root_rows_host, const int32_t 
     std::vector<SGame> games((size_t)n_games);
     std::vector<int64_t> beam((size_t)n_games);
     CKS(c, check_rows(c, "spl_sbatch_create", "game", rows.data(), n_games));
+    bool form = false;
     for (int g = 0; g < n_games; ++g) {
         if (beams[g] < 1) return fail(c, SPL_E_INVALID, "spl_sbatch_create: game %d: beam_width must be >= 1", g);
+        CKS(c, check_heuristic(c, "spl_sbatch_create", heuristics[g]));
+        form |= use_heuristic[g] && is_formula_id(heuristics[g]);
         rows[g].link = ~0ull;
         games[g] = SGame{goals[g], use_heuristic[g] ? 1 : 0, heuristics[g], 0};
         beam[g] = use_heuristic[g] ? beams[g] : INT64_MAX;  // BFS keeps every unique state
     }
-    return open_batch(c, SPEEDRUN_BATCH, games.data(), sizeof(SGame), rows.data(), 32, beam.data(), n_games, keep_links,
-                      "spl_sbatch_create", out, tie_policy, noise);
+    CKS(c, open_batch(c, SPEEDRUN_BATCH, games.data(), sizeof(SGame), rows.data(), 32, beam.data(), n_games, keep_links,
+                      "spl_sbatch_create", out, tie_policy, noise));
+    (*out)->form = form;
+    return SPL_OK;
 }
 
 int32_t spl_sbatch_games(spl_solver *s, spl_rgame_info *out_host, int32_t n_games) {

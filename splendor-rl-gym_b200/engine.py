@@ -8,6 +8,7 @@ import numpy as np
 import torch
 
 from ._lib import Config, Key, LevelInfo, RGameInfo, check, lib
+from .formula import Formula
 
 HEURISTIC_IDS = {'simple': 0, 'balanced': 1, 'aggressive': 2, 'efficiency': 3, 'competitive': 1}
 TIE_IDS = {'stable': 0, 'det': 1, 'key': 1, 'det_ordered': 2}
@@ -137,6 +138,7 @@ class Engine:
         check(lib.spl_create(C.byref(cfg), C.byref(h)))
         self._h = h
         self.host_bytes = [0, 0]  # bytes this Python layer copied host->device / device->host itself (torch tensors)
+        self._formula_ids = {}    # Formula -> its id on this context (spl_add_formula)
 
     @classmethod
     def get(cls, device: int = 0, **kw) -> 'Engine':
@@ -157,6 +159,18 @@ class Engine:
             pass
 
     # -------------------------------------------------------------- helpers
+    def heuristic_id(self, heuristic) -> int:
+        """The library id of a built-in name (unknown names: `simple`), an id, or a Formula.  A formula is registered with
+        this context once (spl_add_formula); its id is valid on this Engine only."""
+        if isinstance(heuristic, Formula):
+            hid = self._formula_ids.get(heuristic)
+            if hid is None:
+                out = C.c_int32()
+                check(lib.spl_add_formula(self._h, C.byref(heuristic.as_c()), C.byref(out)), self._h)
+                hid = self._formula_ids[heuristic] = out.value
+            return hid
+        return heuristic if isinstance(heuristic, int) else heuristic_id(heuristic)
+
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.tdev).cuda_stream)
 
@@ -234,10 +248,11 @@ class Engine:
                             us.data_ptr(), C.byref(m), self._stream()), self._h)
         return uk[:m.value], ua[:m.value], us[:m.value]
 
-    def score(self, heuristic: str, keys: torch.Tensor, aux: torch.Tensor, noise: str = 'const') -> torch.Tensor:
+    def score(self, heuristic, keys: torch.Tensor, aux: torch.Tensor, noise: str = 'const') -> torch.Tensor:
+        """`heuristic`: a built-in name or a Formula"""
         n = keys.shape[0]
         out = torch.empty(n, dtype=torch.float64, device=self.tdev)
-        check(lib.spl_score(self._h, heuristic_id(heuristic), NOISE_IDS[noise], keys.data_ptr(), aux.data_ptr(), n,
+        check(lib.spl_score(self._h, self.heuristic_id(heuristic), NOISE_IDS[noise], keys.data_ptr(), aux.data_ptr(), n,
                             out.data_ptr(), self._stream()), self._h)
         return out
 
@@ -289,15 +304,16 @@ class Engine:
     def sbatch_solver(self, roots_np: np.ndarray, goals, use_heuristic, heuristics, beams, tie: str = 'stable',
                       noise: str = 'const', keep_links: bool = True) -> 'SBatchSolver':
         """spl_sbatch_create: len(roots_np) speedrun games searched in lockstep.  roots_np: 32-byte rows {lo, hi, aux,
-        link} (an [n, 4] uint64 array); goals, use_heuristic, heuristics (names or ids) and beams: one per game."""
+        link} (an [n, 4] uint64 array); goals, use_heuristic, heuristics (names, ids or Formulas) and beams: one per game."""
         return SBatchSolver(self, roots_np, goals, use_heuristic, heuristics, beams, tie, noise, keep_links)
 
     # -------------------------------------------------------------- fused solver
-    def solver(self, root_key: int, root_aux: int, goal_pts: int, use_heuristic: bool, heuristic: str, beam_width: int,
+    def solver(self, root_key: int, root_aux: int, goal_pts: int, use_heuristic: bool, heuristic, beam_width: int,
                tie: str = 'stable', noise: str = 'const', keep_links: bool = True, identity: str = 'key',
                queue: np.ndarray = None) -> 'LevelSolver':
         """With `queue` (an array of 32-byte rows {lo, hi, aux, link} in rank order; links ignored) the solve starts
-        from that level-0 queue instead of the one state (root_key, root_aux), which are then ignored."""
+        from that level-0 queue instead of the one state (root_key, root_aux), which are then ignored.  `heuristic`: a
+        built-in name or a Formula."""
         self.set_identity(identity)
         return LevelSolver(self, root_key, root_aux, goal_pts, use_heuristic, heuristic, beam_width, tie, noise,
                            keep_links, queue)
@@ -321,7 +337,7 @@ class LevelSolver(Stepper):
                  keep_links, queue=None):
         self.eng = eng
         h = C.c_void_p()
-        args = (goal_pts, int(bool(use_heuristic)), heuristic_id(heuristic), beam_width, TIE_IDS[tie], NOISE_IDS[noise],
+        args = (goal_pts, int(bool(use_heuristic)), eng.heuristic_id(heuristic), beam_width, TIE_IDS[tie], NOISE_IDS[noise],
                 int(keep_links), C.byref(h))
         if queue is None:
             k = Key(root_key & M64, root_key >> 64)
@@ -501,7 +517,7 @@ class SBatchSolver(Stepper):
         cols = [goals, use_heuristic, heuristics, beams]
         if any(len(x) != self.n_games for x in cols):
             raise ValueError(f'{self.n_games} roots, but {[len(x) for x in cols]} goals / kinds / heuristics / beam widths')
-        ids = [h if isinstance(h, int) else heuristic_id(h) for h in heuristics]
+        ids = [eng.heuristic_id(h) for h in heuristics]
         g = np.ascontiguousarray(goals, dtype=np.int32)
         u = np.ascontiguousarray([int(bool(x)) for x in use_heuristic], dtype=np.int32)
         h = np.ascontiguousarray(ids, dtype=np.int32)

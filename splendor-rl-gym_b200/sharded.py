@@ -30,7 +30,7 @@ import torch
 import torch.distributed as dist
 
 from ._lib import SPL_E_CAPACITY, Key as _Key, check, lib
-from .engine import NOISE_IDS, TIE_IDS, Engine, Stepper, _DevArray, heuristic_id
+from .engine import NOISE_IDS, TIE_IDS, Engine, Stepper, _DevArray
 
 import os
 import time
@@ -291,7 +291,7 @@ class CudaBackend(_Backend):
     def score(self, heuristic, noise, rows, draws=None):
         n = rows.shape[0]
         out = torch.empty(n, dtype=torch.float64, device=self.device)
-        check(lib.spl_score_rows(self.eng._h, heuristic_id(heuristic), NOISE_IDS[noise], rows.data_ptr(), n, out.data_ptr(),
+        check(lib.spl_score_rows(self.eng._h, self.eng.heuristic_id(heuristic), NOISE_IDS[noise], rows.data_ptr(), n, out.data_ptr(),
                                  draws.data_ptr() if draws is not None else None, self.eng._stream()), self.eng._h)
         return out
 
@@ -759,7 +759,7 @@ class GroupedShardedSolver(Stepper):
         self.C = int(round_parents)   # global ranks per round (all ranks walk the same window of the queue)
         k = _Key(root_key & ((1 << 64) - 1), root_key >> 64)
         h = C.c_void_p()
-        check(lib.spl_gs_create(eng._h, comm.rank, comm.world, C.byref(k), root_aux, goal_pts, heuristic_id(heuristic), beam_width,
+        check(lib.spl_gs_create(eng._h, comm.rank, comm.world, C.byref(k), root_aux, goal_pts, eng.heuristic_id(heuristic), beam_width,
                                 NOISE_IDS[noise], int(keep_links), C.byref(h)), eng._h)
         self._h = h
         self.N = 1

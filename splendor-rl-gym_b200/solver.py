@@ -28,7 +28,8 @@ import torch
 
 from .cardparser import CardIndices, get_deck
 from .color import COLOR_NUM
-from .engine import M64, Engine, heuristic_id, pack_aux, pack_key, unpack_record, _i64
+from .engine import M64, Engine, pack_aux, pack_key, unpack_record, _i64
+from .formula import Formula
 from .gems import MAX_GEMS, Gems, increase_bonus, subtract_with_bonus
 
 deck = get_deck()
@@ -58,7 +59,7 @@ def _engine(device=None) -> Engine:
     return Engine.get(device)
 
 
-def _score_one(name: str, state: 'State') -> float:
+def _score_one(name, state: 'State') -> float:
     eng = _engine()
     k = pack_key(state.cards, state.gems)
     keys = torch.tensor([[_i64(k), _i64(k >> 64)]], dtype=torch.int64, device=eng.tdev)
@@ -101,6 +102,15 @@ HEURISTICS: dict[str, HeuristicFunc] = {
     'efficiency': efficiency_heuristic,
     'competitive': competitive_heuristic,
 }
+
+
+def _heuristic(name):
+    """What solve() scores with for `heuristic_name`: the Formula that HEURISTICS[name] holds (or `name` itself when it is
+    a Formula), else the name, which the library maps to its built-in (unknown names: `simple`, src/solver.py:429)."""
+    if isinstance(name, Formula):
+        return name
+    value = HEURISTICS.get(name)
+    return value if isinstance(value, Formula) else name
 
 
 class State:
@@ -187,10 +197,15 @@ class State:
         ('key' = exact (cards, gems); 'pyhash' = dedup on the reference's own 64-bit
         hash((cards, gems)), src/solver.py:316, so that even hash collisions merge as they do there;
         single GPU only).
+
+        `heuristic_name` is looked up in HEURISTICS once: a Formula found there (or passed directly) is scored as
+        declared (formula.py); any other value, or a missing name, selects the built-in of that name (`simple` for
+        unknown names), as before.
         """
         tie_policy = tie_policy or DEFAULT_TIE_POLICY
         noise = noise or DEFAULT_NOISE
         eng = engine or _engine(device)
+        heuristic = _heuristic(heuristic_name)
         if verbose:
             print('=' * 60)
             print('SPEEDRUN MODE SOLVER')
@@ -211,7 +226,7 @@ class State:
             from .sharded import Comm, CudaBackend, DictionaryOverflow, GroupedShardedSolver, ShardedSolver
 
             def key_sharded():  # exhaustive BFS, key ties, hash / mt noise, pyhash identity: queue sharded by key hash
-                return ShardedSolver(CudaBackend(eng), Comm(eng.tdev), k, a, goal_pts, use_heuristic, heuristic_name,
+                return ShardedSolver(CudaBackend(eng), Comm(eng.tdev), k, a, goal_pts, use_heuristic, heuristic,
                                      beam_width, tie_policy, noise, identity=identity)
 
             def run(sh):
@@ -223,7 +238,7 @@ class State:
                         sh.close()
             if use_heuristic and tie_policy == 'stable' and noise == 'const' and identity == 'key':
                 # queue sharded by card set: gem takes never leave the GPU, only card buys are routed
-                sh = GroupedShardedSolver(eng, Comm(eng.tdev), k, a, goal_pts, heuristic_name, beam_width, noise)
+                sh = GroupedShardedSolver(eng, Comm(eng.tdev), k, a, goal_pts, heuristic, beam_width, noise)
                 try:
                     infos, ordinals = run(sh)
                 except DictionaryOverflow:  # too many distinct scores for the dictionary cut (every rank gets here together)
@@ -240,7 +255,7 @@ class State:
             for o in ordinals:
                 path.append(path[-1]._successors(eng)[o])
             return path
-        sol = eng.solver(k, a, goal_pts, use_heuristic, heuristic_name, beam_width, tie_policy, noise, identity=identity)
+        sol = eng.solver(k, a, goal_pts, use_heuristic, heuristic, beam_width, tie_policy, noise, identity=identity)
         try:
             turn = 0
             max_pts = 0
@@ -281,7 +296,8 @@ class State:
     ) -> list[list['State']]:
         """`root.solve(goal_pts=..., use_heuristic=..., heuristic_name=..., beam_width=..., tie_policy=..., noise=...,
         verbose=False)` for every root of `roots`, searched together on one GPU: the games advance one level at a time
-        in lockstep, and each returns exactly the line its own solve() returns.
+        in lockstep, and each returns exactly the line its own solve() returns.  Formulas (names that HEURISTICS maps to
+        a Formula, or Formula objects) mix freely with the built-ins and BFS games.
 
         `goal_pts`, `use_heuristic`, `heuristic_name` and `beam_width` are one value or one per root; `tie_policy`
         ('stable' | 'det') and `noise` ('const' | 'hash': 'mt' draws would depend on the other games) hold for the
@@ -324,7 +340,7 @@ class State:
             k, a = r.record()
             rows[g] = (k & M64, k >> 64, a, M64)
         eng = engine or _engine(device)
-        sol = eng.sbatch_solver(rows, goals, kinds, [heuristic_id(h) for h in names], beams, tie_policy, noise)
+        sol = eng.sbatch_solver(rows, goals, kinds, [_heuristic(h) for h in names], beams, tie_policy, noise)
         try:
             while not sol.ended:
                 info = sol.step()
