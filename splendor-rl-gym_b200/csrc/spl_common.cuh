@@ -17,6 +17,8 @@ constexpr int NCOL = 5;
 constexpr int TILE = 256;               // parents per CTA tile == threads per CTA
 constexpr uint32_t DEAD = 0xFFFFFFFFu;  // candidate already in the visited set (earlier epoch)
 constexpr uint64_t GEM_MASK = 0x7FFFull;
+constexpr int GEM_STATES = 2898;     // gem hands with every colour <= 7 and at most 10 gems
+constexpr int NODE_BM_WORDS = 46;    // 2944 bits >= GEM_STATES: one bit per gem hand, in gemrank order
 constexpr uint64_t HI_KEY_MASK = (1ull << 41) - 1;  // key bits 64..104
 constexpr int TAG_SHIFT = 41;                       // epoch tag in bits 105..127 of the table slot
 constexpr uint32_t TAG_MAX = (1u << 23) - 1;

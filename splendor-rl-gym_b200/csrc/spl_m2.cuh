@@ -26,8 +26,6 @@
 
 namespace spl {
 
-constexpr int GEM_STATES = 2898;       // gem hands with every colour <= 7 and at most 10 gems
-constexpr int NODE_BM_WORDS = 46;      // 2944 bits >= GEM_STATES
 constexpr int NODE_WORDS = 48;         // 384 B = 6 DRAM bursts: {m0, m1 | OCC, bitmap[46]}
 constexpr uint64_t NODE_OCC = 1ull << 63;
 constexpr int SMALL_ITEMS = 32;        // runs handled by one warp: at most 32 items and SMALL_W candidates
@@ -541,7 +539,8 @@ struct GroupArgs {
     uint32_t warp_max;             // runs of more candidates than this go to the CTA kernel
     const DevTables *tabs;
     const uint32_t *takes_idx;
-    const uint16_t *takes_edges;
+    const uint32_t *takes_pk;      // per take-table edge: gemrank of the child << 16 | child gems
+    const uint64_t *take_rows;     // [GEM_STATES][NODE_BM_WORDS]: the gemranks the takes of a hand (by its gemrank) reach
     const uint16_t *gemrank;
     const uint16_t *rankgems;      // inverse of gemrank: [GEM_STATES] gem hand of a dense index
     uint64_t *nodes;
@@ -600,17 +599,20 @@ __device__ __forceinline__ void load_buy_key(const GroupArgs &A, const SmemTabs 
 }
 
 // per-warp winner staging: records are collected in shared memory and written out 17..48 at a time behind one
-// global atomic (dense output, few same-address atomics)
+// global atomic (dense output, few same-address atomics).  They are scored as they are written out, every lane busy;
+// the least and largest score key written so far are kept per lane in shared memory (registers are what the walk
+// runs short of).
 constexpr int M2_WARPS_ = TILE / 32;
+constexpr int ST_COLS = 6;
 struct WarpStage {
-    uint64_t *st;                        // this warp's slice of st[5][warps][SM_STAGE] in shared memory: one pointer, the
-    uint32_t cnt;                        // five columns sit at compile-time strides (cnt: warp-uniform)
-    uint64_t kmin, kmax;
+    uint64_t *st;                        // this warp's slice of st[ST_COLS][warps][SM_STAGE] in shared memory: one pointer,
+    uint32_t cnt;                        // the columns sit at compile-time strides (cnt: warp-uniform)
     __device__ __forceinline__ uint64_t &lo(uint32_t i) const { return st[i]; }
     __device__ __forceinline__ uint64_t &hi(uint32_t i) const { return st[1 * M2_WARPS_ * SM_STAGE + i]; }
     __device__ __forceinline__ uint64_t &aux(uint32_t i) const { return st[2 * M2_WARPS_ * SM_STAGE + i]; }
     __device__ __forceinline__ uint64_t &link(uint32_t i) const { return st[3 * M2_WARPS_ * SM_STAGE + i]; }
-    __device__ __forceinline__ uint64_t &sk(uint32_t i) const { return st[4 * M2_WARPS_ * SM_STAGE + i]; }
+    __device__ __forceinline__ uint64_t &kmin() const { return st[4 * M2_WARPS_ * SM_STAGE + (threadIdx.x & 31)]; }
+    __device__ __forceinline__ uint64_t &kmax() const { return st[5 * M2_WARPS_ * SM_STAGE + (threadIdx.x & 31)]; }
 };
 __device__ __forceinline__ void stage_flush(const GroupArgs &A, WarpStage &W) {
     const unsigned lane = threadIdx.x & 31;
@@ -621,7 +623,11 @@ __device__ __forceinline__ void stage_flush(const GroupArgs &A, WarpStage &W) {
     for (uint32_t i = lane; i < W.cnt; i += 32) {
         Rec r{W.lo(i), W.hi(i), W.aux(i), W.link(i)};
         st_rec(A.out + base + i, r);
-        if (A.out_sk) A.out_sk[base + i] = W.sk(i);
+        if (A.out_sk) {
+            const uint64_t k = flip_f64((uint64_t)__double_as_longlong(score_state(A.h, A.noise_mode, r.lo, r.hi & HI_KEY_MASK, r.aux, A.L)));
+            A.out_sk[base + i] = k;
+            W.kmin() = min(W.kmin(), k); W.kmax() = max(W.kmax(), k);
+        }
     }
     W.cnt = 0;
     __syncwarp();
@@ -675,43 +681,52 @@ __device__ __forceinline__ void node_close(uint64_t *N, const uint64_t *bm) {
     if (lane < 16) N[32 + lane] = bm[30 + lane];
 }
 
-// One step of the arrival-ordered walk: up to 32 candidates (act lanes), EARLIER arrivals on lower lanes.  `dups`:
-// several lanes may carry the same gem hand (buy records of different parents), then the lowest lane speaks for it.
-// A candidate wins iff its bit was clear; winners are staged with their scores.  Called by all 32 lanes.
-__device__ __forceinline__ void bm_step(const GroupArgs &A, WarpStage &W, uint64_t *bm, bool act, bool dups, uint32_t g,
-                                        uint64_t t, uint64_t clo, uint64_t chi, uint64_t caux) {
+// The arrival-ordered walk goes in steps of up to 32 candidates (lanes), EARLIER arrivals on lower lanes.  The lanes
+// that speak for a gem hand in a step (leads) carry distinct hands, so a lead wins iff its bit is clear in bm as the
+// step found it -- a plain read -- and the step sets its bits only after every lead has read, with plain writes of
+// which no two go to one word.  A step ends with __syncwarp: the next one reads what it wrote.
+__device__ __forceinline__ bool bm_clear(const uint64_t *bm, uint32_t rk) { return !((bm[rk >> 6] >> (rk & 63)) & 1); }
+// bm |= {a, b}: lane l owns words l and l + 32
+__device__ __forceinline__ void bm_or(uint64_t *bm, uint64_t a, uint64_t b) {
     const unsigned lane = threadIdx.x & 31;
-    uint32_t rk = 0;
-    if (act) rk = __ldg(A.gemrank + g);
-    bool lead = act;
-    if (dups) {
-        const unsigned m = __ballot_sync(0xffffffffu, act);
-        if (act) lead = lane == (unsigned)(__ffs(__match_any_sync(m, rk)) - 1);
-    }
-    bool win = false;
-    if (lead) {
-        // (64-bit OR on shared memory compiles to a CAS loop, a quarter of this kernel's instructions; the native 32-bit
-        // ATOMS.OR with a returned value was measured and is slower here: 97 vs 78 ms per beam-30M solve)
-        // Most candidates are duplicates: a set bit is final, so only clear ones pay for the atomic.
-        const unsigned long long bit = 1ull << (rk & 63);
-        if (!(bm[rk >> 6] & bit)) win = !(atomicOr(reinterpret_cast<unsigned long long *>(&bm[rk >> 6]), bit) & bit);
-    }
+    __syncwarp();
+    bm[lane] |= a;
+    if (lane < NODE_BM_WORDS - 32) bm[32 + lane] |= b;
+    __syncwarp();
+}
+// the winners of a step (win lanes) are staged.  Called by all 32 lanes.
+__device__ __forceinline__ void stage_wins(const GroupArgs &A, WarpStage &W, bool win, uint64_t t, uint64_t clo, uint64_t chi,
+                                           uint64_t caux) {
+    const unsigned lane = threadIdx.x & 31;
     const unsigned wb = __ballot_sync(0xffffffffu, win);
     if (win) {
         const uint32_t at = W.cnt + __popc(wb & ((1u << lane) - 1));
         W.lo(at) = clo; W.hi(at) = chi; W.aux(at) = caux; W.link(at) = t;
-        if (A.out_sk) {
-            const uint64_t k = flip_f64((uint64_t)__double_as_longlong(score_state(A.h, A.noise_mode, clo, chi & HI_KEY_MASK, caux, A.L)));
-            W.sk(at) = k;
-            W.kmin = min(W.kmin, k); W.kmax = max(W.kmax, k);
-        }
     }
     W.cnt += __popc(wb);
     if (W.cnt > SM_STAGE - 32) stage_flush(A, W);
 }
+// buy records (act lanes).  Several may carry one gem hand (records of different parents): the lowest lane speaks for
+// it.  The winners of one bitmap word OR their bits over the group, and its lowest lane writes the word.
+__device__ __forceinline__ void buy_step(const GroupArgs &A, WarpStage &W, uint64_t *bm, bool act, const Rec &b) {
+    const unsigned lane = threadIdx.x & 31;
+    const uint32_t rk = act ? (uint32_t)__ldg(A.gemrank + (uint32_t)(b.lo & GEM_MASK)) : 0u;
+    const unsigned am = __ballot_sync(0xffffffffu, act);
+    bool win = false;
+    if (act) win = lane == (unsigned)(__ffs(__match_any_sync(am, rk)) - 1) && bm_clear(bm, rk);
+    const unsigned wm = __ballot_sync(0xffffffffu, win);
+    if (win) {
+        const unsigned peers = __match_any_sync(wm, rk >> 6);
+        const uint32_t bit = 1u << (rk & 31);
+        const uint32_t lo = __reduce_or_sync(peers, rk & 32 ? 0u : bit), hi = __reduce_or_sync(peers, rk & 32 ? bit : 0u);
+        if (lane == (unsigned)(__ffs(peers) - 1)) bm[rk >> 6] |= (uint64_t)hi << 32 | lo;
+    }
+    __syncwarp();
+    stage_wins(A, W, win, b.link, b.lo, b.hi, b.aux);
+}
 // the gem takes of TWO parents in one step: lanes 0..15 the earlier parent (lane P0 of the item window), lanes 16..31
-// the later one (lane P1); both have at most 16 takes.  Their successors may coincide, so the step resolves equal
-// gem hands in lane order (== arrival order).
+// the later one (lane P1); both have at most 16 takes.  Their successors may coincide: the lower lane (the earlier
+// arrival) speaks for a hand.  Then both parents' successor rows are set.
 __device__ __forceinline__ void take_steps_pair(const GroupArgs &A, WarpStage &W, uint64_t *bm, const Rec &it, uint64_t grank,
                                                 uint32_t tk, uint32_t nb, int P0, int P1) {
     const unsigned lane = threadIdx.x & 31;
@@ -721,10 +736,20 @@ __device__ __forceinline__ void take_steps_pair(const GroupArgs &A, WarpStage &W
     const uint32_t ptk = __shfl_sync(0xffffffffu, tk, src), pnb = __shfl_sync(0xffffffffu, nb, src);
     const uint32_t q = lane & 15;
     const bool act = q < (ptk & 0xff);
-    const uint32_t g = act ? (uint32_t)__ldg(A.takes_edges + (ptk >> 8) + q) : 0u;
-    bm_step(A, W, bm, act, true, g, (pgr << 8) | (pnb + q), (plo & ~GEM_MASK) | g, phi, paux);
+    const uint32_t e = act ? __ldg(A.takes_pk + (ptk >> 8) + q) : 0u;
+    const uint32_t prk = __ldg(A.gemrank + (uint32_t)(plo & GEM_MASK));
+    const uint64_t *r0 = A.take_rows + __shfl_sync(0xffffffffu, prk, 0) * NODE_BM_WORDS;
+    const uint64_t *r1 = A.take_rows + __shfl_sync(0xffffffffu, prk, 16) * NODE_BM_WORDS;
+    const uint64_t a = __ldg(r0 + lane) | __ldg(r1 + lane);
+    const uint64_t b = lane < NODE_BM_WORDS - 32 ? __ldg(r0 + 32 + lane) | __ldg(r1 + 32 + lane) : 0;
+    const unsigned am = __ballot_sync(0xffffffffu, act);
+    bool win = false;
+    if (act) win = lane == (unsigned)(__ffs(__match_any_sync(am, e)) - 1) && bm_clear(bm, e >> 16);
+    stage_wins(A, W, win, (pgr << 8) | (pnb + q), (plo & ~GEM_MASK) | (e & GEM_MASK), phi, paux);
+    bm_or(bm, a, b);
 }
-// the gem takes (src/solver.py:381-388) of one parent (fields warp-uniform), 32 table edges per step
+// the gem takes (src/solver.py:381-388) of one parent (fields warp-uniform), 32 table edges per step.  They are pairwise
+// distinct, so every one is tested against bm as the parent found it, and the parent's successor row is set at the end.
 __device__ __forceinline__ void take_steps(const GroupArgs &A, WarpStage &W, uint64_t *bm, uint64_t plo, uint64_t phi, uint64_t paux,
                                            uint64_t pgr, uint32_t ptk, uint32_t pnb) {
     const unsigned lane = threadIdx.x & 31;
@@ -732,9 +757,11 @@ __device__ __forceinline__ void take_steps(const GroupArgs &A, WarpStage &W, uin
     for (uint32_t q0 = 0; q0 < ntk; q0 += 32) {
         const uint32_t q = q0 + lane;
         const bool act = q < ntk;
-        const uint32_t g = act ? (uint32_t)__ldg(A.takes_edges + (ptk >> 8) + q) : 0u;
-        bm_step(A, W, bm, act, false, g, (pgr << 8) | (pnb + q), (plo & ~GEM_MASK) | g, phi, paux);
+        const uint32_t e = act ? __ldg(A.takes_pk + (ptk >> 8) + q) : 0u;
+        stage_wins(A, W, act && bm_clear(bm, e >> 16), (pgr << 8) | (pnb + q), (plo & ~GEM_MASK) | (e & GEM_MASK), phi, paux);
     }
+    const uint64_t *row = A.take_rows + (uint32_t)__ldg(A.gemrank + (uint32_t)(plo & GEM_MASK)) * NODE_BM_WORDS;
+    bm_or(bm, __ldg(row + lane), lane < NODE_BM_WORDS - 32 ? __ldg(row + 32 + lane) : 0);
 }
 // parent item `i` of the sorted list -> record, fan-out, rank, card-set words
 __device__ __forceinline__ void load_parent_item(const GroupArgs &A, const SmemTabs &tabs, uint32_t i, Rec &it, uint32_t &nb,
@@ -751,14 +778,15 @@ __device__ __forceinline__ void warp_epilogue(const GroupArgs &A, WarpStage &W, 
     if (W.cnt) stage_flush(A, W);
     if (lane == 0 && n_fresh) atomicAdd(&A.ctr->n_new_nodes, n_fresh);
     if (A.out_sk) {
+        uint64_t kmin = W.kmin(), kmax = W.kmax();
 #pragma unroll
         for (int d = 16; d; d >>= 1) {
-            W.kmin = min(W.kmin, __shfl_xor_sync(0xffffffffu, W.kmin, d));
-            W.kmax = max(W.kmax, __shfl_xor_sync(0xffffffffu, W.kmax, d));
+            kmin = min(kmin, __shfl_xor_sync(0xffffffffu, kmin, d));
+            kmax = max(kmax, __shfl_xor_sync(0xffffffffu, kmax, d));
         }
-        if (lane == 0 && W.kmin <= W.kmax) {
-            atomicMin(&A.ctr->sk_min, (unsigned long long)W.kmin);
-            atomicMax(&A.ctr->sk_max, (unsigned long long)W.kmax);
+        if (lane == 0 && kmin <= kmax) {
+            atomicMin(&A.ctr->sk_min, (unsigned long long)kmin);
+            atomicMax(&A.ctr->sk_max, (unsigned long long)kmax);
         }
     }
 }
@@ -772,8 +800,12 @@ constexpr int BSORT_MAX = 512;  // buy records of one run the warp kernel can pu
 struct WarpSmem {
     SmemTabs tabs;
     uint64_t bm[M2_WARPS][NODE_BM_WORDS + 2];
-    uint64_t st[5][M2_WARPS][SM_STAGE];  // lo, hi, aux, link, sk
-    uint64_t done[M2_WARPS][MAX_SETS][2]; // card sets of the current run walked so far (rarely more than one)
+    uint64_t st[ST_COLS][M2_WARPS][SM_STAGE];  // lo, hi, aux, link; per lane: least and largest score key flushed
+    uint64_t done[M2_WARPS][MAX_SETS + 1][2]; // card sets of the current run walked so far (rarely more than one), then the one being walked
+    uint64_t *node[M2_WARPS];             // the node of the card set being walked
+    uint32_t fresh[M2_WARPS];             // nodes this warp claimed
+    uint32_t ticket[M2_WARPS], next[M2_WARPS], end[M2_WARPS];  // the warp's next batch; next entry and end of this one
+    uint32_t run_s[M2_WARPS];             // first item of the run being walked
     uint64_t bsort[M2_WARPS][BSORT_MAX]; // UNORDERED only (last member: the arrival-ordered launch leaves it out)
 };
 
@@ -791,20 +823,33 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
     load_tabs(S.tabs, A.tabs);
     __syncthreads();
     uint64_t *bm = S.bm[w];
-    WarpStage W{S.st[0][w], 0, ~0ull, 0};
-    const uint32_t n_list = A.ctr->n_cls[CLS_WARP];
-    uint32_t n_fresh = 0;
+    WarpStage W{S.st[0][w], 0};
+    W.kmin() = ~0ull;
+    W.kmax() = 0;
+    uint32_t &n_fresh = S.fresh[w];  // (lane 0's count)
+    if (lane == 0) n_fresh = 0;
     // Runs weigh 17 .. 1024 candidates and their order in the list is whatever the dispatch kernel's atomics made it:
     // warps draw batches of WARP_BATCH runs from a ticket (the next batch's ticket is in flight while this one is
     // walked) instead of striding over the list, so the launch ends when the work does, not with its unluckiest warp.
-    uint32_t next_base = 0;
-    if (lane == 0) next_base = atomicAdd(&A.ctr->ticket[2], (unsigned)WARP_BATCH);
+    // (The loop state lives in shared memory: registers are short in the walk.)
+    if (lane == 0) {
+        S.ticket[w] = atomicAdd(&A.ctr->ticket[2], (unsigned)WARP_BATCH);
+        S.next[w] = S.end[w] = 0;
+    }
     for (;;) {
-        const uint32_t base = __shfl_sync(0xffffffffu, next_base, 0);
-        if (base >= n_list) break;
-        if (lane == 0) next_base = atomicAdd(&A.ctr->ticket[2], (unsigned)WARP_BATCH);
-        const uint32_t j_end = min(base + (uint32_t)WARP_BATCH, n_list);
-      for (uint32_t j = base; j < j_end; ++j) {
+        __syncwarp();
+        if (lane == 0 && S.next[w] == S.end[w]) {  // the batch is done: open the one whose ticket is in flight
+            const uint32_t base = S.ticket[w], n_list = A.ctr->n_cls[CLS_WARP];
+            S.next[w] = base;
+            S.end[w] = min(base + (uint32_t)WARP_BATCH, n_list);
+            if (base < n_list) S.ticket[w] = atomicAdd(&A.ctr->ticket[2], (unsigned)WARP_BATCH);
+        }
+        __syncwarp();
+        const uint32_t j = S.next[w];
+        if (j >= S.end[w]) break;
+        __syncwarp();
+        if (lane == 0) S.next[w] = j + 1;
+      {
         const uint32_t r = A.cls_list[CLS_WARP][j];
         const uint32_t s = A.run_start[r], e = A.run_start[r + 1];
         // parents [s, pe), buy records [pe, e)
@@ -844,6 +889,8 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
         uint64_t (*done)[2] = S.done[w];  // card sets done so far (shared memory: keeps 16 registers out of the walk)
         int n_done = 0;
         uint32_t lead = s;
+        if (lane == 0) S.run_s[w] = s;
+        __syncwarp();
         while (lead != 0xFFFFFFFFu) {
             uint64_t M0 = 0, M1 = 0;
             if (lane == 0) {
@@ -854,18 +901,21 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
             }
             M0 = __shfl_sync(0xffffffffu, M0, 0); M1 = __shfl_sync(0xffffffffu, M1, 0);
             uint64_t *N = node_open(A, M0, M1, bm, n_fresh);
+            // the set being walked is done[n_done] from here on (shared memory: registers are short in the walk)
+            if (lane == 0) { done[n_done][0] = M0; done[n_done][1] = M1; S.node[w] = N; }
+            __syncwarp();
             uint32_t next_lead = 0xFFFFFFFFu;
             Rec it{0, 0, 0, 0}, bt{0, 0, 0, 0};
             uint32_t nb = 0, tk = 0;
-            uint64_t grank = 0, brank = 0;
-            uint32_t bnext = pe, pnext = s;   // first item not loaded into a window yet
+            uint64_t grank = 0;
+            uint32_t bnext = pe, pnext = S.run_s[w];   // first item not loaded into a window yet
             unsigned bmask = 0, pmask = 0;
             for (;;) {
                 if (!pmask && pnext < pe) {  // refill the parent window
                     const bool valid = pnext + lane < pe;
                     uint64_t m0 = 0, m1 = 0;
                     if (valid) load_parent_item(A, S.tabs, pnext + lane, it, nb, tk, grank, m0, m1);
-                    const bool ok = valid && m0 == M0 && m1 == M1;
+                    const bool ok = valid && m0 == done[n_done][0] && m1 == done[n_done][1];
                     bool other = valid && !ok;  // a card set not walked yet?
 #pragma unroll
                     for (int d = 0; d < MAX_SETS; ++d) other = other && !(d < n_done && done[d][0] == m0 && done[d][1] == m1);
@@ -882,9 +932,8 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
                         const uint32_t at = resort ? pe + (uint32_t)(bs[bnext - pe + lane] & 1023u) : bnext + lane;
                         load_buy<UNORDERED>(A, S.tabs, item_id(A, at), bt);
                         mask_words(bt.lo, bt.hi, m0, m1);
-                        brank = bt.link >> 8;
                     }
-                    const bool ok = valid && m0 == M0 && m1 == M1;
+                    const bool ok = valid && m0 == done[n_done][0] && m1 == done[n_done][1];
                     bool other = valid && !ok;
 #pragma unroll
                     for (int d = 0; d < MAX_SETS; ++d) other = other && !(d < n_done && done[d][0] == m0 && done[d][1] == m1);
@@ -899,9 +948,9 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
                 }
                 if (!pmask && !bmask) break;
                 const uint64_t X = pmask ? __shfl_sync(0xffffffffu, grank, __ffs(pmask) - 1) : ~0ull;
-                const unsigned m = bmask & __ballot_sync(0xffffffffu, brank < X);
+                const unsigned m = bmask & __ballot_sync(0xffffffffu, (bt.link >> 8) < X);
                 if (m) {  // the buy records of the window that arrive before the next parent
-                    bm_step(A, W, bm, (m >> lane) & 1, true, (uint32_t)(bt.lo & GEM_MASK), bt.link, bt.lo, bt.hi, bt.aux);
+                    buy_step(A, W, bm, (m >> lane) & 1, bt);
                     bmask &= ~m;
                 } else {  // pmask != 0 here: every record left in the window arrives after parent X
                     const int P = __ffs(pmask) - 1;
@@ -913,7 +962,7 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
                     if (P1 >= 0) {
                         const uint32_t n0 = __shfl_sync(0xffffffffu, tk, P) & 0xff, n1 = __shfl_sync(0xffffffffu, tk, P1) & 0xff;
                         const uint64_t X1 = __shfl_sync(0xffffffffu, grank, P1);
-                        const unsigned between = bmask & __ballot_sync(0xffffffffu, brank < X1);
+                        const unsigned between = bmask & __ballot_sync(0xffffffffu, (bt.link >> 8) < X1);
                         pair = n0 <= 16 && n1 <= 16 && between == 0 && (bmask != 0 || bnext >= e);
                     }
                     if (pair) {
@@ -925,11 +974,9 @@ __global__ void __launch_bounds__(TILE, SPL_WARP_CTAS) m2_group_warp_kernel(Grou
                     }
                 }
             }
-            node_close(N, bm);
+            node_close(S.node[w], bm);
             if (next_lead != 0xFFFFFFFFu) {
                 if (n_done == MAX_SETS) { if (lane == 0) atomicExch(&A.ctr->error, 3u); break; }
-                if (lane == 0) { done[n_done][0] = M0; done[n_done][1] = M1; }
-                __syncwarp();
                 ++n_done;
             }
             lead = next_lead;
@@ -1099,7 +1146,7 @@ __device__ __forceinline__ void big_enumerate(const GroupArgs &A, BigSmem &S, ui
             derive_parent(S.tabs, A.takes_idx, it.lo, it.hi, it.aux, bl, bh, nb, tk);
             const uint64_t tb = (parent_rank(A, id) << 8) | nb;
             const uint32_t ntk = tk & 0xff;
-            for (uint32_t q = 0; q < ntk; ++q) f((uint32_t)__ldg(A.gemrank + __ldg(A.takes_edges + (tk >> 8) + q)), tb + q, i - s);
+            for (uint32_t q = 0; q < ntk; ++q) f(__ldg(A.takes_pk + (tk >> 8) + q) >> 16, tb + q, i - s);
         }
     }
 }

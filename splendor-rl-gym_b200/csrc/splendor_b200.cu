@@ -174,6 +174,8 @@ struct spl_ctx {
     DevTables *d_tabs = nullptr;
     uint32_t *d_takes_idx = nullptr;
     uint16_t *d_takes_edges = nullptr;
+    uint32_t *d_takes_pk = nullptr;     // HostTables::takes_pk
+    uint64_t *d_take_rows = nullptr;    // HostTables::take_rows
     double *d_lut = nullptr;
     ScoreLuts luts{};
     // formula heuristics (spl_add_formula): device formula table (allocated with the first formula) and one
@@ -341,6 +343,10 @@ int32_t spl_create(const spl_config *cfg, spl_ctx **out) {
     CKC(cudaMemcpy(c->d_takes_idx, T.takes_idx.data(), T.takes_idx.size() * 4, cudaMemcpyHostToDevice));
     CKC(cudaMalloc(&c->d_takes_edges, T.takes_edges.size() * 2));
     CKC(cudaMemcpy(c->d_takes_edges, T.takes_edges.data(), T.takes_edges.size() * 2, cudaMemcpyHostToDevice));
+    CKC(cudaMalloc(&c->d_takes_pk, T.takes_pk.size() * 4));
+    CKC(cudaMemcpy(c->d_takes_pk, T.takes_pk.data(), T.takes_pk.size() * 4, cudaMemcpyHostToDevice));
+    CKC(cudaMalloc(&c->d_take_rows, T.take_rows.size() * 8));
+    CKC(cudaMemcpy(c->d_take_rows, T.take_rows.data(), T.take_rows.size() * 8, cudaMemcpyHostToDevice));
     const size_t n_lut = T.lut_pts.size() + T.lut_saved.size() + T.lut_small.size();
     CKC(cudaMalloc(&c->d_lut, n_lut * 8));
     CKC(cudaMemcpy(c->d_lut, T.lut_pts.data(), T.lut_pts.size() * 8, cudaMemcpyHostToDevice));
@@ -401,7 +407,7 @@ int32_t spl_destroy(spl_ctx *c) {
     if (!c) return SPL_OK;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    cudaFree(c->d_tabs); cudaFree(c->d_takes_idx); cudaFree(c->d_takes_edges);
+    cudaFree(c->d_tabs); cudaFree(c->d_takes_idx); cudaFree(c->d_takes_edges); cudaFree(c->d_takes_pk); cudaFree(c->d_take_rows);
     cudaFree(c->d_lut); cudaFree(c->d_ctr); cudaFreeHost(c->h_ctr); cudaFree(c->d_sel); cudaFreeHost(c->h_sel);
     cudaFree(c->d_hist); cudaFree(c->d_dict); cudaFree(c->d_dict2); cudaFree(c->d_dest); cudaFree(c->d_gemrank); cudaFree(c->d_rankgems);
     cudaFree(c->d_forms);
@@ -1558,7 +1564,7 @@ static int group_round(spl_ctx *c, const GroupRound &R, int64_t *n_new_out, Roun
     A.run_start = c->run_start.as<uint32_t>(); A.run_wpre = c->run_wpre.as<uint32_t>();
     A.np = (uint32_t)R.np; A.rank_base = R.rank_base; A.grank = R.grank; A.unordered = R.unordered;
     A.warp_max = R.unordered ? std::min<uint32_t>(BIG_W, BSORT_MAX) : BIG_W;  // the warp kernel sorts at most BSORT_MAX records of a run itself
-    A.tabs = c->d_tabs; A.takes_idx = c->d_takes_idx; A.takes_edges = c->d_takes_edges; A.gemrank = c->d_gemrank; A.rankgems = c->d_rankgems;
+    A.tabs = c->d_tabs; A.takes_idx = c->d_takes_idx; A.takes_pk = c->d_takes_pk; A.take_rows = c->d_take_rows; A.gemrank = c->d_gemrank; A.rankgems = c->d_rankgems;
     A.nodes = c->nodes.as<uint64_t>(); A.nn = c->nodes.units; A.out = R.out->as<Rec>(); A.out_sk = c->sk.as<uint64_t>(); A.out_base = (uint64_t)R.out_base;
     for (int k = 0; k < NUM_CLS; ++k) A.cls_list[k] = nullptr;
     A.cls_list[CLS_WARP] = c->cls_list.as<uint32_t>();
